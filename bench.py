@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — headline benchmark of the b2048 hot path (see BASELINE.json / DESIGN.md).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
 
 Workload at every N (weak scaling): BASELINE.json configs[1] per GPU — random-action batched env
 stepping on 1,048,576 packed boards (uniform over the legal moves from the Philox action word,
@@ -33,6 +33,10 @@ reset-on-done).  One "step" = one fused `b2048_step_many` launch over all boards
 
 `--impl reference` times the CPU side alone (the reference is pure Python and cannot travel to the GPU
 box; oracle/pyport.py restates it at the same per-environment granularity).
+
+`--dump-outputs DIR` writes the outputs of the last timed env step as .npy files (see dump_outputs).  The boards, seeds
+and step counters depend on the arguments alone, so two builds run with the same arguments can be compared output for
+output.
 """
 from __future__ import annotations
 
@@ -279,6 +283,8 @@ def run_b200(args):
             envs[k % R].step_many(action_mode="random_legal", auto_reset=True)
         t1e.record()
         barrier()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(envs[(K - 1) % R], args.dump_outputs)
     kernel_ms = t0e.elapsed_time(t1e)
     t = torch.tensor([kernel_ms], dtype=torch.float64, device=dev)
     if world > 1:
@@ -518,6 +524,35 @@ def run_b200(args):
         dist.destroy_process_group()
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(env, out_dir: str) -> None:
+    """Writes what the last timed step_many returned to its caller, as out_dir/<name>.npy: reward and flags, and the
+    state it updated in place (packed board as [low, high] 32-bit words, score, step, max tile exponent).  Integers are
+    stored exactly as float32 (8-bit) or float64 (32-bit and wider).  Above 64 MB in all, a fixed seeded sample of the
+    boards is written instead, with its board indices in index.npy."""
+    import numpy as np
+    board = env.board.cpu().numpy().view(np.uint64)
+    out = {"board": np.stack([board & np.uint64(0xFFFFFFFF), board >> np.uint64(32)], axis=1).astype(np.float64),
+           "reward": env.reward.cpu().numpy().astype(np.float32),
+           "flags": env.flags.cpu().numpy().astype(np.float32)}
+    if env.track_state:
+        out["score"] = env.score.cpu().numpy().astype(np.float64)
+        out["step"] = env.step_count.cpu().numpy().astype(np.float64)
+        out["max_exp"] = env.max_exp.cpu().numpy().astype(np.float32)
+    n = len(board)
+    per_board = sum(a.nbytes for a in out.values()) // n
+    if per_board * n > DUMP_LIMIT_BYTES:
+        m = DUMP_LIMIT_BYTES // (per_board + 8)
+        idx = np.sort(np.random.default_rng(0).choice(n, m, replace=False))
+        out = {k: a[idx] for k, a in out.items()}
+        out["index"] = idx.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 _REAL_STDOUT = None
 
 
@@ -551,7 +586,12 @@ def main():
     ap.add_argument("--cpu-seconds", type=float, default=10.0)
     ap.add_argument("--train-boards", type=int, default=65536)
     ap.add_argument("--ac-boards", type=int, default=262144, help="actor-critic leg (BASELINE.json configs[3])")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write rank 0's outputs of the last timed env step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs needs --impl b200: the reference arm only times the CPU")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -463,3 +463,33 @@ def test_step_many_n_equals_single_steps(b2048, mode, auto_reset, track):
     a.step_many(action_mode="random_legal", auto_reset=True)
     b.step_many(action_mode="random_legal", auto_reset=True)
     assert torch.equal(a.board, b.board)
+
+
+def test_bench_dump_outputs_are_the_last_timed_step(b2048, tmp_path):
+    """bench.py --dump-outputs writes the last timed step of its headline leg, which the CPU oracle reproduces bit for bit
+    from the bench's protocol: per batch r (seed 0xB200 + r) a reset and 64 spreading steps, then max(3, W, R) warm-up
+    and K timed launches rotating over the R batches."""
+    import subprocess
+    import sys
+    from helpers import ROOT
+    n, K, W, R = 4096, 7, 3, 2
+    out = tmp_path / "dump"
+    subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--gpus", "1", "--steps", str(K), "--warmup", str(W),
+                    "--boards", str(n), "--batches", str(R), "--no-cpu", "--no-rollout", "--no-numa-bind",
+                    "--dump-outputs", str(out)], check=True, cwd=tmp_path, stdout=subprocess.DEVNULL)
+    got = {f[:-4]: np.load(os.path.join(out, f)) for f in os.listdir(out)}
+    assert sorted(got) == ["board", "flags", "max_exp", "reward", "score", "step"]
+    assert all(a.dtype in (np.float32, np.float64) and len(a) == n for a in got.values())
+    warm = max(3, W, R)
+    last = (K - 1) % R
+    steps = 64 + sum(1 for k in range(warm) if k % R == last) + sum(1 for k in range(K) if k % R == last)
+    cfg = oracle_cfg("runner_default", action_mode="random_legal", auto_reset=True)
+    seed = 0xB200 + last
+    st = oracle.reset_many(n, seed, 0, 0)
+    for t in range(1, steps + 1):
+        o = oracle.step_many(st, cfg, seed, 0, t)
+    w = got["board"].astype(np.uint64)
+    assert ((w[:, 1] << np.uint64(32)) | w[:, 0] == st["board"]).all()
+    assert (got["reward"] == o["reward"]).all() and (got["flags"] == o["flags"]).all()
+    assert (got["score"] == st["score"]).all() and (got["step"] == st["step"]).all()
+    assert (got["max_exp"] == st["max_exp"]).all()

@@ -255,6 +255,56 @@ def test_bench_reads_roofline_traffic_from_the_committed_ncu_summary():
     assert t3 is not None and 2e8 < t3 < 1e9
 
 
+@pytest.mark.parametrize("track", [True, False])
+def test_bench_dump_outputs_format_and_size_cap(tmp_path, monkeypatch, track):
+    """bench.py --dump-outputs: float32 / float64 .npy files that hold the step's outputs exactly (the packed board as
+    two 32-bit words); above the size cap, the same fixed seeded sample of boards every time, with its indices."""
+    import importlib.util
+    import types
+    import torch
+    spec = importlib.util.spec_from_file_location("bench_mod", os.path.join(ROOT, "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    rng = np.random.default_rng(3)
+    n = 1000
+    board = rng.integers(0, 2**64, n, dtype=np.uint64)
+    env = types.SimpleNamespace(
+        board=torch.from_numpy(board.view(np.int64)), reward=torch.from_numpy(rng.random(n, np.float32)),
+        flags=torch.from_numpy(rng.integers(0, 256, n, dtype=np.uint8)), track_state=track,
+        score=torch.from_numpy(rng.integers(0, 2**31, n, dtype=np.int32)) if track else None,
+        step_count=torch.from_numpy(rng.integers(0, 1025, n, dtype=np.int32)) if track else None,
+        max_exp=torch.from_numpy(rng.integers(0, 16, n, dtype=np.uint8)) if track else None)
+    names = ["board", "reward", "flags"] + (["score", "step", "max_exp"] if track else [])
+
+    def load(d):
+        got = {f[:-4]: np.load(os.path.join(d, f)) for f in os.listdir(d)}
+        assert all(a.dtype in (np.float32, np.float64) for a in got.values())
+        return got
+
+    def check(got, idx):
+        w = got["board"].astype(np.uint64)
+        assert ((w[:, 1] << np.uint64(32)) | w[:, 0] == board[idx]).all()
+        assert (got["reward"] == env.reward.numpy()[idx]).all() and (got["flags"] == env.flags.numpy()[idx]).all()
+        if track:
+            assert (got["score"] == env.score.numpy()[idx]).all() and (got["step"] == env.step_count.numpy()[idx]).all()
+            assert (got["max_exp"] == env.max_exp.numpy()[idx]).all()
+
+    bench.dump_outputs(env, str(tmp_path / "full"))
+    got = load(tmp_path / "full")
+    assert sorted(got) == sorted(names)
+    check(got, np.arange(n))
+    monkeypatch.setattr(bench, "DUMP_LIMIT_BYTES", 20000)
+    for d in ("a", "b"):
+        bench.dump_outputs(env, str(tmp_path / d))
+    a, b = load(tmp_path / "a"), load(tmp_path / "b")
+    assert sorted(a) == sorted(names + ["index"])
+    assert sum(x.nbytes for x in a.values()) <= 20000
+    idx = a["index"].astype(np.int64)
+    assert 0 < len(idx) < n and (np.diff(idx) > 0).all()
+    assert all((a[k] == b[k]).all() for k in a)
+    check(a, idx)
+
+
 def test_debug_options_match_the_header():
     """_lib.DEBUG_OPTIONS mirrors the B2048_DBG_* enum of include/b2048.h."""
     import re
