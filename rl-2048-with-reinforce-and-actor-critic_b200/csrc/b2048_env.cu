@@ -20,6 +20,7 @@
 #include <cstdlib>
 
 #include "b2048_internal.h"
+#include "b2048_ptx.cuh"
 #include "b2048_step_fast.cuh"
 
 namespace b2 {
@@ -93,7 +94,24 @@ struct StepArgs {
     long long* debug_clock;   // optional phase timestamps of a few CTAs (B2048_STEP_DEBUG_CLOCK), else NULL
 };
 
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
+// Thread 0 stages args.tables into shared memory with bulk copies that complete on `mbar` (phase 0): the small tables
+// first (needed first, kSmall only), then the row tables in 32 KB pieces.  Ends with every thread past the barrier's
+// initialisation, so any thread may wait on it.  `args` is taken by reference: a by-value table pointer costs
+// step_fast_n_kernel two registers.
+template <bool kSmall, class Args>
+__device__ __forceinline__ void stage_tables(uint8_t* smem, const Args& args, uint64_t* mbar) {
+    const uint32_t bar = s_u32(mbar);
+    if (threadIdx.x == 0) {
+        mbar_init(bar, 1);
+        mbar_init_fence();
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        mbar_expect_tx(bar, kSmall ? (uint32_t)B2048_TABLES_BYTES : (uint32_t)B2048_LUT_BYTES);
+        if (kSmall) bulk_load(s_u32(smem + B2048_LUT_BYTES), args.tables + B2048_LUT_BYTES, (uint32_t)B2048_SMALL_BYTES, bar);
+        bulk_load_chunked<32768u>(s_u32(smem), args.tables, (uint32_t)B2048_LUT_BYTES, bar);
+    }
+}
 
 // 128-bit coalesced observation stores for raw / log2: lane l of store round s writes row (l & 3) of
 // the board held by lane 8s + (l >> 2), so consecutive lanes write consecutive 16-byte chunks.
@@ -158,25 +176,7 @@ __global__ void __launch_bounds__(kThreads, kSmemLut ? 1 : 2) step_kernel(const 
     if (kSmemLut) {
         // Stage both row tables (192 KB) into shared memory with the bulk-copy engine; completion is
         // signalled on an mbarrier so the copy overlaps the first iteration's loads and Philox block.
-        if (tid == 0) {
-            asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(smem_u32(&mbar)));
-            asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-        }
-        __syncthreads();
-        if (tid == 0) {
-            asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(&mbar)),
-                         "r"((uint32_t)B2048_LUT_BYTES)
-                         : "memory");
-            constexpr uint32_t kChunk = 32768;
-#pragma unroll
-            for (uint32_t off = 0; off < (uint32_t)B2048_LUT_BYTES; off += kChunk) {
-                asm volatile(
-                    "cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-                        smem_u32(smem + off)),
-                    "l"(args.tables + off), "r"(kChunk), "r"(smem_u32(&mbar))
-                    : "memory");
-            }
-        }
+        stage_tables<false>(smem, args, &mbar);
         lut_left = reinterpret_cast<const uint16_t*>(smem);
         lut_merge = smem + B2048_LUT_LEFT_BYTES;
     } else {
@@ -215,16 +215,7 @@ __global__ void __launch_bounds__(kThreads, kSmemLut ? 1 : 2) step_kernel(const 
         }
         if (!lut_ready) {
             // all threads wait on phase 0 of the table barrier (returns immediately once complete)
-            uint32_t done = 0;
-            while (!done) {
-                asm volatile(
-                    "{\n\t.reg .pred p;\n\t"
-                    "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], 0;\n\t"
-                    "selp.u32 %0, 1, 0, p;\n\t}"
-                    : "=r"(done)
-                    : "r"(smem_u32(&mbar))
-                    : "memory");
-            }
+            mbar_wait(s_u32(&mbar), 0);
             lut_ready = true;
         }
         bool frozen = false;
@@ -278,34 +269,12 @@ __global__ void __launch_bounds__(1024, 1) step_fast_kernel(const __grid_constan
     const bool dbg = args.debug_clock != nullptr && tid == 0 && (blockIdx.x == 0 || blockIdx.x == 147);
     long long* dc = dbg ? args.debug_clock + (blockIdx.x == 0 ? 0 : 16) : nullptr;
     int dci = 0;
-    if (dbg) { unsigned long long gt; asm volatile("mov.u64 %0, %globaltimer;" : "=l"(gt)); dc[dci++] = (long long)gt; dc[dci++] = clock64(); }
+    if (dbg) { dc[dci++] = (long long)globaltimer(); dc[dci++] = clock64(); }
     // Programmatic dependent launch (no-ops when the launch does not carry the attribute): the NEXT launch in the
     // stream may start placing its CTAs as soon as SMs free up, so its barrier set-up and its 194 KB table staging run
     // under this launch's tail; it reads or writes nothing a previous launch touched before its own griddepcontrol.wait.
-    asm volatile("griddepcontrol.launch_dependents;");
-    if (tid == 0) {
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(smem_u32(&mbar)));
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    __syncthreads();
-    if (tid == 0) {
-        asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(&mbar)),
-                     "r"((uint32_t)B2048_TABLES_BYTES)
-                     : "memory");
-        // small tables first (needed first), then the row tables in 32 KB pieces
-        asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-                         smem_u32(smem + B2048_LUT_BYTES)),
-                     "l"(args.tables + B2048_LUT_BYTES), "r"((uint32_t)B2048_SMALL_BYTES), "r"(smem_u32(&mbar))
-                     : "memory");
-        constexpr uint32_t kChunk = 32768;
-#pragma unroll
-        for (uint32_t off = 0; off < (uint32_t)B2048_LUT_BYTES; off += kChunk) {
-            asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-                             smem_u32(smem + off)),
-                         "l"(args.tables + off), "r"(kChunk), "r"(smem_u32(&mbar))
-                         : "memory");
-        }
-    }
+    pdl_launch_dependents();
+    stage_tables<true>(smem, args, &mbar);
     FastTables T;
     T.left = reinterpret_cast<const uint16_t*>(smem);
     T.merge = smem + B2048_LUT_LEFT_BYTES;
@@ -313,7 +282,7 @@ __global__ void __launch_bounds__(1024, 1) step_fast_kernel(const __grid_constan
     T.sel = reinterpret_cast<const SelEntry*>(smem + B2048_LUT_BYTES + B2048_SMALL_SEL_OFF);
     T.act = smem + B2048_LUT_BYTES + B2048_SMALL_ACT_OFF;
     // everything above touched only the static tables; the boards may have been written by the previous launch
-    asm volatile("griddepcontrol.wait;" ::: "memory");
+    pdl_wait();
 
     const b2048_env_cfg& cfg = args.cfg;
     if constexpr (kPlain) {
@@ -332,18 +301,7 @@ __global__ void __launch_bounds__(1024, 1) step_fast_kernel(const __grid_constan
         // the Philox block of the first board is computed while the tables arrive; later ones at the end of the
         // previous iteration (same instruction count, the first one is off the staging's critical path)
         Rand4 rnd = stream_keyed(args.keys, args.gid0 + (uint64_t)i, args.t, B2048_DOM_STEP);
-        {   // the tables have to be in shared memory before the first lookup
-            uint32_t ok = 0;
-            while (!ok) {
-                asm volatile(
-                    "{\n\t.reg .pred p;\n\t"
-                    "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], 0;\n\t"
-                    "selp.u32 %0, 1, 0, p;\n\t}"
-                    : "=r"(ok)
-                    : "r"(smem_u32(&mbar))
-                    : "memory");
-            }
-        }
+        mbar_wait(s_u32(&mbar), 0);   // the tables have to be in shared memory before the first lookup
         for (; i < n; i += stride) {
             FastIO io;
             io.lo = bw_next.x; io.hi = bw_next.y;
@@ -391,16 +349,7 @@ __global__ void __launch_bounds__(1024, 1) step_fast_kernel(const __grid_constan
         bool frozen = false;
         if (args.ep_len) frozen = args.ep_len[i] != 0;
         if (!ready) {
-            uint32_t ok = 0;
-            while (!ok) {
-                asm volatile(
-                    "{\n\t.reg .pred p;\n\t"
-                    "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], 0;\n\t"
-                    "selp.u32 %0, 1, 0, p;\n\t}"
-                    : "=r"(ok)
-                    : "r"(smem_u32(&mbar))
-                    : "memory");
-            }
+            mbar_wait(s_u32(&mbar), 0);
             ready = true;
             if (dbg) dc[dci++] = clock64();
         }
@@ -424,7 +373,7 @@ __global__ void __launch_bounds__(1024, 1) step_fast_kernel(const __grid_constan
         args.flags[i] = (uint8_t)io.flags;
         if (dbg && dci < 12) dc[dci++] = clock64();
     }
-    if (dbg) { unsigned long long gt; asm volatile("mov.u64 %0, %globaltimer;" : "=l"(gt)); dc[14] = clock64(); dc[15] = (long long)gt; }
+    if (dbg) { const unsigned long long gt = globaltimer(); dc[14] = clock64(); dc[15] = (long long)gt; }
 }
 
 // Launched with cudaLaunchAttributeProgrammaticStreamSerialization (programmatic dependent launch): when the previous
@@ -479,27 +428,7 @@ __global__ void __launch_bounds__(1024, 1) step_fast_n_kernel(const __grid_const
     extern __shared__ __align__(128) uint8_t smem[];
     __shared__ uint64_t mbar;
     const int tid = threadIdx.x;
-    if (tid == 0) {
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(smem_u32(&mbar)));
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    __syncthreads();
-    if (tid == 0) {
-        asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(&mbar)),
-                     "r"((uint32_t)B2048_TABLES_BYTES)
-                     : "memory");
-        asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-                         smem_u32(smem + B2048_LUT_BYTES)),
-                     "l"(args.tables + B2048_LUT_BYTES), "r"((uint32_t)B2048_SMALL_BYTES), "r"(smem_u32(&mbar))
-                     : "memory");
-        constexpr uint32_t kChunk = 32768;
-#pragma unroll
-        for (uint32_t off = 0; off < (uint32_t)B2048_LUT_BYTES; off += kChunk)
-            asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-                             smem_u32(smem + off)),
-                         "l"(args.tables + off), "r"(kChunk), "r"(smem_u32(&mbar))
-                         : "memory");
-    }
+    stage_tables<true>(smem, args, &mbar);
     FastTables T;
     T.left = reinterpret_cast<const uint16_t*>(smem);
     T.merge = smem + B2048_LUT_LEFT_BYTES;
@@ -519,16 +448,7 @@ __global__ void __launch_bounds__(1024, 1) step_fast_n_kernel(const __grid_const
         io.flags = io.mask_in;
         io.reward = 0.0f;
         if (!ready) {
-            uint32_t ok = 0;
-            while (!ok) {
-                asm volatile(
-                    "{\n\t.reg .pred p;\n\t"
-                    "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], 0;\n\t"
-                    "selp.u32 %0, 1, 0, p;\n\t}"
-                    : "=r"(ok)
-                    : "r"(smem_u32(&mbar))
-                    : "memory");
-            }
+            mbar_wait(s_u32(&mbar), 0);
             ready = true;
         }
         float rsum = 0.0f;

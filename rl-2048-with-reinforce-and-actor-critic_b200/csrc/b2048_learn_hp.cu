@@ -140,20 +140,15 @@ struct PipeCtx {
 __device__ __forceinline__ void prog(const PipeCtx& px, int idx, int64_t v) {
     if (px.progress) px.progress[blockIdx.x * 8 + idx] = (int)v;
 }
-__device__ __forceinline__ uint32_t ld_acquire(const uint32_t* p) {
-    uint32_t v;
-    asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-    return v;
-}
 __device__ __forceinline__ void flag_wait(const uint32_t* p) {
-    while (ld_acquire(p) == 0u) __nanosleep(100);
+    while (ld_acquire_gpu(p) == 0u) __nanosleep(100);
 }
 // everything this thread (and, through the mbarriers it waited on, this CTA) wrote before becomes visible to a thread that
 // acquires the flag; bulk-copy (async proxy) writes must have completed (cp.async.bulk.wait_group 0) before the call
 __device__ __forceinline__ void flag_set(uint32_t* p) {
-    asm volatile("fence.proxy.async;" ::: "memory");
+    fence_proxy_async();
     __threadfence();
-    asm volatile("st.release.gpu.global.u32 [%0], %1;" ::"l"(p), "r"(1u) : "memory");
+    st_release_gpu(p, 1u);
 }
 
 // ------------------------------------------------------------------------------------------------ precise forward
@@ -168,9 +163,9 @@ static_assert(FS_RES % 1024 == 0 && (FS_RES + RES_W3H) % 1024 == 0 && (FS_RES + 
               "operand alignment");
 static_assert(FS_TOTAL <= 232448, "fwd_hp_kernel exceeds the shared memory of an sm_100 CTA");
 
-constexpr uint32_t kIdescF16 = (1u << 4) | ((uint32_t)(TC_H >> 3) << 17) | ((uint32_t)(TC_M >> 4) << 24);       // A/B fp16
-constexpr uint32_t kIdescHeadF16 = (1u << 4) | ((uint32_t)(TC_N3 >> 3) << 17) | ((uint32_t)(TC_M >> 4) << 24);
-constexpr uint32_t kIdescHead32F16 = (1u << 4) | ((uint32_t)((2 * TC_N3) >> 3) << 17) | ((uint32_t)(TC_M >> 4) << 24);   // N = 32: [W3 hi | W3 lo]
+constexpr uint32_t kIdescF16 = idesc_f16(TC_M, TC_H);
+constexpr uint32_t kIdescHeadF16 = idesc_f16(TC_M, TC_N3);
+constexpr uint32_t kIdescHead32F16 = idesc_f16(TC_M, 2 * TC_N3);   // N = 32: [W3 hi | W3 lo]
 
 struct FwdHpArgs {
     const uint8_t* img;       // split-weight image (global)
@@ -186,13 +181,9 @@ struct FwdHpArgs {
 
 constexpr int FH_THREADS = 512 + 3 * 32 + 128;   // 16 epilogue warps, MMA warp, weight loader, image storer, 4 I/O warps
 
-__device__ __forceinline__ uint32_t pack_f16(float a, float b) {
-    __half2 p = __floats2half2_rn(a, b);
-    return *reinterpret_cast<uint32_t*>(&p);
-}
 // hi = fp16x2(relu(a), relu(b)) in one instruction; lo = fp16x2(relu(x) - float(hi))
 __device__ __forceinline__ void relu_split(uint32_t a_bits, uint32_t b_bits, uint32_t& hi, uint32_t& lo) {
-    asm("cvt.rn.relu.f16x2.f32 %0, %1, %2;" : "=r"(hi) : "f"(__uint_as_float(b_bits)), "f"(__uint_as_float(a_bits)));
+    hi = relu_pack_f16(a_bits, b_bits);
     const float2 hf = __half22float2(*reinterpret_cast<__half2*>(&hi));
     const float ra = fmaxf(__uint_as_float(a_bits), 0.0f), rb = fmaxf(__uint_as_float(b_bits), 0.0f);
     lo = pack_f16(ra - hf.x, rb - hf.y);
@@ -219,16 +210,14 @@ __device__ __forceinline__ void fwd_role(const FwdHpArgs& args, const PipeCtx& p
         mbar_init(bar_out, 20);          // pipeline mode: every epilogue / I/O warp has written its global outputs of the tile
         for (int i = 0; i < 3; ++i) { mbar_init(w_full0 + 8u * i, 1); mbar_init(w_empty0 + 8u * i, 1); }
         for (int i = 0; i < 2; ++i) { mbar_init(a_full0 + 8u * i, 16); mbar_init(a_free0 + 8u * i, 2); }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        mbar_init_fence();
     }
-    if (warp == 16) {   // D1 = columns 0..255, D2 = 256..511, D3 = 256..271 (over the drained first columns of D2)
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(s_u32(tmem_slot)), "r"(512u)
-                     : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    // The TMEM prologue and epilogue and the two image-load loops of this role stay written out: through tmem_setup(),
+    // tmem_teardown() or bulk_load_chunked() the MMA warp's loop compiles to different (equivalent) SASS.
+    if (warp == 16) tmem_alloc(s_u32(tmem_slot), 512u);   // D1 = columns 0..255, D2 = 256..511, D3 = 256..271 (over D2)
+    tc_fence_before();
     __syncthreads();
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+    tc_fence_after();
     const uint32_t tmem_base = *tmem_slot;
     const int64_t n_tiles = (args.n + TC_M - 1) / TC_M;
     const int64_t first = rank;
@@ -243,13 +232,10 @@ __device__ __forceinline__ void fwd_role(const FwdHpArgs& args, const PipeCtx& p
             const bool leader = lane == 0;
             const uint8_t* gres = args.img + HP_RES;
             if (leader) {
-                asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar_res), "r"((uint32_t)RES_BYTES) : "memory");
+                mbar_expect_tx(bar_res, (uint32_t)RES_BYTES);
                 for (uint32_t off = 0; off < (uint32_t)RES_BYTES; off += 16384u) {
                     uint32_t sz = (uint32_t)RES_BYTES - off < 16384u ? (uint32_t)RES_BYTES - off : 16384u;
-                    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-                                     s_u32(smem + FS_RES + off)),
-                                 "l"(gres + off), "r"(sz), "r"(bar_res)
-                                 : "memory");
+                    bulk_load(s_u32(smem + FS_RES + off), gres + off, sz, bar_res);
                 }
             }
             mbar_wait(bar_res, 0);
@@ -259,7 +245,7 @@ __device__ __forceinline__ void fwd_role(const FwdHpArgs& args, const PipeCtx& p
             const uint32_t lA1 = dlo_ns(sA1), lW1H = dlo_ns(sRes + RES_W1H), lW1L = dlo_ns(sRes + RES_W1L);
             auto issue_layer1 = [&](uint32_t ph) {
                 mbar_wait(bar_a1, ph);
-                asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+                tc_fence_after();
                 if (leader) {
                     umma_w(tmem_base, lA1, DH_NOSW, lW1H, DH_NOSW, kIdescF16, 0u);
                     umma_w(tmem_base, lA1, DH_NOSW, lW1L, DH_NOSW, kIdescF16, 1u);
@@ -284,7 +270,7 @@ __device__ __forceinline__ void fwd_role(const FwdHpArgs& args, const PipeCtx& p
                     const uint32_t st = F & 1u, au = F >> 1;
                     long long c0 = dbg ? clock64() : 0;
                     mbar_wait(a_full0 + 8u * st, au & 1u);
-                    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+                    tc_fence_after();
                     const uint32_t ahi = dlo_sw(sA + st * FS_ASTAGE), alo = ahi + (16384u >> 4);
                     uint32_t slot = U % 3u, use = U / 3u;
                     long long c1 = dbg ? clock64() : 0;
@@ -327,7 +313,7 @@ __device__ __forceinline__ void fwd_role(const FwdHpArgs& args, const PipeCtx& p
                 for (int s = 0; s < 4; ++s) {
                     const uint32_t st = F & 1u, au = F >> 1;
                     mbar_wait(a_full0 + 8u * st, au & 1u);
-                    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+                    tc_fence_after();
                     const uint32_t ahi = dlo_sw(sA + st * FS_ASTAGE), alo = ahi + (16384u >> 4);
                     // An M128 N16 K16 MMA occupies the tensor pipe as long as a full-width one (~110-140 cycles, measured in
                     // b2048_policy_tc.cu), so the three products are issued as TWO instructions per K step: H2hi x [W3hi | W3lo]
@@ -357,14 +343,12 @@ __device__ __forceinline__ void fwd_role(const FwdHpArgs& args, const PipeCtx& p
                     const uint32_t slot = U % 3u, use = U / 3u;
                     if (use > 0) mbar_wait(w_empty0 + 8u * slot, (use - 1u) & 1u);
                     const uint32_t bar = w_full0 + 8u * slot;
-                    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"((uint32_t)HP_UNIT) : "memory");
+                    mbar_expect_tx(bar, (uint32_t)HP_UNIT);
                     const uint8_t* g = args.img + (size_t)j * HP_UNIT;
                     const uint32_t d = s_u32(smem + FS_W) + slot * HP_UNIT;
 #pragma unroll
                     for (uint32_t off = 0; off < (uint32_t)HP_UNIT; off += 16384u)
-                        asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(d + off),
-                                     "l"(g + off), "r"(16384u), "r"(bar)
-                                     : "memory");
+                        bulk_load(d + off, g + off, 16384u, bar);
                 }
             }
         }
@@ -385,12 +369,10 @@ __device__ __forceinline__ void fwd_role(const FwdHpArgs& args, const PipeCtx& p
 #pragma unroll
                             for (int half = 0; half < 2; ++half) {
                                 uint8_t* dst = img + (size_t)((tile % px.R) * 2 + half) * ACT_TILE_BYTES + (size_t)s * ACT_SLAB_BYTES;
-                                asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(dst),
-                                             "r"(src + (uint32_t)half * 8192u), "r"((uint32_t)ACT_SLAB_BYTES)
-                                             : "memory");
+                                bulk_store(dst, src + (uint32_t)half * 8192u, (uint32_t)ACT_SLAB_BYTES);
                             }
-                            asm volatile("cp.async.bulk.commit_group;" ::: "memory");
-                            asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
+                            bulk_commit();
+                            bulk_wait_read();
                         }
                         mbar_arrive(a_free0 + 8u * st);
                     }
@@ -398,12 +380,12 @@ __device__ __forceinline__ void fwd_role(const FwdHpArgs& args, const PipeCtx& p
                 if (piped) {    // publish the tile: masks / head outputs / A1^T written (bar_out), image writes complete
                     prog(px, 4, tile);
                     mbar_wait(bar_out, (uint32_t)((tile - first) / nranks) & 1u);
-                    asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
+                    bulk_wait();
                     flag_set(px.f_done + tile);
                     prog(px, 5, tile);
                 }
             }
-            asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
+            bulk_wait();
         }
         __syncwarp();
     } else if (warp < 16) {
@@ -437,8 +419,8 @@ __device__ __forceinline__ void fwd_role(const FwdHpArgs& args, const PipeCtx& p
                     *reinterpret_cast<uint4*>(base + sw) = make_uint4(hi[0], hi[1], hi[2], hi[3]);
                     *reinterpret_cast<uint4*>(base + 16384 + sw) = make_uint4(lo[0], lo[1], lo[2], lo[3]);
                 }
-                asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-                asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+                fence_proxy_async_smem();
+                tc_fence_before();
                 __syncwarp();
                 if (lane == 0) mbar_arrive(a_full0 + 8u * st);
             }
@@ -451,14 +433,14 @@ __device__ __forceinline__ void fwd_role(const FwdHpArgs& args, const PipeCtx& p
             if (dbg) dc[0] = clock64();
             mbar_wait(bar_d1, ph);
             if (dbg) dc[1] = clock64();
-            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+            tc_fence_after();
             const uint64_t m1 = epilogue(tlane);
             if (dbg) dc[2] = clock64();
             if (piped) mbar_wait(bar_slot, ph);
             if (args.m1) args.m1[(size_t)((tile % px.R) * 4 + g) * TC_M + row] = m1;
             mbar_wait(bar_d2, ph);
             if (dbg) dc[3] = clock64();
-            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+            tc_fence_after();
             const uint64_t m2 = epilogue(tlane + 256u);
             if (dbg) dc[4] = clock64();
             if (args.m2) args.m2[(size_t)((tile % px.R) * 4 + g) * TC_M + row] = m2;
@@ -492,7 +474,7 @@ __device__ __forceinline__ void fwd_role(const FwdHpArgs& args, const PipeCtx& p
             uint8_t* a1 = smem + FS_A1 + (row >> 3) * 256 + (row & 7) * 16;
             *reinterpret_cast<uint4*>(a1) = make_uint4(pk_next[0], pk_next[1], pk_next[2], pk_next[3]);
             *reinterpret_cast<uint4*>(a1 + 128) = make_uint4(pk_next[4], pk_next[5], pk_next[6], pk_next[7]);
-            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+            fence_proxy_async_smem();
             __syncwarp();
             if (lane == 0) mbar_arrive(bar_a1);
         };
@@ -518,12 +500,12 @@ __device__ __forceinline__ void fwd_role(const FwdHpArgs& args, const PipeCtx& p
             const int64_t next = tile + nranks;
             if (next < n_tiles) encode_a1(next);
             mbar_wait(bar_d3, ph);
-            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+            tc_fence_after();
             uint32_t r4[4], r4b[4];
             tmem_ld4_issue(tlane + 256u, r4);
-            tmem_ld4(tlane + 256u + 16u, r4b);                  // the hi x lo partial sums; the wait covers both loads
-            asm volatile("" : "+r"(r4[0]), "+r"(r4[1]), "+r"(r4[2]), "+r"(r4[3]));
-            asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+            tmem_ld4_issue(tlane + 256u + 16u, r4b);            // the hi x lo partial sums
+            tmem_ld_wait(r4);                                   // covers both loads
+            tc_fence_before();
             __syncwarp();
             if (lane == 0) mbar_arrive(bar_d3r);
             if (s < args.n) {
@@ -540,11 +522,9 @@ __device__ __forceinline__ void fwd_role(const FwdHpArgs& args, const PipeCtx& p
         }
     }
 
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    tc_fence_before();
     __syncthreads();
-    if (warp == 16) {
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512u) : "memory");
-    }
+    if (warp == 16) tmem_dealloc(tmem_base, 512u);
 }
 
 __global__ void __launch_bounds__(FH_THREADS, 1) fwd_hp_kernel(const __grid_constant__ FwdHpArgs args) {
@@ -582,20 +562,6 @@ struct BwdArgs {
 
 constexpr int BW_THREADS = 512 + 32 + 128;
 
-__device__ __forceinline__ void bw_store_slab(uint8_t* img, int64_t tile, uint32_t sA2, int g) {
-#pragma unroll
-    for (int half = 0; half < 2; ++half) {
-        uint8_t* dst = img + (size_t)(tile * 2 + half) * ACT_TILE_BYTES + (size_t)g * ACT_SLAB_BYTES;
-        asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(dst),
-                     "r"(sA2 + (uint32_t)g * 16384u + (uint32_t)half * 8192u), "r"((uint32_t)ACT_SLAB_BYTES)
-                     : "memory");
-    }
-}
-__device__ __forceinline__ void bw_stores_read_done() {
-    asm volatile("cp.async.bulk.commit_group;" ::: "memory");
-    asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
-}
-
 // Backward deltas of one 128-sample tile at a time, and the input-layer gradient:
 //   D5 = d3 W3^T in two N = 128 halves (TMEM columns 0..127, the second half once the first is drained)
 //   DL2 = D5 . [z2 > 0]  -> A2 (fp16, the A operand of D4) and the global DL2 image (dW2 is another kernel / role)
@@ -623,17 +589,9 @@ __device__ __forceinline__ void bwd_role(const BwdArgs& args, const PipeCtx& px,
             mbar_init(bar_bslab0 + 8u * g, 16);
             mbar_init(bar_dslab0 + 8u * g, 16);
         }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        mbar_init_fence();
     }
-    if (warp == 16) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(s_u32(tmem_slot)), "r"(512u)
-                     : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    __syncthreads();
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    const uint32_t tmem_base = *tmem_slot;
+    const uint32_t tmem_base = tmem_setup(warp == 16, tmem_slot, 512u);
     const int64_t n_tiles = (args.n + TC_M - 1) / TC_M;
     const int64_t first = rank;
     const int64_t n_local = first < n_tiles ? (n_tiles - first + nranks - 1) / nranks : 0;
@@ -644,25 +602,18 @@ __device__ __forceinline__ void bwd_role(const BwdArgs& args, const PipeCtx& px,
             const uint32_t sA2 = s_u32(smem + SM_A2), sW2 = s_u32(smem + IMG_W2), sW3 = s_u32(smem + IMG_W3);
             const uint32_t sA1T = s_u32(smem + BW_A1T);
             constexpr uint32_t kIdescBwd = kIdescF16 | kIdescBMn;                                                          // M128 N256
-            constexpr uint32_t kIdescD5 = ((1u << 4) | ((uint32_t)(128 >> 3) << 17) | ((uint32_t)(TC_M >> 4) << 24)) | kIdescBMn;   // M128 N128
-            constexpr uint32_t kIdescDw1 = ((1u << 4) | ((uint32_t)(32 >> 3) << 17) | ((uint32_t)(TC_M >> 4) << 24)) | kIdescAMn;   // M128 N32
+            constexpr uint32_t kIdescD5 = idesc_f16(128, 128) | kIdescBMn;
+            constexpr uint32_t kIdescDw1 = idesc_f16(128, 32) | kIdescAMn;
             // only W2 and W3 of the image are read by this kernel
-            asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar_img), "r"((uint32_t)(131072 + 8192)) : "memory");
-            for (uint32_t off = 0; off < 131072u; off += 16384u)
-                asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-                                 s_u32(smem + IMG_W2 + off)),
-                             "l"(args.img + IMG_W2 + off), "r"(16384u), "r"(bar_img)
-                             : "memory");
-            asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-                             s_u32(smem + IMG_W3)),
-                         "l"(args.img + IMG_W3), "r"(8192u), "r"(bar_img)
-                         : "memory");
+            mbar_expect_tx(bar_img, (uint32_t)(131072 + 8192));
+            bulk_load_chunked<16384u>(s_u32(smem + IMG_W2), args.img + IMG_W2, 131072u, bar_img);
+            bulk_load(s_u32(smem + IMG_W3), args.img + IMG_W3, 8192u, bar_img);
             mbar_wait(bar_img, 0);
             auto issue_d5a = [&](uint32_t ph) {
                 // backward through the head, features 0..127: D5 = d3 . W3^T.  A = d3 as fp16 [128 x 16] (K-major, A1's layout);
                 // B = the head's W3 image [j][f] read MN-major (N = f contiguous: 64-wide slabs 2048 B apart, 8 K rows = 1024 B)
                 mbar_wait(bar_dl3, ph);
-                asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+                tc_fence_after();
                 umma_f16(tmem_base, desc_nosw_k16(s_u32(smem + BW_D3A)), desc_sw128_mn(sW3, 2048u), kIdescD5, 0u);
                 umma_commit(bar_d5);
             };
@@ -674,7 +625,7 @@ __device__ __forceinline__ void bwd_role(const BwdArgs& args, const PipeCtx& px,
                 //      MN-major (N = in contiguous: 64-wide slabs 32768 B apart, 8 K rows = 1024 B)
                 for (int g = 0; g < 4; ++g) {
                     mbar_wait(bar_bslab0 + 8u * g, ph);
-                    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+                    tc_fence_after();
                     if (g == 1) {   // slabs 0 and 1 of DL2 are written, i.e. the first half of D5 is drained: features 128..255
                         umma_f16(tmem_base, desc_nosw_k16(s_u32(smem + BW_D3A)), desc_sw128_mn(sW3 + 2u * 2048u, 2048u), kIdescD5, 0u);
                         umma_commit(bar_d5b);
@@ -683,16 +634,17 @@ __device__ __forceinline__ void bwd_role(const BwdArgs& args, const PipeCtx& px,
                     for (int q = 0; q < 4; ++q)
                         umma_f16(tmem_base + 256u, desc_sw128(sA2 + (uint32_t)g * 16384u + (uint32_t)q * 32u),
                                  desc_sw128_mn(sW2 + (uint32_t)(g * 64 + q * 16) * 128u, 32768u), kIdescBwd, (g | q) ? 1u : 0u);
-                    bw_store_slab(args.dl2, tile % px.R, sA2, g);
+                    store_act_slab(args.dl2, tile % px.R, sA2, g);
                 }
-                bw_stores_read_done();                   // epilogue 4 overwrites DL2 once bar_d4 completes
+                bulk_commit();
+                bulk_wait_read();                        // epilogue 4 overwrites DL2 once bar_d4 completes
                 umma_commit(bar_d4);
                 // ---- the next tile's D5 (this tile's D5 was drained by every warp before the DL2 slab arrivals)
                 if (tile + nranks < n_tiles) issue_d5a(ph ^ 1u);
                 // ---- dW1^T += DL1^T [A1 | 1]: A = DL1 in A2 read MN-major (M = features: 64-wide slabs 16384 B apart,
                 //      K = samples: 8 rows = 1024 B), B = the tile's A1^T buffer (K-major, 32 rows: 16 inputs, the ones row, zeros)
                 for (int g = 0; g < 4; ++g) mbar_wait(bar_dslab0 + 8u * g, ph);
-                asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+                tc_fence_after();
                 const uint32_t sB = sA1T + (uint32_t)(lt & 1) * 8192u;
 #pragma unroll
                 for (int kk = 0; kk < 8; ++kk) {         // 16 samples per MMA
@@ -705,13 +657,13 @@ __device__ __forceinline__ void bwd_role(const BwdArgs& args, const PipeCtx& px,
                 umma_commit(bar_free);
                 if (piped) {                             // publish the tile: d3^T written, DL2 image writes complete
                     prog(px, 4, tile);
-                    asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
+                    bulk_wait();
                     flag_set(px.b_done + tile);
                     prog(px, 5, tile);
                 }
                 ph ^= 1u;
             }
-            asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
+            bulk_wait();
         }
         __syncwarp();
     } else if (warp < 16) {
@@ -739,8 +691,8 @@ __device__ __forceinline__ void bwd_role(const BwdArgs& args, const PipeCtx& px,
                 const int sw = ((g * 2 + c) ^ (row & 7)) << 4;
                 *reinterpret_cast<uint4*>(a2_row + s * 16384 + sw) = make_uint4(out[0], out[1], out[2], out[3]);
             }
-            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-            asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+            fence_proxy_async_smem();
+            tc_fence_before();
             __syncwarp();
             if (lane == 0) mbar_arrive(bar0 + 8u * s);
         };
@@ -765,18 +717,18 @@ __device__ __forceinline__ void bwd_role(const BwdArgs& args, const PipeCtx& px,
             if (dbg) dc[1] = clock64();
             if (tile != first) mbar_wait(bar_free, ph ^ 1u);
             if (dbg) dc[2] = clock64();
-            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+            tc_fence_after();
             masked_slab(tlane + (uint32_t)(g * 16), 0, m2, bar_bslab0);
             masked_slab(tlane + (uint32_t)(64 + g * 16), 1, m2, bar_bslab0);
             mbar_wait(bar_d5b, ph);                      // features 128..255 of D5 (same TMEM columns)
-            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+            tc_fence_after();
             masked_slab(tlane + (uint32_t)(g * 16), 2, m2, bar_bslab0);
             masked_slab(tlane + (uint32_t)(64 + g * 16), 3, m2, bar_bslab0);
             if (dbg) dc[3] = clock64();
             // ---- DL1 = D4 [z1 > 0] over DL2 (the backward MMAs have completed); read by the dW1 MMAs
             mbar_wait(bar_d4, ph);
             if (dbg) dc[4] = clock64();
-            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+            tc_fence_after();
 #pragma unroll
             for (int s = 0; s < 4; ++s) masked_slab(tlane + 256u + (uint32_t)(s * 64 + g * 16), s, m1, bar_dslab0);
             if (dbg) dc[5] = clock64();
@@ -785,7 +737,7 @@ __device__ __forceinline__ void bwd_role(const BwdArgs& args, const PipeCtx& px,
         // ---- read-out of dW1^T (columns 0..15) and db1 (column 16): lane quarter q, features hf * 128 + q * 32 + lane
         if (g == 0 && n_local > 0) {
             mbar_wait(bar_free, ph ^ 1u);                // the last tile's dW1 MMAs
-            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+            tc_fence_after();
             const float inv = args.scale[1];
 #pragma unroll
             for (int hf = 0; hf < 2; ++hf) {
@@ -815,7 +767,7 @@ __device__ __forceinline__ void bwd_role(const BwdArgs& args, const PipeCtx& px,
                 const uint32_t v = rowj == 16 ? 0x3C003C00u : 0u;              // fp16 1.0 pairs
                 *reinterpret_cast<uint4*>(smem + BW_A1T + off) = make_uint4(v, v, v, v);
             }
-            asm volatile("bar.sync 1, 128;" ::: "memory");                     // the four I/O warps only
+            bar_sync(1, 128);                     // the four I/O warps only
         }
         const float S = args.scale[0];
         uint32_t ph = 0;
@@ -883,7 +835,7 @@ __device__ __forceinline__ void bwd_role(const BwdArgs& args, const PipeCtx& px,
             }
             if (tile != first) mbar_wait(bar_d5b, ph ^ 1u);                       // the previous tile's D5 (both halves) has read d3a
             *reinterpret_cast<uint4*>(d3a) = make_uint4(p01, p23, 0u, 0u);
-            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+            fence_proxy_async_smem();
             __syncwarp();
             if (lane == 0) mbar_arrive(bar_dl3);
             if (!piped) {
@@ -904,11 +856,7 @@ __device__ __forceinline__ void bwd_role(const BwdArgs& args, const PipeCtx& px,
         }
     }
 
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    __syncthreads();
-    if (warp == 16) {
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512u) : "memory");
-    }
+    tmem_teardown(warp == 16, tmem_base, 512u);
 }
 
 __global__ void __launch_bounds__(BW_THREADS, 1) bwd_tc_kernel(const __grid_constant__ BwdArgs args) {
@@ -958,16 +906,9 @@ __device__ __forceinline__ void dw_role(const DwArgs& args, const PipeCtx& px, c
             mbar_init(bar_empty0 + 8u * i, kWhich == 2 ? 5 : 1);   // the MMA commit (+ the four column-sum warps of the dW2 role)
         }
         mbar_init(bar_done, 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        mbar_init_fence();
     }
-    if (warp == 1) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(s_u32(tmem_slot)), "r"(Cfg::kTmemCols) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    __syncthreads();
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    const uint32_t tmem_base = *tmem_slot;
+    const uint32_t tmem_base = tmem_setup(warp == 1, tmem_slot, Cfg::kTmemCols);
     const int64_t n_my = rank < args.n_tiles ? (args.n_tiles - rank + nranks - 1) / nranks : 0;
     const int64_t n_it = 2 * n_my;                          // 64-sample half tiles
     uint32_t* c_done = kWhich == 2 ? px.c2_done : px.c13_done;      // (c13_done: the dW3 role)
@@ -986,27 +927,18 @@ __device__ __forceinline__ void dw_role(const DwArgs& args, const PipeCtx& px, c
                     flag_wait(px.b_done + tile);             // forward and backward outputs of the tile are in its slot
                     wait_cycles += clock64() - w0;
                     prog(px, 6, wait_cycles >> 10);
-                    asm volatile("fence.proxy.async;" ::: "memory");
+                    fence_proxy_async();
                 }
                 const uint32_t bar = bar_full0 + 8u * st;
-                asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"((uint32_t)Cfg::kStageBytes) : "memory");
+                mbar_expect_tx(bar, (uint32_t)Cfg::kStageBytes);
                 const uint32_t sa = s_u32(smem + st * Cfg::kStageBytes);
                 const uint8_t* ga = (kWhich == 2 ? args.h1 : args.h2) + (size_t)half * ACT_TILE_BYTES;
-#pragma unroll
-                for (uint32_t off = 0; off < (uint32_t)ACT_TILE_BYTES; off += 16384u)
-                    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(sa + off),
-                                 "l"(ga + off), "r"(16384u), "r"(bar) : "memory");
+                bulk_load_chunked<16384u>(sa, ga, (uint32_t)ACT_TILE_BYTES, bar);
                 if (kWhich == 2) {
                     const uint8_t* gb = args.dl2 + (size_t)half * ACT_TILE_BYTES;
-#pragma unroll
-                    for (uint32_t off = 0; off < (uint32_t)ACT_TILE_BYTES; off += 16384u)
-                        asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-                                         sa + (uint32_t)ACT_TILE_BYTES + off),
-                                     "l"(gb + off), "r"(16384u), "r"(bar) : "memory");
+                    bulk_load_chunked<16384u>(sa + (uint32_t)ACT_TILE_BYTES, gb, (uint32_t)ACT_TILE_BYTES, bar);
                 } else {
-                    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-                                     sa + (uint32_t)ACT_TILE_BYTES),
-                                 "l"(args.d3t + (size_t)half * SMALL_TILE_BYTES), "r"((uint32_t)SMALL_TILE_BYTES), "r"(bar) : "memory");
+                    bulk_load(sa + (uint32_t)ACT_TILE_BYTES, args.d3t + (size_t)half * SMALL_TILE_BYTES, (uint32_t)SMALL_TILE_BYTES, bar);
                 }
             }
         }
@@ -1016,19 +948,19 @@ __device__ __forceinline__ void dw_role(const DwArgs& args, const PipeCtx& px, c
         if (lane == 0) {
             for (int64_t j = 0; j < n_it; ++j) {
                 mbar_wait(bar_empty0 + 8u * (uint32_t)(j % Cfg::kStages), (uint32_t)(j / Cfg::kStages) & 1u);
-                if (j & 1) asm volatile("st.release.gpu.global.u32 [%0], %1;" ::"l"(c_done + rank + (j >> 1) * nranks), "r"(1u) : "memory");
+                if (j & 1) st_release_gpu(c_done + rank + (j >> 1) * nranks, 1u);
             }
         }
         __syncwarp();
     } else if (warp == 1) {
         if (lane == 0) {
-            constexpr uint32_t idesc2 = ((1u << 4) | ((uint32_t)(256 >> 3) << 17) | ((uint32_t)(128 >> 4) << 24)) | kIdescAMn | kIdescBMn;
-            constexpr uint32_t idesc16 = ((1u << 4) | ((uint32_t)(16 >> 3) << 17) | ((uint32_t)(128 >> 4) << 24)) | kIdescAMn;
+            constexpr uint32_t idesc2 = idesc_f16(128, 256) | kIdescAMn | kIdescBMn;
+            constexpr uint32_t idesc16 = idesc_f16(128, 16) | kIdescAMn;
             for (int64_t it = 0; it < n_it; ++it) {
                 const int st = (int)(it % Cfg::kStages);
                 const int64_t use = it / Cfg::kStages;
                 mbar_wait(bar_full0 + 8u * st, (uint32_t)use & 1u);
-                asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+                tc_fence_after();
                 const uint32_t sa = s_u32(smem + st * Cfg::kStageBytes), sb = sa + (uint32_t)ACT_TILE_BYTES;
                 const uint32_t acc = it ? 1u : 0u;
 #pragma unroll
@@ -1086,7 +1018,7 @@ __device__ __forceinline__ void dw_role(const DwArgs& args, const PipeCtx& px, c
         // ---- read-out: TMEM lane quarter = warp % 4
         if (n_it > 0) {
             mbar_wait(bar_done, 0);
-            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+            tc_fence_after();
             const int q = warp & 3;
             const uint32_t tlane = tmem_base + ((uint32_t)(q * 32) << 16);
 #pragma unroll
@@ -1114,11 +1046,7 @@ __device__ __forceinline__ void dw_role(const DwArgs& args, const PipeCtx& px, c
             }
         }
     }
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    __syncthreads();
-    if (warp == 1) {
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(Cfg::kTmemCols) : "memory");
-    }
+    tmem_teardown(warp == 1, tmem_base, Cfg::kTmemCols);
 }
 
 // ------------------------------------------------------------------------------------------------ the persistent update pipeline

@@ -81,7 +81,7 @@ __device__ __forceinline__ uint32_t pack_bf16(float a, float b) {
 
 // Epilogues 1 / 2: relu + bf16 pack of this warp's 16 columns in each of the four K slabs into the shared-memory
 // operand of the next MMA.  The same bytes are the global activation image of the tile: the MMA warp streams each
-// finished slab out with bulk async copies (store_slab), so the epilogue threads issue no global stores (a per-thread
+// finished slab out with bulk async copies (store_act_slab), so the epilogue threads issue no global stores (a per-thread
 // 16-byte store at a 128-byte stride costs 32 LSU wavefronts per instruction and was the kernel's bottleneck).
 // Returns the 64 "z > 0" bits of the thread's columns (bit 16 s + 15 - i for column i of slab s).
 __device__ __forceinline__ uint64_t fb_relu_store(uint32_t tcol0, uint8_t* a2_row, int row, int g, int lane, uint32_t bar0) {
@@ -101,8 +101,8 @@ __device__ __forceinline__ uint64_t fb_relu_store(uint32_t tcol0, uint8_t* a2_ro
             const int sw = ((g * 2 + c) ^ (row & 7)) << 4;
             *reinterpret_cast<uint4*>(a2_row + s * 16384 + sw) = v;
         }
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-        asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+        fence_proxy_async_smem();
+        tc_fence_before();
         __syncwarp();
         if (lane == 0) mbar_arrive(bar0 + 8u * s);
     }
@@ -112,21 +112,6 @@ __device__ __forceinline__ uint64_t fb_relu_store(uint32_t tcol0, uint8_t* a2_ro
 __device__ __forceinline__ float bf_lo(uint32_t w) { return __uint_as_float(w << 16); }
 __device__ __forceinline__ float bf_hi(uint32_t w) { return __uint_as_float(w & 0xFFFF0000u); }
 
-// slab g of the [128 rows x 4 slabs] shared-memory tile -> the two 64-row tiles of a global activation image
-__device__ __forceinline__ void store_slab(uint8_t* img, int64_t tile, uint32_t sA2, int g) {
-#pragma unroll
-    for (int half = 0; half < 2; ++half) {
-        uint8_t* dst = img + (size_t)(tile * 2 + half) * ACT_TILE_BYTES + (size_t)g * ACT_SLAB_BYTES;
-        asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(dst),
-                     "r"(sA2 + (uint32_t)g * 16384u + (uint32_t)half * 8192u), "r"((uint32_t)ACT_SLAB_BYTES)
-                     : "memory");
-    }
-}
-// all bulk stores issued so far by this thread have finished READING shared memory
-__device__ __forceinline__ void bulk_stores_read_done() {
-    asm volatile("cp.async.bulk.commit_group;" ::: "memory");
-    asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
-}
 
 constexpr int FB_THREADS = 512 + 32 + 128;
 
@@ -159,17 +144,10 @@ __global__ void __launch_bounds__(FB_THREADS, 1) fb_tc_kernel(const __grid_const
             mbar_init(bar_bslab0 + 8u * g, 16);
             mbar_init(bar_dslab0 + 8u * g, 16);
         }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        mbar_init_fence();
     }
-    if (warp == 16) {   // D1 = columns 0..255 (D3 re-uses 0..15 once D1 is drained), D2 / D4 = columns 256..511
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(s_u32(tmem_slot)), "r"(512u)
-                     : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    __syncthreads();
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    const uint32_t tmem_base = *tmem_slot;
+    // D1 = columns 0..255 (D3 re-uses 0..15 once D1 is drained), D2 / D4 = columns 256..511
+    const uint32_t tmem_base = tmem_setup(warp == 16, tmem_slot, 512u);
     const int64_t n_tiles = (args.n + TC_M - 1) / TC_M;
     const int64_t first = blockIdx.x;
 
@@ -179,24 +157,16 @@ __global__ void __launch_bounds__(FB_THREADS, 1) fb_tc_kernel(const __grid_const
         const uint32_t sW1 = s_u32(smem + IMG_W1), sW2 = s_u32(smem + IMG_W2), sW3 = s_u32(smem + IMG_W3);
         const uint64_t dBias = desc_nosw_k16(s_u32(smem + IMG_BIAS));
         const uint64_t dOnes1 = desc_ones(s_u32(smem + IMG_ONES1)), dOnes2 = desc_ones(s_u32(smem + IMG_ONES2));
-        constexpr uint32_t kIdescBwd = idesc_f16(TC_M, TC_H) | kIdescBMn;
+        constexpr uint32_t kIdescBwd = idesc_bf16(TC_M, TC_H) | kIdescBMn;
         if (lane == 0) {
-            asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar_img), "r"((uint32_t)IMG_BYTES)
-                         : "memory");
-            constexpr uint32_t kChunk = 16384;
-            for (uint32_t off = 0; off < (uint32_t)IMG_BYTES; off += kChunk) {
-                uint32_t sz = (uint32_t)IMG_BYTES - off < kChunk ? (uint32_t)IMG_BYTES - off : kChunk;
-                asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-                                 s_u32(smem + off)),
-                             "l"(args.img + off), "r"(sz), "r"(bar_img)
-                             : "memory");
-            }
+            mbar_expect_tx(bar_img, (uint32_t)IMG_BYTES);
+            bulk_load_chunked<16384u>(s_u32(smem), args.img, (uint32_t)IMG_BYTES, bar_img);
             mbar_wait(bar_img, 0);
         }
         __syncwarp();
         auto issue_layer1 = [&](uint32_t ph) {
             mbar_wait(bar_a1, ph);
-            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+            tc_fence_after();
             umma_f16(tmem_base, desc_nosw_k16(sA1), desc_nosw_k16(sW1), kIdesc, 0u);
             umma_f16(tmem_base, dOnes1, dBias, kIdesc, 1u);
             umma_commit(bar_d1);
@@ -209,63 +179,67 @@ __global__ void __launch_bounds__(FB_THREADS, 1) fb_tc_kernel(const __grid_const
                 //      (its D4 was drained before the DL1 slab arrivals this warp waited for at the end of that tile)
                 for (int g = 0; g < 4; ++g) {
                     mbar_wait(bar_slab0 + 8u * g, ph);
-                    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+                    tc_fence_after();
 #pragma unroll
                     for (int q = 0; q < 4; ++q)
                         umma_f16(tmem_base + 256u, desc_sw128(sA2 + (uint32_t)g * 16384u + (uint32_t)q * 32u),
                                  desc_sw128(sW2 + (uint32_t)g * 32768u + (uint32_t)q * 32u), kIdesc, (g | q) ? 1u : 0u);
-                    store_slab(args.h1, tile, sA2, g);
+                    store_act_slab(args.h1, tile, sA2, g);
                 }
                 umma_f16(tmem_base + 256u, dOnes2, dBias, kIdesc, 1u);
-                bulk_stores_read_done();                 // epilogue 2 overwrites H1 once bar_d2 completes
+                bulk_commit();
+                bulk_wait_read();                        // epilogue 2 overwrites H1 once bar_d2 completes
                 umma_commit(bar_d2);
                 // ---- head: D3 = columns 0..15 (D1 has been drained by every warp before the H1 slab arrivals)
                 for (int g = 0; g < 4; ++g) {
                     mbar_wait(bar_hslab0 + 8u * g, ph);
-                    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+                    tc_fence_after();
 #pragma unroll
                     for (int q = 0; q < 4; ++q)
                         umma_f16(tmem_base, desc_sw128(sA2 + (uint32_t)g * 16384u + (uint32_t)q * 32u),
                                  desc_sw128(sW3 + (uint32_t)g * 2048u + (uint32_t)q * 32u), kIdescHead, (g | q) ? 1u : 0u);
-                    store_slab(args.h2, tile, sA2, g);
+                    store_act_slab(args.h2, tile, sA2, g);
                 }
-                bulk_stores_read_done();                 // epilogue 3 overwrites H2 once bar_d3 completes
+                bulk_commit();
+                bulk_wait_read();                        // epilogue 3 overwrites H2 once bar_d3 completes
                 umma_commit(bar_d3);
                 // ---- backward through the head: D5 = d3 . W3^T into columns 0..255 (D1 / D3 are dead: the I/O warps have
                 //      read D3).  A = d3 as bf16 [128 x 16] (K-major, A1's layout); B = the head's W3 image [j][f]
                 //      read MN-major (N = f contiguous: 64-wide slabs 2048 B apart, 8 K rows = 1024 B).
                 mbar_wait(bar_dl3, ph);
-                asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+                tc_fence_after();
                 umma_f16(tmem_base, desc_nosw_k16(s_u32(smem + FB_D3A)), desc_sw128_mn(sW3, 2048u), kIdescBwd, 0u);
                 umma_commit(bar_d5);
                 // ---- backward through layer 2: D4 = DL2 . W2 over K = out features; B = the W2 image [out][in]
                 //      read MN-major (N = in contiguous: 64-wide slabs 32768 B apart, 8 K rows = 1024 B)
                 for (int g = 0; g < 4; ++g) {
                     mbar_wait(bar_bslab0 + 8u * g, ph);
-                    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+                    tc_fence_after();
 #pragma unroll
                     for (int q = 0; q < 4; ++q)
                         umma_f16(tmem_base + 256u, desc_sw128(sA2 + (uint32_t)g * 16384u + (uint32_t)q * 32u),
                                  desc_sw128_mn(sW2 + (uint32_t)(g * 64 + q * 16) * 128u, 32768u), kIdescBwd,
                                  (g | q) ? 1u : 0u);
-                    store_slab(args.dl2, tile, sA2, g);
+                    store_act_slab(args.dl2, tile, sA2, g);
                 }
-                bulk_stores_read_done();                 // epilogue 4 overwrites DL2 once bar_d4 completes
+                bulk_commit();
+                bulk_wait_read();                        // epilogue 4 overwrites DL2 once bar_d4 completes
                 umma_commit(bar_d4);
                 // ---- the next tile's layer 1 (D5 was drained by every warp before the DL2 slab arrivals)
                 if (tile + gridDim.x < n_tiles) issue_layer1(ph ^ 1u);
                 // ---- DL1 leaves through the same buffer; the next tile's epilogue 1 may reuse it afterwards
                 for (int g = 0; g < 4; ++g) {
                     mbar_wait(bar_dslab0 + 8u * g, ph);
-                    store_slab(args.dl1, tile, sA2, g);
+                    store_act_slab(args.dl1, tile, sA2, g);
                 }
-                bulk_stores_read_done();
+                bulk_commit();
+                bulk_wait_read();
                 mbar_arrive(bar_free);
             }
             __syncwarp();
             ph ^= 1u;
         }
-        if (lane == 0) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");   // image writes complete before exit
+        if (lane == 0) bulk_wait();   // image writes complete before exit
         __syncwarp();
     } else if (warp < 16) {
         // ============================ epilogue warps ============================
@@ -283,19 +257,19 @@ __global__ void __launch_bounds__(FB_THREADS, 1) fb_tc_kernel(const __grid_const
             mbar_wait(bar_d1, ph);
             if (tile != first) mbar_wait(bar_free, ph ^ 1u);
             if (dbg) dc[1] = clock64();
-            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+            tc_fence_after();
             const uint64_t m1 = fb_relu_store(tlane, a2_row, row, g, lane, bar_slab0);
             if (dbg) dc[2] = clock64();
             // ---- epilogue 2: H2 over H1 (layer 2 has completed)
             mbar_wait(bar_d2, ph);
             if (dbg) dc[3] = clock64();
-            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+            tc_fence_after();
             const uint64_t m2 = fb_relu_store(tlane + 256u, a2_row, row, g, lane, bar_hslab0);
             if (dbg) dc[4] = clock64();
             // ---- epilogue 3: DL2 = D5 [z2 > 0] over H2 (D5 complete => the head MMAs that read H2 have completed)
             mbar_wait(bar_d5, ph);
             if (dbg) dc[5] = clock64();
-            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+            tc_fence_after();
 #pragma unroll
             for (int s = 0; s < 4; ++s) {
                 uint32_t rr[16];
@@ -314,8 +288,8 @@ __global__ void __launch_bounds__(FB_THREADS, 1) fb_tc_kernel(const __grid_const
                     const int sw = ((g * 2 + c) ^ (row & 7)) << 4;
                     *reinterpret_cast<uint4*>(a2_row + s * 16384 + sw) = make_uint4(out[0], out[1], out[2], out[3]);
                 }
-                asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-                asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+                fence_proxy_async_smem();
+                tc_fence_before();
                 __syncwarp();
                 if (lane == 0) mbar_arrive(bar_bslab0 + 8u * s);
             }
@@ -323,7 +297,7 @@ __global__ void __launch_bounds__(FB_THREADS, 1) fb_tc_kernel(const __grid_const
             // ---- epilogue 4: DL1 = D4 [z1 > 0] over DL2 (the backward MMAs have completed), streamed out by the MMA warp
             mbar_wait(bar_d4, ph);
             if (dbg) dc[7] = clock64();
-            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+            tc_fence_after();
 #pragma unroll
             for (int s = 0; s < 4; ++s) {
                 uint32_t rr[16];
@@ -342,8 +316,8 @@ __global__ void __launch_bounds__(FB_THREADS, 1) fb_tc_kernel(const __grid_const
                     const int sw = ((g * 2 + c) ^ (row & 7)) << 4;
                     *reinterpret_cast<uint4*>(a2_row + s * 16384 + sw) = make_uint4(out[0], out[1], out[2], out[3]);
                 }
-                asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-                asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+                fence_proxy_async_smem();
+                tc_fence_before();
                 __syncwarp();
                 if (lane == 0) mbar_arrive(bar_dslab0 + 8u * s);
             }
@@ -378,7 +352,7 @@ __global__ void __launch_bounds__(FB_THREADS, 1) fb_tc_kernel(const __grid_const
             uint8_t* a1 = smem + SM_A1 + (row >> 3) * 256 + (row & 7) * 16;
             *reinterpret_cast<uint4*>(a1) = make_uint4(packed[0], packed[1], packed[2], packed[3]);
             *reinterpret_cast<uint4*>(a1 + 128) = make_uint4(packed[4], packed[5], packed[6], packed[7]);
-            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+            fence_proxy_async_smem();
             __syncwarp();
             if (lane == 0) mbar_arrive(bar_a1);
         };
@@ -400,10 +374,10 @@ __global__ void __launch_bounds__(FB_THREADS, 1) fb_tc_kernel(const __grid_const
             const int64_t next = tile + gridDim.x;
             if (next < n_tiles) encode_a1(next);
             mbar_wait(bar_d3, ph);
-            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+            tc_fence_after();
             uint32_t r4[4];
             tmem_ld4(tlane, r4);
-            asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+            tc_fence_before();
             float d0, d1 = 0.0f, d2 = 0.0f, d3 = 0.0f;
             if (args.head_mode == 0) {
                 const float lg0 = __uint_as_float(r4[0]) + sB3[0], lg1 = __uint_as_float(r4[1]) + sB3[1];
@@ -423,7 +397,7 @@ __global__ void __launch_bounds__(FB_THREADS, 1) fb_tc_kernel(const __grid_const
             // d3 as the bf16 A operand of D5 = d3 W3^T (k = 0..3 real), then release the MMA warp
             const uint32_t p01 = pack_bf16(d0, d1), p23 = pack_bf16(d2, d3);
             *reinterpret_cast<uint4*>(d3a) = make_uint4(p01, p23, 0u, 0u);
-            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+            fence_proxy_async_smem();
             __syncwarp();
             if (lane == 0) mbar_arrive(bar_dl3);
             // off the critical path: transposed bf16 copy for dW3 = H2^T d3 (rows >= n_out of the small image stay
@@ -445,11 +419,7 @@ __global__ void __launch_bounds__(FB_THREADS, 1) fb_tc_kernel(const __grid_const
         }
     }
 
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    __syncthreads();
-    if (warp == 16) {
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512u) : "memory");
-    }
+    tmem_teardown(warp == 16, tmem_base, 512u);
 }
 
 // ------------------------------------------------------------------------------------------------ dW GEMM
@@ -472,18 +442,9 @@ __global__ void __launch_bounds__(ATB_THREADS, 1) atb_tc_kernel(const __grid_con
             mbar_init(bar_empty0 + 8u * i, want_colsum ? 5 : 1);
         }
         mbar_init(bar_done, 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        mbar_init_fence();
     }
-    if (warp == 1) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(s_u32(tmem_slot)),
-                     "r"(Cfg::kTmemCols)
-                     : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    __syncthreads();
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    const uint32_t tmem_base = *tmem_slot;
+    const uint32_t tmem_base = tmem_setup(warp == 1, tmem_slot, Cfg::kTmemCols);
     // balanced contiguous ranges of 64-sample tiles (gridDim.x <= tiles64, so every CTA owns at least one)
     const int64_t t0 = args.tiles64 * blockIdx.x / gridDim.x, t1 = args.tiles64 * (blockIdx.x + 1) / gridDim.x;
     const int n_it = (int)(t1 - t0);
@@ -494,34 +455,23 @@ __global__ void __launch_bounds__(ATB_THREADS, 1) atb_tc_kernel(const __grid_con
                 const int st = it % Cfg::kStages, use = it / Cfg::kStages;
                 if (use > 0) mbar_wait(bar_empty0 + 8u * st, (uint32_t)(use - 1) & 1u);
                 const uint32_t bar = bar_full0 + 8u * st;
-                asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar),
-                             "r"((uint32_t)Cfg::kStageBytes)
-                             : "memory");
+                mbar_expect_tx(bar, (uint32_t)Cfg::kStageBytes);
                 const uint8_t* ga = args.A + (size_t)(t0 + it) * ACT_TILE_BYTES;
                 const uint8_t* gb = args.B + (size_t)(t0 + it) * Cfg::kBBytes;
                 uint8_t* sa = smem + st * Cfg::kStageBytes;
-                for (int off = 0; off < ACT_TILE_BYTES; off += 16384)
-                    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-                                     s_u32(sa + off)),
-                                 "l"(ga + off), "r"(16384u), "r"(bar)
-                                 : "memory");
-                constexpr int kBChunk = Cfg::kBBytes < 16384 ? Cfg::kBBytes : 16384;
-                for (int off = 0; off < Cfg::kBBytes; off += kBChunk)
-                    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-                                     s_u32(sa + ACT_TILE_BYTES + off)),
-                                 "l"(gb + off), "r"((uint32_t)kBChunk), "r"(bar)
-                                 : "memory");
+                bulk_load_chunked<16384u>(s_u32(sa), ga, (uint32_t)ACT_TILE_BYTES, bar);
+                bulk_load_chunked<16384u>(s_u32(sa + ACT_TILE_BYTES), gb, (uint32_t)Cfg::kBBytes, bar);
             }
         }
         __syncwarp();
     } else if (warp == 1) {
         if (lane == 0) {
             // kind::f16 operand format bits (7-9: A, 10-12: B): 1 = bf16, 0 = fp16
-            const uint32_t idesc = (idesc_f16(128, NB) & ~(args.f16 ? ((1u << 7) | (1u << 10)) : 0u)) | kIdescAMn | (NB == 256 ? kIdescBMn : 0u);
+            const uint32_t idesc = (args.f16 ? idesc_f16(128, NB) : idesc_bf16(128, NB)) | kIdescAMn | (NB == 256 ? kIdescBMn : 0u);
             for (int it = 0; it < n_it; ++it) {
                 const int st = it % Cfg::kStages, use = it / Cfg::kStages;
                 mbar_wait(bar_full0 + 8u * st, (uint32_t)use & 1u);
-                asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+                tc_fence_after();
                 const uint32_t sa = s_u32(smem + st * Cfg::kStageBytes), sb = sa + ACT_TILE_BYTES;
 #pragma unroll
                 for (int kk = 0; kk < 4; ++kk) {                                   // 16 samples per MMA
@@ -578,7 +528,7 @@ __global__ void __launch_bounds__(ATB_THREADS, 1) atb_tc_kernel(const __grid_con
         // ---- read-out: TMEM lane quarter = warp % 4
         if (n_it > 0) {
             mbar_wait(bar_done, 0);
-            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+            tc_fence_after();
             const int q = warp & 3;
             const uint32_t tlane = tmem_base + ((uint32_t)(q * 32) << 16);
 #pragma unroll
@@ -598,11 +548,7 @@ __global__ void __launch_bounds__(ATB_THREADS, 1) atb_tc_kernel(const __grid_con
         }
     }
 
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    __syncthreads();
-    if (warp == 1) {
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(Cfg::kTmemCols) : "memory");
-    }
+    tmem_teardown(warp == 1, tmem_base, Cfg::kTmemCols);
 }
 
 template <int NB>

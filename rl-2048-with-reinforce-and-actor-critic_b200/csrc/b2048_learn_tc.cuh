@@ -23,6 +23,14 @@ __device__ __forceinline__ size_t small_off(int64_t r, int j) {
     return (size_t)(r >> 6) * SMALL_TILE_BYTES + (size_t)j * 128 + (size_t)(((int)((r & 63) >> 3) ^ (j & 7)) << 4) +
            (size_t)(r & 7) * 2;
 }
+// slab g of the [128 rows x 4 slabs] shared-memory tile at sA2 -> the two 64-row tiles of a global activation image
+__device__ __forceinline__ void store_act_slab(uint8_t* img, int64_t tile, uint32_t sA2, int g) {
+#pragma unroll
+    for (int half = 0; half < 2; ++half) {
+        uint8_t* dst = img + (size_t)(tile * 2 + half) * ACT_TILE_BYTES + (size_t)g * ACT_SLAB_BYTES;
+        bulk_store(dst, sA2 + (uint32_t)g * 16384u + (uint32_t)half * 8192u, (uint32_t)ACT_SLAB_BYTES);
+    }
+}
 
 struct AtbArgs {
     const uint8_t* A;       // activation image (MN-major A operand: M = 256 features, K = samples)

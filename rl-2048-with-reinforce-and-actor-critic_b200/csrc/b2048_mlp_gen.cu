@@ -223,44 +223,8 @@ struct GenArgs {
     long long* dbg;             // optional phase clocks of CTA 0 (B2048_DBG_TC_CLOCKS), 64 slots per tile for the first 4 tiles
 };
 
-__host__ __device__ constexpr uint32_t idesc_h(int m, int n) {          // kind::f16, A/B fp16, D fp32
-    return (1u << 4) | ((uint32_t)(n >> 3) << 17) | ((uint32_t)(m >> 4) << 24);
-}
-// a wait that cannot hang the device: a legitimate wait lasts micro- to milliseconds; after ~2 s the kernel traps
-__device__ __forceinline__ uint32_t gtry(uint32_t bar, uint32_t parity) {
-    uint32_t ok;
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(ok)
-        : "r"(bar), "r"(parity)
-        : "memory");
-    return ok;
-}
-__device__ __forceinline__ void gwait(uint32_t bar, uint32_t parity) {
-    if (gtry(bar, parity)) return;
-    const long long t0 = clock64();
-    while (!gtry(bar, parity))
-        if (clock64() - t0 > 4000000000LL) __trap();
-}
-// umma_w (tcgen05.mma from 32-bit descriptor halves): b2048_tc.cuh
-__device__ __forceinline__ uint32_t gpack(float a, float b) {
-    __half2 p = __floats2half2_rn(a, b);
-    return *reinterpret_cast<uint32_t*>(&p);
-}
-__device__ __forceinline__ void g_bulk_load(uint32_t dst, const uint8_t* src, uint32_t bytes, uint32_t bar) {
-    for (uint32_t off = 0; off < bytes; off += 16384u) {
-        const uint32_t sz = bytes - off < 16384u ? bytes - off : 16384u;
-        asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(dst + off),
-                     "l"(src + off), "r"(sz), "r"(bar)
-                     : "memory");
-    }
-}
 __device__ __forceinline__ void g_bulk_store(uint8_t* dst, uint32_t src, uint32_t bytes) {
-    for (uint32_t off = 0; off < bytes; off += 16384u)
-        asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(dst + off), "r"(src + off), "r"(16384u)
-                     : "memory");
+    for (uint32_t off = 0; off < bytes; off += 16384u) bulk_store(dst + off, src + off, 16384u);
 }
 
 // Row `row` of the network input as fp16 K-major slab rows: slabs slab0 .. slab0 + nslabs - 1 of the input go to dst,
@@ -351,23 +315,23 @@ struct UnitSeq {
         constexpr GGemm gm = SP::P.gemm[G];
         constexpr uint32_t r = SP::P.rec[U];
         constexpr uint32_t ks = (r >> 16) & 7u, kind = (r >> 19) & 3u, slab = (r >> 24) & 7u;
-        constexpr uint32_t idesc = idesc_h(TC_M, gm.N);
+        constexpr uint32_t idesc = idesc_f16(TC_M, gm.N);
         constexpr uint32_t HI_SW = 0x40004040u, HI_NOSW = 0x4010u, HI_ONES = 0x4000u;
         constexpr uint32_t acc0 = U == gm.u0 ? 0u : 1u;
         if constexpr ((r & GR_SLABWAIT) != 0) {
-            gwait(c.bar_slab0 + 8u * slab, (c.spar >> slab) & 1u);
+            mbar_wait_or_trap(c.bar_slab0 + 8u * slab, (c.spar >> slab) & 1u);
             c.spar ^= 1u << slab;
-            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+            tc_fence_after();
         }
         if constexpr ((r & GR_STORE) != 0) {
             if (c.leader) {
                 g_bulk_store(img_dst + (size_t)slab * GN_SLAB, c.sA + slab * GN_SLAB, GN_SLAB);
-                asm volatile("cp.async.bulk.commit_group;" ::: "memory");
+                bulk_commit();
             }
         }
         if constexpr ((r & GR_FIRST) != 0) {
             c.slot = c.U % GN_NSLOT;
-            gwait(c.w_full0 + 8u * c.slot, (c.U / GN_NSLOT) & 1u);
+            mbar_wait_or_trap(c.w_full0 + 8u * c.slot, (c.U / GN_NSLOT) & 1u);
             c.wb_base = (c.sW + c.slot * GN_SLOT) >> 4;
         }
         if (c.leader) {
@@ -405,8 +369,8 @@ struct GemmSeq {
         constexpr GGemm gm = SP::P.gemm[G];
         constexpr bool store = SP::P.fb != 0 && G > 0;
         if constexpr (gm.from_io != 0) {
-            gwait(c.bar_io, c.nio & 1u); ++c.nio;
-            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+            mbar_wait_or_trap(c.bar_io, c.nio & 1u); ++c.nio;
+            tc_fence_after();
         }
         uint8_t* img_dst = nullptr;
         if constexpr (store) {
@@ -415,7 +379,7 @@ struct GemmSeq {
         }
         UnitSeq<SP, G, gm.u0, gm.u0 + gm.nu>::run(c, img_dst);
         if (c.leader) {
-            if constexpr (store) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
+            if constexpr (store) bulk_wait_read();
             umma_commit(gm.head ? c.bar_acc_h : c.bar_acc_e);
         }
         GemmSeq<SP, G + 1, GEND>::run(c, a, tile);
@@ -448,22 +412,15 @@ __global__ void __launch_bounds__(GN_THREADS, 1) gen_mlp_kernel(const __grid_con
         mbar_init(bar_acc_e, 1);     // an accumulator for the epilogue warps is complete
         mbar_init(bar_acc_h, 1);     // the head accumulator (I/O warps) is complete
         mbar_init(bar_free, 1);      // update mode: the tile's last image has left the A buffer
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        mbar_init_fence();
     }
     if (tid < 64) {      // ONES operand: [2 k-chunks][8 rows][8 halves]; chunk 0 of every row = (1, 1, 0, ...)
         const int e = tid & 7, chunk = tid >> 5;
         reinterpret_cast<uint32_t*>(smem + GS_ONES)[tid] = 0u;
         if (chunk == 0 && (e & 3) == 0) reinterpret_cast<uint32_t*>(smem + GS_ONES)[tid] = 0x3C003C00u;
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+        fence_proxy_async_smem();
     }
-    if (warp == 16) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(s_u32(tmem_slot)), "r"(512u) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    __syncthreads();
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    const uint32_t tmem_base = *tmem_slot;
+    const uint32_t tmem_base = tmem_setup(warp == 16, tmem_slot, 512u);
     const int64_t n_eff = a.n_dev ? (int64_t)*a.n_dev : a.n;        // uniform over the grid
     const int64_t n_tiles = (n_eff + TC_M - 1) / TC_M;
     const uint32_t sA = s_u32(smem + GS_A), sW = s_u32(smem + GS_W);
@@ -488,18 +445,18 @@ __global__ void __launch_bounds__(GN_THREADS, 1) gen_mlp_kernel(const __grid_con
                     constexpr int nsl = SP::P.width[0] >> 6;
 #pragma unroll
                     for (int sl = 0; sl < nsl; ++sl) {
-                        gwait(bar_slab0 + 8u * (uint32_t)sl, (c.spar >> sl) & 1u);
+                        mbar_wait_or_trap(bar_slab0 + 8u * (uint32_t)sl, (c.spar >> sl) & 1u);
                         c.spar ^= 1u << sl;
                         if (c.leader) g_bulk_store(a.dlimg[0] + ((size_t)tile * nsl + sl) * GN_SLAB, sA + (uint32_t)sl * GN_SLAB, GN_SLAB);
                     }
                     if (c.leader) {
-                        asm volatile("cp.async.bulk.commit_group;" ::: "memory");
-                        asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
+                        bulk_commit();
+                        bulk_wait_read();
                         mbar_arrive(bar_free);
                     }
                 }
             }
-            if (c.leader) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
+            if (c.leader) bulk_wait();
         } else {
             const bool leader = lane == 0;
             uint32_t U = 0, nio = 0, spar = 0;      // ring fills consumed; I/O hand-offs; phase parity of the four slab barriers
@@ -514,8 +471,8 @@ __global__ void __launch_bounds__(GN_THREADS, 1) gen_mlp_kernel(const __grid_con
                     const bool from_io = gm.from_io != 0;
                     long long wsum = 0;
                     if (from_io) {
-                        gwait(bar_io, nio & 1u); ++nio;
-                        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+                        mbar_wait_or_trap(bar_io, nio & 1u); ++nio;
+                        tc_fence_after();
                         if (dc) dc[1 + 3 * G] = clock64();
                     }
                     // in update mode the A operand of every GEMM but the first is an image the dW GEMMs read
@@ -526,7 +483,7 @@ __global__ void __launch_bounds__(GN_THREADS, 1) gen_mlp_kernel(const __grid_con
                         img_dst = (!gm.bwd ? a.himg[gm.layer - 1] : a.dlimg[gm.layer]) + (size_t)tile * nsl * GN_SLAB;
                     }
                     const uint32_t dcol = tmem_base + (uint32_t)(G & 1) * 256u;
-                    const uint32_t idesc = idesc_h(TC_M, gm.N);
+                    const uint32_t idesc = idesc_f16(TC_M, gm.N);
                     uint32_t acc = 0u;
                     for (int f = gm.f0; f < gm.f0 + gm.nf; ++f, ++U) {
                         const GFill fl = P.fill[f];
@@ -536,19 +493,19 @@ __global__ void __launch_bounds__(GN_THREADS, 1) gen_mlp_kernel(const __grid_con
                             const GUnit un = P.unit[u];
                             if (un.kind == 0 || un.kind == 2) {      // first unit of K slab un.slab
                                 if (!from_io) {
-                                    gwait(bar_slab0 + 8u * (uint32_t)un.slab, (spar >> un.slab) & 1u);
+                                    mbar_wait_or_trap(bar_slab0 + 8u * (uint32_t)un.slab, (spar >> un.slab) & 1u);
                                     spar ^= 1u << un.slab;
-                                    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+                                    tc_fence_after();
                                     if (dc && un.slab == 0) dc[1 + 3 * G] = clock64();
                                 }
                                 if (store && leader) {
                                     g_bulk_store(img_dst + (size_t)un.slab * GN_SLAB, sA + (uint32_t)un.slab * GN_SLAB, GN_SLAB);
-                                    asm volatile("cp.async.bulk.commit_group;" ::: "memory");
+                                    bulk_commit();
                                 }
                             }
                             if (!loaded) {
                                 const long long w0 = dc ? clock64() : 0;
-                                gwait(w_full0 + 8u * slot, use & 1u);
+                                mbar_wait_or_trap(w_full0 + 8u * slot, use & 1u);
                                 if (dc) wsum += clock64() - w0;
                                 loaded = true;
                             }
@@ -588,25 +545,25 @@ __global__ void __launch_bounds__(GN_THREADS, 1) gen_mlp_kernel(const __grid_con
                         if (leader) umma_commit(w_empty0 + 8u * slot);
                     }
                     // the epilogue of this GEMM overwrites the A buffer: the image stores must have read it
-                    if (store && leader) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
+                    if (store && leader) bulk_wait_read();
                     if (leader) umma_commit(gm.head ? bar_acc_h : bar_acc_e);
                     if (dc) { dc[2 + 3 * G] = clock64(); dc[3 + 3 * G] = wsum; }
                 }
                 if (P.fb) {            // delta_0 (the last epilogue's output) is only an image
                     const int nsl = P.width[0] >> 6;
                     for (int sl = 0; sl < nsl; ++sl) {
-                        gwait(bar_slab0 + 8u * (uint32_t)sl, (spar >> sl) & 1u);
+                        mbar_wait_or_trap(bar_slab0 + 8u * (uint32_t)sl, (spar >> sl) & 1u);
                         spar ^= 1u << sl;
                         if (leader) g_bulk_store(a.dlimg[0] + ((size_t)tile * nsl + sl) * GN_SLAB, sA + (uint32_t)sl * GN_SLAB, GN_SLAB);
                     }
                     if (leader) {
-                        asm volatile("cp.async.bulk.commit_group;" ::: "memory");
-                        asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
+                        bulk_commit();
+                        bulk_wait_read();
                         mbar_arrive(bar_free);
                     }
                 }
             }
-            if (leader) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
+            if (leader) bulk_wait();
         }
         __syncwarp();
     } else if (warp == 17) {
@@ -617,10 +574,10 @@ __global__ void __launch_bounds__(GN_THREADS, 1) gen_mlp_kernel(const __grid_con
                 for (int f = 0; f < P.n_fills; ++f, ++U) {
                     const GFill fl = P.fill[f];
                     const uint32_t slot = U % GN_NSLOT, use = U / GN_NSLOT;
-                    if (use > 0) gwait(w_empty0 + 8u * slot, (use - 1u) & 1u);
+                    if (use > 0) mbar_wait_or_trap(w_empty0 + 8u * slot, (use - 1u) & 1u);
                     const uint32_t bar = w_full0 + 8u * slot, bytes = (uint32_t)fl.bytes16 * 16u;
-                    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-                    g_bulk_load(sW + slot * GN_SLOT, a.img + fl.off, bytes, bar);
+                    mbar_expect_tx(bar, bytes);
+                    bulk_load_chunked<16384u>(sW + slot * GN_SLOT, a.img + fl.off, bytes, bar);
                 }
             }
         }
@@ -641,9 +598,9 @@ __global__ void __launch_bounds__(GN_THREADS, 1) gen_mlp_kernel(const __grid_con
             for (int G = 0; G < P.n_gemm; ++G) {
                 const GGemm gm = P.gemm[G];
                 if (gm.head) continue;
-                gwait(bar_acc_e, ne & 1u); ++ne;
+                mbar_wait_or_trap(bar_acc_e, ne & 1u); ++ne;
                 if (dc) dc[32 + 2 * G] = clock64();
-                asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+                tc_fence_after();
                 const uint32_t dcol = tlane + (uint32_t)(G & 1) * 256u + (uint32_t)(g * 16);
                 const int nsl = gm.N >> 6;
                 uint32_t r[2][16];
@@ -664,10 +621,10 @@ __global__ void __launch_bounds__(GN_THREADS, 1) gen_mlp_kernel(const __grid_con
                             for (int k = 0; k < 4; ++k) {
                                 const float s0 = 1.0f / (1.0f + expf(-__uint_as_float(rc[8 * c + 2 * k])));
                                 const float s1 = 1.0f / (1.0f + expf(-__uint_as_float(rc[8 * c + 2 * k + 1])));
-                                hi[k] = gpack(s0, s1);
+                                hi[k] = pack_f16(s0, s1);
                                 const float2 hf = __half22float2(*reinterpret_cast<__half2*>(&hi[k]));
-                                lo[k] = gpack(s0 - hf.x, s1 - hf.y);
-                                dg[4 * c + k] = gpack(s0 * (1.0f - s0), s1 * (1.0f - s1));
+                                lo[k] = pack_f16(s0 - hf.x, s1 - hf.y);
+                                dg[4 * c + k] = pack_f16(s0 * (1.0f - s0), s1 * (1.0f - s1));
                             }
                             const int sw = ((g * 2 + c) ^ (row & 7)) << 4;
                             *reinterpret_cast<uint4*>(a_row + s * GN_SLAB + sw) = make_uint4(hi[0], hi[1], hi[2], hi[3]);
@@ -689,7 +646,7 @@ __global__ void __launch_bounds__(GN_THREADS, 1) gen_mlp_kernel(const __grid_con
 #pragma unroll
                             for (int k = 0; k < 4; ++k) {
                                 const float2 df = __half22float2(*reinterpret_cast<const __half2*>(&dw[k]));
-                                o[k] = gpack(__uint_as_float(rc[8 * c + 2 * k]) * df.x, __uint_as_float(rc[8 * c + 2 * k + 1]) * df.y);
+                                o[k] = pack_f16(__uint_as_float(rc[8 * c + 2 * k]) * df.x, __uint_as_float(rc[8 * c + 2 * k + 1]) * df.y);
                             }
                             const int sw = ((g * 2 + c) ^ (row & 7)) << 4;
                             *reinterpret_cast<uint4*>(a_row + s * GN_SLAB + sw) = make_uint4(o[0], o[1], o[2], o[3]);
@@ -705,10 +662,10 @@ __global__ void __launch_bounds__(GN_THREADS, 1) gen_mlp_kernel(const __grid_con
 #pragma unroll
                             for (int k = 0; k < 4; ++k) {
                                 const uint32_t b0 = rc[8 * c + 2 * k], b1 = rc[8 * c + 2 * k + 1];
-                                asm("cvt.rn.relu.f16x2.f32 %0, %1, %2;" : "=r"(hi[k]) : "f"(__uint_as_float(b1)), "f"(__uint_as_float(b0)));
+                                hi[k] = relu_pack_f16(b0, b1);
                                 if (P.split) {
                                     const float2 hf = __half22float2(*reinterpret_cast<__half2*>(&hi[k]));
-                                    lo[k] = gpack(fmaxf(__uint_as_float(b0), 0.0f) - hf.x, fmaxf(__uint_as_float(b1), 0.0f) - hf.y);
+                                    lo[k] = pack_f16(fmaxf(__uint_as_float(b0), 0.0f) - hf.x, fmaxf(__uint_as_float(b1), 0.0f) - hf.y);
                                 }
                             }
                             const int sw = ((g * 2 + c) ^ (row & 7)) << 4;
@@ -726,14 +683,14 @@ __global__ void __launch_bounds__(GN_THREADS, 1) gen_mlp_kernel(const __grid_con
                                 const int i0 = 8 * c + 2 * k;
                                 const float x0 = (m >> (15 - i0)) & 1u ? __uint_as_float(rc[i0]) : 0.0f;
                                 const float x1 = (m >> (14 - i0)) & 1u ? __uint_as_float(rc[i0 + 1]) : 0.0f;
-                                o[k] = gpack(x0, x1);
+                                o[k] = pack_f16(x0, x1);
                             }
                             const int sw = ((g * 2 + c) ^ (row & 7)) << 4;
                             *reinterpret_cast<uint4*>(a_row + s * GN_SLAB + sw) = make_uint4(o[0], o[1], o[2], o[3]);
                         }
                     }
-                    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-                    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+                    fence_proxy_async_smem();
+                    tc_fence_before();
                     __syncwarp();
                     if (lane == 0) mbar_arrive(bar_slab0 + 8u * (uint32_t)s);
                 }
@@ -770,23 +727,23 @@ __global__ void __launch_bounds__(GN_THREADS, 1) gen_mlp_kernel(const __grid_con
             if (valid && !P.fb && a.action && !a.greedy) w3 = stream_keyed(a.keys, a.gid0 + (uint64_t)s, a.t, B2048_DOM_STEP).w3;
             // the A buffer is free: forward-only, the previous tile's head GEMM has completed (waited for below); update mode,
             // its last image has been read out
-            if (P.fb && lt > 0) gwait(bar_free, (lt - 1u) & 1u);
+            if (P.fb && lt > 0) mbar_wait_or_trap(bar_free, (lt - 1u) & 1u);
             if (dc) dc[61] = clock64();
             if (P.obs_mode == B2048_OBS_ONEHOT) {
                 zero_slabs_128(smem + GS_A, P.in_slabs, tid - 18 * 32);
-                asm volatile("bar.sync 1, 128;" ::: "memory");                     // the four I/O warps only
+                bar_sync(1, 128);                     // the four I/O warps only
             }
             encode_input_row(bd, row, smem + GS_A, 0, P.in_slabs, P.obs_mode, P.obs_scale);
-            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+            fence_proxy_async_smem();
             __syncwarp();
             if (lane == 0) mbar_arrive(bar_io);
             if (dc) dc[62] = clock64();
-            gwait(bar_acc_h, lt & 1u);
+            mbar_wait_or_trap(bar_acc_h, lt & 1u);
             if (dc) dc[63] = clock64();
-            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+            tc_fence_after();
             uint32_t r4[4];
             tmem_ld4(tlane + hcol, r4);
-            asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+            tc_fence_before();
             float lg[4];
 #pragma unroll
             for (int j = 0; j < 4; ++j) lg[j] = __uint_as_float(r4[j]) + b4[j];
@@ -846,9 +803,9 @@ __global__ void __launch_bounds__(GN_THREADS, 1) gen_mlp_kernel(const __grid_con
                 // completed, so the A buffer is free
                 uint8_t* a_row = smem + GS_A + row * 128;
                 const int sw = row & 7;
-                *reinterpret_cast<uint4*>(a_row + ((0 ^ sw) << 4)) = make_uint4(gpack(d[0] * S, d[1] * S), gpack(d[2] * S, d[3] * S), 0u, 0u);
+                *reinterpret_cast<uint4*>(a_row + ((0 ^ sw) << 4)) = make_uint4(pack_f16(d[0] * S, d[1] * S), pack_f16(d[2] * S, d[3] * S), 0u, 0u);
                 *reinterpret_cast<uint4*>(a_row + ((1 ^ sw) << 4)) = make_uint4(0u, 0u, 0u, 0u);
-                asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+                fence_proxy_async_smem();
                 __syncwarp();
                 if (lane == 0) mbar_arrive(bar_io);
                 // head bias gradient (unscaled float32 sum over the warp's 32 samples)
@@ -864,11 +821,7 @@ __global__ void __launch_bounds__(GN_THREADS, 1) gen_mlp_kernel(const __grid_con
         }
     }
 
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    __syncthreads();
-    if (warp == 16) {
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512u) : "memory");
-    }
+    tmem_teardown(warp == 16, tmem_base, 512u);
 }
 
 // ------------------------------------------------------------------------------------------------ dW GEMMs
@@ -904,22 +857,15 @@ __global__ void __launch_bounds__(GD_THREADS, 1) gen_dw_kernel(const __grid_cons
     if (tid == 0) {
         for (int i = 0; i < a.stages; ++i) { mbar_init(full0 + 8u * i, gen ? 5 : 1); mbar_init(empty0 + 8u * i, 1 + ncs); }
         mbar_init(bar_done, 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        mbar_init_fence();
     }
     // a missing second A slab (a 64- or 272-feature input) stays zero for the whole kernel
     for (int i = tid; i < a.stages * 2 * GN_SLAB / 16; i += GD_THREADS) {
         const int st = i / (2 * GN_SLAB / 16), o = i % (2 * GN_SLAB / 16);
         *reinterpret_cast<uint4*>(smem + st * stage_bytes + o * 16) = make_uint4(0u, 0u, 0u, 0u);
     }
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-    if (warp == 1) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(s_u32(tmem_slot)), "r"(a.tmem_cols) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    __syncthreads();
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    const uint32_t tmem_base = *tmem_slot;
+    fence_proxy_async_smem();
+    const uint32_t tmem_base = tmem_setup(warp == 1, tmem_slot, a.tmem_cols);
     const int64_t n_my = ks < a.n_tiles ? (a.n_tiles - ks + a.ksplit - 1) / a.ksplit : 0;
 
     if (warp == 0) {
@@ -927,23 +873,23 @@ __global__ void __launch_bounds__(GD_THREADS, 1) gen_dw_kernel(const __grid_cons
             for (int64_t it = 0; it < n_my; ++it) {
                 const int st = (int)(it % a.stages);
                 const int64_t use = it / a.stages, tile = ks + it * a.ksplit;
-                if (use > 0) gwait(empty0 + 8u * st, (uint32_t)(use - 1) & 1u);
+                if (use > 0) mbar_wait_or_trap(empty0 + 8u * st, (uint32_t)(use - 1) & 1u);
                 const uint32_t bar = full0 + 8u * st;
                 const uint32_t ab = gen ? 0u : (uint32_t)(a_have * GN_SLAB), bb = (uint32_t)(a.b_slabs * GN_SLAB);
-                asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(ab + bb) : "memory");
+                mbar_expect_tx(bar, ab + bb);
                 const uint32_t sa = s_u32(smem + st * stage_bytes);
-                if (!gen) g_bulk_load(sa, a.aimg + ((size_t)tile * a.a_slabs + 2 * mt) * GN_SLAB, ab, bar);
-                g_bulk_load(sa + 2u * GN_SLAB, a.bimg + (size_t)tile * a.b_slabs * GN_SLAB, bb, bar);
+                if (!gen) bulk_load_chunked<16384u>(sa, a.aimg + ((size_t)tile * a.a_slabs + 2 * mt) * GN_SLAB, ab, bar);
+                bulk_load_chunked<16384u>(sa + 2u * GN_SLAB, a.bimg + (size_t)tile * a.b_slabs * GN_SLAB, bb, bar);
             }
         }
         __syncwarp();
     } else if (warp == 1) {
         if (lane == 0) {
-            const uint32_t idesc = idesc_h(128, a.N) | kIdescAMn | kIdescBMn;
+            const uint32_t idesc = idesc_f16(128, a.N) | kIdescAMn | kIdescBMn;
             for (int64_t it = 0; it < n_my; ++it) {
                 const int st = (int)(it % a.stages);
-                gwait(full0 + 8u * st, (uint32_t)(it / a.stages) & 1u);
-                asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+                mbar_wait_or_trap(full0 + 8u * st, (uint32_t)(it / a.stages) & 1u);
+                tc_fence_after();
                 const uint32_t sa = s_u32(smem + st * stage_bytes), sb = sa + 2u * GN_SLAB;
 #pragma unroll
                 for (int kk = 0; kk < 8; ++kk)            // 16 samples per MMA; M = 128 features = two slabs, N = a.N
@@ -964,7 +910,7 @@ __global__ void __launch_bounds__(GD_THREADS, 1) gen_dw_kernel(const __grid_cons
             for (int e = 0; e < 8; ++e) acc[e] = 0.0f;
             for (int64_t it = 0; it < n_my; ++it) {
                 const int st = (int)(it % a.stages);
-                gwait(full0 + 8u * st, (uint32_t)(it / a.stages) & 1u);
+                mbar_wait_or_trap(full0 + 8u * st, (uint32_t)(it / a.stages) & 1u);
                 const uint8_t* x = smem + st * stage_bytes + 2 * GN_SLAB + cw * GN_SLAB;
 #pragma unroll 4
                 for (int r = rsub; r < 128; r += 4) {
@@ -990,8 +936,8 @@ __global__ void __launch_bounds__(GD_THREADS, 1) gen_dw_kernel(const __grid_cons
             }
         }
         if (n_my > 0) {
-            gwait(bar_done, 0);
-            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+            mbar_wait_or_trap(bar_done, 0);
+            tc_fence_after();
             const int q = warp & 3;
             const uint32_t tlane = tmem_base + ((uint32_t)(q * 32) << 16);
             const int m = mt * 128 + q * 32 + lane;                    // input feature
@@ -1004,9 +950,7 @@ __global__ void __launch_bounds__(GD_THREADS, 1) gen_dw_kernel(const __grid_cons
                     if (vec4 && c0 + 16 <= a.N_real) {          // four 128-bit reductions instead of 16 scalar atomics
 #pragma unroll
                         for (int i = 0; i < 16; i += 4)
-                            asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(dst + i), "f"(__uint_as_float(r[i]) * inv),
-                                         "f"(__uint_as_float(r[i + 1]) * inv), "f"(__uint_as_float(r[i + 2]) * inv), "f"(__uint_as_float(r[i + 3]) * inv)
-                                         : "memory");
+                            red_add_v4(dst + i, __uint_as_float(r[i]) * inv, __uint_as_float(r[i + 1]) * inv, __uint_as_float(r[i + 2]) * inv, __uint_as_float(r[i + 3]) * inv);
                     } else {
 #pragma unroll
                         for (int i = 0; i < 16; ++i) {
@@ -1025,22 +969,21 @@ __global__ void __launch_bounds__(GD_THREADS, 1) gen_dw_kernel(const __grid_cons
             const int64_t use = it / a.stages, tile = ks + it * a.ksplit;
             const int64_t s = tile * 128 + row;
             const uint64_t bd = s < a.n ? a.board[s] : 0ull;
-            if (use > 0) gwait(empty0 + 8u * st, (uint32_t)(use - 1) & 1u);
+            if (use > 0) mbar_wait_or_trap(empty0 + 8u * st, (uint32_t)(use - 1) & 1u);
             if (a.obs_mode == B2048_OBS_ONEHOT) {
                 zero_slabs_128(smem + st * stage_bytes, a_have, tid - 6 * 32);
-                asm volatile("bar.sync 2, 128;" ::: "memory");                     // the four generator warps only
+                bar_sync(2, 128);                     // the four generator warps only
             }
             encode_input_row(bd, row, smem + st * stage_bytes, 2 * mt, a_have, a.obs_mode, a.obs_scale);
-            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+            fence_proxy_async_smem();
             __syncwarp();
             if (lane == 0) mbar_arrive(full0 + 8u * st);
         }
     }
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    // written out: tmem_teardown() would load a.tmem_cols ahead of the branch and change the SASS
+    tc_fence_before();
     __syncthreads();
-    if (warp == 1) {
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(a.tmem_cols) : "memory");
-    }
+    if (warp == 1) tmem_dealloc(tmem_base, a.tmem_cols);
 }
 
 // ------------------------------------------------------------------------------------------------ loss scale

@@ -156,18 +156,15 @@ __device__ __forceinline__ void relu_store_tmem(uint32_t tlane_d2, int q, int g,
 #pragma unroll
     for (int s = 0; s < 4; ++s) {
         if (s + 1 < 4) tmem_ld16_issue(tlane_d2 + (uint32_t)((s + 1) * 64 + g * 16), r[(s + 1) & 1]);
-        asm volatile("bar.sync %0, 128;" ::"r"(2 + q) : "memory");              // every warp of the quarter holds slab s in registers
+        bar_sync(2 + q, 128);              // every warp of the quarter holds slab s in registers
         const uint32_t(&v)[16] = r[s & 1];
         uint32_t w[8];
 #pragma unroll
         for (int c = 0; c < 8; ++c) w[c] = relu_pack(v[2 * c], v[2 * c + 1]);
-        asm volatile("tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};" ::"r"(
-                         tlane_d2 + (uint32_t)(kDstCol + s * 32 + g * 8)),
-                     "r"(w[0]), "r"(w[1]), "r"(w[2]), "r"(w[3]), "r"(w[4]), "r"(w[5]), "r"(w[6]), "r"(w[7])
-                     : "memory");
-        asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
+        tmem_st8(tlane_d2 + (uint32_t)(kDstCol + s * 32 + g * 8), w);
+        tmem_st_wait();
         if (s + 1 < 4) tmem_ld_wait(r[(s + 1) & 1]);
-        asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");         // TMEM reads and writes ordered before the hand-off
+        tc_fence_before();         // TMEM reads and writes ordered before the hand-off
         __syncwarp();
         if (lane == 0) mbar_arrive(bar0 + 8u * s);
     }
@@ -204,17 +201,10 @@ __global__ void __launch_bounds__(kRollout ? TC_THREADS + TC_ENV_THREADS : TC_TH
         mbar_init(bar_free, TC_EPI_THREADS / 32 + TC_IO_THREADS / 32);
         for (int g = 0; g < 2; ++g) { mbar_init(bar_act0 + 8u * g, TC_IO_THREADS / 32); mbar_init(bar_step0 + 8u * g, TC_ENV_GROUP / 32); }
         for (int g = 0; g < 4; ++g) { mbar_init(bar_slab0 + 8u * g, TC_EPI_THREADS / 32); mbar_init(bar_hslab0 + 8u * g, TC_EPI_THREADS / 32); }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        mbar_init_fence();
     }
-    if (warp == 16) {   // all 512 TMEM columns: D1 = 0..255, D2 = 256..511, D3 = 256..287 (two partial sums) and H2 (packed bf16) = 288..415 (over D2)
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(s_u32(tmem_slot)), "r"(512u)
-                     : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    __syncthreads();
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    const uint32_t tmem_base = *tmem_slot;
+    // all 512 TMEM columns: D1 = 0..255, D2 = 256..511, D3 = 256..287 (two partial sums) and H2 (packed bf16) = 288..415 (over D2)
+    const uint32_t tmem_base = tmem_setup(warp == 16, tmem_slot, 512u);
     const int64_t n_slots = (kRollout && args.n_dev) ? (int64_t)*args.n_dev : args.n;   // uniform over the grid
     const int64_t n_tiles = (n_slots + TC_M - 1) / TC_M;
     const int64_t first = blockIdx.x;
@@ -239,22 +229,14 @@ __global__ void __launch_bounds__(kRollout ? TC_THREADS + TC_ENV_THREADS : TC_TH
         const uint32_t lBias = dlo_ns(s_u32(smem + IMG_BIAS));
         const uint32_t lOnes1 = dlo_ns(s_u32(smem + IMG_ONES1)), lOnes2 = dlo_ns(s_u32(smem + IMG_ONES2));
         if (leader) {
-            asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar_img), "r"((uint32_t)IMG_BYTES)
-                         : "memory");
-            constexpr uint32_t kChunk = 16384;
-            for (uint32_t off = 0; off < (uint32_t)IMG_BYTES; off += kChunk) {
-                uint32_t sz = (uint32_t)IMG_BYTES - off < kChunk ? (uint32_t)IMG_BYTES - off : kChunk;
-                asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-                                 s_u32(smem + off)),
-                             "l"(args.img + off), "r"(sz), "r"(bar_img)
-                             : "memory");
-            }
+            mbar_expect_tx(bar_img, (uint32_t)IMG_BYTES);
+            bulk_load_chunked<16384u>(s_u32(smem), args.img, (uint32_t)IMG_BYTES, bar_img);
         }
         __syncwarp();
         mbar_wait(bar_img, 0);
         auto issue_layer1 = [&](uint32_t ph) {   // D1 = A1 . W1^T + b1   (called by the whole warp)
             mbar_wait(bar_a1, ph);
-            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+            tc_fence_after();
             if (leader) {
                 umma_w(tmem_base, lA1, DH_NOSW, lW1, DH_NOSW, kIdesc, 0u);
                 umma_w(tmem_base, lOnes1, DH_ONES, lBias, DH_NOSW, kIdesc, 1u);
@@ -272,7 +254,7 @@ __global__ void __launch_bounds__(kRollout ? TC_THREADS + TC_ENV_THREADS : TC_TH
                 mbar_wait(bar_slab0 + 8u * g, ph);
                 if (g == 0 && item != 0) mbar_wait(bar_free, ph ^ 1u);       // D2/D3 drained by the previous tile
                 if (g == 0 && mdbg) args.debug_clock[64 + 4 * item] = clock64();
-                asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+                tc_fence_after();
                 const uint32_t a0 = tmem_base + g * 32u, b0 = lW2 + g * 2048u;
                 if (leader) {
                     umma_w_ts(tmem_base + 256u, a0, b0, DH_SW, kIdesc, g ? 1u : 0u);
@@ -300,7 +282,7 @@ __global__ void __launch_bounds__(kRollout ? TC_THREADS + TC_ENV_THREADS : TC_TH
                 try_layer1();
                 while (!mbar_test(bar_hslab0 + 8u * g, ph)) try_layer1();
                 if (mdbg && g == 3) args.debug_clock[64 + 4 * item + 1] = clock64();
-                asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+                tc_fence_after();
                 const uint32_t a0 = tmem_base + 256u + (uint32_t)TC_H2_COL + g * 32u, b0 = lW3 + g * 128u;
                 if (leader) {
                     umma_w_ts(tmem_base + 256u, a0, b0, DH_SW, kIdescHead, g ? 1u : 0u);
@@ -329,13 +311,13 @@ __global__ void __launch_bounds__(kRollout ? TC_THREADS + TC_ENV_THREADS : TC_TH
             //      operand of layer 2 in tensor memory
             mbar_wait(bar_d1, ph);
             if (dbg) dc[1] = clock64();
-            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+            tc_fence_after();
             relu_store_tmem<0>(tlane, q, g, lane, bar_slab0);
             if (dbg) dc[2] = clock64();
             // ---- epilogue 2: H2 = bf16(relu(D2)), slab by slab, packed back into tensor memory (relu_store_tmem)
             mbar_wait(bar_d2, ph);
             if (dbg) dc[3] = clock64();
-            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+            tc_fence_after();
             relu_store_tmem<TC_H2_COL>(tlane + 256u, q, g, lane, bar_hslab0);
             if (args.debug_clock != nullptr && blockIdx.x == 0 && item < 4 && lane == 0)    // the slowest warp's end of epilogue 2
                 atomicMax(reinterpret_cast<unsigned long long*>(args.debug_clock) + 80 + item, (unsigned long long)clock64());
@@ -403,7 +385,7 @@ __global__ void __launch_bounds__(kRollout ? TC_THREADS + TC_ENV_THREADS : TC_TH
                 uint8_t* a1 = smem + SM_A1 + (row >> 3) * 256 + (row & 7) * 16;
                 *reinterpret_cast<uint4*>(a1) = make_uint4(packed[0], packed[1], packed[2], packed[3]);
                 *reinterpret_cast<uint4*>(a1 + 128) = make_uint4(packed[4], packed[5], packed[6], packed[7]);
-                asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+                fence_proxy_async_smem();
                 __syncwarp();
                 if (lane == 0) mbar_arrive(bar_a1);
             };
@@ -437,12 +419,12 @@ __global__ void __launch_bounds__(kRollout ? TC_THREADS + TC_ENV_THREADS : TC_TH
                 if (dbg && item < 4) args.debug_clock[64 + 4 * item + 3] = clock64();
                 mbar_wait(bar_d3, ph);
                 if (dbg) args.debug_clock[8 * item + 5] = clock64();
-                asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+                tc_fence_after();
                 uint32_t r4[4], r4b[4];
                 tmem_ld4_issue(tlane + 256u, r4);
-                tmem_ld4(tlane + 256u + 16u, r4b);             // waits for both loads
-                asm volatile("" : "+r"(r4[0]), "+r"(r4[1]), "+r"(r4[2]), "+r"(r4[3]));
-                asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+                tmem_ld4_issue(tlane + 256u + 16u, r4b);
+                tmem_ld_wait(r4);                              // waits for both loads
+                tc_fence_before();
                 __syncwarp();
                 if (lane == 0) mbar_arrive(bar_free);
                 const float lg0 = (__uint_as_float(r4[0]) + __uint_as_float(r4b[0])) + sB3[0];
@@ -519,7 +501,7 @@ __global__ void __launch_bounds__(kRollout ? TC_THREADS + TC_ENV_THREADS : TC_TH
                 const uint4* src = reinterpret_cast<const uint4*>(args.tables + B2048_LUT_BYTES);
                 uint4* dst = reinterpret_cast<uint4*>(smem + SM_TBL);
                 for (int i = tid - TC_THREADS; i < B2048_SMALL_BYTES / 16; i += TC_ENV_THREADS) dst[i] = src[i];
-                asm volatile("bar.sync 1, %0;" ::"n"(TC_ENV_THREADS) : "memory");
+                bar_sync(1, TC_ENV_THREADS);
             }
             const int grp = (warp - 21) >> 2;
             const uint32_t bar_act = bar_act0 + 8u * grp, bar_step = bar_step0 + 8u * grp;
@@ -605,11 +587,7 @@ __global__ void __launch_bounds__(kRollout ? TC_THREADS + TC_ENV_THREADS : TC_TH
         }
     }
 
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    __syncthreads();
-    if (warp == 16) {
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512u) : "memory");
-    }
+    tmem_teardown(warp == 16, tmem_base, 512u);
 }
 
 // Builds the bf16 weight image of a 16 -> 256 -> 256 -> n_out (n_out <= 4) network into `img` (IMG_BYTES, device).

@@ -1,10 +1,12 @@
 // b2048_tc.cuh — shared pieces of the tcgen05 / TMEM kernels (policy forward: b2048_policy_tc.cu; training
-// forward + backward and the dW GEMMs: b2048_learn_tc.cu): the bf16 weight image layout, mbarrier / UMMA / TMEM PTX
-// wrappers and the shared-memory / instruction descriptors.
+// forward + backward and the dW GEMMs: b2048_learn_tc.cu, b2048_learn_hp.cu; the generic MLP: b2048_mlp_gen.cu): the bf16
+// weight image layout and the shared-memory / instruction descriptors.  The PTX wrappers are in b2048_ptx.cuh.
 #pragma once
 #include <cuda_bf16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
+
+#include "b2048_ptx.cuh"
 
 namespace b2 {
 
@@ -30,36 +32,7 @@ constexpr int SM_TOTAL2 = SM_BAR + 256;
 static_assert(IMG_W3 % 1024 == 0 && SM_A2 % 1024 == 0 && IMG_BYTES % 16 == 0, "operand alignment");
 static_assert(SM_TOTAL2 <= 232448, "exceeds the 227 KB shared memory of an sm_100 CTA");
 
-// ------------------------------------------------------------------------------------------------ PTX helpers
-__device__ __forceinline__ uint32_t s_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-
-__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count));
-}
-__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
-    uint32_t ok = 0;
-    while (!ok) {
-        asm volatile(
-            "{\n\t.reg .pred p;\n\t"
-            "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-            "selp.u32 %0, 1, 0, p;\n\t}"
-            : "=r"(ok)
-            : "r"(bar), "r"(parity)
-            : "memory");
-    }
-}
-// one non-blocking probe of a barrier phase
-__device__ __forceinline__ bool mbar_test(uint32_t bar, uint32_t parity) {
-    uint32_t ok;
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.test_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(ok)
-        : "r"(bar), "r"(parity)
-        : "memory");
-    return ok != 0u;
-}
+// ------------------------------------------------------------------------------------------------ descriptors
 // SWIZZLE_128B K-major operand: rows of 128 B, 8-row groups 1024 B apart (SBO), version 1 (sm_100)
 __device__ __forceinline__ uint64_t desc_sw128(uint32_t saddr) {
     return (uint64_t)((saddr & 0x3FFFFu) >> 4) | (1ull << 16) | ((uint64_t)(1024 >> 4) << 32) | (1ull << 46) | (2ull << 61);
@@ -74,125 +47,11 @@ __device__ __forceinline__ uint64_t desc_nosw_k16(uint32_t saddr) {
 __device__ __forceinline__ uint64_t desc_ones(uint32_t saddr) {
     return (uint64_t)((saddr & 0x3FFFFu) >> 4) | ((uint64_t)(128 >> 4) << 16) | (1ull << 46);
 }
-// kind::f16 instruction descriptor: D fp32, A/B bf16, both K-major, M = 128, N = 256
-constexpr uint32_t kIdesc = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(TC_H >> 3) << 17) | ((uint32_t)(TC_M >> 4) << 24);
-
-constexpr uint32_t kIdescHead = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(TC_N3 >> 3) << 17) | ((uint32_t)(TC_M >> 4) << 24);
-
-__device__ __forceinline__ void umma_f16(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc, uint32_t accumulate) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "setp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-        ::"r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate)
-        : "memory");
-}
-// the same with the A operand in tensor memory (lane = row, a 32-bit column = two consecutive K elements)
-__device__ __forceinline__ void umma_f16_ts(uint32_t d_tmem, uint32_t a_tmem, uint64_t b_desc, uint32_t idesc, uint32_t accumulate) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "setp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, p;\n\t}"
-        ::"r"(d_tmem), "r"(a_tmem), "l"(b_desc), "r"(idesc), "r"(accumulate)
-        : "memory");
-}
-// tcgen05.mma from the 32-bit halves of the two shared-memory descriptors (upper halves are compile-time constants), so that the
-// descriptor arithmetic of a convergent MMA warp stays in uniform registers (see fwd_role)
-__device__ __forceinline__ void umma_w(uint32_t d_tmem, uint32_t a_lo, uint32_t a_hi, uint32_t b_lo, uint32_t b_hi, uint32_t idesc, uint32_t accumulate) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t.reg .b64 da, db;\n\t"
-        "setp.ne.b32 p, %6, 0;\n\t"
-        "mov.b64 da, {%1, %2};\n\t"
-        "mov.b64 db, {%3, %4};\n\t"
-        "tcgen05.mma.cta_group::1.kind::f16 [%0], da, db, %5, p;\n\t}"
-        ::"r"(d_tmem), "r"(a_lo), "r"(a_hi), "r"(b_lo), "r"(b_hi), "r"(idesc), "r"(accumulate)
-        : "memory");
-}
 constexpr uint32_t DH_SW = 0x40004040u;     // upper word of desc_sw128: SBO 1024, version 1, 128-byte swizzle
 constexpr uint32_t DH_NOSW = 0x4010u;       // desc_nosw_k16: SBO 256, version 1
 constexpr uint32_t DH_ONES = 0x4000u;       // desc_ones: SBO 0, version 1
 __device__ __forceinline__ uint32_t dlo_sw(uint32_t saddr) { return (saddr >> 4) | (1u << 16); }
 __device__ __forceinline__ uint32_t dlo_ns(uint32_t saddr) { return (saddr >> 4) | (8u << 16); }
-
-// the same with the A operand in tensor memory
-__device__ __forceinline__ void umma_w_ts(uint32_t d_tmem, uint32_t a_tmem, uint32_t b_lo, uint32_t b_hi, uint32_t idesc, uint32_t accumulate) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t.reg .b64 db;\n\t"
-        "setp.ne.b32 p, %5, 0;\n\t"
-        "mov.b64 db, {%2, %3};\n\t"
-        "tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], db, %4, p;\n\t}"
-        ::"r"(d_tmem), "r"(a_tmem), "r"(b_lo), "r"(b_hi), "r"(idesc), "r"(accumulate)
-        : "memory");
-}
-
-__device__ __forceinline__ void umma_commit(uint32_t bar) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
-}
-__device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&r)[32]) {
-    asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
-        "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, "
-        "%16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31}, [%32];"
-        : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-          "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]), "=r"(r[16]),
-          "=r"(r[17]), "=r"(r[18]), "=r"(r[19]), "=r"(r[20]), "=r"(r[21]), "=r"(r[22]), "=r"(r[23]), "=r"(r[24]),
-          "=r"(r[25]), "=r"(r[26]), "=r"(r[27]), "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
-        : "r"(taddr));
-    asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-}
-
-__device__ __forceinline__ void tmem_ld4(uint32_t taddr, uint32_t (&r)[4]) {
-    asm volatile("tcgen05.ld.sync.aligned.32x32b.x4.b32 {%0, %1, %2, %3}, [%4];"
-                 : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3])
-                 : "r"(taddr));
-    asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-}
-
-__device__ __forceinline__ void tmem_ld4_issue(uint32_t taddr, uint32_t (&r)[4]) {   // completed by a later tcgen05.wait::ld
-    asm volatile("tcgen05.ld.sync.aligned.32x32b.x4.b32 {%0, %1, %2, %3}, [%4];"
-                 : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3])
-                 : "r"(taddr));
-}
-
-__device__ __forceinline__ void mbar_arrive(uint32_t bar) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
-}
-
-// bf16x2( relu(a), relu(b) ) in ONE instruction (F2FP with the .relu modifier; a in the low half): the epilogues are
-// issue-bound (16 warps on 4 schedulers), so every instruction per column pair counts
-__device__ __forceinline__ uint32_t relu_pack(uint32_t a_bits, uint32_t b_bits) {
-    uint32_t d;
-    asm("cvt.rn.relu.bf16x2.f32 %0, %1, %2;" : "=r"(d) : "f"(__uint_as_float(b_bits)), "f"(__uint_as_float(a_bits)));
-    return d;
-}
-
-__device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t (&r)[16]) {
-    asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x16.b32 "
-        "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
-        : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-          "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
-        : "r"(taddr));
-    asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-}
-
-
-// asynchronous halves of tmem_ld16: issue now, wait later (tcgen05.wait::ld covers every outstanding load of the thread)
-__device__ __forceinline__ void tmem_ld16_issue(uint32_t taddr, uint32_t (&r)[16]) {
-    asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x16.b32 "
-        "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
-        : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-          "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
-        : "r"(taddr));
-}
-// The destination registers of an issued load are valid only after the wait: the empty asm makes every later use of
-// them depend on a statement the compiler keeps behind the wait (asm volatile statements are not reordered).
-__device__ __forceinline__ void tmem_ld_wait(uint32_t (&r)[16]) {
-    asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-    asm volatile("" : "+r"(r[0]), "+r"(r[1]), "+r"(r[2]), "+r"(r[3]), "+r"(r[4]), "+r"(r[5]), "+r"(r[6]), "+r"(r[7]), "+r"(r[8]),
-                      "+r"(r[9]), "+r"(r[10]), "+r"(r[11]), "+r"(r[12]), "+r"(r[13]), "+r"(r[14]), "+r"(r[15]));
-}
 
 // MN-major SWIZZLE_128B operand (the contiguous dimension is M or N, not K): a [K rows][64 MN elements = 128 B] atom
 // of 8 K-rows (1024 B); the next 8 K-rows are SBO = 1024 B away, the next 64 MN elements LBO bytes away.
@@ -200,10 +59,17 @@ __device__ __forceinline__ uint64_t desc_sw128_mn(uint32_t saddr, uint32_t lbo_b
     return (uint64_t)((saddr & 0x3FFFFu) >> 4) | ((uint64_t)(lbo_bytes >> 4) << 16) | ((uint64_t)(1024 >> 4) << 32) |
            (1ull << 46) | (2ull << 61);
 }
-constexpr uint32_t kIdescAMn = 1u << 15;   // instruction-descriptor bit: A is MN-major
-constexpr uint32_t kIdescBMn = 1u << 16;   // instruction-descriptor bit: B is MN-major
-__host__ __device__ constexpr uint32_t idesc_f16(int m, int n) {
+
+// kind::f16 instruction descriptors: D fp32, A and B K-major (or with the MN-major bits below), M x N
+__host__ __device__ constexpr uint32_t idesc_bf16(int m, int n) {   // A/B bf16
     return (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(n >> 3) << 17) | ((uint32_t)(m >> 4) << 24);
 }
+__host__ __device__ constexpr uint32_t idesc_f16(int m, int n) {    // A/B fp16
+    return (1u << 4) | ((uint32_t)(n >> 3) << 17) | ((uint32_t)(m >> 4) << 24);
+}
+constexpr uint32_t kIdescAMn = 1u << 15;   // instruction-descriptor bit: A is MN-major
+constexpr uint32_t kIdescBMn = 1u << 16;   // instruction-descriptor bit: B is MN-major
+constexpr uint32_t kIdesc = idesc_bf16(TC_M, TC_H);
+constexpr uint32_t kIdescHead = idesc_bf16(TC_M, TC_N3);
 
 }  // namespace b2

@@ -35,6 +35,16 @@ def test_header_declares_the_expected_surface():
         assert s in syms
 
 
+
+def test_inline_ptx_only_in_the_wrapper_header():
+    # Each PTX operation, with its operand constraints and clobbers, is written once in b2048_ptx.cuh.  The exception is
+    # b2048_device.cuh: its prmt / mul.hi / lop3 intrinsics sit in a header that also compiles with g++ (host_check),
+    # and their C forms (__byte_perm, __umulhi, an and-or select) compile the step kernels to different SASS.
+    csrc = os.path.join(PKG, "csrc")
+    stmt = re.compile(r"asm\s*(volatile)?\s*\(")
+    with_asm = sorted(f for f in os.listdir(csrc) if stmt.search(open(os.path.join(csrc, f)).read()))
+    assert [f for f in with_asm if f not in ("b2048_ptx.cuh", "b2048_device.cuh")] == []
+
 def test_library_exports_every_declared_symbol(lib_path):
     lib = C.CDLL(lib_path)           # loads without a GPU (CUDA runtime is linked statically)
     for s in header_symbols():
