@@ -571,14 +571,7 @@ using namespace b2;
 
 extern "C" int b2048_create(b2048_handle** out) {
     B2_REQUIRE(out != nullptr, "b2048_create: out is NULL");
-    b2048_handle* h = new b2048_handle();
-    h->tc_image = nullptr;
-    h->hp_image = nullptr;
-    h->gen_image = nullptr;
-    h->gen_image_bytes = 0;
-    h->attrs = 0u;
-    h->debug = 0u;
-    h->pipe_split = 0u;
+    b2048_handle* h = new b2048_handle();   // value-initialised: no buffers yet, no attributes set, every debug option off
     B2_CUDA(cudaGetDevice(&h->device));
     B2_CUDA(cudaDeviceGetAttribute(&h->num_sms, cudaDevAttrMultiProcessorCount, h->device));
     B2_CUDA(cudaDeviceGetAttribute(&h->smem_optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, h->device));
@@ -620,6 +613,8 @@ extern "C" int b2048_destroy(b2048_handle* h) {
     if (h->tc_image) cudaFree(h->tc_image);
     if (h->hp_image) cudaFree(h->hp_image);
     if (h->gen_image) cudaFree(h->gen_image);
+    if (h->dbg_clock) cudaFree(h->dbg_clock);
+    if (h->dbg_progress) cudaFreeHost(h->dbg_progress);
     delete h;
     return B2048_OK;
 }
@@ -673,13 +668,8 @@ extern "C" int b2048_step_many(b2048_handle* h, const uint64_t* board_in, uint64
     a.merge_sum = merge_sum;
     a.reward = reward; a.reward64 = reward64; a.flags = flags; a.obs = obs; a.tables = h->d_tables;
     a.n = n; a.seed = seed; a.gid0 = gid0; a.t = t; a.cfg = *cfg; a.keys = make_keys(seed);
-    a.debug_clock = nullptr;
-    static long long* dbg_buf = nullptr;
-    if (h->debug & (1u << B2048_DBG_STEP_CLOCKS)) {
-        if (!dbg_buf) cudaMalloc(&dbg_buf, 32 * sizeof(long long));
-        a.debug_clock = dbg_buf;
-    }
     cudaStream_t s = (cudaStream_t)stream;
+    a.debug_clock = debug_clock_begin(h, B2048_DBG_STEP_CLOCKS, s);
     // Large batches: persistent CTAs with the tables in shared memory.  Small batches (the B=1
     // drop-in env, unit tests): tables read through L1/L2, no 192 KB staging per launch.
     const bool use_smem = h->smem_optin >= B2048_LUT_BYTES && n >= (int64_t)32768;
@@ -707,8 +697,7 @@ extern "C" int b2048_step_many(b2048_handle* h, const uint64_t* board_in, uint64
     B2_CUDA(cudaGetLastError());
     if (a.debug_clock && fast) {
         long long hb[32];
-        cudaStreamSynchronize(s);
-        cudaMemcpy(hb, a.debug_clock, sizeof(hb), cudaMemcpyDeviceToHost);
+        { int st = debug_clock_read(h, hb, 32, s); if (st != B2048_OK) return st; }
         for (int c = 0; c < 2; ++c) {
             long long* d = hb + 16 * c;
             fprintf(stderr, "[step clock] cta %d: start@%lld ns, staged +%lld cyc, iters:", c ? 147 : 0, d[0] - hb[0], d[2] - d[1]);

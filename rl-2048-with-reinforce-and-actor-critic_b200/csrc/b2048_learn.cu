@@ -19,25 +19,6 @@
 
 namespace b2 {
 
-int validate_mlp(const b2048_mlp_desc* d, MlpDev* out, size_t* smem_bytes, int smem_optin, const char* who);
-// b2048_learn_tc.cu
-bool backward_tc_supported(const b2048_handle* h, const b2048_mlp_desc* mlp);
-int64_t backward_tc_workspace_bytes(int64_t chunk);
-bool backward_hp_supported(const b2048_handle* h, const b2048_mlp_desc* mlp);
-int64_t backward_hp_workspace_bytes(int64_t chunk);
-int launch_backward_hp(b2048_handle* h, const uint64_t* board, const uint8_t* mask_flags, const uint8_t* action,
-                       const float* coef, const b2048_mlp_desc* mlp, float* grads, int64_t n, int head_mode,
-                       uint8_t* workspace, int64_t workspace_bytes, int64_t chunk, cudaStream_t stream);
-bool gen_shape_ok(const b2048_mlp_desc* mlp);
-bool gen_supported(const b2048_handle* h, const b2048_mlp_desc* mlp);
-int64_t gen_workspace_bytes(const b2048_mlp_desc* mlp, int64_t chunk);
-int launch_backward_gen(b2048_handle* h, const uint64_t* board, const uint8_t* mask_flags, const uint8_t* action, const float* coef,
-                        const b2048_mlp_desc* mlp, float* grads, int64_t n, int head_mode, uint8_t* workspace, int64_t chunk,
-                        cudaStream_t stream);
-int launch_backward_tc(b2048_handle* h, const uint64_t* board, const uint8_t* mask_flags, const uint8_t* action,
-                       const float* coef, const b2048_mlp_desc* mlp, float* grads, int64_t n, int head_mode,
-                       uint8_t* workspace, int64_t chunk, cudaStream_t stream);
-
 // ------------------------------------------------------------------------------------------------ K4
 // One thread per board, sequential in t (the recurrence is evaluated in float64 with separately
 // rounded multiply and add exactly like the reference's Python loop, then stored as float32).
@@ -501,7 +482,7 @@ extern "C" int64_t b2048_backward_workspace_floats(const b2048_mlp_desc* mlp, in
     for (int l = 1; l + 1 < mlp->n_layers; ++l) wt += (int64_t)mlp->dims[l] * mlp->dims[l + 1];
     int64_t floats = per * chunk + wt + 64;
     // the tensor-core paths carve their images out of the same workspace
-    if (mlp->n_layers == 3 && mlp->dims[0] == 16 && mlp->dims[1] == 256 && mlp->dims[2] == 256) {
+    if (is_16_256_256(mlp)) {
         const int64_t tc = (backward_tc_workspace_bytes(chunk) + 3) / 4, hp = (backward_hp_workspace_bytes(chunk) + 3) / 4;
         floats = floats > tc ? floats : tc;
         floats = floats > hp ? floats : hp;
@@ -576,13 +557,8 @@ extern "C" int b2048_mlp_backward(b2048_handle* h, const uint64_t* board, const 
         transpose_kernel<<<grd, blk, 0, s>>>(a.mlp.W[l], wt, dims[l], dims[l + 1]);
         a.WT[l] = wt;
     }
-    // flat gradient layout
-    float* gW[B2048_MAX_LAYERS];
-    float* gb[B2048_MAX_LAYERS];
-    {
-        float* g = grads;
-        for (int l = 0; l < L; ++l) { gW[l] = g; g += (int64_t)dims[l] * dims[l + 1]; gb[l] = g; g += dims[l + 1]; }
-    }
+    float *gW[B2048_MAX_LAYERS], *gb[B2048_MAX_LAYERS];
+    carve_grads(mlp, grads, gW, gb);
     B2_CUDA(cudaFuncSetAttribute(mlp_backward_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     for (int64_t c0 = 0; c0 < n; c0 += chunk) {
         const int64_t cn = (n - c0) < chunk ? (n - c0) : chunk;

@@ -33,8 +33,6 @@
 
 namespace b2 {
 
-int ensure_tc_image(b2048_handle* h);
-
 // ------------------------------------------------------------------------------------------------ split-weight image
 constexpr int HP_UNIT = 32768;                  // one streamed unit: a 64-wide K slab of W2 hi or lo, [256 rows x 128 B]
 constexpr int HP_RES = 8 * HP_UNIT;             // units in streaming order hi0, lo0, hi1, lo1, ...; then the resident part
@@ -1116,23 +1114,20 @@ static HpWorkspace hp_workspace(int64_t chunk) {
 bool backward_hp_supported(const b2048_handle* h, const b2048_mlp_desc* mlp) {
     // log2 observations only: fp16 holds them exactly and the hidden activations stay far below 65504; raw tile values
     // (up to 32768 per input) could overflow the fp16 activations
-    return mlp->n_layers == 3 && mlp->dims[0] == 16 && mlp->dims[1] == TC_H && mlp->dims[2] == TC_H && mlp->dims[3] >= 1 &&
-           mlp->dims[3] <= 4 && mlp->activation == B2048_ACTV_RELU && mlp->obs_mode == B2048_OBS_LOG2 &&
-           h->smem_optin >= PIPE_SMEM && h->smem_optin >= AtbCfg<256>::kSmem;
+    return fixed_tc_net(mlp) && mlp->obs_mode == B2048_OBS_LOG2 && h->smem_optin >= PIPE_SMEM && h->smem_optin >= AtbCfg<256>::kSmem;
 }
 
 int64_t backward_hp_workspace_bytes(int64_t chunk) { return hp_workspace(chunk).total + 1024; }
-int64_t forward_hp_workspace_bytes() { return (HP_BYTES + 1023) / 1024 * 1024 + 1024; }
 
 static int hp_attrs(b2048_handle* h) {
-    if (!(h->attrs & 16u)) {
+    if (!(h->attrs & ATTR_HP)) {
         cudaError_t e = cudaFuncSetAttribute(fwd_hp_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, FS_TOTAL);
         if (e != cudaSuccess) return check_cuda(e, "cudaFuncSetAttribute(fwd_hp_kernel)");
         e = cudaFuncSetAttribute(bwd_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, BW_TOTAL);
         if (e != cudaSuccess) return check_cuda(e, "cudaFuncSetAttribute(bwd_tc_kernel)");
         e = cudaFuncSetAttribute(update_pipe_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, PIPE_SMEM);
         if (e != cudaSuccess) return check_cuda(e, "cudaFuncSetAttribute(update_pipe_kernel)");
-        h->attrs |= 16u;
+        h->attrs |= ATTR_HP;
     }
     return B2048_OK;
 }
@@ -1152,23 +1147,16 @@ int launch_forward_hp(b2048_handle* h, const b2048_mlp_desc* mlp, const uint64_t
     { int st = hp_attrs(h); if (st != B2048_OK) return st; }
     { int st = ensure_hp_image(h); if (st != B2048_OK) return st; }
     hp_prepare_kernel<<<64, 256, 0, stream>>>(mlp->W[0], mlp->b[0], mlp->W[1], mlp->b[1], mlp->W[2], mlp->b[2], mlp->dims[3], h->hp_image);
-    FwdHpArgs f;
-    f.img = h->hp_image; f.board = board; f.out = out; f.h1 = nullptr; f.h2 = nullptr; f.m1 = nullptr; f.m2 = nullptr;
-    f.n = n; f.n_out = mlp->dims[3]; f.obs_mode = mlp->obs_mode; f.obs_scale = mlp->obs_log2_scale;
-    f.debug_clock = nullptr;
-    static long long* dbg_buf = nullptr;
-    if (h->debug & (1u << B2048_DBG_TC_CLOCKS)) {
-        if (!dbg_buf) cudaMalloc(&dbg_buf, 80 * sizeof(long long));
-        cudaMemsetAsync(dbg_buf, 0, 80 * sizeof(long long), stream);
-        f.debug_clock = dbg_buf;
-    }
+    FwdHpArgs f{};
+    f.img = h->hp_image; f.board = board; f.out = out; f.n = n; f.n_out = mlp->dims[3]; f.obs_mode = mlp->obs_mode; f.obs_scale = mlp->obs_log2_scale;
+    f.debug_clock = debug_clock_begin(h, B2048_DBG_TC_CLOCKS, stream);
     const int64_t tiles = (n + TC_M - 1) / TC_M;
     const int grid = (int)(tiles < h->num_sms ? tiles : h->num_sms);
     fwd_hp_kernel<<<grid, FH_THREADS, FS_TOTAL, stream>>>(f);
-    if (f.debug_clock) {
+    int st = check_cuda(cudaGetLastError(), "fwd_hp_kernel launch");
+    if (st == B2048_OK && f.debug_clock) {
         long long hb[80];
-        cudaStreamSynchronize(stream);
-        cudaMemcpy(hb, dbg_buf, sizeof(hb), cudaMemcpyDeviceToHost);
+        if ((st = debug_clock_read(h, hb, 80, stream)) != B2048_OK) return st;
         for (int k = 0; k < 5; ++k) {
             long long* d = hb + 6 * k;
             fprintf(stderr, "[fwd_hp clock] tile %d: wait_d1 %lld epi1 %lld wait_d2 %lld epi2 %lld | to next %lld || mma lane: period %lld, "
@@ -1177,7 +1165,37 @@ int launch_forward_hp(b2048_handle* h, const b2048_mlp_desc* mlp, const uint64_t
                     hb[42 + 4 * (k + 1)]);
         }
     }
-    return check_cuda(cudaGetLastError(), "fwd_hp_kernel launch");
+    return st;
+}
+
+int launch_loss_scale(const b2048_handle* h, const float* coef, int64_t n, float* scale, cudaStream_t stream) {
+    cudaError_t e = cudaMemsetAsync(scale, 0, 16, stream);
+    if (e != cudaSuccess) return check_cuda(e, "cudaMemsetAsync(scale)");
+    absmax_kernel<<<h->num_sms * 4, 256, 0, stream>>>(coef, n, reinterpret_cast<uint32_t*>(scale) + 2);
+    scale_from_max_kernel<<<1, 1, 0, stream>>>(scale);
+    return B2048_OK;
+}
+
+// The forward stage over `n` samples from `board`, and the backward stage of the same samples (which start at sample c0
+// of the caller's arrays), on the workspace `ws` laid out as `w`: shared by the pipelined and the chunked update.
+static FwdHpArgs fwd_hp_args(const b2048_mlp_desc* mlp, uint8_t* ws, const HpWorkspace& w, const uint64_t* board, int64_t n) {
+    FwdHpArgs f{};
+    f.img = ws + w.img; f.board = board; f.out = reinterpret_cast<float*>(ws + w.logits);
+    f.h1 = ws + w.h1; f.h2 = ws + w.h2;
+    f.m1 = reinterpret_cast<uint64_t*>(ws + w.m1); f.m2 = reinterpret_cast<uint64_t*>(ws + w.m2);
+    f.n = n; f.n_out = mlp->dims[3]; f.obs_mode = mlp->obs_mode; f.obs_scale = mlp->obs_log2_scale;
+    return f;
+}
+static BwdArgs bwd_args(const FwdHpArgs& f, uint8_t* ws, const HpWorkspace& w, const uint8_t* mask_flags, const uint8_t* action,
+                        const float* coef, int64_t c0, int head_mode, float* const* gW, float* const* gb) {
+    BwdArgs b{};
+    b.img = ws + w.bimg; b.logits = f.out; b.m1 = f.m1; b.m2 = f.m2; b.board = f.board;
+    b.mask_flags = mask_flags ? mask_flags + c0 : nullptr;
+    b.action = action ? action + c0 : nullptr;
+    b.coef = coef + c0; b.scale = reinterpret_cast<const float*>(ws + w.scale);
+    b.dl2 = ws + w.dl2; b.d3t = ws + w.d3t; b.gb3 = gb[2]; b.gW1 = gW[0]; b.gb1 = gb[0];
+    b.n = f.n; b.head_mode = head_mode; b.n_out = f.n_out; b.obs_mode = f.obs_mode; b.obs_scale = f.obs_scale;
+    return b;
 }
 
 // Same contract as the fp32 body of b2048_mlp_backward (grads accumulated, flat layout W_0, b_0, W_1, b_1, ...).
@@ -1193,11 +1211,8 @@ static int launch_backward_hp_piped(b2048_handle* h, const uint64_t* board, cons
     float* scale = reinterpret_cast<float*>(ws + w.scale);
     hp_prepare_kernel<<<64, 256, 0, stream>>>(mlp->W[0], mlp->b[0], mlp->W[1], mlp->b[1], mlp->W[2], mlp->b[2], n_out, ws + w.img);
     bwd_prepare_kernel<<<64, 256, 0, stream>>>(mlp->W[1], mlp->W[2], n_out, ws + w.bimg);
-    cudaError_t e = cudaMemsetAsync(scale, 0, 16, stream);
-    if (e != cudaSuccess) return check_cuda(e, "cudaMemsetAsync(scale)");
-    absmax_kernel<<<h->num_sms * 4, 256, 0, stream>>>(coef, n, reinterpret_cast<uint32_t*>(scale) + 2);
-    scale_from_max_kernel<<<1, 1, 0, stream>>>(scale);
-    e = cudaMemsetAsync(flags, 0, (size_t)n_tiles * 16, stream);
+    { int st = launch_loss_scale(h, coef, n, scale, stream); if (st != B2048_OK) return st; }
+    cudaError_t e = cudaMemsetAsync(flags, 0, (size_t)n_tiles * 16, stream);
     if (e != cudaSuccess) return check_cuda(e, "cudaMemsetAsync(flags)");
     e = cudaMemsetAsync(ws + w.d3t, 0, (size_t)R * 2 * SMALL_TILE_BYTES, stream);     // rows >= n_out of d3^T stay zero
     if (e != cudaSuccess) return check_cuda(e, "cudaMemsetAsync(d3t)");
@@ -1205,31 +1220,19 @@ static int launch_backward_hp_piped(b2048_handle* h, const uint64_t* board, cons
     a.px.f_done = flags; a.px.b_done = flags + n_tiles; a.px.c2_done = flags + 2 * n_tiles; a.px.c13_done = flags + 3 * n_tiles;
     a.px.R = R;
     a.px.progress = nullptr;
-    static int* prog_host = nullptr;
     if (h->debug & (1u << B2048_DBG_TC_CLOCKS)) {
-        if (!prog_host) cudaHostAlloc(&prog_host, 256 * 8 * sizeof(int), cudaHostAllocMapped);
-        for (int i = 0; i < 256 * 8; ++i) prog_host[i] = -1;
+        for (int i = 0; i < DBG_PROGRESS_WORDS; ++i) h->dbg_progress[i] = -1;
         int* dptr = nullptr;
-        cudaHostGetDevicePointer(&dptr, prog_host, 0);
+        e = cudaHostGetDevicePointer(reinterpret_cast<void**>(&dptr), h->dbg_progress, 0);
+        if (e != cudaSuccess) return check_cuda(e, "cudaHostGetDevicePointer(progress)");
         a.px.progress = dptr;
     }
-    a.f.img = ws + w.img; a.f.board = board; a.f.out = reinterpret_cast<float*>(ws + w.logits);
-    a.f.h1 = ws + w.h1; a.f.h2 = ws + w.h2;
-    a.f.m1 = reinterpret_cast<uint64_t*>(ws + w.m1); a.f.m2 = reinterpret_cast<uint64_t*>(ws + w.m2);
-    a.f.n = n; a.f.n_out = n_out; a.f.obs_mode = mlp->obs_mode; a.f.obs_scale = mlp->obs_log2_scale; a.f.debug_clock = nullptr;
-    a.b.img = ws + w.bimg; a.b.logits = a.f.out; a.b.m1 = a.f.m1; a.b.m2 = a.f.m2;
-    a.b.board = board; a.b.mask_flags = mask_flags; a.b.action = action; a.b.coef = coef; a.b.scale = scale;
-    a.b.dl2 = ws + w.dl2; a.b.d3t = ws + w.d3t;
-    a.b.n = n; a.b.head_mode = head_mode; a.b.n_out = n_out; a.b.obs_mode = mlp->obs_mode; a.b.obs_scale = mlp->obs_log2_scale;
-    a.b.debug_clock = nullptr;
-    float* gW1 = grads;
-    float* gb1 = gW1 + 16 * TC_H;
-    float* gW2 = gb1 + TC_H;
-    float* gb2 = gW2 + TC_H * TC_H;
-    float* gW3 = gb2 + TC_H;
-    a.b.gb3 = gW3 + TC_H * n_out; a.b.gW1 = gW1; a.b.gb1 = gb1;
+    float *gW[B2048_MAX_LAYERS], *gb[B2048_MAX_LAYERS];
+    carve_grads(mlp, grads, gW, gb);
+    a.f = fwd_hp_args(mlp, ws, w, board, n);
+    a.b = bwd_args(a.f, ws, w, mask_flags, action, coef, 0, head_mode, gW, gb);
     a.d.h1 = a.f.h1; a.d.h2 = a.f.h2; a.d.dl2 = a.b.dl2; a.d.d3t = a.b.d3t;
-    a.d.gW2 = gW2; a.d.gb2 = gb2; a.d.gW3 = gW3; a.d.inv_scale = scale + 1;
+    a.d.gW2 = gW[1]; a.d.gb2 = gb[1]; a.d.gW3 = gW[2]; a.d.inv_scale = scale + 1;
     a.d.n_tiles = n_tiles; a.d.n_out = n_out;
     // role split (148 SMs -> 78 / 40 / 16 / 14; swept again after the head of the forward role went from 48 to 32 MMAs): per tile the forward role needs ~12 K cycles, the backward role ~7.5 K, the dW2 role ~4.5 K, the dW3 role ~2.5 K (both bound by ~30 B/clk of L2 -> shared-memory bulk copies per SM)
     const int S = h->num_sms;
@@ -1250,7 +1253,7 @@ static int launch_backward_hp_piped(b2048_handle* h, const uint64_t* board, cons
             fprintf(stderr, "[update pipeline] stuck after 3 s; n_tiles %lld R %lld roles F %d B %d dW2 %d dW13 %d\n", (long long)n_tiles,
                     (long long)R, a.nF, a.nB, a.nC2, a.nC13);
             for (int b = 0; b < S; ++b) {
-                const int* q = prog_host + b * 8;
+                const int* q = h->dbg_progress + b * 8;
                 fprintf(stderr, "  cta %3d role %d: [1] %d [2] %d [3] %d [4] %d [5] %d done %d\n", b, q[0], q[1], q[2], q[3], q[4], q[5], q[7]);
             }
             fflush(stderr);
@@ -1260,7 +1263,7 @@ static int launch_backward_hp_piped(b2048_handle* h, const uint64_t* board, cons
         long long tot[4] = {0, 0, 0, 0}, wt[4] = {0, 0, 0, 0};
         int cnt[4] = {0, 0, 0, 0};
         for (int b = 0; b < S; ++b) {
-            const int* q = prog_host + b * 8;
+            const int* q = h->dbg_progress + b * 8;
             const int role = q[0] / 100 - 1;
             if (role < 0 || role > 3) continue;
             cnt[role]++; tot[role] += q[7]; wt[role] += q[6] > 0 ? q[6] : 0;
@@ -1278,12 +1281,6 @@ int launch_backward_hp(b2048_handle* h, const uint64_t* board, const uint8_t* ma
                        uint8_t* workspace, int64_t workspace_bytes, int64_t chunk, cudaStream_t stream) {
     { int st = hp_attrs(h); if (st != B2048_OK) return st; }
     const int n_out = mlp->dims[3];
-    float* gW1 = grads;
-    float* gb1 = gW1 + 16 * TC_H;
-    float* gW2 = gb1 + TC_H;
-    float* gb2 = gW2 + TC_H * TC_H;
-    float* gW3 = gb2 + TC_H;
-    float* gb3 = gW3 + TC_H * n_out;
     uint8_t* ws = reinterpret_cast<uint8_t*>(((uintptr_t)workspace + 1023) & ~(uintptr_t)1023);
     {   // large batches: the persistent pipeline with an L2-resident ring of tile slots
         const int64_t n_tiles = (n + TC_M - 1) / TC_M;
@@ -1299,51 +1296,31 @@ int launch_backward_hp(b2048_handle* h, const uint64_t* board, const uint8_t* ma
         }
     }
     const HpWorkspace w = hp_workspace(chunk);
-    uint8_t* img = ws + w.img;
-    uint8_t* bimg = ws + w.bimg;
     float* scale = reinterpret_cast<float*>(ws + w.scale);
-    hp_prepare_kernel<<<64, 256, 0, stream>>>(mlp->W[0], mlp->b[0], mlp->W[1], mlp->b[1], mlp->W[2], mlp->b[2], n_out, img);
-    bwd_prepare_kernel<<<64, 256, 0, stream>>>(mlp->W[1], mlp->W[2], n_out, bimg);
-    cudaError_t e = cudaMemsetAsync(scale, 0, 16, stream);
-    if (e != cudaSuccess) return check_cuda(e, "cudaMemsetAsync(scale)");
-    absmax_kernel<<<h->num_sms * 4, 256, 0, stream>>>(coef, n, reinterpret_cast<uint32_t*>(scale) + 2);
-    scale_from_max_kernel<<<1, 1, 0, stream>>>(scale);
+    hp_prepare_kernel<<<64, 256, 0, stream>>>(mlp->W[0], mlp->b[0], mlp->W[1], mlp->b[1], mlp->W[2], mlp->b[2], n_out, ws + w.img);
+    bwd_prepare_kernel<<<64, 256, 0, stream>>>(mlp->W[1], mlp->W[2], n_out, ws + w.bimg);
+    { int st = launch_loss_scale(h, coef, n, scale, stream); if (st != B2048_OK) return st; }
+    float *gW[B2048_MAX_LAYERS], *gb[B2048_MAX_LAYERS];
+    carve_grads(mlp, grads, gW, gb);
+    long long* dbg = debug_clock_begin(h, B2048_DBG_TC_CLOCKS, stream);     // clocks of the first chunk's bwd_tc_kernel
     for (int64_t c0 = 0; c0 < n; c0 += chunk) {
         const int64_t cn = (n - c0) < chunk ? (n - c0) : chunk;
         const int64_t tiles = (cn + TC_M - 1) / TC_M;
         const int grid = (int)(tiles < h->num_sms ? tiles : h->num_sms);
-        FwdHpArgs f;
-        f.img = img; f.board = board + c0; f.out = reinterpret_cast<float*>(ws + w.logits);
-        f.h1 = ws + w.h1; f.h2 = ws + w.h2;
-        f.m1 = reinterpret_cast<uint64_t*>(ws + w.m1); f.m2 = reinterpret_cast<uint64_t*>(ws + w.m2);
-        f.n = cn; f.n_out = n_out; f.obs_mode = mlp->obs_mode; f.obs_scale = mlp->obs_log2_scale; f.debug_clock = nullptr;
+        const FwdHpArgs f = fwd_hp_args(mlp, ws, w, board + c0, cn);
         fwd_hp_kernel<<<grid, FH_THREADS, FS_TOTAL, stream>>>(f);
         int st = check_cuda(cudaGetLastError(), "fwd_hp_kernel launch");
         if (st != B2048_OK) return st;
-        BwdArgs b;
-        b.img = bimg; b.logits = f.out; b.m1 = f.m1; b.m2 = f.m2;
-        b.mask_flags = mask_flags ? mask_flags + c0 : nullptr;
-        b.action = action ? action + c0 : nullptr;
-        b.coef = coef + c0; b.scale = scale;
-        b.board = board + c0;
-        b.dl2 = ws + w.dl2; b.d3t = ws + w.d3t; b.gb3 = gb3; b.gW1 = gW1; b.gb1 = gb1;
-        b.n = cn; b.head_mode = head_mode; b.n_out = n_out; b.obs_mode = mlp->obs_mode; b.obs_scale = mlp->obs_log2_scale;
-        b.debug_clock = nullptr;
-        static long long* dbg_buf = nullptr;
-        if ((h->debug & (1u << B2048_DBG_TC_CLOCKS)) && c0 == 0) {
-            if (!dbg_buf) cudaMalloc(&dbg_buf, 64 * sizeof(long long));
-            cudaMemsetAsync(dbg_buf, 0, 64 * sizeof(long long), stream);
-            b.debug_clock = dbg_buf;
-        }
-        e = cudaMemsetAsync(b.d3t, 0, (size_t)tiles * 2 * SMALL_TILE_BYTES, stream);
+        BwdArgs b = bwd_args(f, ws, w, mask_flags, action, coef, c0, head_mode, gW, gb);
+        if (c0 == 0) b.debug_clock = dbg;
+        cudaError_t e = cudaMemsetAsync(b.d3t, 0, (size_t)tiles * 2 * SMALL_TILE_BYTES, stream);
         if (e != cudaSuccess) return check_cuda(e, "cudaMemsetAsync(d3t)");
         bwd_tc_kernel<<<grid, BW_THREADS, BW_TOTAL, stream>>>(b);
         st = check_cuda(cudaGetLastError(), "bwd_tc_kernel launch");
         if (st != B2048_OK) return st;
         if (b.debug_clock) {
             long long hb[64];
-            cudaStreamSynchronize(stream);
-            cudaMemcpy(hb, dbg_buf, sizeof(hb), cudaMemcpyDeviceToHost);
+            if ((st = debug_clock_read(h, hb, 64, stream)) != B2048_OK) return st;
             for (int k = 0; k < 5; ++k) {
                 long long* d = hb + 8 * k;
                 fprintf(stderr, "[bwd_tc clock] tile %d: wait_d5 %lld wait_free %lld epi3 %lld wait_d4 %lld epi4 %lld | to next %lld\n", k,
@@ -1353,10 +1330,10 @@ int launch_backward_hp(b2048_handle* h, const uint64_t* board, const uint8_t* ma
         AtbArgs g;
         g.tiles64 = tiles * 2; g.f16 = 1; g.inv_scale = scale + 1;
         // dW2 = H1^T DL2, db2 = column sums of DL2
-        g.A = f.h1; g.B = b.dl2; g.C = gW2; g.ldm = TC_H; g.ldn = 1; g.n_valid = TC_H; g.colsum = gb2; g.colsum_of_b = 1;
+        g.A = f.h1; g.B = b.dl2; g.C = gW[1]; g.ldm = TC_H; g.ldn = 1; g.n_valid = TC_H; g.colsum = gb[1]; g.colsum_of_b = 1;
         if ((st = launch_atb<256>(h, g, stream)) != B2048_OK) return st;
         // dW3 = H2^T d3
-        g.A = f.h2; g.B = b.d3t; g.C = gW3; g.ldm = n_out; g.ldn = 1; g.n_valid = n_out; g.colsum = nullptr; g.colsum_of_b = 0;
+        g.A = f.h2; g.B = b.d3t; g.C = gW[2]; g.ldm = n_out; g.ldn = 1; g.n_valid = n_out; g.colsum = nullptr; g.colsum_of_b = 0;
         if ((st = launch_atb<16>(h, g, stream)) != B2048_OK) return st;
     }
     return B2048_OK;

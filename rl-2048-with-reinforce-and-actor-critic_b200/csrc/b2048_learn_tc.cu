@@ -40,9 +40,6 @@
 
 namespace b2 {
 
-void launch_tc_prepare(const b2048_mlp_desc* mlp, uint8_t* img, cudaStream_t stream);
-int ensure_tc_image(b2048_handle* h);
-
 // ------------------------------------------------------------------------------------------------ layouts
 constexpr int FB_D3A = SM_BAR + 256;      // head deltas of the tile in flight as a bf16 A operand [128 x 16], A1's layout
 constexpr int FB_TOTAL = FB_D3A + 4096;
@@ -553,7 +550,7 @@ __global__ void __launch_bounds__(ATB_THREADS, 1) atb_tc_kernel(const __grid_con
 
 template <int NB>
 int launch_atb(b2048_handle* h, const AtbArgs& a, cudaStream_t stream) {
-    constexpr unsigned kBit = NB == 256 ? 4u : 8u;
+    constexpr unsigned kBit = NB == 256 ? ATTR_ATB_256 : ATTR_ATB_16;
     if (!(h->attrs & kBit)) {
         cudaError_t e = cudaFuncSetAttribute(atb_tc_kernel<NB>, cudaFuncAttributeMaxDynamicSharedMemorySize, AtbCfg<NB>::kSmem);
         if (e != cudaSuccess) return check_cuda(e, "cudaFuncSetAttribute(atb_tc_kernel)");
@@ -568,10 +565,7 @@ template int launch_atb<256>(b2048_handle*, const AtbArgs&, cudaStream_t);
 template int launch_atb<16>(b2048_handle*, const AtbArgs&, cudaStream_t);
 
 bool backward_tc_supported(const b2048_handle* h, const b2048_mlp_desc* mlp) {
-    return mlp->n_layers == 3 && mlp->dims[0] == 16 && mlp->dims[1] == TC_H && mlp->dims[2] == TC_H && mlp->dims[3] >= 1 &&
-           mlp->dims[3] <= 4 && mlp->activation == B2048_ACTV_RELU &&
-           (mlp->obs_mode == B2048_OBS_RAW || mlp->obs_mode == B2048_OBS_LOG2) && h->smem_optin >= FB_TOTAL &&
-           h->smem_optin >= AtbCfg<256>::kSmem;
+    return fixed_tc_net(mlp) && h->smem_optin >= FB_TOTAL && h->smem_optin >= AtbCfg<256>::kSmem;
 }
 
 int64_t backward_tc_workspace_bytes(int64_t chunk) { return tc_workspace(chunk).total + 1024; }
@@ -581,21 +575,18 @@ int launch_backward_tc(b2048_handle* h, const uint64_t* board, const uint8_t* ma
                        const float* coef, const b2048_mlp_desc* mlp, float* grads, int64_t n, int head_mode,
                        uint8_t* workspace, int64_t chunk, cudaStream_t stream) {
     { int st = ensure_tc_image(h); if (st != B2048_OK) return st; }
-    if (!(h->attrs & 2u)) {
+    if (!(h->attrs & ATTR_FB_TC)) {
         cudaError_t e = cudaFuncSetAttribute(fb_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, FB_TOTAL);
         if (e != cudaSuccess) return check_cuda(e, "cudaFuncSetAttribute(fb_tc_kernel)");
-        h->attrs |= 2u;
+        h->attrs |= ATTR_FB_TC;
     }
     launch_tc_prepare(mlp, h->tc_image, stream);
     const int n_out = mlp->dims[3];
-    float* gW1 = grads;
-    float* gb1 = gW1 + 16 * TC_H;
-    float* gW2 = gb1 + TC_H;
-    float* gb2 = gW2 + TC_H * TC_H;
-    float* gW3 = gb2 + TC_H;
-    float* gb3 = gW3 + TC_H * n_out;
+    float *gW[B2048_MAX_LAYERS], *gb[B2048_MAX_LAYERS];
+    carve_grads(mlp, grads, gW, gb);
     uint8_t* ws = reinterpret_cast<uint8_t*>(((uintptr_t)workspace + 1023) & ~(uintptr_t)1023);
     const TcWorkspace w = tc_workspace(chunk);
+    long long* dbg = debug_clock_begin(h, B2048_DBG_TC_CLOCKS, stream);     // clocks of the first chunk's fb_tc_kernel
     for (int64_t c0 = 0; c0 < n; c0 += chunk) {
         const int64_t cn = (n - c0) < chunk ? (n - c0) : chunk;
         const int64_t tiles = (cn + TC_M - 1) / TC_M;
@@ -606,25 +597,19 @@ int launch_backward_tc(b2048_handle* h, const uint64_t* board, const uint8_t* ma
         a.action = action ? action + c0 : nullptr;
         a.coef = coef + c0;
         a.h1 = ws + w.h1; a.h2 = ws + w.h2; a.dl2 = ws + w.dl2; a.dl1 = ws + w.dl1; a.a1t = ws + w.a1t; a.d3t = ws + w.d3t;
-        a.gb3 = gb3;
+        a.gb3 = gb[2];
         a.n = cn;
         a.head_mode = head_mode; a.n_out = n_out; a.obs_mode = mlp->obs_mode; a.obs_scale = mlp->obs_log2_scale;
         cudaError_t e = cudaMemsetAsync(a.d3t, 0, (size_t)tiles * 2 * SMALL_TILE_BYTES, stream);
         if (e != cudaSuccess) return check_cuda(e, "cudaMemsetAsync(d3t)");
         int grid = (int)(tiles < h->num_sms ? tiles : h->num_sms);
-        a.debug_clock = nullptr;
-        if (h->debug & (1u << B2048_DBG_TC_CLOCKS)) {
-            static long long* dbg_buf = nullptr;
-            if (!dbg_buf) cudaMalloc(&dbg_buf, 80 * sizeof(long long));
-            a.debug_clock = dbg_buf;
-        }
+        a.debug_clock = dbg;
         fb_tc_kernel<<<grid, FB_THREADS, FB_TOTAL, stream>>>(a);
         int st = check_cuda(cudaGetLastError(), "fb_tc_kernel launch");
         if (st != B2048_OK) return st;
-        if (a.debug_clock && c0 == 0) {
+        if (dbg && c0 == 0) {
             long long hb[80];
-            cudaStreamSynchronize(stream);
-            cudaMemcpy(hb, a.debug_clock, sizeof(hb), cudaMemcpyDeviceToHost);
+            if ((st = debug_clock_read(h, hb, 80, stream)) != B2048_OK) return st;
             for (int k = 0; k < 5; ++k) {
                 long long* d = hb + 10 * k;
                 fprintf(stderr, "[fb clock] tile %d: wait_d1 %lld epi1 %lld wait_d2 %lld epi2 %lld wait_d3 %lld epi3 %lld wait_d4 %lld epi4 %lld | to next %lld\n",
@@ -635,13 +620,13 @@ int launch_backward_tc(b2048_handle* h, const uint64_t* board, const uint8_t* ma
         AtbArgs g;
         g.tiles64 = tiles * 2; g.f16 = 0; g.inv_scale = nullptr;
         // dW2 = H1^T DL2, db2 = column sums of DL2
-        g.A = a.h1; g.B = a.dl2; g.C = gW2; g.ldm = TC_H; g.ldn = 1; g.n_valid = TC_H; g.colsum = gb2; g.colsum_of_b = 1;
+        g.A = a.h1; g.B = a.dl2; g.C = gW[1]; g.ldm = TC_H; g.ldn = 1; g.n_valid = TC_H; g.colsum = gb[1]; g.colsum_of_b = 1;
         if ((st = launch_atb<256>(h, g, stream)) != B2048_OK) return st;
         // dW3 = H2^T d3
-        g.A = a.h2; g.B = a.d3t; g.C = gW3; g.ldm = n_out; g.ldn = 1; g.n_valid = n_out; g.colsum = nullptr; g.colsum_of_b = 0;
+        g.A = a.h2; g.B = a.d3t; g.C = gW[2]; g.ldm = n_out; g.ldn = 1; g.n_valid = n_out; g.colsum = nullptr; g.colsum_of_b = 0;
         if ((st = launch_atb<16>(h, g, stream)) != B2048_OK) return st;
         // dW1^T = DL1^T A1, db1 = column sums of DL1
-        g.A = a.dl1; g.B = a.a1t; g.C = gW1; g.ldm = 1; g.ldn = TC_H; g.n_valid = 16; g.colsum = gb1; g.colsum_of_b = 0;
+        g.A = a.dl1; g.B = a.a1t; g.C = gW[0]; g.ldm = 1; g.ldn = TC_H; g.n_valid = 16; g.colsum = gb[0]; g.colsum_of_b = 0;
         if ((st = launch_atb<16>(h, g, stream)) != B2048_OK) return st;
     }
     return B2048_OK;

@@ -986,25 +986,6 @@ __global__ void __launch_bounds__(GD_THREADS, 1) gen_dw_kernel(const __grid_cons
     if (warp == 1) tmem_dealloc(tmem_base, a.tmem_cols);
 }
 
-// ------------------------------------------------------------------------------------------------ loss scale
-// S = the power of two that brings max |coef| into [32, 64) (as b2048_learn_hp.cu): scale[0] = S, scale[1] = 1 / S, [2] = bits of max
-__global__ void __launch_bounds__(256) gen_absmax_kernel(const float* __restrict__ x, int64_t n, uint32_t* __restrict__ out_bits) {
-    float m = 0.0f;
-    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) m = fmaxf(m, fabsf(x[i]));
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) m = fmaxf(m, __shfl_xor_sync(0xFFFFFFFFu, m, o));
-    if ((threadIdx.x & 31) == 0 && m > 0.0f && isfinite(m)) atomicMax(out_bits, __float_as_uint(m));
-}
-__global__ void gen_scale_kernel(float* __restrict__ scale) {
-    const float m = __uint_as_float(reinterpret_cast<uint32_t*>(scale)[2]);
-    int e = 0;
-    if (m > 0.0f) frexpf(m, &e);
-    int sh = 6 - e;
-    sh = sh > 100 ? 100 : (sh < -100 ? -100 : sh);
-    scale[0] = ldexpf(1.0f, sh);
-    scale[1] = ldexpf(1.0f, -sh);
-}
-
 // ------------------------------------------------------------------------------------------------ host side
 // Shapes: 1..4 hidden layers whose sizes are multiples of 64 up to 256, ReLU or Sigmoid, log2 (16-wide) or one-hot (272-wide)
 // input, 1..4 outputs.  (Raw observations reach 32768 per input and could leave the fp16 range in the activations.)
@@ -1052,7 +1033,7 @@ static GenWorkspace gen_workspace(const b2048_mlp_desc* mlp, int64_t chunk, int 
 int64_t gen_workspace_bytes(const b2048_mlp_desc* mlp, int64_t chunk) { return gen_workspace(mlp, chunk, 256).total + 2048; }
 
 static int gen_attrs(b2048_handle* h) {
-    if (!(h->attrs & 32u)) {
+    if (!(h->attrs & ATTR_GEN)) {
         cudaError_t e = cudaSuccess;
         auto set = [&](const void* f) { if (e == cudaSuccess) e = cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, GS_TOTAL); };
         set((const void*)gen_mlp_kernel<B2048_ACTV_RELU, false, 0, false, false>);
@@ -1065,7 +1046,7 @@ static int gen_attrs(b2048_handle* h) {
         if (e != cudaSuccess) return check_cuda(e, "cudaFuncSetAttribute(gen_mlp_kernel)");
         e = cudaFuncSetAttribute(gen_dw_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
         if (e != cudaSuccess) return check_cuda(e, "cudaFuncSetAttribute(gen_dw_kernel)");
-        h->attrs |= 32u;
+        h->attrs |= ATTR_GEN;
     }
     return B2048_OK;
 }
@@ -1090,18 +1071,10 @@ static int ensure_gen_image(b2048_handle* h, size_t bytes) {
     return B2048_OK;
 }
 
-static long long* g_dbg_buf = nullptr;
-static void gen_dbg_begin(b2048_handle* h, GenArgs& a, cudaStream_t stream) {
-    if (!(h->debug & (1u << B2048_DBG_TC_CLOCKS))) return;
-    if (!g_dbg_buf) cudaMalloc(&g_dbg_buf, 256 * sizeof(long long));
-    cudaMemsetAsync(g_dbg_buf, 0, 256 * sizeof(long long), stream);
-    a.dbg = g_dbg_buf;
-}
-static void gen_dbg_end(const GenArgs& a, cudaStream_t stream) {
-    if (!a.dbg) return;
+static int gen_dbg_print(const b2048_handle* h, const GenArgs& a, cudaStream_t stream) {
+    if (!a.dbg) return B2048_OK;
     long long hb[256];
-    cudaStreamSynchronize(stream);
-    cudaMemcpy(hb, g_dbg_buf, sizeof(hb), cudaMemcpyDeviceToHost);
+    { int st = debug_clock_read(h, hb, 256, stream); if (st != B2048_OK) return st; }
     for (int lt = 0; lt < 4; ++lt) {
         const long long* d = hb + 64 * lt;
         const long long t0 = d[0];
@@ -1113,6 +1086,7 @@ static void gen_dbg_end(const GenArgs& a, cudaStream_t stream) {
                     G, a.p.gemm[G].bwd ? "bwd" : "fwd", a.p.gemm[G].layer, a.p.gemm[G].N, a.p.gemm[G].nf, d[1 + 3 * G] - t0, d[2 + 3 * G] - t0,
                     d[3 + 3 * G], a.p.gemm[G].head ? 0 : d[32 + 2 * G] - t0, a.p.gemm[G].head ? 0 : d[33 + 2 * G] - t0);
     }
+    return B2048_OK;
 }
 
 static void gen_launch(const GenArgs& a, int grid, cudaStream_t stream) {
@@ -1164,10 +1138,10 @@ int launch_forward_gen(b2048_handle* h, const b2048_mlp_desc* mlp, const uint64_
     a.slot_map = slot_map; a.n_dev = slot_map ? n_dev : nullptr;
     const int64_t tiles = (n + TC_M - 1) / TC_M;
     const int grid = (int)(tiles < h->num_sms ? tiles : h->num_sms);
-    gen_dbg_begin(h, a, stream);
+    a.dbg = debug_clock_begin(h, B2048_DBG_TC_CLOCKS, stream);
     gen_launch(a, grid, stream);
-    gen_dbg_end(a, stream);
-    return check_cuda(cudaGetLastError(), "gen_mlp_kernel launch");
+    const int st = check_cuda(cudaGetLastError(), "gen_mlp_kernel launch");
+    return st != B2048_OK ? st : gen_dbg_print(h, a, stream);
 }
 
 // Same contract as the fp32 body of b2048_mlp_backward (grads accumulated; flat layout W_0, b_0, W_1, b_1, ...).
@@ -1182,16 +1156,9 @@ int launch_backward_gen(b2048_handle* h, const uint64_t* board, const uint8_t* m
     build_program(mlp, true, true, p);
     { int st = gen_prepare(mlp, p, ws + w.img, stream); if (st != B2048_OK) return st; }
     float* scale = reinterpret_cast<float*>(ws + w.scale);
-    cudaError_t e = cudaMemsetAsync(scale, 0, 16, stream);
-    if (e != cudaSuccess) return check_cuda(e, "cudaMemsetAsync(scale)");
-    gen_absmax_kernel<<<h->num_sms * 4, 256, 0, stream>>>(coef, n, reinterpret_cast<uint32_t*>(scale) + 2);
-    gen_scale_kernel<<<1, 1, 0, stream>>>(scale);
-    float* gW[GN_MAXL];
-    float* gb[GN_MAXL];
-    {
-        float* g = grads;
-        for (int l = 0; l < L; ++l) { gW[l] = g; g += (int64_t)mlp->dims[l] * mlp->dims[l + 1]; gb[l] = g; g += mlp->dims[l + 1]; }
-    }
+    { int st = launch_loss_scale(h, coef, n, scale, stream); if (st != B2048_OK) return st; }
+    float *gW[B2048_MAX_LAYERS], *gb[B2048_MAX_LAYERS];
+    carve_grads(mlp, grads, gW, gb);
     for (int64_t c0 = 0; c0 < n; c0 += chunk) {
         const int64_t cn = (n - c0) < chunk ? (n - c0) : chunk;
         const int64_t tiles = (cn + TC_M - 1) / TC_M;
@@ -1207,11 +1174,10 @@ int launch_backward_gen(b2048_handle* h, const uint64_t* board, const uint8_t* m
         a.gb_head = gb[L - 1];
         if (mlp->activation == B2048_ACTV_SIGMOID) a.dsig_scratch = reinterpret_cast<uint4*>(ws + w.masks);
         else a.mask_scratch = reinterpret_cast<uint16_t*>(ws + w.masks);
-        if (c0 == 0) gen_dbg_begin(h, a, stream);
+        if (c0 == 0) a.dbg = debug_clock_begin(h, B2048_DBG_TC_CLOCKS, stream);
         gen_launch(a, grid, stream);
-        gen_dbg_end(a, stream);
         int st = check_cuda(cudaGetLastError(), "gen_mlp_kernel launch");
-        if (st != B2048_OK) return st;
+        if (st != B2048_OK || (st = gen_dbg_print(h, a, stream)) != B2048_OK) return st;
         for (int l = 0; l < L; ++l) {
             GenDwArgs d;
             memset(&d, 0, sizeof(d));

@@ -145,23 +145,6 @@ __global__ void __launch_bounds__(kMlpThreads, 1) dense_forward_kernel(const __g
     }
 }
 
-int launch_policy_tc(b2048_handle* h, const b2048_mlp_desc* mlp, const uint64_t* board, const uint8_t* mask_flags,
-                     uint8_t* action, float* probs, float* logits, int64_t n, uint64_t seed, uint64_t gid0, uint32_t t,
-                     int greedy, cudaStream_t stream, bool rebuild_image);
-int launch_forward_hp(b2048_handle* h, const b2048_mlp_desc* mlp, const uint64_t* board, float* out, int64_t n, cudaStream_t stream);
-int launch_forward_gen(b2048_handle* h, const b2048_mlp_desc* mlp, const uint64_t* board, const uint8_t* mask_flags, float* out,
-                       uint8_t* action, float* probs, float* logits, int64_t n, uint64_t seed, uint64_t gid0, uint32_t t, int greedy,
-                       int split, bool rebuild_image, cudaStream_t stream, const int32_t* slot_map = nullptr,
-                       const int32_t* n_dev = nullptr);
-bool gen_supported(const b2048_handle* h, const b2048_mlp_desc* mlp);
-int launch_forward_tc(b2048_handle* h, const b2048_mlp_desc* mlp, const uint64_t* board, float* out, int64_t n,
-                      cudaStream_t stream);
-int launch_rollout_tc(b2048_handle* h, const b2048_mlp_desc* mlp, uint64_t* boards, uint8_t* flags, uint8_t* actions,
-                      float* rewards, uint32_t* score, uint32_t* step, uint8_t* max_exp, int32_t* ep_len,
-                      const b2048_env_cfg* cfg, int64_t B, int32_t t_begin, int32_t n_steps, uint64_t seed, uint64_t gid0,
-                      uint32_t t0, int use_mask, int greedy, const int32_t* slot_map, int64_t n_slots, const int32_t* n_slots_dev,
-                      cudaStream_t stream);
-
 int validate_mlp(const b2048_mlp_desc* d, MlpDev* out, size_t* smem_bytes, int smem_optin, const char* who) {
     if (!d) return fail(B2048_ERR_INVALID, std::string(who) + ": mlp descriptor is NULL");
     if (d->n_layers < 1 || d->n_layers > B2048_MAX_LAYERS)

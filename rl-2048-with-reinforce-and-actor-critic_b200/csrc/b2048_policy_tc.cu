@@ -591,41 +591,33 @@ __global__ void __launch_bounds__(kRollout ? TC_THREADS + TC_ENV_THREADS : TC_TH
 }
 
 // Builds the bf16 weight image of a 16 -> 256 -> 256 -> n_out (n_out <= 4) network into `img` (IMG_BYTES, device).
-// Shared with the training kernels (b2048_learn_tc.cu).
 void launch_tc_prepare(const b2048_mlp_desc* mlp, uint8_t* img, cudaStream_t stream) {
     policy_tc_prepare_kernel<<<64, 256, 0, stream>>>(mlp->W[0], mlp->b[0], mlp->W[1], mlp->b[1], mlp->W[2], mlp->b[2],
                                                       mlp->dims[3], img);
 }
 
-// Allocates the handle's weight-image buffer (shared by the policy, rollout and training kernels; also used by
-// b2048_learn_tc.cu) and opts the kernels of this file into their dynamic shared memory sizes.
+// Allocates the handle's weight-image buffer (shared by the policy, rollout and training kernels) and opts the kernels of
+// this file into their dynamic shared memory sizes.
 int ensure_tc_image(b2048_handle* h) {
     if (!h->tc_image) {
         cudaError_t e = cudaMalloc(&h->tc_image, IMG_BYTES);
         if (e != cudaSuccess) return check_cuda(e, "cudaMalloc(tc_image)");
     }
-    if (!(h->attrs & 1u)) {
+    if (!(h->attrs & ATTR_POLICY_TC)) {
         cudaError_t e = cudaFuncSetAttribute(policy_tc_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SM_TOTAL2);
         if (e != cudaSuccess) return check_cuda(e, "cudaFuncSetAttribute(policy_tc_kernel)");
         e = cudaFuncSetAttribute(policy_tc_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SM_TOTAL_RO);
         if (e != cudaSuccess) return check_cuda(e, "cudaFuncSetAttribute(policy_tc_kernel<rollout>)");
         e = cudaFuncSetAttribute(policy_tc_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SM_TOTAL_RO);
         if (e != cudaSuccess) return check_cuda(e, "cudaFuncSetAttribute(policy_tc_kernel<rollout, shaped>)");
-        h->attrs |= 1u;
+        h->attrs |= ATTR_POLICY_TC;
     }
     return B2048_OK;
 }
 
-static long long* debug_clock_buffer(const b2048_handle* h) {
-    static long long* dbg_buf = nullptr;
-    if (!(h->debug & (1u << B2048_DBG_TC_CLOCKS))) return nullptr;
-    if (!dbg_buf) { cudaMalloc(&dbg_buf, 96 * sizeof(long long)); cudaMemset(dbg_buf, 0, 96 * sizeof(long long)); }
-    return dbg_buf;
-}
-static void print_debug_clock(long long* dbg, cudaStream_t stream) {
+static int print_debug_clock(const b2048_handle* h, cudaStream_t stream) {
     long long hbuf[96];
-    cudaStreamSynchronize(stream);
-    cudaMemcpy(hbuf, dbg, sizeof(hbuf), cudaMemcpyDeviceToHost);
+    { int st = debug_clock_read(h, hbuf, 96, stream); if (st != B2048_OK) return st; }
     for (int k = 0; k < 6; ++k)
         fprintf(stderr,
                 "[tc clock] item %d: wait_d1+d3 %lld epi1 %lld wait_d2 %lld epi2 %lld | total %lld | to next %lld | io: d3 seen +%lld, "
@@ -638,75 +630,54 @@ static void print_debug_clock(long long* dbg, cudaStream_t stream) {
                 k, hbuf[64 + 4 * k] - hbuf[8 * k], hbuf[64 + 4 * k + 1] - hbuf[8 * k], hbuf[64 + 4 * k + 2] - hbuf[8 * k],
                 hbuf[64 + 4 * k + 3] - hbuf[8 * k]);
     for (int k = 0; k < 4; ++k) fprintf(stderr, "[tc clock] item %d: slowest epilogue warp leaves epilogue 2 at +%lld\n", k, hbuf[80 + k] - hbuf[8 * k]);
-    cudaMemset(dbg + 80, 0, 16 * sizeof(long long));
+    return B2048_OK;
 }
 
-// Returns B2048_OK if the tensor-core path applies and was launched, B2048_ERR_UNSUPPORTED (without setting an
-// error message) when the shape is outside what this kernel implements.
 int launch_policy_tc(b2048_handle* h, const b2048_mlp_desc* mlp, const uint64_t* board, const uint8_t* mask_flags,
                      uint8_t* action, float* probs, float* logits, int64_t n, uint64_t seed, uint64_t gid0, uint32_t t,
                      int greedy, cudaStream_t stream, bool rebuild_image) {
-    if (mlp->n_layers != 3 || mlp->dims[0] != 16 || mlp->dims[1] != TC_H || mlp->dims[2] != TC_H || mlp->dims[3] != 4 ||
-        mlp->activation != B2048_ACTV_RELU || (mlp->obs_mode != B2048_OBS_RAW && mlp->obs_mode != B2048_OBS_LOG2) ||
-        h->smem_optin < SM_TOTAL2)
-        return B2048_ERR_UNSUPPORTED;
+    if (!fixed_tc_net(mlp) || mlp->dims[3] != 4 || h->smem_optin < SM_TOTAL2) return B2048_ERR_UNSUPPORTED;
     { int st = ensure_tc_image(h); if (st != B2048_OK) return st; }
     // The image is rebuilt on every stand-alone call (71 K parameters): the library never caches weights across
     // calls.  b2048_rollout_many builds it once for the whole loop (parameters cannot change inside one call).
-    if (rebuild_image)
-        policy_tc_prepare_kernel<<<64, 256, 0, stream>>>(mlp->W[0], mlp->b[0], mlp->W[1], mlp->b[1], mlp->W[2], mlp->b[2], 4,
-                                                          h->tc_image);
-    PolicyTcArgs a;
+    if (rebuild_image) launch_tc_prepare(mlp, h->tc_image, stream);
+    PolicyTcArgs a{};
     a.img = h->tc_image; a.board = board; a.mask_flags = mask_flags; a.action = action; a.probs = probs; a.logits = logits;
-    a.head_out = nullptr; a.n_out = 4;
-    a.n = n; a.keys = make_keys(seed); a.gid0 = gid0; a.t = t; a.greedy = greedy; a.obs_mode = mlp->obs_mode;
-    a.obs_scale = mlp->obs_log2_scale;
-    a.debug_clock = nullptr;
-    a.ro_boards = nullptr; a.ro_flags = nullptr; a.ro_actions = nullptr; a.ro_rewards = nullptr; a.score = nullptr;
-    a.step = nullptr; a.max_exp = nullptr; a.ep_len = nullptr; a.tables = nullptr; a.seed = seed; a.t_begin = 0; a.n_steps = 1;
-    a.t0 = 0; a.slot_map = nullptr; a.n_dev = nullptr; a.ro_stride = n;
-    a.debug_clock = debug_clock_buffer(h);
+    a.n_out = 4; a.n = n; a.keys = make_keys(seed); a.gid0 = gid0; a.t = t; a.greedy = greedy; a.obs_mode = mlp->obs_mode;
+    a.obs_scale = mlp->obs_log2_scale; a.seed = seed; a.n_steps = 1; a.ro_stride = n;
+    a.debug_clock = debug_clock_begin(h, B2048_DBG_TC_CLOCKS, stream);
     int64_t tiles = (n + TC_M - 1) / TC_M;
     int grid = (int)(tiles < h->num_sms ? tiles : h->num_sms);
     policy_tc_kernel<false><<<grid, TC_THREADS, SM_TOTAL2, stream>>>(a);
-    if (a.debug_clock) print_debug_clock(a.debug_clock, stream);
-    return check_cuda(cudaGetLastError(), "policy_tc_kernel launch");
+    int st = check_cuda(cudaGetLastError(), "policy_tc_kernel launch");
+    if (st == B2048_OK && a.debug_clock) st = print_debug_clock(h, stream);
+    return st;
 }
 
 // b2048_mlp_forward on the tensor cores: out[n][n_out] = head outputs of a 16-256-256-n_out (n_out <= 4) ReLU network
-// (the critic's V(s) for the TD targets, reinforce_agent.py:425-437).  B2048_ERR_UNSUPPORTED (silent) for other shapes.
+// (the critic's V(s) for the TD targets, reinforce_agent.py:425-437).
 int launch_forward_tc(b2048_handle* h, const b2048_mlp_desc* mlp, const uint64_t* board, float* out, int64_t n,
                       cudaStream_t stream) {
-    if (mlp->n_layers != 3 || mlp->dims[0] != 16 || mlp->dims[1] != TC_H || mlp->dims[2] != TC_H || mlp->dims[3] < 1 ||
-        mlp->dims[3] > 4 || mlp->activation != B2048_ACTV_RELU ||
-        (mlp->obs_mode != B2048_OBS_RAW && mlp->obs_mode != B2048_OBS_LOG2) || h->smem_optin < SM_TOTAL2 || n < 4096)
-        return B2048_ERR_UNSUPPORTED;
+    if (!fixed_tc_net(mlp) || h->smem_optin < SM_TOTAL2 || n < 4096) return B2048_ERR_UNSUPPORTED;
     { int st = ensure_tc_image(h); if (st != B2048_OK) return st; }
     launch_tc_prepare(mlp, h->tc_image, stream);
-    PolicyTcArgs a;
-    a.img = h->tc_image; a.board = board; a.mask_flags = nullptr; a.action = nullptr; a.probs = nullptr; a.logits = nullptr;
-    a.head_out = out; a.n_out = mlp->dims[3]; a.n = n; a.keys = make_keys(0); a.gid0 = 0; a.t = 0; a.greedy = 1;
-    a.obs_mode = mlp->obs_mode; a.obs_scale = mlp->obs_log2_scale; a.debug_clock = nullptr;
-    a.ro_boards = nullptr; a.ro_flags = nullptr; a.ro_actions = nullptr; a.ro_rewards = nullptr; a.score = nullptr;
-    a.step = nullptr; a.max_exp = nullptr; a.ep_len = nullptr; a.tables = nullptr; a.seed = 0; a.t_begin = 0; a.n_steps = 1;
-    a.t0 = 0; a.slot_map = nullptr; a.n_dev = nullptr; a.ro_stride = n;
+    PolicyTcArgs a{};
+    a.img = h->tc_image; a.board = board; a.head_out = out; a.n_out = mlp->dims[3]; a.n = n; a.keys = make_keys(0); a.greedy = 1;
+    a.obs_mode = mlp->obs_mode; a.obs_scale = mlp->obs_log2_scale; a.n_steps = 1; a.ro_stride = n;
     int64_t tiles = (n + TC_M - 1) / TC_M;
     int grid = (int)(tiles < h->num_sms ? tiles : h->num_sms);
     policy_tc_kernel<false><<<grid, TC_THREADS, SM_TOTAL2, stream>>>(a);
     return check_cuda(cudaGetLastError(), "policy_tc_kernel (forward) launch");
 }
 
-// The whole rollout loop of b2048_rollout_many in one launch (policy_tc_kernel<true>).  Returns
-// B2048_ERR_UNSUPPORTED (no error message) when the network / env configuration is outside what the fused kernel
-// implements; the caller then runs the two-kernels-per-step loop.
+// The whole rollout loop of b2048_rollout_many in one launch (policy_tc_kernel<true>).  When the network / env
+// configuration is outside what the fused kernel implements, the caller runs the two-kernels-per-step loop.
 int launch_rollout_tc(b2048_handle* h, const b2048_mlp_desc* mlp, uint64_t* boards, uint8_t* flags, uint8_t* actions,
                       float* rewards, uint32_t* score, uint32_t* step, uint8_t* max_exp, int32_t* ep_len,
                       const b2048_env_cfg* cfg, int64_t B, int32_t t_begin, int32_t n_steps, uint64_t seed, uint64_t gid0,
                       uint32_t t0, int use_mask, int greedy, const int32_t* slot_map, int64_t n_slots, const int32_t* n_slots_dev,
                       cudaStream_t stream) {
-    const bool net_ok = mlp->n_layers == 3 && mlp->dims[0] == 16 && mlp->dims[1] == TC_H && mlp->dims[2] == TC_H &&
-                        mlp->dims[3] == 4 && mlp->activation == B2048_ACTV_RELU &&
-                        (mlp->obs_mode == B2048_OBS_RAW || mlp->obs_mode == B2048_OBS_LOG2) && h->smem_optin >= SM_TOTAL_RO;
+    const bool net_ok = fixed_tc_net(mlp) && mlp->dims[3] == 4 && h->smem_optin >= SM_TOTAL_RO;
     // every action-mask-on reward configuration (step_fast_rnd carries the shaping terms; the counters are always tracked here)
     const bool env_ok = score && step && max_exp && cfg->use_action_mask &&
                         (cfg->reward_mode == B2048_REWARD_SUM || cfg->reward_mode == B2048_REWARD_LOG2);
@@ -718,20 +689,20 @@ int launch_rollout_tc(b2048_handle* h, const b2048_mlp_desc* mlp, uint64_t* boar
     if (n == 0) return B2048_OK;
     { int st = ensure_tc_image(h); if (st != B2048_OK) return st; }
     launch_tc_prepare(mlp, h->tc_image, stream);
-    PolicyTcArgs a;
-    a.img = h->tc_image; a.board = nullptr; a.mask_flags = use_mask ? flags : nullptr; a.action = nullptr; a.probs = nullptr;
-    a.logits = nullptr; a.head_out = nullptr; a.n_out = 4; a.n = n; a.keys = make_keys(seed); a.gid0 = gid0; a.t = 0; a.greedy = greedy;
-    a.obs_mode = mlp->obs_mode; a.obs_scale = mlp->obs_log2_scale; a.debug_clock = nullptr;
+    PolicyTcArgs a{};
+    a.img = h->tc_image; a.mask_flags = use_mask ? flags : nullptr; a.n_out = 4; a.n = n; a.keys = make_keys(seed); a.gid0 = gid0;
+    a.greedy = greedy; a.obs_mode = mlp->obs_mode; a.obs_scale = mlp->obs_log2_scale;
     a.ro_boards = boards; a.ro_flags = flags; a.ro_actions = actions; a.ro_rewards = rewards; a.score = score; a.step = step;
     a.max_exp = max_exp; a.ep_len = ep_len; a.tables = h->d_tables; a.seed = seed; a.t_begin = t_begin; a.n_steps = n_steps;
     a.t0 = t0; a.cfg = *cfg; a.cfg.action_mode = B2048_ACT_BUFFER; a.slot_map = slot_map; a.n_dev = slot_map ? n_slots_dev : nullptr;
     a.ro_stride = B;
     int grid = (int)(tiles < h->num_sms ? tiles : h->num_sms);
-    a.debug_clock = debug_clock_buffer(h);
+    a.debug_clock = debug_clock_begin(h, B2048_DBG_TC_CLOCKS, stream);
     if (cfg_is_shaped(*cfg)) policy_tc_kernel<true, true><<<grid, TC_THREADS + TC_ENV_THREADS, SM_TOTAL_RO, stream>>>(a);
     else policy_tc_kernel<true, false><<<grid, TC_THREADS + TC_ENV_THREADS, SM_TOTAL_RO, stream>>>(a);
-    if (a.debug_clock) print_debug_clock(a.debug_clock, stream);
-    return check_cuda(cudaGetLastError(), "policy_tc_kernel<rollout> launch");
+    int st = check_cuda(cudaGetLastError(), "policy_tc_kernel<rollout> launch");
+    if (st == B2048_OK && a.debug_clock) st = print_debug_clock(h, stream);
+    return st;
 }
 
 }  // namespace b2

@@ -45,6 +45,16 @@ def test_inline_ptx_only_in_the_wrapper_header():
     with_asm = sorted(f for f in os.listdir(csrc) if stmt.search(open(os.path.join(csrc, f)).read()))
     assert [f for f in with_asm if f not in ("b2048_ptx.cuh", "b2048_device.cuh")] == []
 
+
+def test_no_static_pointer_caches():
+    # Buffers belong to a handle (b2048_handle in b2048_internal.h), which lives on one device and frees them in
+    # b2048_destroy.  A function-level or file-level `static T* p` would be shared by every handle of the process.
+    csrc = os.path.join(PKG, "csrc")
+    decl = re.compile(r"^\s*static\s+(?:const\s+)?[\w:<>]+(?:\s+[\w:<>]+)*\s*\*+\s*\w+\s*(?:=[^=;]*)?;", re.M)
+    found = [(f, m.group(0).strip()) for f in sorted(os.listdir(csrc)) if f.endswith(".cu")
+             for m in decl.finditer(open(os.path.join(csrc, f)).read())]
+    assert found == []
+
 def test_library_exports_every_declared_symbol(lib_path):
     lib = C.CDLL(lib_path)           # loads without a GPU (CUDA runtime is linked statically)
     for s in header_symbols():
