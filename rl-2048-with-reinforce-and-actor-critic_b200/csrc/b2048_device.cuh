@@ -187,6 +187,17 @@ B2_HD uint32_t blk_transpose(uint32_t x, uint32_t s) {  // s in {0,12}
 B2_HD uint32_t nib_swap(uint32_t x, uint32_t s) {  // s in {0,4}
     return bitsel(0xF0F0F0F0u, x << s, x >> s);
 }
+// The same two transforms without a data-dependent shift, for the ALU-bound fast step: the shifts become IMADs on
+// the FMA pipe and the choice between transform and identity moves into per-action masks / multipliers.
+//   blk_transpose_m(x, tm) == blk_transpose(x, s) for tm = 0x0F0F0000 (s = 12) or 0 (s = 0)
+//   nib_swap_m(x, nl, nr)  == nib_swap(x, s)      for (nl, nr) = (16, 1) (s = 4) or (1, 16) (s = 0);
+// with s = 0, (x * 16) >> 4 drops only the top nibble, which the 0x0F0F0F0F half of the select does not keep.
+B2_HD uint32_t blk_transpose_m(uint32_t x, uint32_t tm) {
+    return bitsel(tm, x * 4096u, bitsel(shr_fma<12>(tm), shr_fma<12>(x), x));
+}
+B2_HD uint32_t nib_swap_m(uint32_t x, uint32_t nl, uint32_t nr) {
+    return bitsel(0xF0F0F0F0u, x * nl, shr_fma<4>(x * nr));
+}
 
 B2_HD Board canon_fwd(Board b, const Xform& x) {
     uint32_t lo = nib_swap(blk_transpose(b.lo, x.st), x.sm);

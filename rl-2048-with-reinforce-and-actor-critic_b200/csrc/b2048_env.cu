@@ -309,7 +309,7 @@ __global__ void __launch_bounds__(1024, 1) step_fast_kernel(const __grid_constan
             io.action = act_next; io.mask_in = fin_next;
             const uint32_t inext = i + stride;
             if (inext < n) request(inext);
-            step_fast_rnd<kAct, kTrack, false>(io, cfg, rnd, args.seed, args.gid0 + (uint64_t)i, args.t, T);   // kPlain: unshaped rewards
+            step_fast_rnd<kAct, kTrack, false>(io, cfg, rnd, args.keys, args.gid0 + (uint64_t)i, args.t, T);   // kPlain: unshaped rewards
             *reinterpret_cast<uint2*>(args.board_out + i) = make_uint2(io.lo, io.hi);
             if (kTrack) { args.score[i] = io.score; args.step[i] = io.step; args.max_exp[i] = (uint8_t)io.max_exp; }
             args.reward[i] = io.reward;

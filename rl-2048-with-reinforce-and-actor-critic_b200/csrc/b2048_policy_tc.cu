@@ -562,7 +562,7 @@ __global__ void __launch_bounds__(kRollout ? TC_THREADS + TC_ENV_THREADS : TC_TH
                         args.ro_flags[o] = (uint8_t)io.flags;
                     } else {
                         io.action = sAct[grp * TC_M + row];
-                        step_fast_rnd<B2048_ACT_BUFFER, true, kShaped>(io, args.cfg, rr, args.seed, args.gid0 + (uint64_t)b, t_env, T);
+                        step_fast_rnd<B2048_ACT_BUFFER, true, kShaped>(io, args.cfg, rr, args.keys, args.gid0 + (uint64_t)b, t_env, T);
                         if (args.ep_len && (io.flags & (B2048_F_DONE | B2048_F_TRUNC))) {
                             args.ep_len[b] = (int32_t)(slice + 1);
                             cur.ep = (int32_t)(slice + 1);

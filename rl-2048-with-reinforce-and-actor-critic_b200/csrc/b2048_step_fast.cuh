@@ -10,7 +10,10 @@
 //     each row's merge byte and are combined with two adds and two ors;
 //   * the spawn cell is found with one multiply-prefix-sum per half and a byte-lane compare, and the
 //     isolated bit (G & -G) is turned into the tile with one multiply (no find-first-set, no shifts);
-//   * the non-zero masks of the moved board are reused for the legal-move test of the new board.
+//   * the non-zero masks of the moved board are reused for the legal-move test of the new board;
+//   * the canonicalisation has no data-dependent shift (blk_transpose_m / nib_swap_m: IMADs and per-action masks);
+//   * auto-reset looks the two-tile start board and its legal mask up by the cells and values its Philox words pick
+//     (start_board) instead of running the generic reset_board + legal_mask.
 // Host+device like the other step headers.
 #pragma once
 #include "b2048_step.cuh"
@@ -20,7 +23,7 @@ namespace b2 {
 // ---- small tables appended to the row tables (built once by build_small_tables) -----------------
 struct SelEntry {            // per action (0 up, 1 right, 2 down, 3 left)
     uint32_t f_lo, f_hi, i_lo, i_hi;   // PRMT selectors forward / inverse
-    uint32_t st, sm, pad0, pad1;       // in-block transpose shift (0|12), nibble swap shift (0|4)
+    uint32_t tm, nl, nr, pad;          // blk_transpose_m mask, nib_swap_m multipliers (b2048_device.cuh)
 };
 struct AggEntry {            // per merge byte (two 4-bit merged exponents; 0 none, 1 = exponent 16)
     uint32_t agg;            // bits 0-19 sum of merged tiles, 20-27 sum of exponents, 28-31 count
@@ -44,13 +47,74 @@ B2_HD void small_table_entry_agg(uint32_t byte, AggEntry& e) {
 B2_HD void small_table_entry_sel(uint32_t a, SelEntry& s) {
     Xform x = xform_for(a);
     s.f_lo = x.f_lo & 0xFFFFu; s.f_hi = x.f_hi & 0xFFFFu; s.i_lo = x.i_lo & 0xFFFFu; s.i_hi = x.i_hi & 0xFFFFu;
-    s.st = x.st; s.sm = x.sm; s.pad0 = 0; s.pad1 = 0;
+    s.tm = x.st ? 0x0F0F0000u : 0u;
+    s.nl = x.sm ? 16u : 1u;
+    s.nr = x.sm ? 1u : 16u;
+    s.pad = 0;
 }
 // T_act[mask * 4 + j] = j-th legal action of the 4-bit mask (0 when j is out of range)
 B2_HD uint32_t small_table_entry_act(uint32_t mask, uint32_t j) {
     uint32_t m = mask;
     for (uint32_t q = 0; q < j; ++q) m &= m - 1;
     return m ? (uint32_t)ffs0(m) : 0u;
+}
+
+// ---- auto-reset by table lookup --------------------------------------------------------------------
+// reset_board(seed, gid, t) spawns on the empty board from the words w of stream(seed, gid, t, B2048_DOM_RESET): the
+// first tile goes to cell c1 = mulhi(w0, 16), the second to the k2-th (k2 = mulhi(w2, 15)) of the 15 cells left, that
+// is cell c2 = k2 + (k2 >= c1); a tile is 4 (exponent 2) when its value word is >= 0xE6666667, else 2.  start_board
+// looks the board and its legal mask up by (c1, k2, v1, v2) instead of two place_kth_empty and a legal_mask.  The
+// tables sit in constant memory: only the lanes that reset read them, so the step kernels stage nothing more into
+// shared memory for them.
+struct StartTables {               // index (c1 * 16 + k2) * 4 + 2 * (v1 - 1) + (v2 - 1)
+    Board board[1024];
+    uint8_t mask[1024];
+};
+// legal mask of a board given cell by cell (exponent per cell, row-major): bit a set iff some tile has an empty or
+// equal neighbour in direction a (0 up, 1 right, 2 down, 3 left).  Plain loops, so it can build the tables at compile time.
+constexpr uint32_t cells_legal_mask(const uint8_t (&e)[16]) {
+    const int dr[4] = {-1, 0, 1, 0}, dc[4] = {0, 1, 0, -1};
+    uint32_t m = 0;
+    for (int c = 0; c < 16; ++c)
+        for (int a = 0; a < 4; ++a) {
+            const int r2 = c / 4 + dr[a], c2 = c % 4 + dc[a];
+            if (e[c] && r2 >= 0 && r2 < 4 && c2 >= 0 && c2 < 4 && (e[4 * r2 + c2] == 0 || e[4 * r2 + c2] == e[c])) m |= 1u << a;
+        }
+    return m;
+}
+constexpr StartTables make_start_tables() {
+    StartTables s{};
+    for (uint32_t c1 = 0; c1 < 16; ++c1)
+        for (uint32_t k2 = 0; k2 < 16; ++k2) {
+            const uint32_t c2 = (k2 + (k2 >= c1 ? 1u : 0u)) & 15u;   // k2 = 15 never occurs (mulhi(w2, 15) < 15)
+            for (uint32_t v = 0; v < 4; ++v) {
+                uint8_t e[16] = {};
+                e[c2] = (uint8_t)(1 + (v & 1));
+                e[c1] = (uint8_t)(1 + (v >> 1));
+                uint64_t b = 0;
+                for (int c = 0; c < 16; ++c) b |= (uint64_t)e[c] << (4 * c);
+                s.board[(c1 * 16 + k2) * 4 + v] = Board{(uint32_t)b, (uint32_t)(b >> 32)};
+                s.mask[(c1 * 16 + k2) * 4 + v] = (uint8_t)cells_legal_mask(e);
+            }
+        }
+    return s;
+}
+#if defined(__CUDACC__)
+static __constant__ StartTables g_start_tables_dev = make_start_tables();
+#endif
+static constexpr StartTables g_start_tables_host = make_start_tables();
+
+// reset_board from the Philox words of (gid, t, B2048_DOM_RESET); also returns the board's legal mask
+B2_HD Board start_board(const Rand4& w, uint32_t& mask) {
+#if defined(__CUDA_ARCH__)
+    const StartTables& S = g_start_tables_dev;
+#else
+    const StartTables& S = g_start_tables_host;
+#endif
+    const uint32_t i = (mulhi(w.w0, 16u) * 16u + mulhi(w.w2, 15u)) * 4u + (w.w1 >= 0xE6666667u ? 2u : 0u) +
+                       (w.w3 >= 0xE6666667u ? 1u : 0u);
+    mask = S.mask[i];
+    return S.board[i];
 }
 
 struct FastTables {
@@ -73,12 +137,12 @@ struct FastIO {
 
 // kAct: B2048_ACT_*; kTrack: score / step / max_exp kept (and truncation evaluated)
 // step_fast_rnd takes the board's Philox block of (gid, t, B2048_DOM_STEP) from the caller (the fused rollout kernel
-// shares it with the policy's sampling word); step_fast computes it.
+// shares it with the policy's sampling word); step_fast computes it.  keys = make_keys(seed) of the env's seed.
 // kShaped = false: the caller guarantees empty_tile_reward = merge_reward = endgame_penalty = 0 and bonus off (the env-only
 // headline kernel: no instruction spent on them).
 template <int kAct, bool kTrack, bool kShaped = true>
-B2_HD void step_fast_rnd(FastIO& io, const b2048_env_cfg& cfg, const Rand4& rnd, uint64_t seed, uint64_t gid, uint32_t t,
-                         const FastTables& T) {
+B2_HD void step_fast_rnd(FastIO& io, const b2048_env_cfg& cfg, const Rand4& rnd, const PhiloxKeys& keys, uint64_t gid,
+                         uint32_t t, const FastTables& T) {
 
     uint32_t a;
     if (kAct == B2048_ACT_BUFFER) a = io.action & 3u;
@@ -92,7 +156,7 @@ B2_HD void step_fast_rnd(FastIO& io, const b2048_env_cfg& cfg, const Rand4& rnd,
 
     // ---- move: canonicalise, four row lookups, merge statistics, de-canonicalise
     const SelEntry s = T.sel[a];
-    uint32_t clo = nib_swap(blk_transpose(io.lo, s.st), s.sm), chi = nib_swap(blk_transpose(io.hi, s.st), s.sm);
+    uint32_t clo = nib_swap_m(blk_transpose_m(io.lo, s.tm), s.nl, s.nr), chi = nib_swap_m(blk_transpose_m(io.hi, s.tm), s.nl, s.nr);
     uint32_t flo = prmt(clo, chi, s.f_lo), fhi = prmt(clo, chi, s.f_hi);
     uint32_t i0 = flo & 0xFFFFu, i1 = shr_fma<16>(flo), i2 = fhi & 0xFFFFu, i3 = shr_fma<16>(fhi);
     uint32_t r0 = T.left[i0], r1 = T.left[i1], r2 = T.left[i2], r3 = T.left[i3];
@@ -101,7 +165,7 @@ B2_HD void step_fast_rnd(FastIO& io, const b2048_env_cfg& cfg, const Rand4& rnd,
     uint32_t orm = g0.orm | g1.orm | g2.orm | g3.orm;
     uint32_t mlo = r0 + (r1 << 16), mhi = r2 + (r3 << 16);
     uint32_t plo = prmt(mlo, mhi, s.i_lo), phi = prmt(mlo, mhi, s.i_hi);
-    uint32_t vlo = blk_transpose(nib_swap(plo, s.sm), s.st), vhi = blk_transpose(nib_swap(phi, s.sm), s.st);
+    uint32_t vlo = blk_transpose_m(nib_swap_m(plo, s.nl, s.nr), s.tm), vhi = blk_transpose_m(nib_swap_m(phi, s.nl, s.nr), s.tm);
     const bool changed = ((vlo ^ io.lo) | (vhi ^ io.hi)) != 0u;
 
     const uint32_t msum = agg & 0xFFFFFu;
@@ -180,19 +244,18 @@ B2_HD void step_fast_rnd(FastIO& io, const b2048_env_cfg& cfg, const Rand4& rnd,
     uint32_t f = (changed ? B2048_F_CHANGED : 0u) | (done ? B2048_F_DONE : 0u) | (trunc ? B2048_F_TRUNC : 0u) |
                  ((orm >> 16) & 1u ? B2048_F_OVERFLOW : 0u);
     if (cfg.auto_reset && (done | trunc)) {
-        Board nbd = reset_board(seed, gid, t);
+        const Board nbd = start_board(stream_keyed(keys, gid, t, B2048_DOM_RESET), mask);   // == reset_board(seed, gid, t)
         nlo = nbd.lo; nhi = nbd.hi;
         if (kTrack) { io.score = 0u; io.step = 0u; io.max_exp = 2u; }
-        mask = legal_mask(nbd);
     }
     io.lo = nlo; io.hi = nhi;
     io.flags = f | mask;
 }
 
 template <int kAct, bool kTrack, bool kShaped = true>
-B2_HD void step_fast(FastIO& io, const b2048_env_cfg& cfg, const PhiloxKeys& keys, uint64_t seed, uint64_t gid,
-                     uint32_t t, const FastTables& T) {
-    step_fast_rnd<kAct, kTrack, kShaped>(io, cfg, stream_keyed(keys, gid, t, B2048_DOM_STEP), seed, gid, t, T);
+B2_HD void step_fast(FastIO& io, const b2048_env_cfg& cfg, const PhiloxKeys& keys, uint64_t /* seed: carried by keys */,
+                     uint64_t gid, uint32_t t, const FastTables& T) {
+    step_fast_rnd<kAct, kTrack, kShaped>(io, cfg, stream_keyed(keys, gid, t, B2048_DOM_STEP), keys, gid, t, T);
 }
 // host side: does this configuration need the shaping terms?
 inline bool cfg_is_shaped(const b2048_env_cfg& c) {
