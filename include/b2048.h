@@ -35,6 +35,8 @@
  * spawn(wp, wv): n = #empty; n == 0 -> no-op; k = mulhi32(wp, n); the k-th
  * empty cell in row-major order (np.argwhere order, game2048.py:109) receives
  * exponent 2 if wv >= 0xE6666667 (u = wv/2^32 >= 0.9, game2048.py:117) else 1.
+ * The reference's own NumPy streams (default_rng(env_seed) / default_rng(policy_seed)) are a second, per-board
+ * family: see b2048_np_rng below.
  */
 #ifndef B2048_H_
 #define B2048_H_
@@ -252,6 +254,43 @@ int b2048_rollout_many(b2048_handle* h, uint64_t* boards, uint8_t* flags, uint8_
  * count is a device int32 (zeroed by the call).  Order is unspecified (a board's results do not depend on its slot). */
 int b2048_compact_live(b2048_handle* h, const int32_t* ep_len, int64_t B, int32_t* slot_map, int32_t* count,
                        void* stream);
+
+/* ---------------- reference-seeded streams ----------------
+ * The reference seeds each episode with two integers (runner.py:244-261): np.random.default_rng(env_seed) draws the
+ * spawns (game2048.py:102-118) and np.random.default_rng(policy_seed) the sampled actions (rng.choice(4, p=probs),
+ * reinforce_agent.py:187).  b2048_np_rng is the state of one such generator — NumPy's PCG64 with its 32-bit output
+ * buffer — kept per board on the device, so that a batch plays exactly the episodes run_episode(env_seed, policy_seed)
+ * plays.  Field order and meaning follow numpy's bit_generator.state: state = state_hi << 64 | state_lo,
+ * inc = inc_hi << 64 | inc_lo (odd), has_uint32 / uinteger the buffered high half of the last 64-bit output. */
+typedef struct b2048_np_rng {
+    uint64_t state_hi, state_lo, inc_hi, inc_lo;
+    uint32_t has_uint32, uinteger;
+    uint64_t reserved;                    /* pads the state to 48 bytes */
+} b2048_np_rng;
+
+/* rng[i] = np.random.default_rng(seeds[i]) (PCG64 seeded through SeedSequence) for n device-side seeds in [0, 2^64). */
+int b2048_np_rng_seed(const uint64_t* seeds, b2048_np_rng* rng, int64_t n, void* stream);
+
+/* b2048_reset_many with the two spawns of Game2048.reset drawn from each board's env stream env_rng[i] (advanced in
+ * place): board i is the board Game2048.reset(seed) returns when env_rng[i] = default_rng(seed).  score / step /
+ * max_exp / flags as in b2048_reset_many (each may be NULL). */
+int b2048_reset_many_np(b2048_handle* h, uint64_t* board, uint32_t* score, uint32_t* step, uint8_t* max_exp,
+                        uint8_t* flags, b2048_np_rng* env_rng, int64_t n, void* stream);
+
+/* b2048_rollout_many's run-to-termination loop on the reference's own random streams: the spawns of board b come from
+ * env_rng[b] (as left by b2048_reset_many_np), its sampled actions from policy_rng[b] = default_rng(policy_seed)
+ * (greedy = 1 draws nothing), both advanced in place; a finished board draws nothing more.  The policy is the fp32
+ * CUDA-core kernel only: the tensor-core policies compute other probabilities and would therefore sample other actions.
+ * ep_len is required (zero on entry for the boards still playing).  slot_map / n_slots / n_slots_dev as in
+ * b2048_rollout_many (slot_map may be NULL: every board): the policy visits only the listed boards; the step kernel
+ * passes the finished ones through.  Per board the result does not depend on the board's position in the batch or in
+ * the list. */
+int b2048_rollout_many_np(b2048_handle* h, uint64_t* boards, uint8_t* flags, uint8_t* actions, float* rewards,
+                          uint32_t* score, uint32_t* step, uint8_t* max_exp, int32_t* ep_len,
+                          const b2048_env_cfg* cfg /* host */, const b2048_mlp_desc* mlp /* host */, int64_t B,
+                          int32_t t_begin, int32_t n_steps, b2048_np_rng* env_rng, b2048_np_rng* policy_rng,
+                          int32_t use_mask, int32_t greedy, const int32_t* slot_map, int64_t n_slots,
+                          const int32_t* n_slots_dev, void* stream);
 
 /* forward_logits only (MLP.py:159-196): out[n, n_out] = logits (actor) or V(s) (critic, n_out = 1).
  *   precision : 0 = fp32 CUDA cores; 1 = single-precision tcgen05 (1e-2 class; n >= 4096: bf16 for 16-256-256-(<=4) ReLU on raw /

@@ -7,7 +7,7 @@ through the C ABI in include/b2048.h (libb2048.so, bound with ctypes in ``_lib``
 """
 from . import _lib
 from ._lib import B2048Error
-from .batched_env import Batched2048Env, Game2048EnvConfig, debug_set, get_handle, make_env_cfg
+from .batched_env import Batched2048Env, Game2048EnvConfig, debug_set, get_handle, make_env_cfg, make_fixed_seed_iter
 from .game2048 import Game2048
 from .env import Game2048Env
 from .MLP import (MLPConfig, DeviceMLP, encode_observation, init_model_params, load_model_params, save_model_params,
@@ -20,4 +20,4 @@ from . import dist
 __all__ = ["B2048Error", "Batched2048Env", "Game2048EnvConfig", "debug_set", "get_handle", "make_env_cfg", "Game2048",
            "Game2048Env", "MLPConfig", "DeviceMLP", "encode_observation", "init_model_params", "load_model_params",
            "save_model_params", "forward_logits", "logits_to_probs", "ReinforceAgent", "ReinforceAgentConfig",
-           "Rollout", "SharedTrunkActorCritic"]
+           "Rollout", "SharedTrunkActorCritic", "make_fixed_seed_iter"]

@@ -11,6 +11,7 @@ PKG_DIR = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(PKG_DIR, "libb2048.so")
 
 B2048_MAX_LAYERS = 8
+NP_RNG_WORDS = 6        # sizeof(b2048_np_rng) / 8: one NumPy PCG64 generator state per board
 
 REWARD = {"sum": 0, "log2": 1}
 BONUS = {"off": 0, "raw": 1, "log2": 2}
@@ -72,6 +73,10 @@ SIGNATURES = {
     "b2048_rollout_many": [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, C.POINTER(EnvCfg), C.POINTER(MlpDesc), _i64, _i32, _i32,
                            _u64, _u64, _u32, _i32, _i32, _i32, _vp, _i64, _vp, _vp],
     "b2048_compact_live": [_vp, _vp, _i64, _vp, _vp, _vp],
+    "b2048_np_rng_seed": [_vp, _vp, _i64, _vp],
+    "b2048_reset_many_np": [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _vp],
+    "b2048_rollout_many_np": [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, C.POINTER(EnvCfg), C.POINTER(MlpDesc), _i64, _i32,
+                              _i32, _vp, _vp, _i32, _i32, _vp, _i64, _vp, _vp],
     "b2048_mlp_forward": [_vp, _vp, C.POINTER(MlpDesc), _vp, _i64, _i32, _vp],
     "b2048_dense_forward": [_vp, _vp, C.POINTER(MlpDesc), _vp, _vp, _i64, _vp],
     "b2048_reverse_scan": [_vp, _vp, _vp, _f32, _i32, _i64, _vp],

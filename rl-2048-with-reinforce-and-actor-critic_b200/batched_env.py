@@ -12,6 +12,7 @@ import ctypes as C
 from dataclasses import dataclass
 from typing import Any
 
+import numpy as np
 import torch
 
 from . import _lib
@@ -93,6 +94,34 @@ def debug_get(option: str) -> bool:
     return _debug.get(option, False)
 
 
+def make_fixed_seed_iter(base_seed: int):
+    """The reference runner's per-episode seed iterator (runner.py:244-261): an endless stream of int64 seeds drawn
+    from np.random.default_rng(base_seed).  runner.py draws env seeds from make_fixed_seed_iter(env base seed) and
+    policy seeds from make_fixed_seed_iter(policy base seed), one of each per episode."""
+    rng = np.random.default_rng(base_seed)
+    while True:
+        yield int(rng.integers(low=0, high=np.iinfo(np.int64).max, dtype=np.int64))
+
+
+def np_seed_streams(seeds, device: torch.device) -> torch.Tensor:
+    """One np.random.default_rng(seed) state per seed on `device` (b2048_np_rng_seed): int64 [n, 6].
+    Seeds must be integers in [0, 2^64); anything else raises ValueError, as default_rng does for negative seeds."""
+    vals = []
+    for s in seeds:
+        if isinstance(s, (bool, np.bool_)) or not isinstance(s, (int, np.integer)):
+            raise ValueError(f"seed {s!r} is not an integer")
+        s = int(s)
+        if not 0 <= s < 2**64:
+            raise ValueError(f"seed {s} is outside [0, 2^64)")
+        vals.append(s)
+    n = len(vals)
+    host = torch.from_numpy(np.array(vals, dtype=np.uint64).view(np.int64))
+    rng = torch.empty((n, _lib.NP_RNG_WORDS), dtype=torch.int64, device=device)
+    with torch.cuda.device(device):
+        _lib.check(_lib.load().b2048_np_rng_seed(_ptr(host.to(device)), _ptr(rng), n, _stream()), "b2048_np_rng_seed")
+    return rng
+
+
 def _ptr(t: torch.Tensor | None):
     return None if t is None else C.c_void_p(t.data_ptr())
 
@@ -132,14 +161,27 @@ class Batched2048Env:
         self.max_exp = torch.full((n,), 2, dtype=torch.uint8, device=dev) if track_state else None
         self.reward = torch.zeros(n, dtype=torch.float32, device=dev)
         self.obs_width = 272 if self.config.obs_mode == "onehot" else 16
+        self.env_rng: torch.Tensor | None = None   # per-board NumPy env streams (reset_many(env_seeds=...))
 
     # ------------------------------------------------------------------ reset
-    def reset_many(self, seed: int | None = None, spawn_replay: torch.Tensor | None = None
+    def reset_many(self, seed: int | None = None, spawn_replay: torch.Tensor | None = None, env_seeds=None
                    ) -> tuple[torch.Tensor, torch.Tensor]:
-        """Game2048Env.reset for every board; returns (packed boards, flags)."""
+        """Game2048Env.reset for every board; returns (packed boards, flags).
+        env_seeds (one integer per board): board i is reset from np.random.default_rng(env_seeds[i]) exactly like
+        Game2048Env.reset(seed=env_seeds[i]), and that generator is kept on the device in ``env_rng`` (int64
+        [num_envs, 6]) for the spawns of ReinforceAgent.run_episodes."""
         if seed is not None:
             self.seed = int(seed) & (2**64 - 1)
         self.t = 0
+        if env_seeds is not None:
+            if len(env_seeds) != self.num_envs:
+                raise ValueError(f"{len(env_seeds)} env seeds for {self.num_envs} boards")
+            self.env_rng = np_seed_streams(env_seeds, self.device)
+            with torch.cuda.device(self.device):
+                _lib.check(self._lib.b2048_reset_many_np(self._h, _ptr(self.board), _ptr(self.score), _ptr(self.step_count),
+                                                         _ptr(self.max_exp), _ptr(self.flags), _ptr(self.env_rng), self.num_envs,
+                                                         _stream()), "b2048_reset_many_np")
+            return self.board, self.flags
         with torch.cuda.device(self.device):
             _lib.check(self._lib.b2048_reset_many(self._h, _ptr(self.board), _ptr(self.score), _ptr(self.step_count),
                                                   _ptr(self.max_exp), _ptr(self.flags), _ptr(spawn_replay), self.num_envs, self.seed,

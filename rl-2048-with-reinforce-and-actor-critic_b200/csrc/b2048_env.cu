@@ -3,6 +3,8 @@
 //   K0 build_lut_kernel   Game2048._row_move_left tabulated over all 65,536 rows (game2048.py:120-137)
 //   K1 reset_kernel       Game2048.reset + Game2048Env.reset              (game2048.py:26-34, env.py:174-194)
 //   K2 step_kernel        fused Game2048.step + Game2048Env.step          (game2048.py:40-70, env.py:197-302)
+//      np_seed_kernel / reset_np_kernel / step_np_kernel: the same with the spawns drawn from per-board NumPy streams
+//                         (np.random.default_rng(env_seed), b2048_np_rng.cuh) — the reference's own seeded episodes
 //      move_kernel        Game2048._move preview                          (game2048.py:158-165)
 //      obs_kernel         Game2048Env._preprocess_board                   (env.py:131-150)
 //
@@ -63,6 +65,31 @@ __global__ void __launch_bounds__(256) reset_kernel(uint64_t* __restrict__ board
         if (score) score[i] = 0u;
         if (step) step[i] = 0u;
         if (max_exp) max_exp[i] = 2u;  // max_tile_seen = 4 (env.py:183)
+        if (flags) flags[i] = (uint8_t)legal_mask(b);
+    }
+}
+
+// ------------------------------------------------------------------------------------------------ NumPy streams
+// rng[i] = np.random.default_rng(seeds[i]): one thread per seed (b2048_np_rng.cuh)
+__global__ void __launch_bounds__(256) np_seed_kernel(const uint64_t* __restrict__ seeds, b2048_np_rng* __restrict__ rng,
+                                                       int64_t n) {
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x)
+        rng[i] = np::seed(seeds[i]);
+}
+
+// Game2048.reset with both spawns drawn from the board's env stream (K1 otherwise)
+__global__ void __launch_bounds__(256) reset_np_kernel(uint64_t* __restrict__ board, uint32_t* __restrict__ score,
+                                                        uint32_t* __restrict__ step, uint8_t* __restrict__ max_exp,
+                                                        uint8_t* __restrict__ flags, b2048_np_rng* __restrict__ env_rng,
+                                                        int64_t n) {
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+        b2048_np_rng r = env_rng[i];
+        const Board b = np::reset_board(r);
+        env_rng[i] = r;
+        board[i] = to_u64(b);
+        if (score) score[i] = 0u;
+        if (step) step[i] = 0u;
+        if (max_exp) max_exp[i] = 2u;
         if (flags) flags[i] = (uint8_t)legal_mask(b);
     }
 }
@@ -163,12 +190,15 @@ __device__ __forceinline__ void store_obs_onehot(float* __restrict__ obs, Board 
     }
 }
 
-template <bool kSmemLut, int kThreads>
-__global__ void __launch_bounds__(kThreads, kSmemLut ? 1 : 2) step_kernel(const __grid_constant__ StepArgs args) {
+// The body of step_kernel and of its reference-seeded variant step_np_kernel (kNp: spawns from the boards' NumPy env
+// streams env_rng, advanced in place; buffer actions, no auto-reset).
+template <bool kSmemLut, int kThreads, bool kNp>
+__device__ __forceinline__ void step_loop(const StepArgs& args, b2048_np_rng* env_rng) {
     extern __shared__ __align__(128) uint8_t smem[];
     __shared__ uint64_t mbar;
 
     const int tid = threadIdx.x;
+    __builtin_assume(tid < kThreads);   // the launch bound, which the kernel's range analysis does not see through the inlined body
     const int lane = tid & 31;
     const uint16_t* lut_left;
     const uint8_t* lut_merge;
@@ -221,7 +251,12 @@ __global__ void __launch_bounds__(kThreads, kSmemLut ? 1 : 2) step_kernel(const 
         bool frozen = false;
         Board board_before = io.board;
         if (args.ep_len && valid) frozen = args.ep_len[i] != 0;
-        step_one(io, cfg, opt, args.seed, args.gid0 + (uint64_t)i, args.t, lut_left, lut_merge);
+        b2048_np_rng rng;
+        if constexpr (kNp) {
+            if (valid && !frozen) rng = env_rng[i];
+        }
+        step_one<decltype(lut_left), decltype(lut_merge), kNp>(io, cfg, opt, args.seed, args.gid0 + (uint64_t)i, args.t,
+                                                              lut_left, lut_merge, &rng, valid && !frozen);
         if (valid && frozen) {
             // finished episode of a run-to-termination rollout: pass the terminal state through untouched
             uint32_t m = legal_mask(board_before);
@@ -245,6 +280,9 @@ __global__ void __launch_bounds__(kThreads, kSmemLut ? 1 : 2) step_kernel(const 
             if (args.reward) args.reward[i] = (float)io.reward;
             if (args.reward64) args.reward64[i] = io.reward;
             args.flags[i] = (uint8_t)io.flags;
+            if constexpr (kNp) {
+                if (io.flags & B2048_F_CHANGED) env_rng[i] = rng;   // only a changed board drew a spawn
+            }
         }
         if (args.obs != nullptr && cfg.obs_mode != B2048_OBS_NONE) {
             const int64_t warp_base = base + (tid & ~31);
@@ -252,6 +290,17 @@ __global__ void __launch_bounds__(kThreads, kSmemLut ? 1 : 2) step_kernel(const 
             else store_obs16(args.obs, io.board, warp_base, args.n, lane, cfg.obs_mode, cfg.obs_log2_scale);
         }
     }
+}
+
+template <bool kSmemLut, int kThreads>
+__global__ void __launch_bounds__(kThreads, kSmemLut ? 1 : 2) step_kernel(const __grid_constant__ StepArgs args) {
+    step_loop<kSmemLut, kThreads, false>(args, nullptr);
+}
+
+template <bool kSmemLut, int kThreads>
+__global__ void __launch_bounds__(kThreads, kSmemLut ? 1 : 2) step_np_kernel(const __grid_constant__ StepArgs args,
+                                                                              b2048_np_rng* __restrict__ env_rng) {
+    step_loop<kSmemLut, kThreads, true>(args, env_rng);
 }
 
 // ------------------------------------------------------------------------------------------------ K2 (fast path)
@@ -583,6 +632,8 @@ extern "C" int b2048_create(b2048_handle** out) {
     if (h->smem_optin >= B2048_LUT_BYTES) {
         B2_CUDA(cudaFuncSetAttribute(step_kernel<true, 1024>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                      B2048_LUT_BYTES));
+        B2_CUDA(cudaFuncSetAttribute(step_np_kernel<true, 1024>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                     B2048_LUT_BYTES));
     }
     if (h->smem_optin >= B2048_TABLES_BYTES) {
 #define B2_SET(A, TR)                                                                                                       \
@@ -637,6 +688,46 @@ extern "C" int b2048_reset_many(b2048_handle* h, uint64_t* board, uint32_t* scor
     if (n == 0) return B2048_OK;
     reset_kernel<<<grid_for(n, 256, h->num_sms, 8), 256, 0, (cudaStream_t)stream>>>(board, score, step, max_exp, flags,
                                                                                    spawn_replay, n, seed, gid0, t);
+    B2_CUDA(cudaGetLastError());
+    return B2048_OK;
+}
+
+extern "C" int b2048_np_rng_seed(const uint64_t* seeds, b2048_np_rng* rng, int64_t n, void* stream) {
+    B2_REQUIRE(n >= 0, "b2048_np_rng_seed: n < 0");
+    if (n == 0) return B2048_OK;
+    B2_REQUIRE(seeds && rng, "b2048_np_rng_seed: seeds / rng is NULL");
+    const int64_t blocks = (n + 255) / 256;
+    np_seed_kernel<<<(unsigned)(blocks < 65536 ? blocks : 65536), 256, 0, (cudaStream_t)stream>>>(seeds, rng, n);
+    B2_CUDA(cudaGetLastError());
+    return B2048_OK;
+}
+
+extern "C" int b2048_reset_many_np(b2048_handle* h, uint64_t* board, uint32_t* score, uint32_t* step, uint8_t* max_exp,
+                                   uint8_t* flags, b2048_np_rng* env_rng, int64_t n, void* stream) {
+    B2_REQUIRE(h != nullptr, "b2048_reset_many_np: handle is NULL");
+    B2_REQUIRE(n >= 0, "b2048_reset_many_np: n < 0");
+    if (n == 0) return B2048_OK;
+    B2_REQUIRE(board && env_rng, "b2048_reset_many_np: board / env_rng is NULL");
+    reset_np_kernel<<<grid_for(n, 256, h->num_sms, 8), 256, 0, (cudaStream_t)stream>>>(board, score, step, max_exp, flags,
+                                                                                       env_rng, n);
+    B2_CUDA(cudaGetLastError());
+    return B2048_OK;
+}
+
+// One step of b2048_rollout_many_np: b2048_step_many in rollout mode (buffer actions, ep_len bookkeeping, float32
+// rewards, no auto-reset) on the generic step kernel, spawns drawn from env_rng.
+int b2::launch_step_np(b2048_handle* h, const uint64_t* board_in, uint64_t* board_out, uint32_t* score, uint32_t* step,
+                   uint8_t* max_exp, const uint8_t* action, const uint8_t* flags_in, const b2048_env_cfg* cfg, float* reward,
+                   uint8_t* flags, int32_t* ep_len, uint32_t ep_t, int64_t n, b2048_np_rng* env_rng, cudaStream_t s) {
+    StepArgs a = {};
+    a.board_in = board_in; a.board_out = board_out; a.score = score; a.step = step; a.max_exp = max_exp;
+    a.action = action; a.flags_in = flags_in; a.ep_len = ep_len; a.ep_t = ep_t;
+    a.reward = reward; a.flags = flags; a.tables = h->d_tables; a.n = n; a.cfg = *cfg;
+    if (h->smem_optin >= B2048_LUT_BYTES && n >= (int64_t)32768) {
+        step_np_kernel<true, 1024><<<grid_for(n, 1024, h->num_sms, 1), 1024, B2048_LUT_BYTES, s>>>(a, env_rng);
+    } else {
+        step_np_kernel<false, 256><<<grid_for(n, 256, h->num_sms, 8), 256, 0, s>>>(a, env_rng);
+    }
     B2_CUDA(cudaGetLastError());
     return B2048_OK;
 }

@@ -126,6 +126,11 @@ int launch_backward_gen(b2048_handle* h, const uint64_t* board, const uint8_t* m
                         const b2048_mlp_desc* mlp, float* grads, int64_t n, int head_mode, uint8_t* workspace, int64_t chunk,
                         cudaStream_t stream);
 
+// ---- b2048_env.cu: the step of b2048_rollout_many_np (generic step kernel, spawns from the boards' NumPy env streams)
+int launch_step_np(b2048_handle* h, const uint64_t* board_in, uint64_t* board_out, uint32_t* score, uint32_t* step,
+                   uint8_t* max_exp, const uint8_t* action, const uint8_t* flags_in, const b2048_env_cfg* cfg, float* reward,
+                   uint8_t* flags, int32_t* ep_len, uint32_t ep_t, int64_t n, b2048_np_rng* env_rng, cudaStream_t s);
+
 }  // namespace b2
 
 #define B2_CUDA(expr)                                              \

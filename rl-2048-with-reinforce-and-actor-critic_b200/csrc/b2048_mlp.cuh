@@ -47,13 +47,15 @@ __device__ __forceinline__ float activate_grad(float a, int mode) {
 }
 
 // Layer-0 input rows: raw / log2 -> 16 floats; onehot -> 16 exponents stored as int bits.
+// slots != NULL: row s of the tile is board slots[s] (a live-board list), else board s.
 __device__ __forceinline__ void encode_input(float* x0 /*[kTileM][16+pad]*/, const uint64_t* __restrict__ board,
-                                             int64_t s0, int64_t n, int obs_mode, float scale) {
+                                             int64_t s0, int64_t n, int obs_mode, float scale,
+                                             const int32_t* __restrict__ slots = nullptr) {
     for (int idx = threadIdx.x; idx < kTileM * 16; idx += kMlpThreads) {
         int b = idx >> 4, cell = idx & 15;
         int64_t s = s0 + b;
         uint32_t e = 0;
-        if (s < n) e = (uint32_t)((board[s] >> (4 * cell)) & 0xFull);
+        if (s < n) e = (uint32_t)((board[slots ? (int64_t)slots[s] : s] >> (4 * cell)) & 0xFull);
         float v;
         if (obs_mode == B2048_OBS_ONEHOT) v = __int_as_float((int)e);
         else if (obs_mode == B2048_OBS_RAW) v = e ? (float)(1u << e) : 0.0f;
@@ -167,8 +169,9 @@ __device__ __forceinline__ void tile_layer0_onehot(const float* __restrict__ X0,
 // arena + act_offset(l).  If gact != nullptr, hidden activations a_l (l >= 1) are also written to
 // gact[l][s][dim_l] for the weight-gradient GEMMs.  Ends with __syncthreads().
 __device__ __forceinline__ void tile_forward_hidden(float* arena, const MlpDev& m, const uint64_t* __restrict__ board,
-                                                    int64_t s0, int64_t n, float* const* gact) {
-    encode_input(arena, board, s0, n, m.obs_mode, m.obs_scale);
+                                                    int64_t s0, int64_t n, float* const* gact,
+                                                    const int32_t* __restrict__ slots = nullptr) {
+    encode_input(arena, board, s0, n, m.obs_mode, m.obs_scale, slots);
     __syncthreads();
     const int L = m.n_layers;
     for (int l = 0; l + 1 < L; ++l) {

@@ -4,12 +4,15 @@
 //                        (src/MLP.py:22-43, :139-196; src/reinforce_agent.py:126-192) fused: the packed
 //                        board is the only per-board input, the action byte (+ optional probs / logits)
 //                        the only output; activations never leave shared memory.
+//   policy_step_np_kernel  the same over a live-board list, sampling rng.choice(4, p) on per-board NumPy streams
+//                        (b2048_rollout_many_np: the reference's own seeded episodes)
 //   mlp_forward_kernel   forward_logits only (critic values V(s), logits for tests / update)
 #include <cuda_runtime.h>
 
 #include "b2048_device.cuh"
 #include "b2048_internal.h"
 #include "b2048_mlp.cuh"
+#include "b2048_np_rng.cuh"
 
 namespace b2 {
 
@@ -26,18 +29,37 @@ struct PolicyArgs {
     int greedy;
 };
 
-__global__ void __launch_bounds__(kMlpThreads, 1) policy_step_kernel(const __grid_constant__ PolicyArgs args) {
+// Extra inputs of the reference-seeded variant policy_step_np_kernel (b2048_rollout_many_np)
+struct PolicyNpArgs {
+    b2048_np_rng* rng;         // per board: the NumPy policy stream rng.choice draws from, advanced in place
+    const int32_t* ep_len;     // a finished board (ep_len != 0) draws nothing and gets no action
+    const int32_t* slot_map;   // live-board list: sample s is board slot_map[s] (NULL: board s)
+    const int32_t* n_dev;      // with slot_map: the number of listed boards, read on the device
+};
+
+// kNp: actions sampled by rng.choice(4, p) on the board's NumPy stream (b2048_np_rng.cuh) over the listed boards; a
+// board's probabilities are the same arithmetic whatever its tile or row, so they do not depend on its position.
+template <bool kNp>
+__device__ __forceinline__ void policy_step_body(const PolicyArgs& args, const PolicyNpArgs& npa) {
     extern __shared__ __align__(16) float arena[];
     const MlpDev& m = args.mlp;
     const int n_out = m.dims[m.n_layers];
-    const int64_t n_tiles = (args.n + kTileM - 1) / kTileM;
+    int64_t n = args.n;
+    if constexpr (kNp) {
+        if (npa.n_dev) n = *npa.n_dev;   // uniform over the grid
+    }
+    const int64_t n_tiles = (n + kTileM - 1) / kTileM;
     for (int64_t tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
         const int64_t s0 = tile * kTileM;
-        tile_forward_hidden(arena, m, args.board, s0, args.n, nullptr);
+        tile_forward_hidden(arena, m, args.board, s0, n, nullptr, kNp ? npa.slot_map : nullptr);
         float logit = tile_head(arena, m);
         const int b = threadIdx.x >> 2, j = threadIdx.x & 3;
-        const int64_t s = s0 + b;
-        const bool valid = s < args.n;
+        int64_t s = s0 + b;
+        bool valid = s < n;
+        if constexpr (kNp) {
+            if (valid && npa.slot_map) s = npa.slot_map[s];
+            if (valid && npa.ep_len[s] != 0) valid = false;   // finished: nothing drawn, nothing written
+        }
         uint32_t fl = 0xFu;
         const bool use_mask = args.mask_flags != nullptr;
         if (use_mask && valid) fl = args.mask_flags[s];
@@ -63,6 +85,10 @@ __global__ void __launch_bounds__(kMlpThreads, 1) policy_step_kernel(const __gri
                 if (q1 > best) { best = q1; a = 1; }
                 if (q2 > best) { best = q2; a = 2; }
                 if (q3 > best) { best = q3; a = 3; }
+            } else if constexpr (kNp) {
+                b2048_np_rng r = npa.rng[s];
+                a = np::choice4(r, p0, p1, p2, p3);   // rng.choice(4, p=probs) (reinforce_agent.py:187)
+                npa.rng[s] = r;
             } else {
                 // rng.choice(4, p=probs) == inverse CDF on one uniform (reinforce_agent.py:187); the uniform
                 // is word 3 of the board's Philox block for this step
@@ -83,6 +109,15 @@ __global__ void __launch_bounds__(kMlpThreads, 1) policy_step_kernel(const __gri
         }
         __syncthreads();  // arena is reused by the next tile
     }
+}
+
+__global__ void __launch_bounds__(kMlpThreads, 1) policy_step_kernel(const __grid_constant__ PolicyArgs args) {
+    policy_step_body<false>(args, PolicyNpArgs{});
+}
+
+__global__ void __launch_bounds__(kMlpThreads, 1) policy_step_np_kernel(const __grid_constant__ PolicyArgs args,
+                                                                         const __grid_constant__ PolicyNpArgs npa) {
+    policy_step_body<true>(args, npa);
 }
 
 struct ForwardArgs {
@@ -259,6 +294,55 @@ extern "C" int b2048_rollout_many(b2048_handle* h, uint64_t* boards, uint8_t* fl
         st = b2048_step_many(h, b_in, b_in + B, score, step, max_exp, actions + t * B, nullptr, f_in, nullptr, &c, nullptr,
                              rewards + t * B, nullptr, f_in + B, nullptr, ep_len, (uint32_t)(t + 1), B, seed, gid0, t_env,
                              stream);
+        if (st != B2048_OK) return st;
+    }
+    return B2048_OK;
+}
+
+// b2048_rollout_many's run-to-termination loop with the reference's NumPy streams: policy_step_np_kernel (fp32) over the
+// listed boards, then the generic step kernel's NumPy variant over all B (it passes the finished boards through).
+extern "C" int b2048_rollout_many_np(b2048_handle* h, uint64_t* boards, uint8_t* flags, uint8_t* actions, float* rewards,
+                                     uint32_t* score, uint32_t* step, uint8_t* max_exp, int32_t* ep_len,
+                                     const b2048_env_cfg* cfg, const b2048_mlp_desc* mlp, int64_t B, int32_t t_begin,
+                                     int32_t n_steps, b2048_np_rng* env_rng, b2048_np_rng* policy_rng, int32_t use_mask,
+                                     int32_t greedy, const int32_t* slot_map, int64_t n_slots, const int32_t* n_slots_dev,
+                                     void* stream) {
+    B2_REQUIRE(h != nullptr, "b2048_rollout_many_np: handle is NULL");
+    B2_REQUIRE(B >= 0 && n_steps >= 0 && t_begin >= 0, "b2048_rollout_many_np: negative size");
+    if (B == 0 || n_steps == 0) return B2048_OK;
+    B2_REQUIRE(boards && flags && actions && rewards && cfg && mlp && ep_len && env_rng && policy_rng,
+               "b2048_rollout_many_np: NULL buffer (ep_len, env_rng and policy_rng are required)");
+    B2_REQUIRE(!cfg->auto_reset, "b2048_rollout_many_np: run-to-termination only (cfg->auto_reset must be 0)");
+    B2_REQUIRE(cfg->reward_mode == B2048_REWARD_SUM || cfg->reward_mode == B2048_REWARD_LOG2,
+               "b2048_rollout_many_np: unsupported reward mode");
+    B2_REQUIRE(cfg->bonus_mode >= B2048_BONUS_OFF && cfg->bonus_mode <= B2048_BONUS_LOG2,
+               "b2048_rollout_many_np: unsupported bonus mode");
+    B2_REQUIRE(slot_map == nullptr || (n_slots >= 0 && n_slots <= B), "b2048_rollout_many_np: n_slots out of range");
+    b2048_env_cfg c = *cfg;
+    c.action_mode = B2048_ACT_BUFFER;
+    c.obs_mode = B2048_OBS_NONE;
+    PolicyArgs a;
+    size_t smem = 0;
+    int st = validate_mlp(mlp, &a.mlp, &smem, h->smem_optin, "b2048_rollout_many_np");
+    if (st != B2048_OK) return st;
+    const int64_t n_pol = slot_map ? n_slots : B;
+    if (n_pol == 0) return B2048_OK;
+    B2_CUDA(cudaFuncSetAttribute(policy_step_np_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    const int64_t tiles = (n_pol + kTileM - 1) / kTileM;
+    const int grid = (int)(tiles < h->num_sms ? tiles : h->num_sms);
+    cudaStream_t s = (cudaStream_t)stream;
+    PolicyNpArgs npa;
+    npa.rng = policy_rng; npa.ep_len = ep_len; npa.slot_map = slot_map; npa.n_dev = slot_map ? n_slots_dev : nullptr;
+    a.probs = nullptr; a.logits = nullptr; a.n = n_pol; a.seed = 0; a.gid0 = 0; a.t = 0; a.greedy = greedy;
+    for (int32_t k = 0; k < n_steps; ++k) {
+        const int64_t t = (int64_t)t_begin + k;
+        uint64_t* b_in = boards + t * B;
+        uint8_t* f_in = flags + t * B;
+        a.board = b_in; a.mask_flags = use_mask ? f_in : nullptr; a.action = actions + t * B;
+        policy_step_np_kernel<<<grid, kMlpThreads, smem, s>>>(a, npa);
+        B2_CUDA(cudaGetLastError());
+        st = launch_step_np(h, b_in, b_in + B, score, step, max_exp, actions + t * B, f_in, &c, rewards + t * B, f_in + B, ep_len,
+                            (uint32_t)(t + 1), B, env_rng, s);
         if (st != B2048_OK) return st;
     }
     return B2048_OK;

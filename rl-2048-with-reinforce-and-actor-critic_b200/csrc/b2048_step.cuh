@@ -9,6 +9,7 @@
 #pragma once
 #include "../../include/b2048.h"
 #include "b2048_device.cuh"
+#include "b2048_np_rng.cuh"
 
 namespace b2 {
 
@@ -40,10 +41,15 @@ struct StepOpts {
     bool track_step, track_max, want_sum;
 };
 
-template <typename LutL, typename LutM>
+// kNp: the spawn is drawn from the board's NumPy env stream *np_rng (b2048_np_rng.cuh) instead of Philox, and only
+// when np_draw is set.  That variant serves buffer actions without auto-reset only, so it computes no Philox block.
+template <typename LutL, typename LutM, bool kNp = false>
 B2_HD void step_one(StepIO& io, const b2048_env_cfg& cfg, const StepOpts& opt, uint64_t seed, uint64_t gid,
-                    uint32_t t, LutL lut_left, LutM lut_merge) {
-    Rand4 rnd = stream(seed, gid, t, B2048_DOM_STEP);
+                    uint32_t t, LutL lut_left, LutM lut_merge, b2048_np_rng* np_rng = nullptr,
+                    bool np_draw = false) {
+    Rand4 rnd;
+    if constexpr (kNp) rnd = Rand4{0u, 0u, 0u, 0u};
+    else rnd = stream(seed, gid, t, B2048_DOM_STEP);
 
     uint32_t a;
     if (cfg.action_mode == B2048_ACT_BUFFER) {
@@ -67,8 +73,13 @@ B2_HD void step_one(StepIO& io, const b2048_env_cfg& cfg, const StepOpts& opt, u
 
     Board nb = mv.board;
     if (changed) {  // game2048.py:56-58
-        if (io.replay & 0x80u) nb = place_kth_empty(nb, io.replay & 0xFu, (io.replay & 0x10u) ? 2u : 1u);
-        else nb = spawn(nb, rnd.w0, rnd.w1);
+        if constexpr (kNp) {
+            if (np_draw) nb = np::spawn(*np_rng, nb);
+        } else if (io.replay & 0x80u) {
+            nb = place_kth_empty(nb, io.replay & 0xFu, (io.replay & 0x10u) ? 2u : 1u);
+        } else {
+            nb = spawn(nb, rnd.w0, rnd.w1);
+        }
     }
     uint32_t mask = legal_mask(nb);
     bool done = (mask == 0u) & ((nb.lo | nb.hi) != 0u);  // == _is_done() for every board incl. the empty one

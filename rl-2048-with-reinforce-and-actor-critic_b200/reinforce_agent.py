@@ -417,41 +417,15 @@ class ReinforceAgent:
             ((self._fused_shape() and not debug_get("no_fused_rollout")) or (not self._fused_shape() and self._generic_tc_shape()))
         if compact:
             rewards.zero_()
-            # Live-board bookkeeping stays on the device: after every chunk b2048_compact_live rebuilds the list and its
-            # count, the next chunk's kernel reads the count from device memory, and the host only looks at the count
-            # of the chunk BEFORE the one it has just enqueued (pinned copy + event) — the GPU never waits for the host.
-            slot_buf = self._buf("ro_slot_map", (B,), torch.int32)
-            count_dev = self._buf("ro_live_count", (1,), torch.int32)
-            n_max = (cap + check_every - 1) // check_every + 1
-            count_host = getattr(self, "_ro_count_host", None)
-            if count_host is None or count_host.numel() < n_max:
-                count_host = self._ro_count_host = torch.zeros(n_max, dtype=torch.int32).pin_memory()
-            events: list[torch.cuda.Event] = []
-            upper, k = B, 0
-            while T < cap:
-                chunk = min(check_every, cap - T)
-                with torch.cuda.device(self.device):
-                    _lib.check(self._lib.b2048_rollout_many(
-                        self._h, _ptr(boards), _ptr(flags), _ptr(actions), _ptr(rewards), _ptr(benv.score),
-                        _ptr(benv.step_count), _ptr(benv.max_exp), _ptr(length), C.byref(cfg), C.byref(self._actor.desc), B, T,
-                        chunk, benv.seed, benv.gid0, t0, int(self._use_mask), int(greedy), 1,
-                        _ptr(slot_buf) if k > 0 else None, upper, _ptr(count_dev) if k > 0 else None, _stream()),
-                        "b2048_rollout_many")
-                    _lib.check(self._lib.b2048_compact_live(self._h, _ptr(length), B, _ptr(slot_buf), _ptr(count_dev), _stream()),
-                               "b2048_compact_live")
-                count_host[k: k + 1].copy_(count_dev, non_blocking=True)
-                ev = torch.cuda.Event()
-                ev.record()
-                events.append(ev)
-                T += chunk
-                if k >= 1:                      # boards alive after chunk k - 1 (that copy finished before chunk k started)
-                    events[k - 1].synchronize()
-                    alive = int(count_host[k - 1])
-                    if alive == 0:              # chunk k found nothing to play
-                        T -= chunk
-                        break
-                    upper = alive
-                k += 1
+
+            def launch(T, chunk, slot_map, upper, count):
+                _lib.check(self._lib.b2048_rollout_many(
+                    self._h, _ptr(boards), _ptr(flags), _ptr(actions), _ptr(rewards), _ptr(benv.score),
+                    _ptr(benv.step_count), _ptr(benv.max_exp), _ptr(length), C.byref(cfg), C.byref(self._actor.desc), B, T,
+                    chunk, benv.seed, benv.gid0, t0, int(self._use_mask), int(greedy), 1, slot_map, upper, count, _stream()),
+                    "b2048_rollout_many")
+
+            T = self._live_chunks(launch, length, cap, check_every)
         while not compact and T < cap:
             chunk = min(check_every if not fixed else 256, cap - T)
             with torch.cuda.device(self.device):
@@ -479,6 +453,85 @@ class ReinforceAgent:
         benv.board = boards[T]
         benv.flags = flags[T]
         return Rollout(boards[: T + 1], flags[: T + 1], actions[:T], rewards[:T], length, T, auto_reset=fixed)
+
+    def _live_chunks(self, launch, length: torch.Tensor, cap: int, check_every: int) -> int:
+        """Run-to-termination chunks on the live-board list: launch(T, chunk, slot_map, upper, count) enqueues steps
+        [T, T + chunk) for the listed boards (every board for the first chunk).  Live-board bookkeeping stays on the
+        device: after every chunk b2048_compact_live rebuilds the list and its count, the next chunk's kernels read the
+        count from device memory, and the host only looks at the count of the chunk BEFORE the one it has just enqueued
+        (pinned copy + event) — the GPU never waits for the host.  Returns the number of steps played."""
+        B = int(length.numel())
+        slot_buf = self._buf("ro_slot_map", (B,), torch.int32)
+        count_dev = self._buf("ro_live_count", (1,), torch.int32)
+        n_max = (cap + check_every - 1) // check_every + 1
+        count_host = getattr(self, "_ro_count_host", None)
+        if count_host is None or count_host.numel() < n_max:
+            count_host = self._ro_count_host = torch.zeros(n_max, dtype=torch.int32).pin_memory()
+        events: list[torch.cuda.Event] = []
+        T, upper, k = 0, B, 0
+        while T < cap:
+            chunk = min(check_every, cap - T)
+            with torch.cuda.device(self.device):
+                launch(T, chunk, _ptr(slot_buf) if k > 0 else None, upper, _ptr(count_dev) if k > 0 else None)
+                _lib.check(self._lib.b2048_compact_live(self._h, _ptr(length), B, _ptr(slot_buf), _ptr(count_dev), _stream()),
+                           "b2048_compact_live")
+            count_host[k: k + 1].copy_(count_dev, non_blocking=True)
+            ev = torch.cuda.Event()
+            ev.record()
+            events.append(ev)
+            T += chunk
+            if k >= 1:                      # boards alive after chunk k - 1 (that copy finished before chunk k started)
+                events[k - 1].synchronize()
+                alive = int(count_host[k - 1])
+                if alive == 0:              # chunk k found nothing to play
+                    T -= chunk
+                    break
+                upper = alive
+            k += 1
+        return T
+
+    def run_episodes(self, benv: Batched2048Env, env_seeds, policy_seeds, use_greedy: bool = False,
+                     max_steps: int | None = None, check_every: int = 48, live_list: bool = True) -> Rollout:
+        """The batched run_episode(env_seed, policy_seed) (reinforce_agent.py:195-252): board b plays exactly the episode
+        run_episode(env_seeds[b], policy_seeds[b]) plays — its spawns come from np.random.default_rng(env_seeds[b]) and
+        its sampled actions from rng.choice(4, p=probs) on np.random.default_rng(policy_seeds[b]), both kept on the
+        device (b2048_rollout_many_np).  The policy runs on the fp32 kernel, the one run_episode uses: a tensor-core
+        policy computes other probabilities and would sample other actions.  len(env_seeds) == len(policy_seeds) ==
+        benv.num_envs; seeds are integers in [0, 2^64).  Every board plays to termination / truncation (max_steps caps
+        the length like rollout_many); after the first chunk the policy visits only the boards still playing
+        (live_list=False: every board every step — the same episodes, for testing).  Returns a run-to-termination
+        Rollout for update_from_rollout; the episodes' max tiles are 2 ** benv.max_exp."""
+        B = benv.num_envs
+        if len(env_seeds) != B or len(policy_seeds) != B:
+            raise ValueError(f"{len(env_seeds)} env seeds and {len(policy_seeds)} policy seeds for {B} boards")
+        from .batched_env import make_env_cfg, np_seed_streams
+        policy_rng = np_seed_streams(policy_seeds, self.device)
+        benv.reset_many(env_seeds=env_seeds)
+        cap = int(max_steps or benv.config.max_steps or 4096)
+        boards = self._buf("ro_boards", (cap + 1, B), torch.int64)
+        flags = self._buf("ro_flags", (cap + 1, B), torch.uint8)
+        actions = self._buf("ro_actions", (cap, B), torch.uint8)
+        rewards = self._buf("ro_rewards", (cap, B), torch.float32)
+        length = torch.zeros(B, dtype=torch.int32, device=self.device)
+        boards[0].copy_(benv.board)
+        flags[0].copy_(benv.flags)
+        actions.zero_()                 # the policy writes no action for a finished board
+        rewards.zero_()
+        cfg = make_env_cfg(benv.config, "buffer", auto_reset=False, emit_obs=False)
+
+        def launch(T, chunk, slot_map, upper, count):
+            _lib.check(self._lib.b2048_rollout_many_np(
+                self._h, _ptr(boards), _ptr(flags), _ptr(actions), _ptr(rewards), _ptr(benv.score), _ptr(benv.step_count),
+                _ptr(benv.max_exp), _ptr(length), C.byref(cfg), C.byref(self._actor.desc), B, T, chunk, _ptr(benv.env_rng),
+                _ptr(policy_rng), int(self._use_mask), int(use_greedy), slot_map if live_list else None, upper, count,
+                _stream()), "b2048_rollout_many_np")
+
+        T = self._live_chunks(launch, length, cap, check_every)
+        benv.t = T
+        length = torch.where(length == 0, torch.full_like(length, T), length)   # cut off by the cap
+        benv.board = boards[T]          # the step kernel passes finished boards through: slice T is every final state
+        benv.flags = flags[T]
+        return Rollout(boards[: T + 1], flags[: T + 1], actions[:T], rewards[:T], length, T)
 
     # ------------------------------------------------------------------ reference API: learning
     def compute_returns(self, rewards: list[float]) -> np.ndarray:

@@ -7,7 +7,10 @@ runner.py:10-63, defaults runner.py:116-173) and writes the same artefacts (``co
 with the full optimiser state every ``train.checkpoint_every`` batches).  One training batch =
 ``train.batch_size`` episodes played in parallel on the GPU (``rollout_many``) followed by one
 ``update_from_rollout``; evaluation = greedy rollouts with the max-tile histogram (runner.py:737-828).
-Extra keys: ``train.precision`` ("auto" | 0 | 1), ``train.exchange`` ("default" | "one_message": one all-reduce per update),
+Extra keys: ``train.seed_streams`` ("philox", the default: fresh counter-based streams per batch | "numpy": the reference's
+own seeded episodes — episode i of batch k plays run_episode(env_seed, policy_seed) with the (k * batch_size + i)-th seed
+of make_fixed_seed_iter(``train.env_base_seed``) / make_fixed_seed_iter(``train.policy_base_seed``), the order
+runner.py:587-608 draws them, on the fp32 policy kernel; evaluation keeps the Philox streams), ``train.precision`` ("auto" | 0 | 1), ``train.exchange`` ("default" | "one_message": one all-reduce per update),
 ``seed``, and an optional section ``shared_trunk`` ({"value_coef", "gae_lambda"}: one network with a policy and a value head).  Under torchrun the episodes are sharded over ranks.
 
     python -m torch.distributed.run ... b2048_runner.py -conf cfg.json      (or: python b2048_runner.py -conf cfg.json)
@@ -26,7 +29,7 @@ import torch
 
 from . import dist as bd
 from .MLP import MLPConfig
-from .batched_env import Batched2048Env, Game2048EnvConfig
+from .batched_env import Batched2048Env, Game2048EnvConfig, make_fixed_seed_iter
 from .reinforce_agent import ReinforceAgent, ReinforceAgentConfig
 
 DEFAULTS: dict[str, Any] = {
@@ -39,7 +42,8 @@ DEFAULTS: dict[str, Any] = {
     "agent": dict(gamma=0.99, learning_rate=1e-4, baseline_mode="batch", model_seed=0, reward_rank_weights=None,
                   optimizer="sgd", adam_beta1=0.9, adam_beta2=0.999, augmentation=False, use_critic=False,
                   critic_learning_rate=1e-5, critic_loss_type="mse", huber_delta=1.0),
-    "train": dict(batch_size=256, num_batches=256, precision="auto", out_dir="training_history"),
+    "train": dict(batch_size=256, num_batches=256, precision="auto", out_dir="training_history", seed_streams="philox",
+                  env_base_seed=3, policy_base_seed=7),
     "eval": dict(num_episodes=2048, model_path=None, use_greedy=True),
 }
 TILE_BINS = [16, 32, 64, 128, 256, 512, 1024, 2048, 4096]      # runner.py:557
@@ -117,11 +121,26 @@ def training(cfg: dict[str, Any], info: bd.DistInfo | None = None, device=None, 
     if tr.get("resume"):
         agent.load_checkpoint(tr["resume"])
     ckpt_every = int(tr.get("checkpoint_every", 50))
+    streams = tr.get("seed_streams", "philox")
+    if streams not in ("philox", "numpy"):
+        raise ValueError(f"Unknown train.seed_streams: {streams}")
+    if streams == "numpy":
+        # the runner's seed iterators, advanced past the batches already played; this rank plays its contiguous slice
+        # [gid0, gid0 + num_envs) of every batch's global seed list, so the episodes do not depend on the world size
+        bs = int(tr["batch_size"])
+        env_it = make_fixed_seed_iter(int(tr.get("env_base_seed", 3)))
+        pol_it = make_fixed_seed_iter(int(tr.get("policy_base_seed", 7)))
+        for _ in range(start * bs):
+            next(env_it), next(pol_it)
     for step in range(start, int(tr["num_batches"])):
         t0 = time.perf_counter()
         global_step = step + 1                                                             # 1-based like runner.py:610
-        env.seed = (int(cfg["seed"]) + 0x9E3779B97F4A7C15 * (step + 1)) & (2**64 - 1)      # fresh episodes every batch
-        ro = agent.rollout_many(env, precision=tr.get("precision", "auto"))
+        if streams == "numpy":
+            pairs = [(next(env_it), next(pol_it)) for _ in range(bs)][env.gid0: env.gid0 + env.num_envs]
+            ro = agent.run_episodes(env, [e for e, _ in pairs], [p for _, p in pairs])
+        else:
+            env.seed = (int(cfg["seed"]) + 0x9E3779B97F4A7C15 * (step + 1)) & (2**64 - 1)  # fresh episodes every batch
+            ro = agent.rollout_many(env, precision=tr.get("precision", "auto"))
         total = ro.total_reward()
         avg, mx, mn = _global_stats(total, info)
         hist = tile_histogram(env.max_exp, info)
