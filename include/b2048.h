@@ -341,6 +341,37 @@ int b2048_td_errors(b2048_handle* h, const float* reward, const float* value, co
                     const float* ep_weight, float gamma, int32_t huber, float huber_delta, float n_traj,
                     int32_t T, int64_t B, float* td, float* gcoef, void* stream);
 
+/* ---------------- fixed-horizon windows ----------------
+ * A window is a b2048_rollout_many fixed-horizon rollout with reset-on-done: T steps of B lanes, a lane holds several
+ * episodes.  e[t,b] = (flags[t+1,b] & (B2048_F_DONE | B2048_F_TRUNC)) != 0 ends an episode at step t (boards[t+1] is
+ * the reset board); a truncated episode is not bootstrapped, like update_batch's last step. */
+
+/* Per-lane targets of a window (one thread per lane, float64 recurrence).  rewards [T,B], flags [T+1,B].
+ *   value == NULL (REINFORCE): v = G_t = r_t + gamma (1 - e_t) G_{t+1}; valid_len[b] = 1 + the lane's last boundary (0 if
+ *                none): later slots belong to an episode that does not end in the window, and v is 0 there.
+ *   value [T+1,B] (actor-critic, V(boards[t]) for every slice): td = delta_t = r_t + gamma (1 - e_t) V_{t+1} - V_t (V_T
+ *                bootstraps the cut-off tail); v = A_t = delta_t + gamma lambda (1 - e_t) A_{t+1}; gcoef = dLoss/dV of
+ *                delta (mse, or its Huber clip with huber != 0, _get_grad_logits_critic) / (T n_traj); valid_len = T.
+ * td / gcoef are required with a value and unused without. */
+int b2048_segment_targets(b2048_handle* h, const float* reward, const uint8_t* flags, const float* value, double gamma,
+                          double lambda, int32_t huber, float huber_delta, float n_traj, int32_t T, int64_t B, float* v,
+                          float* td, float* gcoef, int32_t* valid_len, void* stream);
+
+/* b2048_advantages for a window: the samples of lane b are t < valid_len[b] and coef = adv / (T n_traj) (an episode's
+ * length is not known inside a window).  baseline_mode 0 off, 2 batch, 3 batch_norm; stats / stats_precomputed as in
+ * b2048_advantages (b2048_weighted_stats with len = valid_len gives the sums). */
+int b2048_advantages_window(b2048_handle* h, const float* v, const int32_t* valid_len, int32_t baseline_mode, float n_traj,
+                            int32_t T, int64_t B, float* adv, float* coef, double* stats, int32_t stats_precomputed,
+                            void* stream);
+
+/* Episodes completed inside a window, for logging.  ep_return[B] (device double, in/out) carries the undiscounted return
+ * of each lane's running episode from window to window (zero it with the reset).  Each episode that ends in the window
+ * is ADDED into stats (device double[21]) = {count, sum of returns, max (init -inf), min (init +inf), then 17 counts by
+ * the exponent of its max tile}: max(4, the largest tile after its last move, boards[t] with actions[t]), 16 for a
+ * 32768+32768 merge.  boards [T+1,B] (slices 0..T-1 read), actions [T,B]. */
+int b2048_horizon_episodes(b2048_handle* h, const float* reward, const uint8_t* flags, const uint64_t* board,
+                           const uint8_t* action, int32_t T, int64_t B, double* ep_return, double* stats, void* stream);
+
 /* Gradient accumulation of update_batch's actor / critic blocks (reinforce_agent.py:403-555, _backpropagation
  * :639-678) over n samples (flattened [T,B] rollout; samples with coef == 0 contribute nothing).
  * grads is a flat float32 vector laid out W_0, b_0, W_1, b_1, ... and is ACCUMULATED into (zero it first).

@@ -84,6 +84,10 @@ SIGNATURES = {
     "b2048_advantages": [_vp, _vp, _vp, _vp, _i32, _f32, _i32, _i64, _vp, _vp, _vp, _i32, _vp, _vp],
     "b2048_weighted_stats": [_vp, _vp, _vp, _vp, _i32, _i64, _vp, _vp],
     "b2048_td_errors": [_vp, _vp, _vp, _vp, _vp, _f32, _i32, _f32, _f32, _i32, _i64, _vp, _vp, _vp],
+    "b2048_segment_targets": [_vp, _vp, _vp, _vp, C.c_double, C.c_double, _i32, _f32, _f32, _i32, _i64, _vp, _vp, _vp, _vp,
+                              _vp],
+    "b2048_advantages_window": [_vp, _vp, _vp, _i32, _f32, _i32, _i64, _vp, _vp, _vp, _i32, _vp],
+    "b2048_horizon_episodes": [_vp, _vp, _vp, _vp, _vp, _i32, _i64, _vp, _vp, _vp],
     "b2048_backward_workspace_floats": [C.POINTER(MlpDesc), _i64],
     "b2048_mlp_backward": [_vp, _vp, _vp, _vp, _vp, C.POINTER(MlpDesc), _vp, _i64, _i32, _vp, _i64, _i64, _i32, _vp],
     "b2048_backward_tc_layout": [_i64, _vp],

@@ -5,6 +5,9 @@
 //   K5 weighted_stats_kernel     _compute_weighted_stats    src/reinforce_agent.py:864-881
 //      advantage_kernel          _compute_advantages        src/reinforce_agent.py:276-325 (+ the 1/(T n) weight, :533-534)
 //      td_error_kernel           TD(0) targets / errors     src/reinforce_agent.py:439-447, :884-910
+//      segment_targets_kernel    returns / TD / GAE of fixed-horizon windows (episode boundaries inside a lane)
+//      advantage_window_kernel   advantage_kernel with the window's T n_traj divisor
+//      horizon_episodes_kernel   episodes completed inside a window (logging)
 //   K6 mlp_backward_kernel       _backpropagation per tile  src/reinforce_agent.py:639-678 (deltas + activations)
 //      atb_kernel                dW_l = A_l^T D_l           (sum over samples of np.outer, :666)
 //      colsum_kernel             db_l = sum_s D_l
@@ -14,6 +17,7 @@
 // the per-board scans are fully coalesced.
 #include <cuda_runtime.h>
 
+#include "b2048_horizon.cuh"
 #include "b2048_internal.h"
 #include "b2048_mlp.cuh"
 
@@ -132,6 +136,122 @@ __global__ void __launch_bounds__(256) advantage_kernel(const float* __restrict_
         if (adv) adv[i] = a;
         if (coef) coef[i] = cf;
     }
+}
+
+// ------------------------------------------------------------------------------------------------ fixed-horizon windows
+// advantage_kernel's modes 0 / 2 / 3 for a fixed-horizon window: the samples of lane b are t < valid_len[b] and the divisor
+// is T n_traj (an episode's length is not known inside the window).  A kernel of its own so that advantage_kernel's code
+// stays as it is.
+__global__ void __launch_bounds__(256) advantage_window_kernel(const float* __restrict__ v, const int32_t* __restrict__ valid_len,
+                                                                const double* __restrict__ acc, int mode, float n_traj,
+                                                                int T, int64_t B, float* __restrict__ adv,
+                                                                float* __restrict__ coef) {
+    float mean = 0.0f, stdv = 1.0f;
+    if (mode >= 2) {                                         // same statistics as advantage_kernel
+        double sw = acc[0];
+        if (sw >= 1e-8) {
+            double m = acc[1] / sw, var = acc[2] / sw - m * m;
+            mean = (float)m;
+            stdv = (float)sqrt(var > 0.0 ? var : 0.0);
+        }
+        if (stdv < 1e-8f) stdv = 1e-8f;
+    }
+    const float inv = 1.0f / ((float)T * n_traj);
+    const int64_t total = (int64_t)T * B;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
+        const int t = (int)(i / B);
+        float a = 0.0f, cf = 0.0f;
+        if (t < valid_len[i % B]) {
+            const float val = v[i];
+            a = mode == 0 ? val : (mode == 2 ? val - mean : (val - mean) / stdv);
+            cf = a * inv;
+        }
+        adv[i] = a;
+        coef[i] = cf;
+    }
+}
+
+// One thread per lane, reverse in t (segment_lane, b2048_horizon.cuh).
+__global__ void __launch_bounds__(256) segment_targets_kernel(const float* __restrict__ reward, const uint8_t* __restrict__ flags,
+                                                               const float* __restrict__ value, float gamma, double c,
+                                                               int huber, float huber_delta, float inv_div, int T, int64_t B,
+                                                               float* __restrict__ v, float* __restrict__ td,
+                                                               float* __restrict__ gcoef, int32_t* __restrict__ valid_len) {
+    const int64_t b = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (b >= B) return;
+    valid_len[b] = segment_lane(reward + b, flags + b, value ? value + b : nullptr, B, T, gamma, c, huber, huber_delta,
+                                inv_div, v + b, td ? td + b : nullptr, gcoef ? gcoef + b : nullptr);
+}
+
+__device__ __forceinline__ void atomic_max_f64(double* a, double v) {
+    unsigned long long* p = reinterpret_cast<unsigned long long*>(a);
+    unsigned long long old = *p;
+    while (__longlong_as_double(old) < v) {
+        const unsigned long long prev = atomicCAS(p, old, (unsigned long long)__double_as_longlong(v));
+        if (prev == old) break;
+        old = prev;
+    }
+}
+__device__ __forceinline__ void atomic_min_f64(double* a, double v) {
+    unsigned long long* p = reinterpret_cast<unsigned long long*>(a);
+    unsigned long long old = *p;
+    while (__longlong_as_double(old) > v) {
+        const unsigned long long prev = atomicCAS(p, old, (unsigned long long)__double_as_longlong(v));
+        if (prev == old) break;
+        old = prev;
+    }
+}
+
+// Episodes completed inside a window: ep_return[b] carries the undiscounted return of the lane's running episode
+// across windows (float64); at each boundary the episode is added to acc = {count, sum, max, min, hist[17] by max-tile
+// exponent}.  One thread per lane; per block, register / shared-memory partials and one set of global atomics.
+__global__ void __launch_bounds__(256) horizon_episodes_kernel(const float* __restrict__ reward, const uint8_t* __restrict__ flags,
+                                                                const uint64_t* __restrict__ board,
+                                                                const uint8_t* __restrict__ action,
+                                                                const uint16_t* __restrict__ lut_left,
+                                                                const uint8_t* __restrict__ lut_merge, int T, int64_t B,
+                                                                double* __restrict__ ep_return, double* __restrict__ acc) {
+    __shared__ unsigned hist[17];
+    __shared__ double part[4][8];
+    if (threadIdx.x < 17) hist[threadIdx.x] = 0u;
+    __syncthreads();
+    const int64_t b = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    double n = 0.0, sum = 0.0, mx = -INFINITY, mn = INFINITY;
+    if (b < B) {
+        double carry = ep_return[b];
+        for (int t = 0; t < T; ++t) {
+            const int64_t i = (int64_t)t * B + b;
+            carry += (double)reward[i];
+            if (flags[i + B] & (B2048_F_DONE | B2048_F_TRUNC)) {
+                n += 1.0;
+                sum += carry;
+                mx = fmax(mx, carry);
+                mn = fmin(mn, carry);
+                atomicAdd(&hist[final_max_exp(board[i], action[i], lut_left, lut_merge)], 1u);
+                carry = 0.0;
+            }
+        }
+        ep_return[b] = carry;
+    }
+    for (int d = 16; d > 0; d >>= 1) {
+        n += __shfl_down_sync(0xFFFFFFFFu, n, d); sum += __shfl_down_sync(0xFFFFFFFFu, sum, d);
+        mx = fmax(mx, __shfl_down_sync(0xFFFFFFFFu, mx, d)); mn = fmin(mn, __shfl_down_sync(0xFFFFFFFFu, mn, d));
+    }
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    if (lane == 0) { part[0][warp] = n; part[1][warp] = sum; part[2][warp] = mx; part[3][warp] = mn; }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        for (int k = 1; k < 8; ++k) {
+            n += part[0][k]; sum += part[1][k]; mx = fmax(mx, part[2][k]); mn = fmin(mn, part[3][k]);
+        }
+        if (n != 0.0) {
+            atomicAdd(acc + 0, n);
+            atomicAdd(acc + 1, sum);
+            atomic_max_f64(acc + 2, mx);
+            atomic_min_f64(acc + 3, mn);
+        }
+    }
+    if (threadIdx.x < 17 && hist[threadIdx.x] != 0u) atomicAdd(acc + 4 + threadIdx.x, (double)hist[threadIdx.x]);
 }
 
 // per-episode mean of v over t < len (baseline "each", reinforce_agent.py:296-302)
@@ -469,6 +589,58 @@ extern "C" int b2048_td_errors(b2048_handle* h, const float* reward, const float
     B2_REQUIRE(reward && value && td, "b2048_td_errors: NULL buffer");
     td_error_kernel<<<ew_grid((int64_t)T * B, h->num_sms), 256, 0, (cudaStream_t)stream>>>(
         reward, value, len, ep_weight, gamma, huber, huber_delta, n_traj, T, B, td, gcoef);
+    B2_CUDA(cudaGetLastError());
+    return B2048_OK;
+}
+
+extern "C" int b2048_segment_targets(b2048_handle* h, const float* reward, const uint8_t* flags, const float* value,
+                                     double gamma, double lambda, int32_t huber, float huber_delta, float n_traj, int32_t T,
+                                     int64_t B, float* v, float* td, float* gcoef, int32_t* valid_len, void* stream) {
+    B2_REQUIRE(h != nullptr, "b2048_segment_targets: handle is NULL");
+    B2_REQUIRE(T >= 0 && B >= 0, "b2048_segment_targets: negative size");
+    if (T == 0 || B == 0) return B2048_OK;
+    B2_REQUIRE(reward && flags && v && valid_len, "b2048_segment_targets: NULL buffer");
+    B2_REQUIRE(!value || (td && gcoef), "b2048_segment_targets: td and gcoef are required with values");
+    B2_REQUIRE(n_traj > 0.0f, "b2048_segment_targets: n_traj must be positive");
+    const double c = value ? gamma * lambda : gamma;
+    const float inv_div = 1.0f / ((float)T * n_traj);
+    segment_targets_kernel<<<(unsigned)((B + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
+        reward, flags, value, (float)gamma, c, huber, huber_delta, inv_div, T, B, v, value ? td : nullptr,
+        value ? gcoef : nullptr, valid_len);
+    B2_CUDA(cudaGetLastError());
+    return B2048_OK;
+}
+
+extern "C" int b2048_advantages_window(b2048_handle* h, const float* v, const int32_t* valid_len, int32_t baseline_mode,
+                                       float n_traj, int32_t T, int64_t B, float* adv, float* coef, double* stats,
+                                       int32_t stats_precomputed, void* stream) {
+    B2_REQUIRE(h != nullptr, "b2048_advantages_window: handle is NULL");
+    B2_REQUIRE(baseline_mode == 0 || baseline_mode == 2 || baseline_mode == 3,
+               "b2048_advantages_window: baseline mode must be 0 (off), 2 (batch) or 3 (batch_norm)");
+    B2_REQUIRE(T >= 0 && B >= 0, "b2048_advantages_window: negative size");
+    if (T == 0 || B == 0) return B2048_OK;
+    B2_REQUIRE(v && valid_len && stats, "b2048_advantages_window: v/valid_len/stats is NULL");
+    cudaStream_t s = (cudaStream_t)stream;
+    const int64_t total = (int64_t)T * B;
+    if (baseline_mode >= 2 && !stats_precomputed) {
+        B2_CUDA(cudaMemsetAsync(stats, 0, 4 * sizeof(double), s));
+        weighted_stats_kernel<<<ew_grid(total, h->num_sms), 256, 0, s>>>(v, valid_len, nullptr, T, B, stats);
+    }
+    advantage_window_kernel<<<ew_grid(total, h->num_sms), 256, 0, s>>>(v, valid_len, stats, baseline_mode, n_traj, T, B,
+                                                                        adv, coef);
+    B2_CUDA(cudaGetLastError());
+    return B2048_OK;
+}
+
+extern "C" int b2048_horizon_episodes(b2048_handle* h, const float* reward, const uint8_t* flags, const uint64_t* board,
+                                      const uint8_t* action, int32_t T, int64_t B, double* ep_return, double* stats,
+                                      void* stream) {
+    B2_REQUIRE(h != nullptr, "b2048_horizon_episodes: handle is NULL");
+    B2_REQUIRE(T >= 0 && B >= 0, "b2048_horizon_episodes: negative size");
+    if (T == 0 || B == 0) return B2048_OK;
+    B2_REQUIRE(reward && flags && board && action && ep_return && stats, "b2048_horizon_episodes: NULL buffer");
+    horizon_episodes_kernel<<<(unsigned)((B + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
+        reward, flags, board, action, lut_left_ptr(h), lut_merge_ptr(h), T, B, ep_return, stats);
     B2_CUDA(cudaGetLastError());
     return B2048_OK;
 }

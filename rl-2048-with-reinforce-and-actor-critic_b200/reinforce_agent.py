@@ -8,7 +8,8 @@ errors, back-propagation, global-norm clip, SGD / Adam — is a CUDA kernel reac
 
 Added surface: ``rollout_many`` (run-to-termination or fixed-horizon rollouts of a whole
 ``Batched2048Env``) and ``update_from_rollout``; ``update_batch`` packs reference-style trajectories
-into the same rollout buffers and calls the same kernels.
+into the same rollout buffers and calls the same kernels.  ``update_from_horizon`` trains on fixed-horizon
+windows with reset-on-done (segment-aware returns / TD / GAE, ``horizon_episode_stats`` for logging).
 """
 from __future__ import annotations
 
@@ -645,16 +646,7 @@ class ReinforceAgent:
         accumulates g_A (coefficient w v / (T n)) and g_B (coefficient w / (T n)) locally, one float64 message
         [g_A | g_B | critic gradient | sums] is summed over ranks and g = (g_A - mean g_B) / std is formed afterwards.
         It costs a second actor backward pass, which is why it is an opt-in."""
-        prec = 2 if precision == "auto" else int(precision)
-        if exchange not in ("default", "one_message"):
-            raise ValueError(f"Unknown exchange: {exchange}")
-        cfg = self.agent_config
-        if cfg.baseline_mode not in BASELINE:
-            raise ValueError(f"Unknown baseline mode: {cfg.baseline_mode}")          # reinforce_agent.py:325
-        if cfg.optimizer not in OPTIMIZER:
-            raise ValueError(f"Unknown optimizer: {cfg.optimizer}")                  # reinforce_agent.py:582
-        if cfg.use_critic and cfg.critic_loss_type not in ("mse", "huber"):
-            raise ValueError(f"Unknown critic loss type: {cfg.critic_loss_type}")    # reinforce_agent.py:908
+        cfg = self._check_update_config(exchange)
         if ro.B == 0 or ro.T == 0:
             return {}
         if ro.auto_reset:
@@ -663,7 +655,8 @@ class ReinforceAgent:
             # holds several episodes: returns would run across the resets and TD targets would bootstrap from the
             # reset board.  Roll out to termination / truncation instead (horizon=None; max_steps bounds the length).
             raise ValueError("update_from_rollout: fixed-horizon rollouts with reset-on-done hold several episodes per "
-                             "lane and are not a reference-equivalent update batch; use rollout_many(horizon=None)")
+                             "lane and are not a reference-equivalent update batch; use rollout_many(horizon=None), or "
+                             "update_from_horizon for the segment-aware update")
         if ro.ep_weight is None and cfg.reward_rank_weights:
             # global reward ranks on the device (all-gathered over ranks when the episodes are sharded), computed on
             # the ORIGINAL episodes and repeated by the augmentation like the reference (reinforce_agent.py:369-384, :806)
@@ -673,6 +666,107 @@ class ReinforceAgent:
             ro.ep_weight = bd.episode_rank_weights(ro.total_reward(), cfg.reward_rank_weights, dinfo)
         if cfg.augmentation:
             ro = self._augment_rollout(ro)
+        return self._update(ro, False, chunk, allreduce, precision, exchange)
+
+    def update_from_horizon(self, ro: Rollout, allreduce=None, precision: int | str = "auto", chunk: int = 1 << 20,
+                            exchange: str = "default") -> dict[str, Any]:
+        """One policy-gradient update from a fixed-horizon window: a rollout_many(horizon=H) rollout with reset-on-done,
+        whose lanes keep playing across updates (synchronous A2C / REINFORCE on segments).  Episode boundaries inside a lane
+        (flags DONE | TRUNC after step t) restart the returns, TD targets and advantages (b2048_segment_targets; a truncated
+        episode is not bootstrapped, like update_batch's last step):
+          REINFORCE     G_t = r_t + gamma (1 - e_t) G_{t+1}; only the slots of episodes that end inside the window are samples
+                        (the tail after a lane's last boundary is not used);
+          actor-critic  V on all T + 1 slices, delta_t = r_t + gamma (1 - e_t) V(s_{t+1}) - V(s_t), the cut-off tail
+                        bootstrapped from V(boards[T]); A_t = delta_t + gamma lambda (1 - e_t) A_{t+1} (lambda = gae_lambda,
+                        0 = TD(0)); every slot is a sample.
+        Baselines off / batch / batch_norm over the samples; per-sample weight adv / (T n_traj) with n_traj = ro.n_traj (the
+        global lane count under sharding; x8 with augmentation), i.e. the mean over all slots of the window.  Baseline
+        'each', reward_rank_weights (both need whole episodes), exchange='one_message' and rollouts without reset-on-done
+        raise ValueError.  The episodes the window completes are added to horizon_episode_stats().
+        allreduce / precision / chunk as in update_from_rollout."""
+        cfg = self._check_update_config(exchange)
+        if not ro.auto_reset:
+            raise ValueError("update_from_horizon needs a fixed-horizon rollout with reset-on-done (rollout_many(horizon=H))")
+        if cfg.baseline_mode == "each":
+            raise ValueError("baseline 'each' needs whole episodes: not available on fixed-horizon windows")
+        if cfg.reward_rank_weights or ro.ep_weight is not None:
+            raise ValueError("reward rank weights need whole episodes: not available on fixed-horizon windows")
+        if exchange == "one_message":
+            raise ValueError("exchange='one_message' is not implemented for fixed-horizon windows")
+        if ro.B == 0 or ro.T == 0:
+            return {}
+        self._horizon_account(ro)
+        if cfg.augmentation:
+            ro = self._augment_rollout(ro)
+        return self._update(ro, True, chunk, allreduce, precision, exchange)
+
+    def _segment_targets(self, rewards, flags, values, lam, n_traj, v, td, gcoef, valid_len) -> None:
+        cfg = self.agent_config
+        T, B = rewards.shape
+        with torch.cuda.device(self.device):
+            _lib.check(self._lib.b2048_segment_targets(
+                self._h, _ptr(rewards), _ptr(flags), _ptr(values), float(cfg.gamma), float(lam),
+                int(cfg.critic_loss_type == "huber"), float(cfg.huber_delta), float(n_traj), T, B, _ptr(v), _ptr(td),
+                _ptr(gcoef), _ptr(valid_len), _stream()), "b2048_segment_targets")
+
+    def _horizon_account(self, ro: Rollout) -> None:
+        """Adds the episodes that end inside the window to the device sums behind horizon_episode_stats; each lane's
+        running return is carried to the next window (windows of one set of envs follow each other: a different lane
+        count starts the carries from zero)."""
+        carry = getattr(self, "_hz_carry", None)
+        if carry is None or carry.numel() != ro.B:
+            self._hz_carry = carry = torch.zeros(ro.B, dtype=torch.float64, device=self.device)
+        if getattr(self, "_hz_stats", None) is None:
+            self._hz_stats = torch.zeros(21, dtype=torch.float64, device=self.device)
+            self._hz_stats[2:4] = torch.tensor([-np.inf, np.inf], dtype=torch.float64)
+        with torch.cuda.device(self.device):
+            _lib.check(self._lib.b2048_horizon_episodes(
+                self._h, _ptr(ro.rewards[: ro.T].contiguous()), _ptr(ro.flags[: ro.T + 1].contiguous()),
+                _ptr(ro.boards[: ro.T + 1].contiguous()), _ptr(ro.actions[: ro.T].contiguous()), ro.T, ro.B, _ptr(carry),
+                _ptr(self._hz_stats), _stream()), "b2048_horizon_episodes")
+
+    def horizon_episode_stats(self, reset: bool = True, info=None) -> dict[str, Any]:
+        """The episodes completed by the windows update_from_horizon consumed since the last reset:
+        {episodes, avg_reward, max_reward, min_reward, max_tile_counts} with the undiscounted episode returns and the
+        episodes per max tile in trainer.TILE_BINS order (16 .. 4096).  Stats of no episode are NaN.  info (a dist.DistInfo
+        with world_size > 1): summed / maxed over ranks."""
+        st = getattr(self, "_hz_stats", None)
+        if st is None:
+            st = torch.tensor([0.0, 0.0, -np.inf, np.inf] + [0.0] * 17, dtype=torch.float64, device=self.device)
+        st = st.clone()
+        if info is not None and info.is_distributed:
+            from . import dist as bd
+            sums = torch.cat([st[:2], st[4:]])
+            ext = torch.stack([st[2], -st[3]])
+            bd.allreduce_sum_(sums)
+            bd.allreduce_max_(ext)
+            st = torch.cat([sums[:2], ext[:1], -ext[1:], sums[2:]])
+        h = st.cpu().numpy()
+        n = int(h[0])
+        if reset and getattr(self, "_hz_stats", None) is not None:
+            self._hz_stats.zero_()
+            self._hz_stats[2:4] = torch.tensor([-np.inf, np.inf], dtype=torch.float64)
+        nan = float("nan")
+        return {"episodes": n, "avg_reward": float(h[1] / n) if n else nan, "max_reward": float(h[2]) if n else nan,
+                "min_reward": float(h[3]) if n else nan, "max_tile_counts": [int(c) for c in h[4 + 4: 4 + 13]]}
+
+    def _check_update_config(self, exchange: str) -> ReinforceAgentConfig:
+        if exchange not in ("default", "one_message"):
+            raise ValueError(f"Unknown exchange: {exchange}")
+        cfg = self.agent_config
+        if cfg.baseline_mode not in BASELINE:
+            raise ValueError(f"Unknown baseline mode: {cfg.baseline_mode}")          # reinforce_agent.py:325
+        if cfg.optimizer not in OPTIMIZER:
+            raise ValueError(f"Unknown optimizer: {cfg.optimizer}")                  # reinforce_agent.py:582
+        if cfg.use_critic and cfg.critic_loss_type not in ("mse", "huber"):
+            raise ValueError(f"Unknown critic loss type: {cfg.critic_loss_type}")    # reinforce_agent.py:908
+        return cfg
+
+    def _update(self, ro: Rollout, window: bool, chunk: int, allreduce, precision: int | str, exchange: str) -> dict[str, Any]:
+        """The body of update_from_rollout (window=False: one episode per lane, t < length) and update_from_horizon
+        (window=True: a fixed-horizon window, targets from b2048_segment_targets)."""
+        prec = 2 if precision == "auto" else int(precision)
+        cfg = self.agent_config
         T, B = ro.T, ro.B
         n_traj = float(ro.n_traj if ro.n_traj is not None else B)
         lib, h, dev = self._lib, self._h, self.device
@@ -681,7 +775,19 @@ class ReinforceAgent:
         mflags = ro.flags[:T].reshape(-1)
         acts = ro.actions[:T].reshape(-1)
         rewards = ro.rewards[:T].contiguous()
+        critic = cfg.use_critic and self._critic is not None
+        lam = float(getattr(self, "gae_lambda", 0.0))            # shared_trunk.py; 0 = the reference's TD(0) advantages
         length = ro.length
+        if window:
+            # the samples of lane b are t < valid_len[b]: every slot with a critic, else the slots of the episodes that end
+            # inside the window (known from the flags alone, before the compaction below)
+            length = self._buf("valid_len", (B,), torch.int32)
+            flags_w = ro.flags[: T + 1].contiguous()
+            if critic:
+                length.fill_(T)
+            else:
+                returns = self._buf("returns", (T, B), torch.float32)
+                self._segment_targets(rewards, flags_w, None, lam, n_traj, returns, None, None, length)
         # Run-to-termination rollouts are ragged: slots with t >= len[b] carry no sample.  The per-sample work
         # (forward / backward GEMMs) runs on the compacted list of live slots; the [T, B] grid is kept only for
         # the per-episode time recurrences (returns scan, TD shift).  Pure index plumbing (torch).
@@ -711,6 +817,10 @@ class ReinforceAgent:
                                                         _ptr(stats), _stream()), "b2048_weighted_stats")
                     allreduce(stats)
                     pre = 1
+                if window:
+                    _lib.check(lib.b2048_advantages_window(h, _ptr(values), _ptr(length), mode, n_traj, T, B, _ptr(adv),
+                                                           _ptr(coef), _ptr(stats), pre, _stream()), "b2048_advantages_window")
+                    return
                 _lib.check(lib.b2048_advantages(h, _ptr(values), _ptr(length), _ptr(ro.ep_weight), mode, n_traj, T, B,
                                                 _ptr(adv), _ptr(coef), _ptr(stats), pre, _ptr(ep_mean), _stream()),
                            "b2048_advantages")
@@ -744,41 +854,50 @@ class ReinforceAgent:
                                                   int(t_adam), _ptr(sumsq), _stream()), "b2048_apply_update")
             return sumsq
 
-        if cfg.use_critic and self._critic is not None:
+        if critic:
             # critic block (reinforce_agent.py:403-498): V(s_t) for every stored state, TD(0) errors, critic grads
-            values = self._buf("values", (T, B), torch.float32)
+            # (a window also evaluates V(boards[T]), which bootstraps the cut-off tail; none of its slots is compacted)
+            nv = T + 1 if window else T
+            vboards = ro.boards[:nv].reshape(-1) if window else boards
+            values = self._buf("values", (nv, B), torch.float32)
             vc = values.view(-1) if live is None else self._buf("values_c", (n,), torch.float32)
-            self._values(boards, vc, prec)
+            self._values(vboards, vc, prec)
             if prec in (2, 3) and not bool(torch.isfinite(vc).all()):        # fp16 range exceeded in the value forward
                 fell_back.append(1)
-                self._values(boards, vc, 0)
+                self._values(vboards, vc, 0)
             if live is not None:
                 values.zero_()
                 values.view(-1)[live] = vc
             td = self._buf("td", (T, B), torch.float32)
             gcoef = self._buf("gcoef", (T, B), torch.float32)
-            with torch.cuda.device(dev):
-                _lib.check(lib.b2048_td_errors(h, _ptr(rewards), _ptr(values), _ptr(length), _ptr(ro.ep_weight),
-                                               float(cfg.gamma), int(cfg.critic_loss_type == "huber"),
-                                               float(cfg.huber_delta), n_traj, T, B, _ptr(td), _ptr(gcoef), _stream()),
-                           "b2048_td_errors")
+            if window:                                               # TD errors and A_t = delta_t + gamma lambda A_{t+1}
+                gae = self._buf("gae", (T, B), torch.float32)
+                self._segment_targets(rewards, flags_w, values, lam, n_traj, gae, td, gcoef, length)
+            else:
+                with torch.cuda.device(dev):
+                    _lib.check(lib.b2048_td_errors(h, _ptr(rewards), _ptr(values), _ptr(length), _ptr(ro.ep_weight),
+                                                   float(cfg.gamma), int(cfg.critic_loss_type == "huber"),
+                                                   float(cfg.huber_delta), n_traj, T, B, _ptr(td), _ptr(gcoef), _stream()),
+                               "b2048_td_errors")
             backward(self._critic, gcoef.reshape(-1), 1)
-            base_values = td                                         # advantages := baseline-processed TD errors (:495-498)
+            base_values = gae if window else td                      # advantages := baseline-processed TD errors (:495-498)
             info["td"] = td
-            lam = float(getattr(self, "gae_lambda", 0.0))            # shared_trunk.py; 0 = the reference's TD(0) advantages
-            if lam > 0.0:
+            if lam > 0.0 and not window:
                 gae = self._buf("gae", (T, B), torch.float32)        # A_t = delta_t + gamma lambda A_{t+1}: the returns scan
                 with torch.cuda.device(dev):
                     _lib.check(lib.b2048_reverse_scan_f64(_ptr(td), _ptr(gae), _ptr(length), float(cfg.gamma) * lam, T, B,
                                                           _stream()), "b2048_reverse_scan_f64")
                 base_values = gae
         else:
-            returns = self._buf("returns", (T, B), torch.float32)
-            with torch.cuda.device(dev):
-                _lib.check(lib.b2048_reverse_scan_f64(_ptr(rewards), _ptr(returns), _ptr(length), float(cfg.gamma), T, B,
-                                                      _stream()), "b2048_reverse_scan_f64")
+            if not window:
+                returns = self._buf("returns", (T, B), torch.float32)
+                with torch.cuda.device(dev):
+                    _lib.check(lib.b2048_reverse_scan_f64(_ptr(rewards), _ptr(returns), _ptr(length), float(cfg.gamma), T, B,
+                                                          _stream()), "b2048_reverse_scan_f64")
             base_values = returns
             info["returns"] = returns
+        if window:
+            info["valid_len"] = length
         shared = getattr(self, "_shared_net", None)                  # shared_trunk.py: one network, two heads, one optimizer
         if one_msg and shared is not None:
             raise ValueError("exchange='one_message' is implemented for separate actor / critic networks")

@@ -52,7 +52,8 @@ def transform_flags(flags: torch.Tensor, variant: int) -> torch.Tensor:
 
 def augment_rollout(ro):
     """Rollout with 8x the episodes (every dihedral variant), weights repeated, n_traj = 8 x the caller's n_traj (the
-    GLOBAL episode count when the episodes are sharded over ranks; B when it was not set)."""
+    GLOBAL episode count when the episodes are sharded over ranks; B when it was not set).  A fixed-horizon window stays
+    one (auto_reset is kept: the DONE / TRUNC flag bits travel with the boards)."""
     import ctypes as C
     from . import _lib
     from .batched_env import get_handle
@@ -74,4 +75,5 @@ def augment_rollout(ro):
     rewards = ro.rewards.repeat(1, 8)
     length = ro.length.repeat(8)
     w = None if ro.ep_weight is None else ro.ep_weight.repeat(8)
-    return Rollout(boards, flags, actions, rewards.contiguous(), length, T, w, 8 * (ro.n_traj if ro.n_traj is not None else B))
+    return Rollout(boards, flags, actions, rewards.contiguous(), length, T, w, 8 * (ro.n_traj if ro.n_traj is not None else B),
+                   ro.auto_reset)

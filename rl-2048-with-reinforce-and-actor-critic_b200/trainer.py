@@ -12,6 +12,11 @@ own seeded episodes — episode i of batch k plays run_episode(env_seed, policy_
 of make_fixed_seed_iter(``train.env_base_seed``) / make_fixed_seed_iter(``train.policy_base_seed``), the order
 runner.py:587-608 draws them, on the fp32 policy kernel; evaluation keeps the Philox streams), ``train.precision`` ("auto" | 0 | 1), ``train.exchange`` ("default" | "one_message": one all-reduce per update),
 ``seed``, and an optional section ``shared_trunk`` ({"value_coef", "gae_lambda"}: one network with a policy and a value head).  Under torchrun the episodes are sharded over ranks.
+``train.horizon`` (default None: the batches above): an integer H trains on fixed-horizon windows instead — the
+``train.batch_size`` envs are reset once and keep playing (reset-on-done); each batch is ``rollout_many(horizon=H,
+reset=False)`` followed by one ``update_from_horizon`` (segment-aware returns / TD / GAE, the cut-off tail bootstrapped by
+the critic when there is one).  The CSV rows then describe the episodes that ended inside the batch's window (NaN stats
+and zero counts when none did); a resumed run starts from fresh resets.  Not combinable with ``seed_streams="numpy"``.
 
     python -m torch.distributed.run ... b2048_runner.py -conf cfg.json      (or: python b2048_runner.py -conf cfg.json)
 """
@@ -98,6 +103,13 @@ def _global_stats(values: torch.Tensor, info: bd.DistInfo):
 def training(cfg: dict[str, Any], info: bd.DistInfo | None = None, device=None, log=print) -> list[dict[str, Any]]:
     info = info or bd.DistInfo()
     tr = cfg["train"]
+    horizon = tr.get("horizon")
+    if horizon is not None:
+        horizon = int(horizon)
+        if horizon < 1:
+            raise ValueError(f"train.horizon must be a positive number of steps, got {horizon}")
+        if tr.get("seed_streams", "philox") == "numpy":
+            raise ValueError("train.horizon needs seed_streams='philox': the reference-seeded episodes play to termination")
     env, agent = build(cfg, int(tr["batch_size"]), info, device)
     out_dir = tr.get("out_dir")
     rows: list[dict[str, Any]] = []
@@ -124,6 +136,8 @@ def training(cfg: dict[str, Any], info: bd.DistInfo | None = None, device=None, 
     streams = tr.get("seed_streams", "philox")
     if streams not in ("philox", "numpy"):
         raise ValueError(f"Unknown train.seed_streams: {streams}")
+    if horizon is not None:
+        env.reset_many(seed=(int(cfg["seed"]) + 0x9E3779B97F4A7C15 * (start + 1)) & (2**64 - 1))
     if streams == "numpy":
         # the runner's seed iterators, advanced past the batches already played; this rank plays its contiguous slice
         # [gid0, gid0 + num_envs) of every batch's global seed list, so the episodes do not depend on the world size
@@ -135,24 +149,31 @@ def training(cfg: dict[str, Any], info: bd.DistInfo | None = None, device=None, 
     for step in range(start, int(tr["num_batches"])):
         t0 = time.perf_counter()
         global_step = step + 1                                                             # 1-based like runner.py:610
-        if streams == "numpy":
+        if horizon is not None:
+            row, ro, upd = _horizon_batch(agent, env, info, tr, horizon, global_step, best, out_dir)
+            avg, mx, mn = row["avg_reward"], row["max_reward"], row["min_reward"]
+            if avg > best:
+                best = avg
+            rows.append(dict(row, steps=ro.T * ro.B, seconds=time.perf_counter() - t0, grad_norm=upd.get("actor_grad_norm")))
+        elif streams == "numpy":
             pairs = [(next(env_it), next(pol_it)) for _ in range(bs)][env.gid0: env.gid0 + env.num_envs]
             ro = agent.run_episodes(env, [e for e, _ in pairs], [p for _, p in pairs])
         else:
             env.seed = (int(cfg["seed"]) + 0x9E3779B97F4A7C15 * (step + 1)) & (2**64 - 1)  # fresh episodes every batch
             ro = agent.rollout_many(env, precision=tr.get("precision", "auto"))
-        total = ro.total_reward()
-        avg, mx, mn = _global_stats(total, info)
-        hist = tile_histogram(env.max_exp, info)
-        is_record = avg > best                                                             # runner.py:643-660
-        if is_record:
-            best = avg
-        if global_step > 30 and is_record and info.rank == 0 and out_dir:
-            agent.save_model(os.path.join(out_dir, f"best_avg_{avg:.2f}_step_{global_step}.npz"))
-        upd = bd.sharded_update(agent, ro, info, total_episodes=int(tr["batch_size"]), exchange=tr.get("exchange", "default"))
-        row = {"batch": global_step, "avg_reward": avg, "max_reward": mx, "min_reward": mn, "max_tile_counts": json.dumps(hist)}
-        rows.append(dict(row, steps=int(ro.length.sum().item()), seconds=time.perf_counter() - t0,
-                         grad_norm=upd.get("actor_grad_norm")))
+        if horizon is None:
+            total = ro.total_reward()
+            avg, mx, mn = _global_stats(total, info)
+            hist = tile_histogram(env.max_exp, info)
+            is_record = avg > best                                                         # runner.py:643-660
+            if is_record:
+                best = avg
+            if global_step > 30 and is_record and info.rank == 0 and out_dir:
+                agent.save_model(os.path.join(out_dir, f"best_avg_{avg:.2f}_step_{global_step}.npz"))
+            upd = bd.sharded_update(agent, ro, info, total_episodes=int(tr["batch_size"]), exchange=tr.get("exchange", "default"))
+            row = {"batch": global_step, "avg_reward": avg, "max_reward": mx, "min_reward": mn, "max_tile_counts": json.dumps(hist)}
+            rows.append(dict(row, steps=int(ro.length.sum().item()), seconds=time.perf_counter() - t0,
+                             grad_norm=upd.get("actor_grad_norm")))
         if writer:
             writer.writerow(row)
             fcsv.flush()
@@ -168,6 +189,27 @@ def training(cfg: dict[str, Any], info: bd.DistInfo | None = None, device=None, 
         agent.save_model(os.path.join(out_dir, "final.npz"))
         agent.save_checkpoint(os.path.join(out_dir, "final_checkpoint.npz"))
     return rows
+
+
+def _horizon_batch(agent, env, info: bd.DistInfo, tr: dict[str, Any], horizon: int, global_step: int, best: float,
+                   out_dir: str | None):
+    """One fixed-horizon batch: the window, its update, and the CSV row of the episodes that ended inside it (over all
+    ranks).  A record average is checkpointed with the parameters that played the window, as the episode batches are."""
+    ro = agent.rollout_many(env, horizon=horizon, reset=False, precision=tr.get("precision", "auto"))
+    saving = global_step > 30 and info.rank == 0 and bool(out_dir)
+    before = agent.save_state() if saving else None
+    upd = bd.sharded_update(agent, ro, info, total_episodes=int(tr["batch_size"]), exchange=tr.get("exchange", "default"),
+                            fixed_horizon=True)
+    es = agent.horizon_episode_stats(reset=True, info=info)
+    avg = es["avg_reward"]
+    if saving and avg > best:                                                              # runner.py:643-660
+        after = agent.save_state()
+        agent.load_state(before)
+        agent.save_model(os.path.join(out_dir, f"best_avg_{avg:.2f}_step_{global_step}.npz"))
+        agent.load_state(after)
+    row = {"batch": global_step, "avg_reward": avg, "max_reward": es["max_reward"], "min_reward": es["min_reward"],
+           "max_tile_counts": json.dumps(es["max_tile_counts"])}
+    return row, ro, upd
 
 
 def evaluation(cfg: dict[str, Any], info: bd.DistInfo | None = None, device=None, agent=None) -> dict[str, Any]:
