@@ -372,6 +372,26 @@ int b2048_advantages_window(b2048_handle* h, const float* v, const int32_t* vali
 int b2048_horizon_episodes(b2048_handle* h, const float* reward, const uint8_t* flags, const uint64_t* board,
                            const uint8_t* action, int32_t T, int64_t B, double* ep_return, double* stats, void* stream);
 
+/* Bootstrapping at truncation.  A TRUNC flag ends an episode only because the step budget ran out, so the episode's last
+ * target is r + gamma V(s'), with s' the board the episode was cut on.
+ *
+ * b2048_replay_pre_reset: s' of a fixed-horizon window played with auto-reset (where boards[t + 1] already holds the reset
+ * board).  For each listed slot s = t * B + b of the [T, B] window, out[k] = the board after actions[s] on boards[s] and the
+ * Philox spawn of (seed, gid0 + b, t0 + t + 1) -- the counter b2048_rollout_many used for that step -- with no spawn when
+ * the move changed nothing.  It is the step body with auto-reset off, so it equals b2048_step_many on the same inputs.
+ * boards [T+1, B], actions [T, B], slots [K] (device, int64, each >= 0 and < T * B), out [K] (device).  The slot list is
+ * checked on the host: the call waits for `stream`.
+ *
+ * b2048_fold_bootstrap: reward_out[i] = reward[i] for i in [0, n), except reward_out[slots[k]] = reward[slots[k]] +
+ * gamma * value[k] with the multiply and the add rounded separately.  Fed to b2048_segment_targets or b2048_td_errors,
+ * whose target at an episode's last step is r + gamma * 0, this gives the bootstrapped target, TD error, advantage and
+ * critic coefficient bit for bit.  slots [K] distinct and in [0, n) (checked on the host: the call waits for `stream`);
+ * reward_out may be reward. */
+int b2048_replay_pre_reset(b2048_handle* h, const uint64_t* boards, const uint8_t* actions, const int64_t* slots, int64_t K,
+                           int64_t B, uint64_t seed, uint64_t gid0, uint32_t t0, uint64_t* out, void* stream);
+int b2048_fold_bootstrap(b2048_handle* h, const float* reward, const int64_t* slots, const float* value, int64_t K, int64_t n,
+                         float gamma, float* reward_out, void* stream);
+
 /* Gradient accumulation of update_batch's actor / critic blocks (reinforce_agent.py:403-555, _backpropagation
  * :639-678) over n samples (flattened [T,B] rollout; samples with coef == 0 contribute nothing).
  * grads is a flat float32 vector laid out W_0, b_0, W_1, b_1, ... and is ACCUMULATED into (zero it first).

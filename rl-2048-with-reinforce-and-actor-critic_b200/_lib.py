@@ -88,6 +88,8 @@ SIGNATURES = {
                               _vp],
     "b2048_advantages_window": [_vp, _vp, _vp, _i32, _f32, _i32, _i64, _vp, _vp, _vp, _i32, _vp],
     "b2048_horizon_episodes": [_vp, _vp, _vp, _vp, _vp, _i32, _i64, _vp, _vp, _vp],
+    "b2048_replay_pre_reset": [_vp, _vp, _vp, _vp, _i64, _i64, _u64, _u64, _u32, _vp, _vp],
+    "b2048_fold_bootstrap": [_vp, _vp, _vp, _vp, _i64, _i64, _f32, _vp, _vp],
     "b2048_backward_workspace_floats": [C.POINTER(MlpDesc), _i64],
     "b2048_mlp_backward": [_vp, _vp, _vp, _vp, _vp, C.POINTER(MlpDesc), _vp, _i64, _i32, _vp, _i64, _i64, _i32, _vp],
     "b2048_backward_tc_layout": [_i64, _vp],

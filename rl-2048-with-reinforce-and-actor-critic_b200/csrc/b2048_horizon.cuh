@@ -13,9 +13,17 @@
 // B2_HD so that tests/host_check compiles the recurrence with g++ (-ffp-contract=off) and compares it bit for bit with a
 // NumPy float64 restatement: the float32 TD arithmetic uses separately rounded operations (no FMA contraction) on both
 // sides, the recurrence runs in float64 like reverse_scan_kernel.
+//
+// Bootstrapping at truncation (opt-in, ReinforceAgent.update_from_horizon / update_from_rollout(bootstrap_truncation=True)):
+// a TRUNC boundary ends an episode only because the step budget ran out, so its target is r + gamma V(s') with s' the
+// board the episode was cut on.  fold_bootstrap folds gamma V(s') into a copy of the rewards; segment_lane (vn = 0 at a
+// boundary: r' + gamma 0 == r' exactly) then computes every target, TD error, GAE term and gcoef bit for bit as with
+// vn = V(s') at that boundary.  s' is gone from a reset-on-done window (boards[t + 1] is the reset board), but spawns are
+// counter-based: pre_reset_board replays it from (boards[t], actions[t], seed, gid, t_env) with step_one itself.
 #pragma once
 #include "../../include/b2048.h"
 #include "b2048_device.cuh"
+#include "b2048_step.cuh"
 
 namespace b2 {
 
@@ -75,6 +83,27 @@ B2_HD int segment_lane(const float* reward, const uint8_t* flags, const float* v
         v[i] = (value || t < valid) ? (float)G : 0.0f;
     }
     return valid;
+}
+
+// The bootstrapped reward of a truncated episode's last step: r + gamma V(s'), each operation rounded separately.
+B2_HD float fold_bootstrap(float r, float gamma, float v_next) { return f32_add(r, f32_mul(gamma, v_next)); }
+
+// The board after `a` on `board` at env counter t_env of lane gid, before an auto-reset replaced it: the move, then the
+// Philox spawn of (seed, gid, t_env) when the move changed the board.  step_one with auto-reset off computes exactly that;
+// counters, rewards and flags are not needed.
+template <typename LutL, typename LutM>
+B2_HD uint64_t pre_reset_board(uint64_t board, uint32_t a, uint64_t seed, uint64_t gid, uint32_t t_env, LutL lut_left,
+                               LutM lut_merge) {
+    b2048_env_cfg cfg = {};
+    cfg.action_mode = B2048_ACT_BUFFER;
+    cfg.use_action_mask = 1;
+    StepIO io = {};
+    io.board = make_board(board);
+    io.max_exp = 2u;
+    io.action = a;
+    const StepOpts opt = {false, false, false};
+    step_one(io, cfg, opt, seed, gid, t_env, lut_left, lut_merge);
+    return to_u64(io.board);
 }
 
 // The largest tile of an episode that ended with the move `a` on `board` (max_tile_seen): every tile >= 8 came from a

@@ -8,6 +8,8 @@
 //      segment_targets_kernel    returns / TD / GAE of fixed-horizon windows (episode boundaries inside a lane)
 //      advantage_window_kernel   advantage_kernel with the window's T n_traj divisor
 //      horizon_episodes_kernel   episodes completed inside a window (logging)
+//      replay_pre_reset_kernel   the boards truncated episodes were cut on (bootstrapping at truncation)
+//      fold_bootstrap_kernel     r + gamma V(s') at the truncated slots of a copy of the rewards
 //   K6 mlp_backward_kernel       _backpropagation per tile  src/reinforce_agent.py:639-678 (deltas + activations)
 //      atb_kernel                dW_l = A_l^T D_l           (sum over samples of np.outer, :666)
 //      colsum_kernel             db_l = sum_s D_l
@@ -16,6 +18,8 @@
 // Rollout buffers are time-major [T, B] (board index contiguous) so that every per-step kernel and
 // the per-board scans are fully coalesced.
 #include <cuda_runtime.h>
+
+#include <vector>
 
 #include "b2048_horizon.cuh"
 #include "b2048_internal.h"
@@ -252,6 +256,43 @@ __global__ void __launch_bounds__(256) horizon_episodes_kernel(const float* __re
         }
     }
     if (threadIdx.x < 17 && hist[threadIdx.x] != 0u) atomicAdd(acc + 4 + threadIdx.x, (double)hist[threadIdx.x]);
+}
+
+// One thread per listed slot s = t B + b of a window: the board lane b was cut on by step t (pre_reset_board: step_one
+// with auto-reset off at the rollout's counter t0 + t + 1).
+__global__ void __launch_bounds__(256) replay_pre_reset_kernel(const uint64_t* __restrict__ board, const uint8_t* __restrict__ action,
+                                                                const int64_t* __restrict__ slots, int64_t K, int64_t B,
+                                                                uint64_t seed, uint64_t gid0, uint32_t t0,
+                                                                const uint16_t* __restrict__ lut_left,
+                                                                const uint8_t* __restrict__ lut_merge, uint64_t* __restrict__ out) {
+    const int64_t k = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= K) return;
+    const int64_t s = slots[k];
+    const int64_t t = s / B, b = s - t * B;
+    out[k] = pre_reset_board(board[s], action[s], seed, gid0 + (uint64_t)b, t0 + (uint32_t)t + 1u, lut_left, lut_merge);
+}
+
+// out[slots[k]] = reward[slots[k]] + gamma value[k] (fold_bootstrap); the other elements are copied by the launcher.
+// (reward and out may be the same buffer)
+__global__ void __launch_bounds__(256) fold_bootstrap_kernel(const float* reward, const int64_t* __restrict__ slots,
+                                                              const float* __restrict__ value, int64_t K, float gamma, float* out) {
+    const int64_t k = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= K) return;
+    const int64_t s = slots[k];
+    out[s] = fold_bootstrap(reward[s], gamma, value[k]);
+}
+
+// The slot list lives on the device: copy it to the host and check every index against [lo, hi).
+static int check_slots(const int64_t* slots, int64_t K, int64_t lo, int64_t hi, cudaStream_t s, const char* who) {
+    std::vector<int64_t> host((size_t)K);
+    B2_CUDA(cudaMemcpyAsync(host.data(), slots, (size_t)K * sizeof(int64_t), cudaMemcpyDefault, s));
+    B2_CUDA(cudaStreamSynchronize(s));
+    for (int64_t k = 0; k < K; ++k)
+        if (host[(size_t)k] < lo || host[(size_t)k] >= hi)
+            return fail(B2048_ERR_INVALID, std::string(who) + ": slot " + std::to_string(host[(size_t)k]) + " at index " +
+                                               std::to_string(k) + " is outside [" + std::to_string(lo) + ", " +
+                                               std::to_string(hi) + ")");
+    return B2048_OK;
 }
 
 // per-episode mean of v over t < len (baseline "each", reinforce_agent.py:296-302)
@@ -641,6 +682,42 @@ extern "C" int b2048_horizon_episodes(b2048_handle* h, const float* reward, cons
     B2_REQUIRE(reward && flags && board && action && ep_return && stats, "b2048_horizon_episodes: NULL buffer");
     horizon_episodes_kernel<<<(unsigned)((B + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
         reward, flags, board, action, lut_left_ptr(h), lut_merge_ptr(h), T, B, ep_return, stats);
+    B2_CUDA(cudaGetLastError());
+    return B2048_OK;
+}
+
+extern "C" int b2048_replay_pre_reset(b2048_handle* h, const uint64_t* boards, const uint8_t* actions, const int64_t* slots,
+                                      int64_t K, int64_t B, uint64_t seed, uint64_t gid0, uint32_t t0, uint64_t* out,
+                                      void* stream) {
+    B2_REQUIRE(h != nullptr, "b2048_replay_pre_reset: handle is NULL");
+    B2_REQUIRE(K >= 0 && B >= 0, "b2048_replay_pre_reset: negative size");
+    if (K == 0) return B2048_OK;
+    B2_REQUIRE(B > 0, "b2048_replay_pre_reset: slots listed for a window of no lanes");
+    B2_REQUIRE(boards && actions && slots && out, "b2048_replay_pre_reset: NULL buffer");
+    cudaStream_t s = (cudaStream_t)stream;
+    // the window's length is not an argument: only the lower bound of the slots can be checked
+    int st = check_slots(slots, K, 0, INT64_MAX, s, "b2048_replay_pre_reset");
+    if (st != B2048_OK) return st;
+    replay_pre_reset_kernel<<<(unsigned)((K + 255) / 256), 256, 0, s>>>(boards, actions, slots, K, B, seed, gid0, t0,
+                                                                          lut_left_ptr(h), lut_merge_ptr(h), out);
+    B2_CUDA(cudaGetLastError());
+    return B2048_OK;
+}
+
+extern "C" int b2048_fold_bootstrap(b2048_handle* h, const float* reward, const int64_t* slots, const float* value, int64_t K,
+                                    int64_t n, float gamma, float* reward_out, void* stream) {
+    B2_REQUIRE(h != nullptr, "b2048_fold_bootstrap: handle is NULL");
+    B2_REQUIRE(K >= 0 && n >= 0, "b2048_fold_bootstrap: negative size");
+    if (n == 0 && K == 0) return B2048_OK;
+    B2_REQUIRE(reward && reward_out && (K == 0 || (slots && value)), "b2048_fold_bootstrap: NULL buffer");
+    cudaStream_t s = (cudaStream_t)stream;
+    if (K > 0) {
+        int st = check_slots(slots, K, 0, n, s, "b2048_fold_bootstrap");
+        if (st != B2048_OK) return st;
+    }
+    if (reward_out != reward) B2_CUDA(cudaMemcpyAsync(reward_out, reward, (size_t)n * sizeof(float), cudaMemcpyDeviceToDevice, s));
+    if (K > 0)
+        fold_bootstrap_kernel<<<(unsigned)((K + 255) / 256), 256, 0, s>>>(reward, slots, value, K, gamma, reward_out);
     B2_CUDA(cudaGetLastError());
     return B2048_OK;
 }

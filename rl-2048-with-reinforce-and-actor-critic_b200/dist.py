@@ -125,13 +125,14 @@ def make_sharded_env(total_boards: int, config, info: DistInfo, seed: int = 0, d
 
 
 def sharded_update(agent, rollout, info: DistInfo, total_episodes: int | None = None, precision="auto",
-                   exchange: str = "default", fixed_horizon: bool = False):
+                   exchange: str = "default", fixed_horizon: bool = False, bootstrap_truncation: bool = False):
     """update_from_rollout with gradients / baseline sums all-reduced over ranks; n_traj = global episode count
     so that every rank applies exactly the update a single process holding all episodes would apply.
     exchange="one_message": exactly one all-reduce per update (see ReinforceAgent.update_from_rollout); pass
     total_episodes as well, otherwise the episode count is one more (8-byte) collective.
     fixed_horizon=True: update_from_horizon on a fixed-horizon window; total_episodes is then the global lane count, the
-    per-sample weight 1 / (T n_traj) needs no further exchange (the 32-byte baseline sums, then one gradient all-reduce)."""
+    per-sample weight 1 / (T n_traj) needs no further exchange (the 32-byte baseline sums, then one gradient all-reduce).
+    bootstrap_truncation: passed to the update; it adds no message (the boards are replayed from global ids, V(s') is local)."""
     if total_episodes is None:
         n = torch.tensor([rollout.B], dtype=torch.int64, device=rollout.length.device)
         allreduce_sum_(n)
@@ -139,9 +140,9 @@ def sharded_update(agent, rollout, info: DistInfo, total_episodes: int | None = 
     rollout.n_traj = total_episodes
     if fixed_horizon:
         return agent.update_from_horizon(rollout, allreduce=allreduce_sum_ if info.is_distributed else None,
-                                         precision=precision, exchange=exchange)
+                                         precision=precision, exchange=exchange, bootstrap_truncation=bootstrap_truncation)
     return agent.update_from_rollout(rollout, allreduce=allreduce_sum_ if info.is_distributed else None, precision=precision,
-                                     exchange=exchange)
+                                     exchange=exchange, bootstrap_truncation=bootstrap_truncation)
 
 
 def episode_rank_weights(total_reward: torch.Tensor, weights_conf, info: DistInfo | None = None) -> torch.Tensor:

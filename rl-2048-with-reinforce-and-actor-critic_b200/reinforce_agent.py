@@ -9,7 +9,8 @@ errors, back-propagation, global-norm clip, SGD / Adam — is a CUDA kernel reac
 Added surface: ``rollout_many`` (run-to-termination or fixed-horizon rollouts of a whole
 ``Batched2048Env``) and ``update_from_rollout``; ``update_batch`` packs reference-style trajectories
 into the same rollout buffers and calls the same kernels.  ``update_from_horizon`` trains on fixed-horizon
-windows with reset-on-done (segment-aware returns / TD / GAE, ``horizon_episode_stats`` for logging).
+windows with reset-on-done (segment-aware returns / TD / GAE, ``horizon_episode_stats`` for logging).  Both updates can
+bootstrap truncated episodes from the critic (``bootstrap_truncation=True``).
 """
 from __future__ import annotations
 
@@ -17,7 +18,7 @@ import ctypes as C
 import logging
 import os
 from collections.abc import Callable
-from dataclasses import dataclass
+from dataclasses import dataclass, replace
 from typing import Any
 
 import numpy as np
@@ -74,6 +75,12 @@ class Rollout:
     ep_weight: torch.Tensor | None = None   # float32 [B] episode rank weights (None = 1)
     n_traj: int | None = None               # divisor of the per-episode weight (defaults to B)
     auto_reset: bool = False                # fixed-horizon rollout with reset-on-done: a lane holds SEVERAL episodes
+    # The Philox env streams the rollout played on (rollout_many): the env seed, the global id of lane 0 and the env
+    # counter before the first step (step t of lane b spawned from counter t0 + t + 1).  A window needs them to replay
+    # the boards its truncated episodes were cut on (update_from_horizon(bootstrap_truncation=True)).
+    seed: int | None = None
+    gid0: int | None = None
+    t0: int | None = None
 
     @property
     def B(self) -> int:
@@ -450,10 +457,12 @@ class ReinforceAgent:
             fl = flags[: T + 1].gather(0, idx).reshape(-1)
             # like the frozen pass-through of the step kernel: an episode that ended before T no longer reports "changed"
             benv.flags = torch.where(length < T, fl & 0xEF, fl)
-            return Rollout(boards[: T + 1], flags[: T + 1], actions[:T], rewards[:T], length, T)
+            return Rollout(boards[: T + 1], flags[: T + 1], actions[:T], rewards[:T], length, T, seed=benv.seed, gid0=benv.gid0,
+                           t0=t0)
         benv.board = boards[T]
         benv.flags = flags[T]
-        return Rollout(boards[: T + 1], flags[: T + 1], actions[:T], rewards[:T], length, T, auto_reset=fixed)
+        return Rollout(boards[: T + 1], flags[: T + 1], actions[:T], rewards[:T], length, T, auto_reset=fixed, seed=benv.seed,
+                       gid0=benv.gid0, t0=t0)
 
     def _live_chunks(self, launch, length: torch.Tensor, cap: int, check_every: int) -> int:
         """Run-to-termination chunks on the live-board list: launch(T, chunk, slot_map, upper, count) enqueues steps
@@ -633,7 +642,8 @@ class ReinforceAgent:
         self.update_from_rollout(ro)
 
     def update_from_rollout(self, ro: Rollout, chunk: int = 1 << 20, allreduce=None,
-                            precision: int | str = "auto", exchange: str = "default") -> dict[str, Any]:
+                            precision: int | str = "auto", exchange: str = "default",
+                            bootstrap_truncation: bool = False) -> dict[str, Any]:
         """One policy-gradient update from device-resident rollout buffers.  `allreduce(tensor)` (optional) sums
         a tensor over ranks in place: the flat gradients and the advantage statistics are the only exchange.
         precision: 0 = fp32 CUDA cores, "auto" (default) = the float32-grade tensor-core path (split-fp16 forward, fp16
@@ -645,8 +655,14 @@ class ReinforceAgent:
         one all-reduce per update (SURVEY.md 8e): the backward deltas are linear in the per-sample coefficient, so each rank
         accumulates g_A (coefficient w v / (T n)) and g_B (coefficient w / (T n)) locally, one float64 message
         [g_A | g_B | critic gradient | sums] is summed over ranks and g = (g_A - mean g_B) / std is formed afterwards.
-        It costs a second actor backward pass, which is why it is an opt-in."""
+        It costs a second actor backward pass, which is why it is an opt-in.
+        bootstrap_truncation (needs a critic or a value head): an episode truncated by the env's max_steps (flags[len[b], b]
+        has TRUNC) gets the target r + gamma V(boards[len[b], b]) at its last step instead of r, like Gymnasium's `truncated`
+        (see _update_bootstrapped).  Episodes cut by rollout_many's own max_steps cap carry no TRUNC flag and are not
+        bootstrapped.  The default keeps update_batch's targets."""
         cfg = self._check_update_config(exchange)
+        if bootstrap_truncation:
+            self._check_bootstrap(ro, window=False)
         if ro.B == 0 or ro.T == 0:
             return {}
         if ro.auto_reset:
@@ -664,12 +680,13 @@ class ReinforceAgent:
             dinfo = bd.DistInfo(int(os.environ.get("RANK", "0")), int(os.environ.get("WORLD_SIZE", "1")),
                                 int(os.environ.get("LOCAL_RANK", "0"))) if allreduce is not None else None
             ro.ep_weight = bd.episode_rank_weights(ro.total_reward(), cfg.reward_rank_weights, dinfo)
+        boot = self._truncated_episode_ends(ro) if bootstrap_truncation else None
         if cfg.augmentation:
             ro = self._augment_rollout(ro)
-        return self._update(ro, False, chunk, allreduce, precision, exchange)
+        return self._update_bootstrapped(ro, boot, chunk, allreduce, precision, exchange, window=False)
 
     def update_from_horizon(self, ro: Rollout, allreduce=None, precision: int | str = "auto", chunk: int = 1 << 20,
-                            exchange: str = "default") -> dict[str, Any]:
+                            exchange: str = "default", bootstrap_truncation: bool = False) -> dict[str, Any]:
         """One policy-gradient update from a fixed-horizon window: a rollout_many(horizon=H) rollout with reset-on-done,
         whose lanes keep playing across updates (synchronous A2C / REINFORCE on segments).  Episode boundaries inside a lane
         (flags DONE | TRUNC after step t) restart the returns, TD targets and advantages (b2048_segment_targets; a truncated
@@ -683,7 +700,11 @@ class ReinforceAgent:
         global lane count under sharding; x8 with augmentation), i.e. the mean over all slots of the window.  Baseline
         'each', reward_rank_weights (both need whole episodes), exchange='one_message' and rollouts without reset-on-done
         raise ValueError.  The episodes the window completes are added to horizon_episode_stats().
-        allreduce / precision / chunk as in update_from_rollout."""
+        allreduce / precision / chunk as in update_from_rollout.
+        bootstrap_truncation (needs a critic or a value head, and ro.seed / ro.t0 from rollout_many): a TRUNC boundary
+        after step t (the env's max_steps ran out, the game was not over) uses V(s') instead of 0, s' being the board the
+        episode was cut on: delta_t = r_t + gamma V(s') - V(s_t).  boards[t + 1] already holds the reset board; s' is replayed
+        on the device from boards[t], actions[t] and the env streams (b2048_replay_pre_reset)."""
         cfg = self._check_update_config(exchange)
         if not ro.auto_reset:
             raise ValueError("update_from_horizon needs a fixed-horizon rollout with reset-on-done (rollout_many(horizon=H))")
@@ -693,12 +714,85 @@ class ReinforceAgent:
             raise ValueError("reward rank weights need whole episodes: not available on fixed-horizon windows")
         if exchange == "one_message":
             raise ValueError("exchange='one_message' is not implemented for fixed-horizon windows")
+        if bootstrap_truncation:
+            self._check_bootstrap(ro, window=True)
         if ro.B == 0 or ro.T == 0:
             return {}
-        self._horizon_account(ro)
+        self._horizon_account(ro)                                   # the episode returns are the undiscounted env rewards
+        boot = self._truncated_window_steps(ro) if bootstrap_truncation else None
         if cfg.augmentation:
             ro = self._augment_rollout(ro)
-        return self._update(ro, True, chunk, allreduce, precision, exchange)
+        return self._update_bootstrapped(ro, boot, chunk, allreduce, precision, exchange, window=True)
+
+    # ------------------------------------------------------------------ bootstrapping at truncation
+    def _check_bootstrap(self, ro: Rollout, window: bool) -> None:
+        if not (self.agent_config.use_critic and getattr(self, "_critic", None) is not None):
+            raise ValueError("bootstrap_truncation needs a value function: use_critic=True or SharedTrunkActorCritic")
+        if window and (ro.seed is None or ro.t0 is None):
+            raise ValueError("bootstrap_truncation on a window needs its env streams (Rollout.seed and Rollout.t0, which "
+                             "rollout_many(horizon=H) sets) to replay the boards truncated episodes were cut on")
+
+    def _truncated_window_steps(self, ro: Rollout) -> tuple[torch.Tensor, torch.Tensor]:
+        """(slots, s'): the steps t * B + b of a window after which an episode was truncated (TRUNC without DONE), in
+        row-major [T, B] order, and the boards those episodes were cut on, replayed on the device."""
+        T, B = ro.T, ro.B
+        ends = ro.flags[1: T + 1] & (_lib.F_DONE | _lib.F_TRUNC)
+        slots = torch.nonzero((ends == _lib.F_TRUNC).reshape(-1)).reshape(-1)
+        nxt = torch.empty(slots.numel(), dtype=torch.int64, device=self.device)
+        with torch.cuda.device(self.device):
+            _lib.check(self._lib.b2048_replay_pre_reset(
+                self._h, _ptr(ro.boards[: T + 1].contiguous()), _ptr(ro.actions[:T].contiguous()), _ptr(slots), slots.numel(), B,
+                int(ro.seed) & (2**64 - 1), int(ro.gid0 or 0), int(ro.t0), _ptr(nxt), _stream()), "b2048_replay_pre_reset")
+        return slots, nxt
+
+    def _truncated_episode_ends(self, ro: Rollout) -> tuple[torch.Tensor, torch.Tensor]:
+        """(slots, s') of a run-to-termination rollout: the last step (len[b] - 1) * B + b of every lane whose episode was
+        truncated (flags[len[b], b] has TRUNC, not DONE), and its final board boards[len[b], b]."""
+        T, B = ro.T, ro.B
+        L = ro.length.long().clamp(0, T)
+        last = L.unsqueeze(0)
+        fin = ro.flags[: T + 1].gather(0, last).reshape(-1) & (_lib.F_DONE | _lib.F_TRUNC)
+        lanes = torch.nonzero((fin == _lib.F_TRUNC) & (L > 0)).reshape(-1)
+        slots = (L[lanes] - 1) * B + lanes
+        return slots, ro.boards[: T + 1].gather(0, last).reshape(-1)[lanes]
+
+    def _update_bootstrapped(self, ro: Rollout, boot, chunk: int, allreduce, precision: int | str, exchange: str,
+                             window: bool) -> dict[str, Any]:
+        """_update on a copy of the rewards with gamma V(s') folded in at the truncated steps (boot = (slots, s') of the
+        rollout before augmentation; None: no bootstrap).  The target kernels use V = 0 after an episode's last step, so
+        r' = r + gamma V(s') (each operation rounded separately, b2048_fold_bootstrap) makes every target, TD error,
+        advantage and critic coefficient the bootstrapped one.  With augmentation variant v of step (t, b) is column
+        v B + b, and it folds the value of variant v of s'."""
+        if boot is None or boot[0].numel() == 0:
+            return self._update(ro, window, chunk, allreduce, precision, exchange)
+        slots, nxt = boot
+        lib, h, dev = self._lib, self._h, self.device
+        T, B = ro.T, ro.B
+        if self.agent_config.augmentation:                         # ro is the augmented rollout: B = 8 x the original
+            K, B0 = slots.numel(), B // 8
+            nxt8 = torch.empty(8 * K, dtype=torch.int64, device=dev)
+            with torch.cuda.device(dev):
+                _lib.check(lib.b2048_symmetries(h, _ptr(nxt), None, None, _ptr(nxt8), None, None, 1, K, _stream()),
+                           "b2048_symmetries")                      # variant v of board k at v K + k
+            t, b = slots // B0, slots % B0
+            slots = ((t * B + b).unsqueeze(0) + B0 * torch.arange(8, device=dev).unsqueeze(1)).reshape(-1)
+            nxt = nxt8
+        K = slots.numel()
+        prec = 2 if precision == "auto" else int(precision)
+        # the tensor-core forwards take 4096 boards or more; a shorter list runs where "auto" would put it
+        vprec = prec if (K >= 4096 or prec in (0, 2)) else (2 if prec == 3 else 0)
+        values = torch.empty(K, dtype=torch.float32, device=dev)
+        self._values(nxt, values, vprec)
+        if vprec in (2, 3) and not bool(torch.isfinite(values).all()):   # fp16 range exceeded: as in _update
+            self._values(nxt, values, 0)
+        rewards = torch.empty((T, B), dtype=torch.float32, device=dev)
+        with torch.cuda.device(dev):
+            _lib.check(lib.b2048_fold_bootstrap(h, _ptr(ro.rewards[:T].contiguous()), _ptr(slots), _ptr(values), K, T * B,
+                                                float(self.agent_config.gamma), _ptr(rewards), _stream()),
+                       "b2048_fold_bootstrap")
+        info = self._update(replace(ro, rewards=rewards), window, chunk, allreduce, precision, exchange)
+        info.update(bootstrap_slots=slots, bootstrap_boards=nxt, bootstrap_values=values)
+        return info
 
     def _segment_targets(self, rewards, flags, values, lam, n_traj, v, td, gcoef, valid_len) -> None:
         cfg = self.agent_config

@@ -17,6 +17,9 @@ runner.py:587-608 draws them, on the fp32 policy kernel; evaluation keeps the Ph
 reset=False)`` followed by one ``update_from_horizon`` (segment-aware returns / TD / GAE, the cut-off tail bootstrapped by
 the critic when there is one).  The CSV rows then describe the episodes that ended inside the batch's window (NaN stats
 and zero counts when none did); a resumed run starts from fresh resets.  Not combinable with ``seed_streams="numpy"``.
+``train.bootstrap_truncation`` (default false; needs ``agent.use_critic`` or a ``shared_trunk`` section): in both modes, an
+episode truncated by ``env.max_steps`` gets the target r + gamma V(s') at its last step, s' being the board it was cut on,
+instead of r (``update_from_rollout`` / ``update_from_horizon(bootstrap_truncation=True)``).
 
     python -m torch.distributed.run ... b2048_runner.py -conf cfg.json      (or: python b2048_runner.py -conf cfg.json)
 """
@@ -170,7 +173,8 @@ def training(cfg: dict[str, Any], info: bd.DistInfo | None = None, device=None, 
                 best = avg
             if global_step > 30 and is_record and info.rank == 0 and out_dir:
                 agent.save_model(os.path.join(out_dir, f"best_avg_{avg:.2f}_step_{global_step}.npz"))
-            upd = bd.sharded_update(agent, ro, info, total_episodes=int(tr["batch_size"]), exchange=tr.get("exchange", "default"))
+            upd = bd.sharded_update(agent, ro, info, total_episodes=int(tr["batch_size"]), exchange=tr.get("exchange", "default"),
+                                    bootstrap_truncation=bool(tr.get("bootstrap_truncation", False)))
             row = {"batch": global_step, "avg_reward": avg, "max_reward": mx, "min_reward": mn, "max_tile_counts": json.dumps(hist)}
             rows.append(dict(row, steps=int(ro.length.sum().item()), seconds=time.perf_counter() - t0,
                              grad_norm=upd.get("actor_grad_norm")))
@@ -199,7 +203,7 @@ def _horizon_batch(agent, env, info: bd.DistInfo, tr: dict[str, Any], horizon: i
     saving = global_step > 30 and info.rank == 0 and bool(out_dir)
     before = agent.save_state() if saving else None
     upd = bd.sharded_update(agent, ro, info, total_episodes=int(tr["batch_size"]), exchange=tr.get("exchange", "default"),
-                            fixed_horizon=True)
+                            fixed_horizon=True, bootstrap_truncation=bool(tr.get("bootstrap_truncation", False)))
     es = agent.horizon_episode_stats(reset=True, info=info)
     avg = es["avg_reward"]
     if saving and avg > best:                                                              # runner.py:643-660
