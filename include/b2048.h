@@ -32,6 +32,8 @@
  *   domain B2048_DOM_STEP : w0 spawn cell, w1 spawn value, w2 env-side random
  *                           action, w3 policy-sampling uniform
  *   domain B2048_DOM_RESET: (w0, w1) first spawn, (w2, w3) second spawn
+ *   domain B2048_DOM_PPO  : the PPO minibatch shuffle (b2048_ppo_minibatches): counter (R, round, epoch, domain),
+ *                           key = the shuffle seed, w0 the Feistel round function
  * spawn(wp, wv): n = #empty; n == 0 -> no-op; k = mulhi32(wp, n); the k-th
  * empty cell in row-major order (np.argwhere order, game2048.py:109) receives
  * exponent 2 if wv >= 0xE6666667 (u = wv/2^32 >= 0.9, game2048.py:117) else 1.
@@ -63,6 +65,7 @@ typedef enum {
 
 #define B2048_DOM_STEP  0u
 #define B2048_DOM_RESET 1u
+#define B2048_DOM_PPO   2u
 
 enum { B2048_REWARD_SUM = 0, B2048_REWARD_LOG2 = 1 };            /* env.py:212-223 */
 enum { B2048_BONUS_OFF = 0, B2048_BONUS_RAW = 1, B2048_BONUS_LOG2 = 2 }; /* env.py:242-249 */
@@ -391,6 +394,40 @@ int b2048_replay_pre_reset(b2048_handle* h, const uint64_t* boards, const uint8_
                            int64_t B, uint64_t seed, uint64_t gid0, uint32_t t0, uint64_t* out, void* stream);
 int b2048_fold_bootstrap(b2048_handle* h, const float* reward, const int64_t* slots, const float* value, int64_t K, int64_t n,
                          float gamma, float* reward_out, void* stream);
+
+/* PPO on a window: several epochs of clipped-ratio minibatch steps on the same T x n_traj samples.
+ *
+ * b2048_ppo_minibatches: mb_out[t B + b] (int32 [T, B]) = the minibatch, in [0, minibatches), of the window slot (t, b) in
+ * epoch `epoch`.  Its global sample index is g = t n_traj + gid0 + b (n_traj = the global lane count, gid0 = the global
+ * lane id of this shard's lane 0; gid0 + B <= n_traj, T n_traj <= 2^32).  A keyed Feistel bijection P_e of [0, N),
+ * N = T n_traj, on the Philox stream of domain B2048_DOM_PPO (counter (R, round, epoch, domain), key seed) places g, and
+ * the minibatch is floor(P_e(g) minibatches / N): minibatch m holds ceil((m + 1) N / M) - ceil(m N / M) samples over all
+ * shards, so the partition does not depend on the world size and needs no message (csrc/b2048_ppo.cuh).
+ *
+ * b2048_ppo_logp: logp_out[i] (double) = log pi(action[i] | s_i) from logits [n, 4] (b2048_mlp_forward of the actor) in
+ * float64: log-softmax with the illegal actions of mask_flags[i] (low nibble; NULL = every action legal) filled with -1e9
+ * like logits_to_probs.
+ *
+ * b2048_ppo_coefficients: one minibatch of n samples; sample i is window slot slots[i] (int64).  logits [n, 4] and
+ * value [n] are the minibatch's forward outputs at the current parameters; mask_flags (may be NULL), action, logp_old
+ * (double), adv (the baseline-processed advantages), a_raw (the advantages before the baseline) and v_old (V at the
+ * window's parameters) are [T B] window arrays read at the slot.  With r = exp(logp - logp_old), R = a_raw + v_old
+ * (float32) and m = mb_size, the minibatch's global size:
+ *   coef[i]  = adv r / m, or 0 when (adv > 0 and r > 1 + clip_eps) or (adv < 0 and r < 1 - clip_eps)
+ *              (b2048_mlp_backward head 0: the gradient of the mean clipped surrogate);
+ *   gcoef[i] = dLoss/dV / m (head 1, descent): V - R, or with value_clip_eps > 0 and V_c = v_old + clamp(V - v_old,
+ *              -value_clip_eps, value_clip_eps) the gradient of max((V - R)^2, (V_c - R)^2): (V - R) unless (V_c - R)^2 is
+ *              larger, then (V_c - R) when |V - v_old| < value_clip_eps, else 0; huber != 0 clips it to +-huber_delta.
+ * Arithmetic in float64, coef / gcoef rounded to float32.  stats (device double[5]) is ADDED to: {clipped count, sum r,
+ * sum (r - 1 - log r), sum min(r adv, clip(r) adv), sum of the value loss (0.5 e^2, or Huber, of the selected error)}. */
+int b2048_ppo_minibatches(b2048_handle* h, int32_t T, int64_t B, int64_t n_traj, int64_t gid0, int64_t minibatches,
+                          uint64_t seed, uint32_t epoch, int32_t* mb_out, void* stream);
+int b2048_ppo_logp(b2048_handle* h, const float* logits, const uint8_t* mask_flags, const uint8_t* action, int64_t n,
+                   double* logp_out, void* stream);
+int b2048_ppo_coefficients(b2048_handle* h, const int64_t* slots, int64_t n, const float* logits, const float* value,
+                           const uint8_t* mask_flags, const uint8_t* action, const double* logp_old, const float* adv,
+                           const float* a_raw, const float* v_old, double mb_size, double clip_eps, double value_clip_eps,
+                           int32_t huber, float huber_delta, float* coef, float* gcoef, double* stats, void* stream);
 
 /* Gradient accumulation of update_batch's actor / critic blocks (reinforce_agent.py:403-555, _backpropagation
  * :639-678) over n samples (flattened [T,B] rollout; samples with coef == 0 contribute nothing).

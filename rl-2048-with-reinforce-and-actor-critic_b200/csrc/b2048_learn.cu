@@ -10,6 +10,9 @@
 //      horizon_episodes_kernel   episodes completed inside a window (logging)
 //      replay_pre_reset_kernel   the boards truncated episodes were cut on (bootstrapping at truncation)
 //      fold_bootstrap_kernel     r + gamma V(s') at the truncated slots of a copy of the rewards
+//      ppo_minibatch_kernel      PPO: the minibatch of every slot of a window (keyed Feistel permutation, b2048_ppo.cuh)
+//      ppo_logp_kernel           PPO: log pi_old(a | s) from the learner's logits
+//      ppo_coef_kernel           PPO: ratio, clipped-surrogate and clipped-value coefficients of one minibatch
 //   K6 mlp_backward_kernel       _backpropagation per tile  src/reinforce_agent.py:639-678 (deltas + activations)
 //      atb_kernel                dW_l = A_l^T D_l           (sum over samples of np.outer, :666)
 //      colsum_kernel             db_l = sum_s D_l
@@ -24,6 +27,7 @@
 #include "b2048_horizon.cuh"
 #include "b2048_internal.h"
 #include "b2048_mlp.cuh"
+#include "b2048_ppo.cuh"
 
 namespace b2 {
 
@@ -548,6 +552,57 @@ __global__ void __launch_bounds__(256) adam_kernel(float* __restrict__ theta, fl
     }
 }
 
+// ------------------------------------------------------------------------------------------------ PPO on windows
+// One thread per slot i = t B + b of a window: the minibatch of global sample t n_traj + gid0 + b in epoch `epoch`.
+__global__ void __launch_bounds__(256) ppo_minibatch_kernel(int T, int64_t B, int64_t n_traj, int64_t gid0, uint64_t N,
+                                                             uint64_t M, uint64_t seed, uint32_t epoch,
+                                                             int32_t* __restrict__ mb) {
+    const int64_t total = (int64_t)T * B;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
+        const int64_t t = i / B, b = i - t * B;
+        mb[i] = (int32_t)ppo_minibatch((uint64_t)(t * n_traj + gid0 + b), N, M, seed, epoch);
+    }
+}
+
+__global__ void __launch_bounds__(256) ppo_logp_kernel(const float* __restrict__ logits, const uint8_t* __restrict__ mask_flags,
+                                                        const uint8_t* __restrict__ action, int64_t n, double* __restrict__ out) {
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x)
+        out[i] = ppo_logp(logits + 4 * i, mask_flags ? (uint32_t)(mask_flags[i] & 0xF) : 0xFu, action[i]);
+}
+
+// Sample i of a minibatch is window slot slots[i]; logits / value are the minibatch's forward outputs (row i), the other
+// inputs are window-wide [T B] arrays read at the slot.  R = A_raw + V_old, rounded in float32.  stats (double[5]) +=
+// {clipped count, sum r, sum (r - 1 - log r), sum surrogate, sum value loss}.
+__global__ void __launch_bounds__(256) ppo_coef_kernel(const int64_t* __restrict__ slots, int64_t n, const float* __restrict__ logits,
+                                                        const float* __restrict__ value, const uint8_t* __restrict__ mask_flags,
+                                                        const uint8_t* __restrict__ action, const double* __restrict__ logp_old,
+                                                        const float* __restrict__ adv, const float* __restrict__ a_raw,
+                                                        const float* __restrict__ v_old, double mb_size, double clip_eps,
+                                                        double vclip_eps, int huber, double huber_delta, float* __restrict__ coef,
+                                                        float* __restrict__ gcoef, double* __restrict__ stats) {
+    double acc[5] = {0.0, 0.0, 0.0, 0.0, 0.0};
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+        const int64_t s = slots[i];
+        const PpoSample p = ppo_sample(logits + 4 * i, mask_flags ? (uint32_t)(mask_flags[s] & 0xF) : 0xFu, action[s],
+                                       logp_old[s], adv[s], f32_add(a_raw[s], v_old[s]), v_old[s], value[i], mb_size,
+                                       clip_eps, vclip_eps, huber, huber_delta);
+        coef[i] = (float)p.coef;
+        gcoef[i] = (float)p.gcoef;
+        acc[0] += p.clipped; acc[1] += p.ratio; acc[2] += p.kl; acc[3] += p.surrogate; acc[4] += p.value_loss;
+    }
+    __shared__ double part[5][8];
+    for (int k = 0; k < 5; ++k) {
+        for (int d = 16; d > 0; d >>= 1) acc[k] += __shfl_down_sync(0xFFFFFFFFu, acc[k], d);
+        if ((threadIdx.x & 31) == 0) part[k][threadIdx.x >> 5] = acc[k];
+    }
+    __syncthreads();
+    if (threadIdx.x < 5) {
+        double t = 0.0;
+        for (int w = 0; w < 8; ++w) t += part[threadIdx.x][w];
+        atomicAdd(stats + threadIdx.x, t);
+    }
+}
+
 static int ew_grid(int64_t n, int num_sms) {
     int64_t b = (n + 255) / 256;
     int64_t cap = (int64_t)num_sms * 8;
@@ -718,6 +773,51 @@ extern "C" int b2048_fold_bootstrap(b2048_handle* h, const float* reward, const 
     if (reward_out != reward) B2_CUDA(cudaMemcpyAsync(reward_out, reward, (size_t)n * sizeof(float), cudaMemcpyDeviceToDevice, s));
     if (K > 0)
         fold_bootstrap_kernel<<<(unsigned)((K + 255) / 256), 256, 0, s>>>(reward, slots, value, K, gamma, reward_out);
+    B2_CUDA(cudaGetLastError());
+    return B2048_OK;
+}
+
+extern "C" int b2048_ppo_minibatches(b2048_handle* h, int32_t T, int64_t B, int64_t n_traj, int64_t gid0, int64_t minibatches,
+                                     uint64_t seed, uint32_t epoch, int32_t* mb_out, void* stream) {
+    B2_REQUIRE(h != nullptr, "b2048_ppo_minibatches: handle is NULL");
+    B2_REQUIRE(T >= 0 && B >= 0 && gid0 >= 0, "b2048_ppo_minibatches: negative size");
+    if (T == 0 || B == 0) return B2048_OK;
+    B2_REQUIRE(mb_out != nullptr, "b2048_ppo_minibatches: mb_out is NULL");
+    B2_REQUIRE(gid0 + B <= n_traj, "b2048_ppo_minibatches: the shard [gid0, gid0 + B) is not inside [0, n_traj)");
+    B2_REQUIRE(n_traj <= ((int64_t)1 << 32) / T, "b2048_ppo_minibatches: T n_traj exceeds 2^32 samples");
+    const int64_t N = (int64_t)T * n_traj;
+    B2_REQUIRE(minibatches >= 1 && minibatches <= N, "b2048_ppo_minibatches: minibatches must be in [1, T n_traj]");
+    ppo_minibatch_kernel<<<ew_grid((int64_t)T * B, h->num_sms), 256, 0, (cudaStream_t)stream>>>(
+        T, B, n_traj, gid0, (uint64_t)N, (uint64_t)minibatches, seed, epoch, mb_out);
+    B2_CUDA(cudaGetLastError());
+    return B2048_OK;
+}
+
+extern "C" int b2048_ppo_logp(b2048_handle* h, const float* logits, const uint8_t* mask_flags, const uint8_t* action, int64_t n,
+                              double* logp_out, void* stream) {
+    B2_REQUIRE(h != nullptr, "b2048_ppo_logp: handle is NULL");
+    B2_REQUIRE(n >= 0, "b2048_ppo_logp: n < 0");
+    if (n == 0) return B2048_OK;
+    B2_REQUIRE(logits && action && logp_out, "b2048_ppo_logp: NULL buffer");
+    ppo_logp_kernel<<<ew_grid(n, h->num_sms), 256, 0, (cudaStream_t)stream>>>(logits, mask_flags, action, n, logp_out);
+    B2_CUDA(cudaGetLastError());
+    return B2048_OK;
+}
+
+extern "C" int b2048_ppo_coefficients(b2048_handle* h, const int64_t* slots, int64_t n, const float* logits, const float* value,
+                                      const uint8_t* mask_flags, const uint8_t* action, const double* logp_old,
+                                      const float* adv, const float* a_raw, const float* v_old, double mb_size, double clip_eps,
+                                      double value_clip_eps, int32_t huber, float huber_delta, float* coef, float* gcoef,
+                                      double* stats, void* stream) {
+    B2_REQUIRE(h != nullptr, "b2048_ppo_coefficients: handle is NULL");
+    B2_REQUIRE(n >= 0, "b2048_ppo_coefficients: n < 0");
+    if (n == 0) return B2048_OK;
+    B2_REQUIRE(slots && logits && value && action && logp_old && adv && a_raw && v_old && coef && gcoef && stats,
+               "b2048_ppo_coefficients: NULL buffer");
+    B2_REQUIRE(mb_size >= 1.0 && clip_eps > 0.0, "b2048_ppo_coefficients: mb_size must be >= 1 and clip_eps > 0");
+    ppo_coef_kernel<<<ew_grid(n, h->num_sms), 256, 0, (cudaStream_t)stream>>>(
+        slots, n, logits, value, mask_flags, action, logp_old, adv, a_raw, v_old, mb_size, clip_eps, value_clip_eps, huber,
+        (double)huber_delta, coef, gcoef, stats);
     B2_CUDA(cudaGetLastError());
     return B2048_OK;
 }

@@ -9,7 +9,8 @@ errors, back-propagation, global-norm clip, SGD / Adam — is a CUDA kernel reac
 Added surface: ``rollout_many`` (run-to-termination or fixed-horizon rollouts of a whole
 ``Batched2048Env``) and ``update_from_rollout``; ``update_batch`` packs reference-style trajectories
 into the same rollout buffers and calls the same kernels.  ``update_from_horizon`` trains on fixed-horizon
-windows with reset-on-done (segment-aware returns / TD / GAE, ``horizon_episode_stats`` for logging).  Both updates can
+windows with reset-on-done (segment-aware returns / TD / GAE, ``horizon_episode_stats`` for logging); ``update_ppo`` runs
+several epochs of clipped-ratio minibatch steps on such a window.  The window updates and ``update_from_rollout`` can
 bootstrap truncated episodes from the critic (``bootstrap_truncation=True``).
 """
 from __future__ import annotations
@@ -291,9 +292,71 @@ class ReinforceAgent:
         return self._fused_shape() or self._generic_tc_shape()
 
     def _values(self, boards: torch.Tensor, out: torch.Tensor, precision: int = 0) -> None:
+        self._net_forward(self._critic, boards, out, precision)
+
+    def _net_forward(self, net: DeviceMLP, boards: torch.Tensor, out: torch.Tensor, precision: int = 0) -> None:
         with torch.cuda.device(self.device):
-            _lib.check(self._lib.b2048_mlp_forward(self._h, _ptr(boards), C.byref(self._critic.desc), _ptr(out),
-                                                   boards.numel(), int(precision), _stream()), "b2048_mlp_forward")
+            _lib.check(self._lib.b2048_mlp_forward(self._h, _ptr(boards), C.byref(net.desc), _ptr(out), boards.numel(),
+                                                   int(precision), _stream()), "b2048_mlp_forward")
+
+    def _forward_checked(self, net: DeviceMLP, boards: torch.Tensor, out: torch.Tensor, prec: int) -> bool:
+        """b2048_mlp_forward at prec.  The split-fp16 path keeps activations in fp16: a network whose activations leave the
+        fp16 range gives non-finite outputs, which are recomputed on the fp32 kernels.  True when that happened."""
+        self._net_forward(net, boards, out, prec)
+        if prec in (2, 3) and not bool(torch.isfinite(out).all()):
+            self._net_forward(net, boards, out, 0)
+            return True
+        return False
+
+    @staticmethod
+    def _small_batch_precision(prec: int, n: int) -> int:
+        """The tensor-core kernels take 4096 boards or more; a shorter batch runs where "auto" (2) would put it."""
+        return prec if (n >= 4096 or prec in (0, 2)) else (2 if prec == 3 else 0)
+
+    def _backward(self, net: DeviceMLP, boards, mflags, acts, cf: torch.Tensor, n: int, head_mode: int, prec: int, chunk: int,
+                  fell_back: list) -> None:
+        """net.grad = b2048_mlp_backward of the n samples (head 0: sum cf log pi(a|s), head 1: sum cf V(s)) at prec.  A
+        non-finite split-fp16 gradient (fp16 range exceeded) is never applied: the pass is redone in fp32 and head_mode is
+        appended to fell_back."""
+        lib, h = self._lib, self._h
+        ws_floats = int(lib.b2048_backward_workspace_floats(C.byref(net.desc), min(chunk, n)))
+        ws = self._buf("bwd_ws", (ws_floats,), torch.float32)
+        for p_try in ((prec, 0) if prec in (2, 3) else (prec,)):
+            net.grad.zero_()
+            with torch.cuda.device(self.device):
+                _lib.check(lib.b2048_mlp_backward(h, _ptr(boards), _ptr(mflags) if self._use_mask else None, _ptr(acts),
+                                                  _ptr(cf), C.byref(net.desc), _ptr(net.grad), n, head_mode, _ptr(ws),
+                                                  ws_floats, min(chunk, n), p_try, _stream()), "b2048_mlp_backward")
+            if p_try == 0 or bool(torch.isfinite(net.grad).all()):
+                break
+            fell_back.append(head_mode)
+            self._logger.warning("tensor-core gradient not finite (fp16 range exceeded); recomputing on the fp32 kernels")
+
+    def _apply(self, net, lr: float, sign: float, t_adam: int) -> torch.Tensor:
+        """b2048_apply_update (global-norm clip, SGD / Adam) of net.grad; returns the device double[1] squared norm."""
+        cfg = self.agent_config
+        sumsq = self._buf("sumsq_" + str(sign), (1,), torch.float64)
+        with torch.cuda.device(self.device):
+            _lib.check(self._lib.b2048_apply_update(self._h, _ptr(net.theta), _ptr(net.grad), _ptr(net.adam_m), _ptr(net.adam_v),
+                                                    net.n_params, OPTIMIZER[cfg.optimizer], float(lr), float(sign),
+                                                    float(cfg.max_grad_norm), float(cfg.adam_beta1), float(cfg.adam_beta2),
+                                                    int(t_adam), _ptr(sumsq), _stream()), "b2048_apply_update")
+        return sumsq
+
+    def _optimizer_step(self) -> tuple[torch.Tensor, torch.Tensor | None]:
+        """One optimizer step of the actor (or the shared network) and of a separate critic, each Adam counter advanced
+        once; returns their squared gradient norms (device double[1]; None without a separate critic)."""
+        cfg = self.agent_config
+        shared = getattr(self, "_shared_net", None)
+        if cfg.optimizer == "adam":
+            self._adam_t += 1
+        ss_a = self._apply(self._actor if shared is None else shared, cfg.learning_rate, +1.0, self._adam_t)
+        ss_c = None
+        if cfg.use_critic and self._critic is not None and shared is None:
+            if cfg.optimizer == "adam":
+                self._adam_t_c += 1
+            ss_c = self._apply(self._critic, cfg.critic_learning_rate, -1.0, getattr(self, "_adam_t_c", 0))
+        return ss_a, ss_c
 
     # ------------------------------------------------------------------ reference API: acting
     def _obs_to_packed(self, obs) -> tuple[int, int]:
@@ -724,6 +787,181 @@ class ReinforceAgent:
             ro = self._augment_rollout(ro)
         return self._update_bootstrapped(ro, boot, chunk, allreduce, precision, exchange, window=True)
 
+    # ------------------------------------------------------------------ PPO on windows
+    def update_ppo(self, ro: Rollout, epochs: int = 4, minibatches: int = 4, clip_eps: float = 0.2,
+                   value_clip_eps: float | None = None, shuffle_seed: int = 0, allreduce=None, precision: int | str = "auto",
+                   bootstrap_truncation: bool = False) -> dict[str, Any]:
+        """PPO on a fixed-horizon window (rollout_many(horizon=H), reset-on-done): `epochs` passes over the window's
+        N = T n_traj samples, each split into `minibatches` minibatches, one clipped-surrogate step per minibatch
+        (epochs x minibatches optimizer steps).  Needs a value function (use_critic=True or SharedTrunkActorCritic).
+        Once, at the window's parameters theta_old: V_old on all T + 1 slices, the segment-aware GAE A_raw
+        (b2048_segment_targets; lambda = gae_lambda, 0 = TD(0)), the advantages A of the configured baseline (off / batch /
+        batch_norm, per window), the value target R = A_raw + V_old, and logp_old = log pi_theta_old(a|s) from the learner's
+        own forward at the update's precision (not the rollout's probabilities).
+        Minibatches: b2048_ppo_minibatches, a keyed permutation of the global sample index t n_traj + gid0 + b per epoch
+        (shuffle_seed, epoch); it depends on neither the world size nor the shard, and every rank knows each minibatch's
+        global size.  Per minibatch: forward of actor and critic, r = exp(logp - logp_old), the clipped-surrogate coefficient
+        A r / |mb| (0 where clipped), the value coefficient (V - R) / |mb| (value_clip_eps: PPO's clipped value loss; mse or
+        Huber as configured), b2048_mlp_backward for both heads, ONE all-reduce of the flat gradient when sharded, the
+        global-norm clip and SGD / Adam (the Adam counters advance once per minibatch).
+        The window's episodes are added to horizon_episode_stats() as update_from_horizon does.
+        Returns per-epoch lists (rank-local): clip_fraction, approx_kl (mean r - 1 - log r), mean_ratio, surrogate
+        (mean min(r A, clip(r) A)) and value_loss; per-step actor_grad_norms / critic_grad_norms; advantages (A), gae
+        (A_raw), values_old ([T + 1, B]) and logp_old ([T B], float64) of the window; precision.  The tensors are scratch
+        buffers, valid until the next update.
+        allreduce / precision / bootstrap_truncation as in update_from_horizon.  Refused (ValueError): no value function,
+        a rollout without reset-on-done, augmentation, reward rank weights, baseline 'each', epochs < 1, minibatches
+        outside [1, N], clip_eps <= 0, value_clip_eps <= 0, and a shard (n_traj > B) without ro.gid0."""
+        cfg = self._check_update_config("default")
+        if not (cfg.use_critic and getattr(self, "_critic", None) is not None):
+            raise ValueError("update_ppo needs a value function: use_critic=True or SharedTrunkActorCritic")
+        if not ro.auto_reset:
+            raise ValueError("update_ppo needs a fixed-horizon rollout with reset-on-done (rollout_many(horizon=H))")
+        if cfg.augmentation:
+            raise ValueError("update_ppo does not implement augmentation")
+        if cfg.reward_rank_weights or ro.ep_weight is not None:
+            raise ValueError("reward rank weights need whole episodes: not available on fixed-horizon windows")
+        if cfg.baseline_mode == "each":
+            raise ValueError("baseline 'each' needs whole episodes: not available on fixed-horizon windows")
+        n_traj = int(ro.n_traj if ro.n_traj is not None else ro.B)
+        N = ro.T * n_traj
+        if int(epochs) < 1:
+            raise ValueError(f"update_ppo: epochs must be >= 1, got {epochs}")
+        if not 1 <= int(minibatches) <= max(N, 1):
+            raise ValueError(f"update_ppo: minibatches must be in [1, {N}] (the window's samples), got {minibatches}")
+        if not clip_eps > 0:
+            raise ValueError(f"update_ppo: clip_eps must be positive, got {clip_eps}")
+        if value_clip_eps is not None and not value_clip_eps > 0:
+            raise ValueError(f"update_ppo: value_clip_eps must be positive or None, got {value_clip_eps}")
+        if n_traj > ro.B and ro.gid0 is None:
+            raise ValueError("update_ppo on a shard (n_traj > B) needs Rollout.gid0, the global id of its lane 0, to place "
+                             "its samples in the global minibatches")
+        if bootstrap_truncation:
+            self._check_bootstrap(ro, window=True)
+        if ro.B == 0 or ro.T == 0:
+            return {}
+        self._horizon_account(ro)
+        prec = 2 if precision == "auto" else int(precision)
+        if bootstrap_truncation:
+            boot = self._truncated_window_steps(ro)
+            if boot[0].numel():
+                ro = self._fold_truncation(ro, boot, precision)[0]
+        return self._ppo(ro, int(epochs), int(minibatches), float(clip_eps), value_clip_eps, int(shuffle_seed), allreduce, prec,
+                         n_traj)
+
+    def ppo_minibatch_lists(self, T: int, B: int, n_traj: int, gid0: int, minibatches: int, shuffle_seed: int,
+                            epoch: int) -> tuple[torch.Tensor, list[int]]:
+        """The local slots t B + b of a [T, B] window grouped by minibatch for one epoch of update_ppo: (order, counts) with
+        the slots of minibatch m at order[sum(counts[:m]) : sum(counts[:m + 1])], ascending.  gid0 = the global id of lane 0
+        (0 for a whole window)."""
+        mb = self._buf("ppo_mb", (T, B), torch.int32)
+        with torch.cuda.device(self.device):
+            _lib.check(self._lib.b2048_ppo_minibatches(self._h, T, B, n_traj, gid0, minibatches, shuffle_seed & (2**64 - 1),
+                                                       epoch, _ptr(mb), _stream()), "b2048_ppo_minibatches")
+        mb = mb.reshape(-1)
+        order = torch.sort(mb, stable=True).indices           # grouping only: the order inside a minibatch is by slot
+        counts = torch.bincount(mb, minlength=minibatches).cpu().tolist()
+        return order, counts
+
+    def _ppo(self, ro: Rollout, epochs: int, M: int, clip_eps: float, value_clip_eps, shuffle_seed: int, allreduce, prec: int,
+             n_traj: int) -> dict[str, Any]:
+        cfg = self.agent_config
+        lib, h, dev = self._lib, self._h, self.device
+        T, B = ro.T, ro.B
+        n, N = T * B, T * n_traj
+        gid0 = int(ro.gid0) if n_traj > B else 0
+        lam = float(getattr(self, "gae_lambda", 0.0))
+        boards = ro.boards[:T].reshape(-1)
+        mflags = ro.flags[:T].reshape(-1)
+        acts = ro.actions[:T].reshape(-1)
+        fell_back: list = []
+        # ---- once per window, at theta_old
+        values = self._buf("values", (T + 1, B), torch.float32)
+        if self._forward_checked(self._critic, ro.boards[: T + 1].reshape(-1), values.view(-1), prec):
+            fell_back.append(1)
+        gae, td, gcoef = (self._buf(k, (T, B), torch.float32) for k in ("gae", "td", "gcoef"))
+        valid = self._buf("valid_len", (B,), torch.int32)
+        self._segment_targets(ro.rewards[:T].contiguous(), ro.flags[: T + 1].contiguous(), values, lam, float(n_traj), gae, td,
+                              gcoef, valid)
+        mode = BASELINE[cfg.baseline_mode]
+        stats = self._buf("stats", (4,), torch.float64)
+        adv, coef = self._buf("adv", (T, B), torch.float32), self._buf("coef", (T, B), torch.float32)
+        pre = 0
+        with torch.cuda.device(dev):
+            if allreduce is not None and mode >= 2:            # the window is sharded: the baseline sums are global
+                stats.zero_()
+                _lib.check(lib.b2048_weighted_stats(h, _ptr(gae), _ptr(valid), None, T, B, _ptr(stats), _stream()),
+                           "b2048_weighted_stats")
+                allreduce(stats)
+                pre = 1
+            _lib.check(lib.b2048_advantages_window(h, _ptr(gae), _ptr(valid), mode, float(n_traj), T, B, _ptr(adv), _ptr(coef),
+                                                   _ptr(stats), pre, _stream()), "b2048_advantages_window")
+        logits = self._buf("ppo_logits", (n, 4), torch.float32)
+        if self._forward_checked(self._actor, boards, logits, prec):
+            fell_back.append(0)
+        logp_old = self._buf("ppo_logp_old", (n,), torch.float64)
+        with torch.cuda.device(dev):
+            _lib.check(lib.b2048_ppo_logp(h, _ptr(logits), _ptr(mflags) if self._use_mask else None, _ptr(acts), n,
+                                          _ptr(logp_old), _stream()), "b2048_ppo_logp")
+        # ---- epochs x minibatches clipped steps
+        shared = getattr(self, "_shared_net", None)
+        ep_stats = torch.zeros((epochs, 5), dtype=torch.float64, device=dev)
+        norms = torch.zeros((epochs * M, 2), dtype=torch.float64, device=dev)
+        vclip = float(value_clip_eps) if value_clip_eps is not None else 0.0
+        huber = int(cfg.critic_loss_type == "huber")
+        chunk = 1 << 20
+        for e in range(epochs):
+            order, counts = self.ppo_minibatch_lists(T, B, n_traj, gid0, M, shuffle_seed, e)
+            off = 0
+            for m in range(M):
+                k = counts[m]
+                idx = order[off: off + k]
+                off += k
+                size = (-(-(m + 1) * N // M)) - (-(-m * N // M))   # the minibatch's global size, ceil((m+1)N/M) - ceil(mN/M)
+                if k > 0:
+                    p = self._small_batch_precision(prec, k)
+                    bx, fx, ax = boards.index_select(0, idx), mflags.index_select(0, idx), acts.index_select(0, idx)
+                    z = self._buf("ppo_z", (k, 4), torch.float32)
+                    v = self._buf("ppo_v", (k,), torch.float32)
+                    if self._forward_checked(self._actor, bx, z, p):
+                        fell_back.append(0)
+                    if self._forward_checked(self._critic, bx, v, p):
+                        fell_back.append(1)
+                    cf, gc = self._buf("ppo_coef", (k,), torch.float32), self._buf("ppo_gcoef", (k,), torch.float32)
+                    with torch.cuda.device(dev):
+                        _lib.check(lib.b2048_ppo_coefficients(
+                            h, _ptr(idx), k, _ptr(z), _ptr(v), _ptr(mflags) if self._use_mask else None, _ptr(acts),
+                            _ptr(logp_old), _ptr(adv), _ptr(gae), _ptr(values), float(size), clip_eps, vclip, huber,
+                            float(cfg.huber_delta), _ptr(cf), _ptr(gc), _ptr(ep_stats[e]), _stream()), "b2048_ppo_coefficients")
+                    self._backward(self._actor, bx, fx, ax, cf, k, 0, p, chunk, fell_back)
+                    self._backward(self._critic, bx, fx, ax, gc, k, 1, p, chunk, fell_back)
+                else:                                          # this shard holds none of the minibatch's samples
+                    self._actor.grad.zero_()
+                    self._critic.grad.zero_()
+                if shared is not None:
+                    self._merge_shared_grads()
+                if allreduce is not None:
+                    allreduce(self._grad_all)                  # ONE message per minibatch step
+                ss_a, ss_c = self._optimizer_step()
+                norms[e * M + m, 0] = ss_a[0]
+                if ss_c is not None:
+                    norms[e * M + m, 1] = ss_c[0]
+        st = ep_stats.cpu().numpy() / n
+        nr = norms.sqrt().cpu().numpy()
+        info: dict[str, Any] = {
+            "clip_fraction": st[:, 0].tolist(), "mean_ratio": st[:, 1].tolist(), "approx_kl": st[:, 2].tolist(),
+            "surrogate": st[:, 3].tolist(), "value_loss": st[:, 4].tolist(), "actor_grad_norms": nr[:, 0].tolist(),
+            "advantages": adv, "gae": gae, "values_old": values, "logp_old": logp_old,
+            "precision": self._update_mode_name(prec, n) + (" [fell back to fp32: non-finite fp16 intermediates]" if fell_back else "")}
+        info["actor_grad_norm"] = info["actor_grad_norms"][-1]
+        if shared is None:
+            info["critic_grad_norms"] = nr[:, 1].tolist()
+            info["critic_grad_norm"] = info["critic_grad_norms"][-1]
+        self.last_update_info = info
+        if self._logger.isEnabledFor(logging.INFO):
+            self._logger.info(f"PPO: clip fraction {info['clip_fraction']}, approx KL {info['approx_kl']}")
+        return info
+
     # ------------------------------------------------------------------ bootstrapping at truncation
     def _check_bootstrap(self, ro: Rollout, window: bool) -> None:
         if not (self.agent_config.use_critic and getattr(self, "_critic", None) is not None):
@@ -765,6 +1003,13 @@ class ReinforceAgent:
         v B + b, and it folds the value of variant v of s'."""
         if boot is None or boot[0].numel() == 0:
             return self._update(ro, window, chunk, allreduce, precision, exchange)
+        folded, slots, nxt, values = self._fold_truncation(ro, boot, precision)
+        info = self._update(folded, window, chunk, allreduce, precision, exchange)
+        info.update(bootstrap_slots=slots, bootstrap_boards=nxt, bootstrap_values=values)
+        return info
+
+    def _fold_truncation(self, ro: Rollout, boot, precision: int | str):
+        """(ro with the rewards r + gamma V(s') at the truncated steps, slots, s', V(s')); see _update_bootstrapped."""
         slots, nxt = boot
         lib, h, dev = self._lib, self._h, self.device
         T, B = ro.T, ro.B
@@ -779,20 +1024,14 @@ class ReinforceAgent:
             nxt = nxt8
         K = slots.numel()
         prec = 2 if precision == "auto" else int(precision)
-        # the tensor-core forwards take 4096 boards or more; a shorter list runs where "auto" would put it
-        vprec = prec if (K >= 4096 or prec in (0, 2)) else (2 if prec == 3 else 0)
         values = torch.empty(K, dtype=torch.float32, device=dev)
-        self._values(nxt, values, vprec)
-        if vprec in (2, 3) and not bool(torch.isfinite(values).all()):   # fp16 range exceeded: as in _update
-            self._values(nxt, values, 0)
+        self._forward_checked(self._critic, nxt, values, self._small_batch_precision(prec, K))
         rewards = torch.empty((T, B), dtype=torch.float32, device=dev)
         with torch.cuda.device(dev):
             _lib.check(lib.b2048_fold_bootstrap(h, _ptr(ro.rewards[:T].contiguous()), _ptr(slots), _ptr(values), K, T * B,
                                                 float(self.agent_config.gamma), _ptr(rewards), _stream()),
                        "b2048_fold_bootstrap")
-        info = self._update(replace(ro, rewards=rewards), window, chunk, allreduce, precision, exchange)
-        info.update(bootstrap_slots=slots, bootstrap_boards=nxt, bootstrap_values=values)
-        return info
+        return replace(ro, rewards=rewards), slots, nxt, values
 
     def _segment_targets(self, rewards, flags, values, lam, n_traj, v, td, gcoef, valid_len) -> None:
         cfg = self.agent_config
@@ -924,29 +1163,7 @@ class ReinforceAgent:
         def backward(net: DeviceMLP, cf: torch.Tensor, head_mode: int):
             if live is not None:
                 cf = cf.index_select(0, live)
-            ws_floats = int(lib.b2048_backward_workspace_floats(C.byref(net.desc), min(chunk, n)))
-            ws = self._buf("bwd_ws", (ws_floats,), torch.float32)
-            for p_try in ((prec, 0) if prec in (2, 3) else (prec,)):
-                net.grad.zero_()
-                with torch.cuda.device(dev):
-                    _lib.check(lib.b2048_mlp_backward(h, _ptr(boards), _ptr(mflags) if self._use_mask else None, _ptr(acts),
-                                                      _ptr(cf), C.byref(net.desc), _ptr(net.grad), n, head_mode, _ptr(ws),
-                                                      ws_floats, min(chunk, n), p_try, _stream()), "b2048_mlp_backward")
-                # The split-fp16 path keeps activations and (loss-scaled) deltas in fp16: a network whose activations leave
-                # the fp16 range (> 65504) would give a non-finite gradient.  Never apply that: redo the pass in fp32.
-                if p_try == 0 or bool(torch.isfinite(net.grad).all()):
-                    break
-                fell_back.append(head_mode)
-                self._logger.warning("tensor-core gradient not finite (fp16 range exceeded); recomputing on the fp32 kernels")
-
-        def apply(net: DeviceMLP, lr: float, sign: float, t_adam: int) -> float:
-            sumsq = self._buf("sumsq_" + str(sign), (1,), torch.float64)
-            with torch.cuda.device(dev):
-                _lib.check(lib.b2048_apply_update(h, _ptr(net.theta), _ptr(net.grad), _ptr(net.adam_m), _ptr(net.adam_v),
-                                                  net.n_params, OPTIMIZER[cfg.optimizer], float(lr), float(sign),
-                                                  float(cfg.max_grad_norm), float(cfg.adam_beta1), float(cfg.adam_beta2),
-                                                  int(t_adam), _ptr(sumsq), _stream()), "b2048_apply_update")
-            return sumsq
+            self._backward(net, boards, mflags, acts, cf, n, head_mode, prec, chunk, fell_back)
 
         if critic:
             # critic block (reinforce_agent.py:403-498): V(s_t) for every stored state, TD(0) errors, critic grads
@@ -955,10 +1172,8 @@ class ReinforceAgent:
             vboards = ro.boards[:nv].reshape(-1) if window else boards
             values = self._buf("values", (nv, B), torch.float32)
             vc = values.view(-1) if live is None else self._buf("values_c", (n,), torch.float32)
-            self._values(vboards, vc, prec)
-            if prec in (2, 3) and not bool(torch.isfinite(vc).all()):        # fp16 range exceeded in the value forward
+            if self._forward_checked(self._critic, vboards, vc, prec):
                 fell_back.append(1)
-                self._values(vboards, vc, 0)
             if live is not None:
                 values.zero_()
                 values.view(-1)[live] = vc
@@ -1006,14 +1221,7 @@ class ReinforceAgent:
             if allreduce is not None:
                 allreduce(self._grad_all)    # ONE message per update: [actor gradient | critic gradient]
 
-        if cfg.optimizer == "adam":
-            self._adam_t += 1
-        ss_a = apply(self._actor if shared is None else shared, cfg.learning_rate, +1.0, self._adam_t)
-        ss_c = None
-        if cfg.use_critic and self._critic is not None and shared is None:
-            if cfg.optimizer == "adam":
-                self._adam_t_c += 1
-            ss_c = apply(self._critic, cfg.critic_learning_rate, -1.0, getattr(self, "_adam_t_c", 0))
+        ss_a, ss_c = self._optimizer_step()
         info["advantages"] = adv
         info["precision"] = self._update_mode_name(prec, n) + (" [fell back to fp32: non-finite fp16 intermediates]" if fell_back else "")
         info["actor_grad_norm"] = float(ss_a.cpu()[0]) ** 0.5

@@ -20,6 +20,9 @@ and zero counts when none did); a resumed run starts from fresh resets.  Not com
 ``train.bootstrap_truncation`` (default false; needs ``agent.use_critic`` or a ``shared_trunk`` section): in both modes, an
 episode truncated by ``env.max_steps`` gets the target r + gamma V(s') at its last step, s' being the board it was cut on,
 instead of r (``update_from_rollout`` / ``update_from_horizon(bootstrap_truncation=True)``).
+``train.ppo`` (default None; needs ``train.horizon`` and ``agent.use_critic`` or a ``shared_trunk`` section): a dict with any of
+``epochs`` (4), ``minibatches`` (4), ``clip_eps`` (0.2), ``value_clip_eps`` (None) trains every window with
+``update_ppo`` instead; the shuffle seed of batch k is derived from ``seed`` and k.  The CSV columns are unchanged.
 
     python -m torch.distributed.run ... b2048_runner.py -conf cfg.json      (or: python b2048_runner.py -conf cfg.json)
 """
@@ -55,6 +58,7 @@ DEFAULTS: dict[str, Any] = {
     "eval": dict(num_episodes=2048, model_path=None, use_greedy=True),
 }
 TILE_BINS = [16, 32, 64, 128, 256, 512, 1024, 2048, 4096]      # runner.py:557
+PPO_KEYS = {"epochs", "minibatches", "clip_eps", "value_clip_eps"}
 
 
 def merge_config(user: dict[str, Any] | None) -> dict[str, Any]:
@@ -113,6 +117,15 @@ def training(cfg: dict[str, Any], info: bd.DistInfo | None = None, device=None, 
             raise ValueError(f"train.horizon must be a positive number of steps, got {horizon}")
         if tr.get("seed_streams", "philox") == "numpy":
             raise ValueError("train.horizon needs seed_streams='philox': the reference-seeded episodes play to termination")
+    ppo = tr.get("ppo")
+    if ppo is not None:
+        if horizon is None:
+            raise ValueError("train.ppo needs train.horizon: PPO trains on fixed-horizon windows")
+        if not (cfg["agent"].get("use_critic") or cfg.get("shared_trunk") is not None):
+            raise ValueError("train.ppo needs a value function: agent.use_critic or a shared_trunk section")
+        unknown = set(ppo) - PPO_KEYS
+        if unknown:
+            raise ValueError(f"train.ppo: unknown keys {sorted(unknown)} (allowed: {sorted(PPO_KEYS)})")
     env, agent = build(cfg, int(tr["batch_size"]), info, device)
     out_dir = tr.get("out_dir")
     rows: list[dict[str, Any]] = []
@@ -153,7 +166,7 @@ def training(cfg: dict[str, Any], info: bd.DistInfo | None = None, device=None, 
         t0 = time.perf_counter()
         global_step = step + 1                                                             # 1-based like runner.py:610
         if horizon is not None:
-            row, ro, upd = _horizon_batch(agent, env, info, tr, horizon, global_step, best, out_dir)
+            row, ro, upd = _horizon_batch(agent, env, info, tr, horizon, global_step, best, out_dir, int(cfg["seed"]))
             avg, mx, mn = row["avg_reward"], row["max_reward"], row["min_reward"]
             if avg > best:
                 best = avg
@@ -196,14 +209,17 @@ def training(cfg: dict[str, Any], info: bd.DistInfo | None = None, device=None, 
 
 
 def _horizon_batch(agent, env, info: bd.DistInfo, tr: dict[str, Any], horizon: int, global_step: int, best: float,
-                   out_dir: str | None):
+                   out_dir: str | None, seed: int):
     """One fixed-horizon batch: the window, its update, and the CSV row of the episodes that ended inside it (over all
     ranks).  A record average is checkpointed with the parameters that played the window, as the episode batches are."""
     ro = agent.rollout_many(env, horizon=horizon, reset=False, precision=tr.get("precision", "auto"))
     saving = global_step > 30 and info.rank == 0 and bool(out_dir)
     before = agent.save_state() if saving else None
+    ppo = tr.get("ppo")
+    if ppo is not None:                                    # a fresh minibatch shuffle for every window, the same on every rank
+        ppo = dict(ppo, shuffle_seed=(seed * 0x9E3779B97F4A7C15 + 0xBF58476D1CE4E5B9 * global_step) & (2**64 - 1))
     upd = bd.sharded_update(agent, ro, info, total_episodes=int(tr["batch_size"]), exchange=tr.get("exchange", "default"),
-                            fixed_horizon=True, bootstrap_truncation=bool(tr.get("bootstrap_truncation", False)))
+                            fixed_horizon=True, bootstrap_truncation=bool(tr.get("bootstrap_truncation", False)), ppo=ppo)
     es = agent.horizon_episode_stats(reset=True, info=info)
     avg = es["avg_reward"]
     if saving and avg > best:                                                              # runner.py:643-660
