@@ -451,6 +451,17 @@ int b2048_mlp_backward(b2048_handle* h, const uint64_t* board, const uint8_t* ma
                        const uint8_t* action, const float* coef, const b2048_mlp_desc* mlp, float* grads,
                        int64_t n, int32_t head_mode, float* workspace, int64_t workspace_floats,
                        int64_t chunk, int32_t precision, void* stream);
+/* The policy head with an entropy bonus (A2C / PPO's +beta H(pi(.|s))):
+ *   grads += d/dtheta sum_s [coef[s] log pi(action[s] | board[s]) + ent_coef[s] H_s],  H_s = -sum_{legal j} p_j log p_j
+ * over the legal actions of the masked softmax (outputs j >= n_out are padding).  The head delta is
+ * d_j = coef (1[a = j] - p_j) - ent_coef p_j (log p_j + H_s): exactly 0 for illegal / padded outputs and for a board with one
+ * legal move.  ent_sum (nullable, device double[1]) += sum_s H_s.  Precisions 0, 2 and 3 dispatch exactly as b2048_mlp_backward
+ * (the same kernel families, in their entropy variants; the fp16 loss scale comes from max(|coef| + 1.5 |ent_coef|)); precision 1 returns
+ * B2048_ERR_UNSUPPORTED.  Workspace as b2048_mlp_backward (b2048_backward_workspace_floats). */
+int b2048_mlp_backward_entropy(b2048_handle* h, const uint64_t* board, const uint8_t* mask_flags, const uint8_t* action,
+                               const float* coef, const float* ent_coef, const b2048_mlp_desc* mlp, float* grads, int64_t n,
+                               float* workspace, int64_t workspace_floats, int64_t chunk, int32_t precision,
+                               double* ent_sum, void* stream);
 /* Test / debug access to the tensor-core path's workspace: byte offsets (from the workspace pointer rounded up to
  * 1024 B) of the bf16 images H1, H2, DL2, DL1 ([64-sample tile][4 feature slabs][64 rows][128 B, 128-byte
  * swizzle]) and A1^T, d3^T ([tile][16 rows][128 B]), then the total. */

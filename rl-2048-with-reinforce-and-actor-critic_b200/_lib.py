@@ -96,6 +96,8 @@ SIGNATURES = {
                                _f32, _vp, _vp, _vp, _vp],
     "b2048_backward_workspace_floats": [C.POINTER(MlpDesc), _i64],
     "b2048_mlp_backward": [_vp, _vp, _vp, _vp, _vp, C.POINTER(MlpDesc), _vp, _i64, _i32, _vp, _i64, _i64, _i32, _vp],
+    "b2048_mlp_backward_entropy": [_vp, _vp, _vp, _vp, _vp, _vp, C.POINTER(MlpDesc), _vp, _i64, _vp, _i64, _i64, _i32, _vp,
+                                   _vp],
     "b2048_backward_tc_layout": [_i64, _vp],
     "b2048_apply_update": [_vp, _vp, _vp, _vp, _vp, _i64, _i32, _f32, _f32, _f32, _f32, _f32, _i32, _vp, _vp],
 }

@@ -111,10 +111,13 @@ int64_t backward_hp_workspace_bytes(int64_t chunk);
 int launch_forward_hp(b2048_handle* h, const b2048_mlp_desc* mlp, const uint64_t* board, float* out, int64_t n, cudaStream_t stream);
 int launch_backward_hp(b2048_handle* h, const uint64_t* board, const uint8_t* mask_flags, const uint8_t* action,
                        const float* coef, const b2048_mlp_desc* mlp, float* grads, int64_t n, int head_mode,
-                       uint8_t* workspace, int64_t workspace_bytes, int64_t chunk, cudaStream_t stream);
+                       uint8_t* workspace, int64_t workspace_bytes, int64_t chunk, cudaStream_t stream,
+                       const float* ent_coef = nullptr, double* ent_sum = nullptr);
 // scale[0] = S, the power of two that brings max |coef[0 .. n)| into [32, 64); scale[1] = 1 / S; scale[2] = bits of the max.
-// The fp16 backward passes multiply their deltas by S.
-int launch_loss_scale(const b2048_handle* h, const float* coef, int64_t n, float* scale, cudaStream_t stream);
+// The fp16 backward passes multiply their deltas by S.  ent_coef != NULL (the entropy bonus): the max is taken of
+// |coef| + 1.5 |ent_coef|, a bound of the head delta (b2048_entropy.cuh).
+int launch_loss_scale(const b2048_handle* h, const float* coef, int64_t n, float* scale, cudaStream_t stream,
+                      const float* ent_coef = nullptr);
 
 // ---- b2048_mlp_gen.cu: the shape-generic kernels
 int64_t gen_workspace_bytes(const b2048_mlp_desc* mlp, int64_t chunk);
@@ -124,7 +127,7 @@ int launch_forward_gen(b2048_handle* h, const b2048_mlp_desc* mlp, const uint64_
                        const int32_t* n_dev = nullptr);
 int launch_backward_gen(b2048_handle* h, const uint64_t* board, const uint8_t* mask_flags, const uint8_t* action, const float* coef,
                         const b2048_mlp_desc* mlp, float* grads, int64_t n, int head_mode, uint8_t* workspace, int64_t chunk,
-                        cudaStream_t stream);
+                        cudaStream_t stream, const float* ent_coef = nullptr, double* ent_sum = nullptr);
 
 // ---- b2048_env.cu: the step of b2048_rollout_many_np (generic step kernel, spawns from the boards' NumPy env streams)
 int launch_step_np(b2048_handle* h, const uint64_t* board_in, uint64_t* board_out, uint32_t* score, uint32_t* step,

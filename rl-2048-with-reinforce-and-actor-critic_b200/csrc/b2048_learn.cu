@@ -14,6 +14,7 @@
 //      ppo_logp_kernel           PPO: log pi_old(a | s) from the learner's logits
 //      ppo_coef_kernel           PPO: ratio, clipped-surrogate and clipped-value coefficients of one minibatch
 //   K6 mlp_backward_kernel       _backpropagation per tile  src/reinforce_agent.py:639-678 (deltas + activations)
+//                                (<BackwardEntArgs>: the policy head's delta with the entropy bonus, b2048_entropy.cuh)
 //      atb_kernel                dW_l = A_l^T D_l           (sum over samples of np.outer, :666)
 //      colsum_kernel             db_l = sum_s D_l
 //      sumsq / clip / sgd / adam clip_grads_global_norm :835-861, SGD :565-575, _adam_update :719-770
@@ -22,8 +23,10 @@
 // the per-board scans are fully coalesced.
 #include <cuda_runtime.h>
 
+#include <type_traits>
 #include <vector>
 
+#include "b2048_entropy.cuh"
 #include "b2048_horizon.cuh"
 #include "b2048_internal.h"
 #include "b2048_mlp.cuh"
@@ -352,7 +355,36 @@ struct BackwardArgs {
     int head_mode;                   // 0: actor, d_L = coef * (onehot(a) - pi);  1: value head, d_L = coef
 };
 
-__global__ void __launch_bounds__(kMlpThreads, 1) mlp_backward_kernel(const __grid_constant__ BackwardArgs args) {
+// The entropy variant's extra arguments (b2048_mlp_backward_entropy): per-sample ecoef and the optional sum of H.
+struct BackwardEntArgs : BackwardArgs {
+    const float* ent_coef;
+    double* ent_sum;                 // nullable: += sum_s H_s over the valid samples
+};
+
+// Quad softmax of mlp_backward_kernel with the entropy term t_j of b2048_entropy.cuh (H from a two-step shfl_xor over the quad).
+__device__ __forceinline__ float quad_softmax_entropy(float logit, bool legal, bool use_mask, bool live, uint32_t legal_row,
+                                                      float& t, float& H) {
+    float l = (use_mask && !legal) ? -1e9f : logit;
+    float mx = fmaxf(l, __shfl_xor_sync(0xFFFFFFFFu, l, 1));
+    mx = fmaxf(mx, __shfl_xor_sync(0xFFFFFFFFu, mx, 2));
+    const float z = l - mx;
+    float e = expf(z);
+    float s = e + __shfl_xor_sync(0xFFFFFFFFu, e, 1);
+    s = s + __shfl_xor_sync(0xFFFFFFFFu, s, 2);
+    const float p = e / s, lse = logf(s);
+    float pz = entropy_pz(z, p, live);
+    pz += __shfl_xor_sync(0xFFFFFFFFu, pz, 1);
+    pz += __shfl_xor_sync(0xFFFFFFFFu, pz, 2);
+    H = entropy_h(lse, pz, legal_row != 0u);
+    t = entropy_term(z, lse, p, H, live);
+    return p;
+}
+
+// A = BackwardArgs: the delta of update_batch's policy / value head; A = BackwardEntArgs: the policy head with the entropy
+// bonus, d_j = coef (1[a = j] - p_j) - ecoef t_j (b2048_entropy.cuh)
+template <class A>
+__global__ void __launch_bounds__(kMlpThreads, 1) mlp_backward_kernel(const __grid_constant__ A args) {
+    constexpr bool kEnt = std::is_same<A, BackwardEntArgs>::value;
     extern __shared__ __align__(16) float arena[];
     const MlpDev& m = args.mlp;
     const int L = m.n_layers;
@@ -373,9 +405,25 @@ __global__ void __launch_bounds__(kMlpThreads, 1) mlp_backward_kernel(const __gr
             const bool use_mask = args.mask_flags != nullptr;
             if (use_mask && valid) fl = args.mask_flags[s];
             if (j >= n_out) out = -INFINITY;
-            float p = quad_softmax(out, (fl >> j) & 1u, use_mask);
-            uint32_t a = valid ? args.action[s] : 0u;
-            d = cf * ((a == (uint32_t)j ? 1.0f : 0.0f) - p);  // reinforce_agent.py:340-344
+            if constexpr (kEnt) {
+                // legal outputs of the row: the mask's bits below n_out (every output below n_out without a mask)
+                const uint32_t legal_row = (use_mask ? fl : 0xFu) & ((1u << n_out) - 1u);
+                float t, H;
+                const float p = quad_softmax_entropy(out, (fl >> j) & 1u, use_mask, (legal_row >> j) & 1u, legal_row, t, H);
+                const float ecf = valid ? args.ent_coef[s] : 0.0f;
+                uint32_t a = valid ? args.action[s] : 0u;
+                d = cf * ((a == (uint32_t)j ? 1.0f : 0.0f) - p) - ecf * t;
+                if (args.ent_sum) {             // H of the warp's 8 samples (lane j == 0 of each quad): one float64 atomic per warp
+                    float hs = (valid && j == 0) ? H : 0.0f;
+#pragma unroll
+                    for (int o = 16; o > 0; o >>= 1) hs += __shfl_xor_sync(0xFFFFFFFFu, hs, o);
+                    if ((threadIdx.x & 31) == 0 && hs != 0.0f) atomicAdd(args.ent_sum, (double)hs);
+                }
+            } else {
+                float p = quad_softmax(out, (fl >> j) & 1u, use_mask);
+                uint32_t a = valid ? args.action[s] : 0u;
+                d = cf * ((a == (uint32_t)j ? 1.0f : 0.0f) - p);  // reinforce_agent.py:340-344
+            }
         } else {
             d = cf;
         }
@@ -845,52 +893,59 @@ extern "C" int64_t b2048_backward_workspace_floats(const b2048_mlp_desc* mlp, in
 // Accumulates into grads (flat, same layout as the flat parameter vector: W_0, b_0, W_1, b_1, ...):
 //   head_mode 0: d/dtheta sum_s coef[s] * log pi(action[s] | board[s])        (policy gradient, ascent direction)
 //   head_mode 1: d/dtheta sum_s coef[s] * V(board[s])                          (value head; coef = dLoss/dV * weight)
-extern "C" int b2048_mlp_backward(b2048_handle* h, const uint64_t* board, const uint8_t* mask_flags,
-                                  const uint8_t* action, const float* coef, const b2048_mlp_desc* mlp, float* grads,
-                                  int64_t n, int32_t head_mode, float* workspace, int64_t workspace_floats,
-                                  int64_t chunk, int32_t precision, void* stream) {
-    B2_REQUIRE(h != nullptr, "b2048_mlp_backward: handle is NULL");
-    B2_REQUIRE(n >= 0, "b2048_mlp_backward: n < 0");
+// ent_coef != NULL (policy head only): + d/dtheta sum_s ent_coef[s] * H(pi(. | board[s])) on the entropy variants of the
+// kernels, ent_sum (nullable) += sum_s H.  `who` names the entry point in the error messages.
+static int mlp_backward(b2048_handle* h, const uint64_t* board, const uint8_t* mask_flags, const uint8_t* action,
+                        const float* coef, const float* ent_coef, const b2048_mlp_desc* mlp, float* grads, int64_t n,
+                        int32_t head_mode, float* workspace, int64_t workspace_floats, int64_t chunk, int32_t precision,
+                        double* ent_sum, void* stream, const std::string& who) {
+    B2_REQUIRE(h != nullptr, who + ": handle is NULL");
+    B2_REQUIRE(n >= 0, who + ": n < 0");
     if (n == 0) return B2048_OK;
-    B2_REQUIRE(board && coef && grads && workspace, "b2048_mlp_backward: NULL buffer");
-    B2_REQUIRE(head_mode == 1 || action != nullptr, "b2048_mlp_backward: action required for the policy head");
-    B2_REQUIRE(chunk > 0, "b2048_mlp_backward: chunk must be positive");
+    B2_REQUIRE(board && coef && grads && workspace, who + ": NULL buffer");
+    B2_REQUIRE(head_mode == 1 || action != nullptr, who + ": action required for the policy head");
+    B2_REQUIRE(chunk > 0, who + ": chunk must be positive");
     B2_REQUIRE(precision >= 0 && precision <= 3,
-               "b2048_mlp_backward: precision must be 0 (fp32), 1 (bf16 tcgen05), 2 (auto) or 3 (split-fp16 tcgen05)");
+               who + ": precision must be 0 (fp32), 1 (bf16 tcgen05), 2 (auto) or 3 (split-fp16 tcgen05)");
+    const bool ent = ent_coef != nullptr;
     if (precision == 2 || precision == 3) {   // float32-grade tensor-core path (what "auto" selects)
         const bool ok = backward_hp_supported(h, mlp) && n >= 4096 &&
                         workspace_floats * 4 >= backward_hp_workspace_bytes(chunk < n ? chunk : n);
         if (ok)
             return launch_backward_hp(h, board, mask_flags, action, coef, mlp, grads, n, head_mode,
                                       reinterpret_cast<uint8_t*>(workspace), workspace_floats * 4 - 1024, chunk < n ? chunk : n,
-                                      (cudaStream_t)stream);
+                                      (cudaStream_t)stream, ent_coef, ent_sum);
         // every other ReLU shape with 64-multiple hidden layers (the reference's documented one-hot [256, 128, 64] network):
         // the shape-generic kernels of b2048_mlp_gen.cu, same arithmetic
         if (!backward_hp_supported(h, mlp) && gen_supported(h, mlp) && n >= 4096 &&
             workspace_floats * 4 >= gen_workspace_bytes(mlp, chunk < n ? chunk : n))
             return launch_backward_gen(h, board, mask_flags, action, coef, mlp, grads, n, head_mode,
-                                       reinterpret_cast<uint8_t*>(workspace), chunk < n ? chunk : n, (cudaStream_t)stream);
+                                       reinterpret_cast<uint8_t*>(workspace), chunk < n ? chunk : n, (cudaStream_t)stream,
+                                       ent_coef, ent_sum);
         if (precision == 3)
             return fail(B2048_ERR_UNSUPPORTED,
-                        "b2048_mlp_backward: the split-fp16 tcgen05 path needs a ReLU network with 1-4 hidden layers of 64 / 128 / "
+                        who + ": the split-fp16 tcgen05 path needs a ReLU network with 1-4 hidden layers of 64 / 128 / "
                         "192 / 256 units, log2 or one-hot observations, n >= 4096 and a workspace of "
                         "b2048_backward_workspace_floats()");
     }
     if (precision == 1) {                     // single-bf16 tensor cores: an explicit opt-in (5 % class gradient error)
+        if (ent)
+            return fail(B2048_ERR_UNSUPPORTED, who + ": the single-bf16 path (precision 1) has no entropy variant");
         const bool ok = backward_tc_supported(h, mlp) && n >= 4096 &&
                         workspace_floats * 4 >= backward_tc_workspace_bytes(chunk < n ? chunk : n);
         if (ok)
             return launch_backward_tc(h, board, mask_flags, action, coef, mlp, grads, n, head_mode,
                                       reinterpret_cast<uint8_t*>(workspace), chunk < n ? chunk : n, (cudaStream_t)stream);
         return fail(B2048_ERR_UNSUPPORTED,
-                    "b2048_mlp_backward: the tcgen05 path needs a 16-256-256-(<=4) ReLU network, raw/log2 observations, "
+                    who + ": the tcgen05 path needs a 16-256-256-(<=4) ReLU network, raw/log2 observations, "
                     "n >= 4096 and a workspace of b2048_backward_workspace_floats()");
     }
-    BackwardArgs a;
+    BackwardEntArgs ea;
+    BackwardArgs& a = ea;
     size_t smem = 0;
-    int st = validate_mlp(mlp, &a.mlp, &smem, h->smem_optin, "b2048_mlp_backward");
+    int st = validate_mlp(mlp, &a.mlp, &smem, h->smem_optin, who.c_str());
     if (st != B2048_OK) return st;
-    B2_REQUIRE(workspace_floats >= b2048_backward_workspace_floats(mlp, chunk), "b2048_mlp_backward: workspace too small");
+    B2_REQUIRE(workspace_floats >= b2048_backward_workspace_floats(mlp, chunk), who + ": workspace too small");
     const int L = a.mlp.n_layers;
     const int* dims = a.mlp.dims;
     cudaStream_t s = (cudaStream_t)stream;
@@ -908,7 +963,8 @@ extern "C" int b2048_mlp_backward(b2048_handle* h, const uint64_t* board, const 
     }
     float *gW[B2048_MAX_LAYERS], *gb[B2048_MAX_LAYERS];
     carve_grads(mlp, grads, gW, gb);
-    B2_CUDA(cudaFuncSetAttribute(mlp_backward_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    if (ent) B2_CUDA(cudaFuncSetAttribute(mlp_backward_kernel<BackwardEntArgs>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    else B2_CUDA(cudaFuncSetAttribute(mlp_backward_kernel<BackwardArgs>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     for (int64_t c0 = 0; c0 < n; c0 += chunk) {
         const int64_t cn = (n - c0) < chunk ? (n - c0) : chunk;
         a.board = board + c0;
@@ -919,7 +975,13 @@ extern "C" int b2048_mlp_backward(b2048_handle* h, const uint64_t* board, const 
         a.head_mode = head_mode;
         int64_t tiles = (cn + kTileM - 1) / kTileM;
         int grid = (int)(tiles < h->num_sms ? tiles : h->num_sms);
-        mlp_backward_kernel<<<grid, kMlpThreads, smem, s>>>(a);
+        if (ent) {
+            ea.ent_coef = ent_coef + c0;
+            ea.ent_sum = ent_sum;
+            mlp_backward_kernel<BackwardEntArgs><<<grid, kMlpThreads, smem, s>>>(ea);
+        } else {
+            mlp_backward_kernel<BackwardArgs><<<grid, kMlpThreads, smem, s>>>(a);
+        }
         for (int l = 0; l < L; ++l) {
             const int Mi = dims[l], N = dims[l + 1];
             int split = (int)((cn + 4095) / 4096);
@@ -939,6 +1001,25 @@ extern "C" int b2048_mlp_backward(b2048_handle* h, const uint64_t* board, const 
     }
     B2_CUDA(cudaGetLastError());
     return B2048_OK;
+}
+
+extern "C" int b2048_mlp_backward(b2048_handle* h, const uint64_t* board, const uint8_t* mask_flags,
+                                  const uint8_t* action, const float* coef, const b2048_mlp_desc* mlp, float* grads,
+                                  int64_t n, int32_t head_mode, float* workspace, int64_t workspace_floats,
+                                  int64_t chunk, int32_t precision, void* stream) {
+    return mlp_backward(h, board, mask_flags, action, coef, nullptr, mlp, grads, n, head_mode, workspace, workspace_floats, chunk,
+                        precision, nullptr, stream, "b2048_mlp_backward");
+}
+
+// The policy head with the entropy bonus: grads += d/dtheta sum_s [coef[s] log pi(action[s] | board[s]) + ent_coef[s] H_s]
+// (b2048_entropy.cuh); ent_sum (nullable, device double) += sum_s H_s.  Dispatch as b2048_mlp_backward; precision 1 is refused.
+extern "C" int b2048_mlp_backward_entropy(b2048_handle* h, const uint64_t* board, const uint8_t* mask_flags, const uint8_t* action,
+                                          const float* coef, const float* ent_coef, const b2048_mlp_desc* mlp, float* grads,
+                                          int64_t n, float* workspace, int64_t workspace_floats, int64_t chunk,
+                                          int32_t precision, double* ent_sum, void* stream) {
+    B2_REQUIRE(n <= 0 || ent_coef != nullptr, "b2048_mlp_backward_entropy: NULL buffer");
+    return mlp_backward(h, board, mask_flags, action, coef, ent_coef, mlp, grads, n, 0, workspace, workspace_floats, chunk,
+                        precision, ent_sum, stream, "b2048_mlp_backward_entropy");
 }
 
 // clip by global norm + optimiser step on a flat parameter vector (actor or critic).

@@ -19,14 +19,18 @@
 //                  power-of-two loss scale (the coefficients are ~1e-8).  Rounding the backward operands perturbs the
 //                  gradient linearly (no mask flips): 0.04 % at fp16.
 //  atb_tc_kernel   (b2048_learn_tc.cu) the dW GEMMs on the fp16 images, un-scaled on the way out.
+//  bwd_tc_ent_kernel / update_pipe_ent_kernel   bwd_tc_kernel / update_pipe_kernel with the entropy bonus in the policy head's
+//                  delta (b2048_mlp_backward_entropy, b2048_entropy.cuh)
 #include <cuda_fp16.h>
 #include <cuda_runtime.h>
 
 #include <cstdio>
 #include <ctime>
+#include <type_traits>
 #include <unistd.h>
 
 #include "b2048_device.cuh"
+#include "b2048_entropy.cuh"
 #include "b2048_internal.h"
 #include "b2048_tc.cuh"
 #include "b2048_learn_tc.cuh"
@@ -558,6 +562,16 @@ struct BwdArgs {
     long long* debug_clock;   // optional phase timestamps of CTA 0 (B2048_DBG_TC_CLOCKS), else NULL
 };
 
+// The entropy variant's extra arguments: per-sample ecoef and the optional sum of H over the valid samples.
+struct BwdEnt {
+    const float* ent_coef;
+    double* ent_sum;              // nullable
+};
+struct BwdEntArgs {
+    BwdArgs b;
+    BwdEnt e;
+};
+
 constexpr int BW_THREADS = 512 + 32 + 128;
 
 // Backward deltas of one 128-sample tile at a time, and the input-layer gradient:
@@ -566,7 +580,10 @@ constexpr int BW_THREADS = 512 + 32 + 128;
 //   D4 = DL2 W2 (TMEM columns 256..511)  ->  DL1 = D4 . [z1 > 0]  -> A2
 //   dW1^T += DL1^T [A1 | 1]  (TMEM columns 128..191, N = 32: columns 0..15 = the 16 inputs, column 16 = the bias gradient);
 //   DL1 never leaves the SM; the accumulators stay in TMEM for all tiles of the CTA and are added to the gradient once.
-__device__ __forceinline__ void bwd_role(const BwdArgs& args, const PipeCtx& px, const int rank, const int nranks, uint8_t* smem) {
+// kEnt: the policy head's delta carries the entropy bonus, d_j = coef (1[a = j] - p_j) - ecoef t_j (b2048_entropy.cuh)
+template <bool kEnt>
+__device__ __forceinline__ void bwd_role(const BwdArgs& args, const BwdEnt& ent, const PipeCtx& px, const int rank, const int nranks,
+                                         uint8_t* smem) {
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const bool piped = px.f_done != nullptr;
     uint64_t* bars = reinterpret_cast<uint64_t*>(smem + SM_BAR);
@@ -776,7 +793,7 @@ __device__ __forceinline__ void bwd_role(const BwdArgs& args, const PipeCtx& px,
             const bool valid = s < args.n;
             const bool use_mask = args.mask_flags != nullptr;
             uint32_t fl = 0xFu, act = 0;
-            float cf = 0.0f, lg[4] = {0.0f, 0.0f, 0.0f, 0.0f};
+            float cf = 0.0f, ecf = 0.0f, lg[4] = {0.0f, 0.0f, 0.0f, 0.0f};
             const uint64_t bd = valid ? args.board[s] : 0ull;
             if (piped) {
                 if (lane == 0) flag_wait(px.f_done + tile);
@@ -786,6 +803,7 @@ __device__ __forceinline__ void bwd_role(const BwdArgs& args, const PipeCtx& px,
                 if (use_mask) fl = args.mask_flags[s];
                 if (args.action) act = args.action[s];
                 cf = args.coef[s];
+                if constexpr (kEnt) ecf = ent.ent_coef[s];
                 if (args.head_mode == 0) {
 #pragma unroll
                     for (int j = 0; j < 4; ++j)
@@ -801,8 +819,23 @@ __device__ __forceinline__ void bwd_role(const BwdArgs& args, const PipeCtx& px,
                 float e[4], sum = 0.0f;
 #pragma unroll
                 for (int j = 0; j < 4; ++j) { e[j] = expf(m[j] - mx); sum += e[j]; }
+                if constexpr (kEnt) {
+                    float z[4], p[4], t[4];
 #pragma unroll
-                for (int j = 0; j < 4; ++j) d[j] = cf * ((act == (uint32_t)j ? 1.0f : 0.0f) - e[j] / sum);   // reinforce_agent.py:340-344
+                    for (int j = 0; j < 4; ++j) { z[j] = m[j] - mx; p[j] = e[j] / sum; }
+                    const float H = entropy_row(z, logf(sum), p, use_mask ? fl : 0xFu, args.n_out, t);
+#pragma unroll
+                    for (int j = 0; j < 4; ++j) d[j] = cf * ((act == (uint32_t)j ? 1.0f : 0.0f) - p[j]) - ecf * t[j];
+                    if (ent.ent_sum) {                                            // one float64 atomic per warp and tile
+                        float hs = valid ? H : 0.0f;
+#pragma unroll
+                        for (int o = 16; o > 0; o >>= 1) hs += __shfl_xor_sync(0xFFFFFFFFu, hs, o);
+                        if (lane == 0 && hs != 0.0f) atomicAdd(ent.ent_sum, (double)hs);
+                    }
+                } else {
+#pragma unroll
+                    for (int j = 0; j < 4; ++j) d[j] = cf * ((act == (uint32_t)j ? 1.0f : 0.0f) - e[j] / sum);   // reinforce_agent.py:340-344
+                }
             } else {
                 d[0] = cf;                                                        // value head: dLoss/dV * weight
             }
@@ -862,7 +895,15 @@ __global__ void __launch_bounds__(BW_THREADS, 1) bwd_tc_kernel(const __grid_cons
     PipeCtx px;
     px.f_done = nullptr; px.b_done = nullptr; px.c2_done = nullptr; px.c13_done = nullptr;
     px.R = (args.n + TC_M - 1) / TC_M + 1;      // stand-alone: slot == tile
-    bwd_role(args, px, (int)blockIdx.x, (int)gridDim.x, smem);
+    bwd_role<false>(args, BwdEnt{}, px, (int)blockIdx.x, (int)gridDim.x, smem);
+}
+
+__global__ void __launch_bounds__(BW_THREADS, 1) bwd_tc_ent_kernel(const __grid_constant__ BwdEntArgs args) {
+    extern __shared__ __align__(1024) uint8_t smem[];
+    PipeCtx px;
+    px.f_done = nullptr; px.b_done = nullptr; px.c2_done = nullptr; px.c13_done = nullptr;
+    px.R = (args.b.n + TC_M - 1) / TC_M + 1;    // stand-alone: slot == tile
+    bwd_role<true>(args.b, args.e, px, (int)blockIdx.x, (int)gridDim.x, smem);
 }
 
 // ------------------------------------------------------------------------------------------------ dW roles
@@ -1065,7 +1106,28 @@ __global__ void __launch_bounds__(FH_THREADS, 1) update_pipe_kernel(const __grid
     const long long t0 = clock64();
     if (threadIdx.x == 0) prog(a.px, 0, r < a.nF ? 100 : (r < a.nF + a.nB ? 200 : (r < a.nF + a.nB + a.nC2 ? 300 : 400)));
     if (r < a.nF) fwd_role(a.f, a.px, r, a.nF, smem);
-    else if (r < a.nF + a.nB) bwd_role(a.b, a.px, r - a.nF, a.nB, smem);
+    else if (r < a.nF + a.nB) bwd_role<false>(a.b, BwdEnt{}, a.px, r - a.nF, a.nB, smem);
+    else if (r < a.nF + a.nB + a.nC2) dw_role<2>(a.d, a.px, r - a.nF - a.nB, a.nC2, smem);
+    else dw_role<3>(a.d, a.px, r - a.nF - a.nB - a.nC2, a.nC13, smem);
+    if (threadIdx.x == 0) prog(a.px, 7, (clock64() - t0) >> 10);
+}
+
+// The pipeline with the entropy bonus in the backward role: same roles, role split and shared memory as update_pipe_kernel.
+struct PipeEntArgs {
+    FwdHpArgs f;
+    BwdArgs b;
+    DwArgs d;
+    PipeCtx px;
+    int nF, nB, nC2, nC13;
+    BwdEnt e;
+};
+__global__ void __launch_bounds__(FH_THREADS, 1) update_pipe_ent_kernel(const __grid_constant__ PipeEntArgs a) {
+    extern __shared__ __align__(1024) uint8_t smem[];
+    int r = (int)blockIdx.x;
+    const long long t0 = clock64();
+    if (threadIdx.x == 0) prog(a.px, 0, r < a.nF ? 100 : (r < a.nF + a.nB ? 200 : (r < a.nF + a.nB + a.nC2 ? 300 : 400)));
+    if (r < a.nF) fwd_role(a.f, a.px, r, a.nF, smem);
+    else if (r < a.nF + a.nB) bwd_role<true>(a.b, a.e, a.px, r - a.nF, a.nB, smem);
     else if (r < a.nF + a.nB + a.nC2) dw_role<2>(a.d, a.px, r - a.nF - a.nB, a.nC2, smem);
     else dw_role<3>(a.d, a.px, r - a.nF - a.nB - a.nC2, a.nC13, smem);
     if (threadIdx.x == 0) prog(a.px, 7, (clock64() - t0) >> 10);
@@ -1077,6 +1139,16 @@ __global__ void __launch_bounds__(FH_THREADS, 1) update_pipe_kernel(const __grid
 __global__ void __launch_bounds__(256) absmax_kernel(const float* __restrict__ x, int64_t n, uint32_t* __restrict__ out_bits) {
     float m = 0.0f;
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) m = fmaxf(m, fabsf(x[i]));
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) m = fmaxf(m, __shfl_xor_sync(0xFFFFFFFFu, m, o));
+    if ((threadIdx.x & 31) == 0 && m > 0.0f && isfinite(m)) atomicMax(out_bits, __float_as_uint(m));
+}
+// max(|coef| + 1.5 |ecoef|): the bound of the head delta with the entropy bonus (|t_j| <= ln 4 < 1.5, b2048_entropy.cuh)
+__global__ void __launch_bounds__(256) absmax_ent_kernel(const float* __restrict__ x, const float* __restrict__ ex, int64_t n,
+                                                          uint32_t* __restrict__ out_bits) {
+    float m = 0.0f;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x)
+        m = fmaxf(m, fmaf(1.5f, fabsf(ex[i]), fabsf(x[i])));
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) m = fmaxf(m, __shfl_xor_sync(0xFFFFFFFFu, m, o));
     if ((threadIdx.x & 31) == 0 && m > 0.0f && isfinite(m)) atomicMax(out_bits, __float_as_uint(m));
@@ -1127,6 +1199,10 @@ static int hp_attrs(b2048_handle* h) {
         if (e != cudaSuccess) return check_cuda(e, "cudaFuncSetAttribute(bwd_tc_kernel)");
         e = cudaFuncSetAttribute(update_pipe_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, PIPE_SMEM);
         if (e != cudaSuccess) return check_cuda(e, "cudaFuncSetAttribute(update_pipe_kernel)");
+        e = cudaFuncSetAttribute(bwd_tc_ent_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, BW_TOTAL);
+        if (e != cudaSuccess) return check_cuda(e, "cudaFuncSetAttribute(bwd_tc_ent_kernel)");
+        e = cudaFuncSetAttribute(update_pipe_ent_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, PIPE_SMEM);
+        if (e != cudaSuccess) return check_cuda(e, "cudaFuncSetAttribute(update_pipe_ent_kernel)");
         h->attrs |= ATTR_HP;
     }
     return B2048_OK;
@@ -1168,10 +1244,11 @@ int launch_forward_hp(b2048_handle* h, const b2048_mlp_desc* mlp, const uint64_t
     return st;
 }
 
-int launch_loss_scale(const b2048_handle* h, const float* coef, int64_t n, float* scale, cudaStream_t stream) {
+int launch_loss_scale(const b2048_handle* h, const float* coef, int64_t n, float* scale, cudaStream_t stream, const float* ent_coef) {
     cudaError_t e = cudaMemsetAsync(scale, 0, 16, stream);
     if (e != cudaSuccess) return check_cuda(e, "cudaMemsetAsync(scale)");
-    absmax_kernel<<<h->num_sms * 4, 256, 0, stream>>>(coef, n, reinterpret_cast<uint32_t*>(scale) + 2);
+    if (ent_coef) absmax_ent_kernel<<<h->num_sms * 4, 256, 0, stream>>>(coef, ent_coef, n, reinterpret_cast<uint32_t*>(scale) + 2);
+    else absmax_kernel<<<h->num_sms * 4, 256, 0, stream>>>(coef, n, reinterpret_cast<uint32_t*>(scale) + 2);
     scale_from_max_kernel<<<1, 1, 0, stream>>>(scale);
     return B2048_OK;
 }
@@ -1201,9 +1278,12 @@ static BwdArgs bwd_args(const FwdHpArgs& f, uint8_t* ws, const HpWorkspace& w, c
 // Same contract as the fp32 body of b2048_mlp_backward (grads accumulated, flat layout W_0, b_0, W_1, b_1, ...).
 // The whole update of n samples as ONE persistent cooperative launch (see PipeCtx): the SMs are split into forward,
 // backward and dW roles; R tile slots of images (R x 206 KB, L2-resident) connect them.
+// PA = PipeArgs, or PipeEntArgs (update_pipe_ent_kernel) with ent_coef / ent_sum.
+template <class PA>
 static int launch_backward_hp_piped(b2048_handle* h, const uint64_t* board, const uint8_t* mask_flags, const uint8_t* action,
                                     const float* coef, const b2048_mlp_desc* mlp, float* grads, int64_t n, int head_mode,
-                                    uint8_t* ws, int64_t R, cudaStream_t stream) {
+                                    uint8_t* ws, int64_t R, cudaStream_t stream, const float* ent_coef, double* ent_sum) {
+    constexpr bool kEnt = std::is_same<PA, PipeEntArgs>::value;
     const int n_out = mlp->dims[3];
     const int64_t n_tiles = (n + TC_M - 1) / TC_M;
     const HpWorkspace w = hp_workspace(R * TC_M);
@@ -1211,12 +1291,12 @@ static int launch_backward_hp_piped(b2048_handle* h, const uint64_t* board, cons
     float* scale = reinterpret_cast<float*>(ws + w.scale);
     hp_prepare_kernel<<<64, 256, 0, stream>>>(mlp->W[0], mlp->b[0], mlp->W[1], mlp->b[1], mlp->W[2], mlp->b[2], n_out, ws + w.img);
     bwd_prepare_kernel<<<64, 256, 0, stream>>>(mlp->W[1], mlp->W[2], n_out, ws + w.bimg);
-    { int st = launch_loss_scale(h, coef, n, scale, stream); if (st != B2048_OK) return st; }
+    { int st = launch_loss_scale(h, coef, n, scale, stream, ent_coef); if (st != B2048_OK) return st; }
     cudaError_t e = cudaMemsetAsync(flags, 0, (size_t)n_tiles * 16, stream);
     if (e != cudaSuccess) return check_cuda(e, "cudaMemsetAsync(flags)");
     e = cudaMemsetAsync(ws + w.d3t, 0, (size_t)R * 2 * SMALL_TILE_BYTES, stream);     // rows >= n_out of d3^T stay zero
     if (e != cudaSuccess) return check_cuda(e, "cudaMemsetAsync(d3t)");
-    PipeArgs a;
+    PA a;
     a.px.f_done = flags; a.px.b_done = flags + n_tiles; a.px.c2_done = flags + 2 * n_tiles; a.px.c13_done = flags + 3 * n_tiles;
     a.px.R = R;
     a.px.progress = nullptr;
@@ -1234,6 +1314,7 @@ static int launch_backward_hp_piped(b2048_handle* h, const uint64_t* board, cons
     a.d.h1 = a.f.h1; a.d.h2 = a.f.h2; a.d.dl2 = a.b.dl2; a.d.d3t = a.b.d3t;
     a.d.gW2 = gW[1]; a.d.gb2 = gb[1]; a.d.gW3 = gW[2]; a.d.inv_scale = scale + 1;
     a.d.n_tiles = n_tiles; a.d.n_out = n_out;
+    if constexpr (kEnt) { a.e.ent_coef = ent_coef; a.e.ent_sum = ent_sum; }
     // role split (148 SMs -> 78 / 40 / 16 / 14; swept again after the head of the forward role went from 48 to 32 MMAs): per tile the forward role needs ~12 K cycles, the backward role ~7.5 K, the dW2 role ~4.5 K, the dW3 role ~2.5 K (both bound by ~30 B/clk of L2 -> shared-memory bulk copies per SM)
     const int S = h->num_sms;
     a.nB = (h->pipe_split & 0xFF) ? (h->pipe_split & 0xFF) : (S * 27 + 50) / 100;
@@ -1242,8 +1323,8 @@ static int launch_backward_hp_piped(b2048_handle* h, const uint64_t* board, cons
     a.nF = S - a.nB - a.nC2 - a.nC13;
     if (a.nF < 1 || a.nB < 1 || a.nC2 < 1 || a.nC13 < 1) return fail(B2048_ERR_INVALID, "update pipeline: bad role split");
     void* params[] = {&a};
-    e = cudaLaunchCooperativeKernel(reinterpret_cast<const void*>(update_pipe_kernel), dim3((unsigned)S), dim3(FH_THREADS), params,
-                                    (size_t)PIPE_SMEM, stream);
+    const void* kernel = kEnt ? reinterpret_cast<const void*>(update_pipe_ent_kernel) : reinterpret_cast<const void*>(update_pipe_kernel);
+    e = cudaLaunchCooperativeKernel(kernel, dim3((unsigned)S), dim3(FH_THREADS), params, (size_t)PIPE_SMEM, stream);
     if (e == cudaSuccess && a.px.progress) {      // debug watchdog: a stuck pipeline is reported and the process ends
         for (int ms = 0; ms < 3000 && cudaStreamQuery(stream) == cudaErrorNotReady; ++ms) {
             struct timespec ts = {0, 1000000};
@@ -1278,7 +1359,8 @@ static int launch_backward_hp_piped(b2048_handle* h, const uint64_t* board, cons
 
 int launch_backward_hp(b2048_handle* h, const uint64_t* board, const uint8_t* mask_flags, const uint8_t* action,
                        const float* coef, const b2048_mlp_desc* mlp, float* grads, int64_t n, int head_mode,
-                       uint8_t* workspace, int64_t workspace_bytes, int64_t chunk, cudaStream_t stream) {
+                       uint8_t* workspace, int64_t workspace_bytes, int64_t chunk, cudaStream_t stream, const float* ent_coef,
+                       double* ent_sum) {
     { int st = hp_attrs(h); if (st != B2048_OK) return st; }
     const int n_out = mlp->dims[3];
     uint8_t* ws = reinterpret_cast<uint8_t*>(((uintptr_t)workspace + 1023) & ~(uintptr_t)1023);
@@ -1288,7 +1370,10 @@ int launch_backward_hp(b2048_handle* h, const uint64_t* board, const uint8_t* ma
         const int64_t R = n_tiles < Rmax ? n_tiles : Rmax;
         const int64_t need = hp_workspace(R * TC_M).total + n_tiles * 16 + 2048;
         if (!(h->debug & (1u << B2048_DBG_NO_UPDATE_PIPE)) && n_tiles >= 4 * (int64_t)h->num_sms && need <= workspace_bytes) {
-            const int st = launch_backward_hp_piped(h, board, mask_flags, action, coef, mlp, grads, n, head_mode, ws, R, stream);
+            const int st = ent_coef ? launch_backward_hp_piped<PipeEntArgs>(h, board, mask_flags, action, coef, mlp, grads, n, head_mode,
+                                                                            ws, R, stream, ent_coef, ent_sum)
+                                    : launch_backward_hp_piped<PipeArgs>(h, board, mask_flags, action, coef, mlp, grads, n, head_mode, ws,
+                                                                         R, stream, nullptr, nullptr);
             if (st == B2048_OK) return st;
             // the cooperative launch was refused (e.g. the device cannot hold all CTAs at once because it is shared): nothing of
             // the pipeline has run, so the chunked kernel sequence below does the same work
@@ -1299,7 +1384,7 @@ int launch_backward_hp(b2048_handle* h, const uint64_t* board, const uint8_t* ma
     float* scale = reinterpret_cast<float*>(ws + w.scale);
     hp_prepare_kernel<<<64, 256, 0, stream>>>(mlp->W[0], mlp->b[0], mlp->W[1], mlp->b[1], mlp->W[2], mlp->b[2], n_out, ws + w.img);
     bwd_prepare_kernel<<<64, 256, 0, stream>>>(mlp->W[1], mlp->W[2], n_out, ws + w.bimg);
-    { int st = launch_loss_scale(h, coef, n, scale, stream); if (st != B2048_OK) return st; }
+    { int st = launch_loss_scale(h, coef, n, scale, stream, ent_coef); if (st != B2048_OK) return st; }
     float *gW[B2048_MAX_LAYERS], *gb[B2048_MAX_LAYERS];
     carve_grads(mlp, grads, gW, gb);
     long long* dbg = debug_clock_begin(h, B2048_DBG_TC_CLOCKS, stream);     // clocks of the first chunk's bwd_tc_kernel
@@ -1315,7 +1400,13 @@ int launch_backward_hp(b2048_handle* h, const uint64_t* board, const uint8_t* ma
         if (c0 == 0) b.debug_clock = dbg;
         cudaError_t e = cudaMemsetAsync(b.d3t, 0, (size_t)tiles * 2 * SMALL_TILE_BYTES, stream);
         if (e != cudaSuccess) return check_cuda(e, "cudaMemsetAsync(d3t)");
-        bwd_tc_kernel<<<grid, BW_THREADS, BW_TOTAL, stream>>>(b);
+        if (ent_coef) {
+            BwdEntArgs be;
+            be.b = b; be.e.ent_coef = ent_coef + c0; be.e.ent_sum = ent_sum;
+            bwd_tc_ent_kernel<<<grid, BW_THREADS, BW_TOTAL, stream>>>(be);
+        } else {
+            bwd_tc_kernel<<<grid, BW_THREADS, BW_TOTAL, stream>>>(b);
+        }
         st = check_cuda(cudaGetLastError(), "bwd_tc_kernel launch");
         if (st != B2048_OK) return st;
         if (b.debug_clock) {

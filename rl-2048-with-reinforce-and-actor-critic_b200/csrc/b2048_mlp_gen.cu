@@ -14,6 +14,7 @@
 //                    log2 inputs are exact in fp16, so layer 0 needs two), or one MMA (rollout policy steps).  Backward:
 //                    fp16 deltas with a power-of-two loss scale, as in b2048_learn_hp.cu.  For the dW GEMMs the hi halves of
 //                    the activations and the deltas leave as slab images (bulk shared -> global copies by the MMA lane).
+//  gen_mlp_ent_kernel  gen_mlp_kernel in update mode with the entropy bonus in the policy head's delta (b2048_entropy.cuh)
 //  gen_dw_kernel     dW_l = A_{l-1}^T DL_l (_backpropagation, src/reinforce_agent.py:639-678) for one layer: the slab
 //                    images are read back MN-major; split over 128-feature M tiles and sample ranges; the one-hot / log2
 //                    input of layer 0 is regenerated from the packed boards in shared memory instead of being stored.
@@ -24,6 +25,7 @@
 #include <cstring>
 
 #include "b2048_device.cuh"
+#include "b2048_entropy.cuh"
 #include "b2048_internal.h"
 #include "b2048_tc.cuh"
 
@@ -394,8 +396,19 @@ struct GemmSeq<SP, GEND, GEND> {
 // kAct: the hidden activation is a compile-time choice (the Sigmoid epilogue would cost the ReLU one registers);
 // kDbg compiles the phase clocks in (B2048_DBG_TC_CLOCKS)
 // kSpec != 0: the MMA warp runs the compile-time program of SpecProg<kSpec, kSplit, kFb> (the host launches it only for that network)
-template <int kAct, bool kDbg, int kSpec, bool kSplit, bool kFb>
-__global__ void __launch_bounds__(GN_THREADS, 1) gen_mlp_kernel(const __grid_constant__ GenArgs a) {
+// kEnt (update mode, policy head): the head delta carries the entropy bonus, d_j = coef (1[a = j] - p_j) - ecoef t_j
+// (b2048_entropy.cuh), and ent.ent_sum (nullable) += sum_s H_s
+struct GenEnt {
+    const float* ent_coef;
+    double* ent_sum;
+};
+struct GenEntArgs {
+    GenArgs g;
+    GenEnt e;
+};
+
+template <int kAct, bool kDbg, int kSpec, bool kSplit, bool kFb, bool kEnt>
+__device__ __forceinline__ void gen_mlp_body(const GenArgs& a, const GenEnt& ent) {
     extern __shared__ __align__(1024) uint8_t smem[];
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     uint64_t* bars = reinterpret_cast<uint64_t*>(smem + GS_BAR);
@@ -718,10 +731,11 @@ __global__ void __launch_bounds__(GN_THREADS, 1) gen_mlp_kernel(const __grid_con
             const int64_t s = (valid && a.slot_map) ? (int64_t)a.slot_map[slot] : slot;     // the board behind the slot
             const uint64_t bd = valid ? a.board[s] : 0ull;
             uint32_t fl = 0xFu, act = 0u;
-            float cf = 0.0f;
+            float cf = 0.0f, ecf = 0.0f;
             if (valid) {
                 if (use_mask) fl = a.mask_flags[s];
                 if (P.fb) { cf = a.coef[s]; if (a.act_in) act = a.act_in[s]; }
+                if constexpr (kEnt) ecf = ent.ent_coef[s];
             }
             uint32_t w3 = 0u;
             if (valid && !P.fb && a.action && !a.greedy) w3 = stream_keyed(a.keys, a.gid0 + (uint64_t)s, a.t, B2048_DOM_STEP).w3;
@@ -748,6 +762,7 @@ __global__ void __launch_bounds__(GN_THREADS, 1) gen_mlp_kernel(const __grid_con
 #pragma unroll
             for (int j = 0; j < 4; ++j) lg[j] = __uint_as_float(r4[j]) + b4[j];
             float p[4] = {0.0f, 0.0f, 0.0f, 0.0f};
+            float ent_t[4] = {0.0f, 0.0f, 0.0f, 0.0f}, ent_h = 0.0f;
             if (!P.fb || a.head_mode == 0) {
                 float m[4];
 #pragma unroll
@@ -759,6 +774,12 @@ __global__ void __launch_bounds__(GN_THREADS, 1) gen_mlp_kernel(const __grid_con
                 const float inv = 1.0f / sum;
 #pragma unroll
                 for (int j = 0; j < 4; ++j) p[j] *= inv;
+                if constexpr (kEnt) {
+                    float z[4];
+#pragma unroll
+                    for (int j = 0; j < 4; ++j) z[j] = m[j] - mx;
+                    ent_h = entropy_row(z, logf(sum), p, use_mask ? fl : 0xFu, P.n_out, ent_t);
+                }
             }
             if (!P.fb) {
                 if (valid) {
@@ -795,7 +816,18 @@ __global__ void __launch_bounds__(GN_THREADS, 1) gen_mlp_kernel(const __grid_con
                 if (a.head_mode == 0) {
 #pragma unroll
                     for (int j = 0; j < 4; ++j)
-                        if (j < P.n_out) d[j] = cf * ((act == (uint32_t)j ? 1.0f : 0.0f) - p[j]);     // reinforce_agent.py:340-344
+                        if (j < P.n_out) {
+                            if constexpr (kEnt) d[j] = cf * ((act == (uint32_t)j ? 1.0f : 0.0f) - p[j]) - ecf * ent_t[j];
+                            else d[j] = cf * ((act == (uint32_t)j ? 1.0f : 0.0f) - p[j]);     // reinforce_agent.py:340-344
+                        }
+                    if constexpr (kEnt) {
+                        if (ent.ent_sum) {                                                            // one float64 atomic per warp and tile
+                            float hs = valid ? ent_h : 0.0f;
+#pragma unroll
+                            for (int o = 16; o > 0; o >>= 1) hs += __shfl_xor_sync(0xFFFFFFFFu, hs, o);
+                            if (lane == 0 && hs != 0.0f) atomicAdd(ent.ent_sum, (double)hs);
+                        }
+                    }
                 } else {
                     d[0] = cf;                                                                        // dLoss/dV * weight
                 }
@@ -822,6 +854,17 @@ __global__ void __launch_bounds__(GN_THREADS, 1) gen_mlp_kernel(const __grid_con
     }
 
     tmem_teardown(warp == 16, tmem_base, 512u);
+}
+
+template <int kAct, bool kDbg, int kSpec, bool kSplit, bool kFb>
+__global__ void __launch_bounds__(GN_THREADS, 1) gen_mlp_kernel(const __grid_constant__ GenArgs a) {
+    gen_mlp_body<kAct, kDbg, kSpec, kSplit, kFb, false>(a, GenEnt{});
+}
+
+// update mode with the entropy bonus in the policy head's delta
+template <int kAct, int kSpec, bool kSplit, bool kFb>
+__global__ void __launch_bounds__(GN_THREADS, 1) gen_mlp_ent_kernel(const __grid_constant__ GenEntArgs a) {
+    gen_mlp_body<kAct, false, kSpec, kSplit, kFb, true>(a.g, a.e);
 }
 
 // ------------------------------------------------------------------------------------------------ dW GEMMs
@@ -1043,6 +1086,9 @@ static int gen_attrs(b2048_handle* h) {
         set((const void*)gen_mlp_kernel<B2048_ACTV_RELU, false, 1, false, false>);
         set((const void*)gen_mlp_kernel<B2048_ACTV_RELU, false, 1, true, false>);
         set((const void*)gen_mlp_kernel<B2048_ACTV_RELU, false, 1, true, true>);
+        set((const void*)gen_mlp_ent_kernel<B2048_ACTV_RELU, 0, false, false>);
+        set((const void*)gen_mlp_ent_kernel<B2048_ACTV_SIGMOID, 0, false, false>);
+        set((const void*)gen_mlp_ent_kernel<B2048_ACTV_RELU, 1, true, true>);
         if (e != cudaSuccess) return check_cuda(e, "cudaFuncSetAttribute(gen_mlp_kernel)");
         e = cudaFuncSetAttribute(gen_dw_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
         if (e != cudaSuccess) return check_cuda(e, "cudaFuncSetAttribute(gen_dw_kernel)");
@@ -1108,6 +1154,17 @@ static void gen_launch(const GenArgs& a, int grid, cudaStream_t stream) {
     }
 }
 
+// update mode with the entropy bonus: the kernels of gen_launch's update-mode choices without the debug clocks
+static void gen_launch_ent(const GenEntArgs& a, int grid, cudaStream_t stream) {
+    const GenProg& p = a.g.p;
+    const bool sig = p.act == B2048_ACTV_SIGMOID;
+    const bool spec1 = !sig && p.L == 4 && p.kin == 272 && p.obs_mode == B2048_OBS_ONEHOT && p.width[0] == 256 && p.width[1] == 128 &&
+                       p.width[2] == 64 && p.split == 1;
+    if (spec1) gen_mlp_ent_kernel<B2048_ACTV_RELU, 1, true, true><<<grid, GN_THREADS, GS_TOTAL, stream>>>(a);
+    else if (sig) gen_mlp_ent_kernel<B2048_ACTV_SIGMOID, 0, false, false><<<grid, GN_THREADS, GS_TOTAL, stream>>>(a);
+    else gen_mlp_ent_kernel<B2048_ACTV_RELU, 0, false, false><<<grid, GN_THREADS, GS_TOTAL, stream>>>(a);
+}
+
 static void gen_fill_common(GenArgs& a, const b2048_mlp_desc* mlp, const GenProg& p) {
     memset(&a, 0, sizeof(a));
     a.p = p;
@@ -1147,7 +1204,7 @@ int launch_forward_gen(b2048_handle* h, const b2048_mlp_desc* mlp, const uint64_
 // Same contract as the fp32 body of b2048_mlp_backward (grads accumulated; flat layout W_0, b_0, W_1, b_1, ...).
 int launch_backward_gen(b2048_handle* h, const uint64_t* board, const uint8_t* mask_flags, const uint8_t* action, const float* coef,
                         const b2048_mlp_desc* mlp, float* grads, int64_t n, int head_mode, uint8_t* workspace, int64_t chunk,
-                        cudaStream_t stream) {
+                        cudaStream_t stream, const float* ent_coef, double* ent_sum) {
     { int st = gen_attrs(h); if (st != B2048_OK) return st; }
     const int L = mlp->n_layers;
     uint8_t* ws = reinterpret_cast<uint8_t*>(((uintptr_t)workspace + 1023) & ~(uintptr_t)1023);
@@ -1156,7 +1213,7 @@ int launch_backward_gen(b2048_handle* h, const uint64_t* board, const uint8_t* m
     build_program(mlp, true, true, p);
     { int st = gen_prepare(mlp, p, ws + w.img, stream); if (st != B2048_OK) return st; }
     float* scale = reinterpret_cast<float*>(ws + w.scale);
-    { int st = launch_loss_scale(h, coef, n, scale, stream); if (st != B2048_OK) return st; }
+    { int st = launch_loss_scale(h, coef, n, scale, stream, ent_coef); if (st != B2048_OK) return st; }
     float *gW[B2048_MAX_LAYERS], *gb[B2048_MAX_LAYERS];
     carve_grads(mlp, grads, gW, gb);
     for (int64_t c0 = 0; c0 < n; c0 += chunk) {
@@ -1174,8 +1231,14 @@ int launch_backward_gen(b2048_handle* h, const uint64_t* board, const uint8_t* m
         a.gb_head = gb[L - 1];
         if (mlp->activation == B2048_ACTV_SIGMOID) a.dsig_scratch = reinterpret_cast<uint4*>(ws + w.masks);
         else a.mask_scratch = reinterpret_cast<uint16_t*>(ws + w.masks);
-        if (c0 == 0) a.dbg = debug_clock_begin(h, B2048_DBG_TC_CLOCKS, stream);
-        gen_launch(a, grid, stream);
+        if (ent_coef) {                              // the entropy kernels carry no phase clocks
+            GenEntArgs ea;
+            ea.g = a; ea.e.ent_coef = ent_coef + c0; ea.e.ent_sum = ent_sum;
+            gen_launch_ent(ea, grid, stream);
+        } else {
+            if (c0 == 0) a.dbg = debug_clock_begin(h, B2048_DBG_TC_CLOCKS, stream);
+            gen_launch(a, grid, stream);
+        }
         int st = check_cuda(cudaGetLastError(), "gen_mlp_kernel launch");
         if (st != B2048_OK || (st = gen_dbg_print(h, a, stream)) != B2048_OK) return st;
         for (int l = 0; l < L; ++l) {

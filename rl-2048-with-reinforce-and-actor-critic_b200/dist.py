@@ -126,7 +126,7 @@ def make_sharded_env(total_boards: int, config, info: DistInfo, seed: int = 0, d
 
 def sharded_update(agent, rollout, info: DistInfo, total_episodes: int | None = None, precision="auto",
                    exchange: str = "default", fixed_horizon: bool = False, bootstrap_truncation: bool = False,
-                   ppo: dict | None = None):
+                   ppo: dict | None = None, entropy_coef: float = 0.0):
     """update_from_rollout with gradients / baseline sums all-reduced over ranks; n_traj = global episode count
     so that every rank applies exactly the update a single process holding all episodes would apply.
     exchange="one_message": exactly one all-reduce per update (see ReinforceAgent.update_from_rollout); pass
@@ -136,11 +136,15 @@ def sharded_update(agent, rollout, info: DistInfo, total_episodes: int | None = 
     bootstrap_truncation: passed to the update; it adds no message (the boards are replayed from global ids, V(s') is local).
     ppo (with fixed_horizon=True): keyword arguments of ReinforceAgent.update_ppo (epochs, minibatches, clip_eps,
     value_clip_eps, shuffle_seed); the window is trained with PPO instead, one gradient all-reduce per minibatch step (the
-    minibatches are keyed on global sample ids: no message places them).  exchange="one_message" is refused."""
+    minibatches are keyed on global sample ids: no message places them).  exchange="one_message" is refused.
+    entropy_coef: the entropy bonus of the three updates; its per-sample weight is beta times the policy term's, so it adds
+    no message."""
     if ppo is not None and not fixed_horizon:
         raise ValueError("sharded_update: ppo needs fixed_horizon=True (PPO trains on fixed-horizon windows)")
     if ppo is not None and exchange != "default":
         raise ValueError("sharded_update: exchange='one_message' is not implemented for PPO")
+    if entropy_coef != 0.0:      # refused configurations raise before the episode-count collective
+        type(agent)._check_entropy(entropy_coef, exchange, precision)
     if total_episodes is None:
         n = torch.tensor([rollout.B], dtype=torch.int64, device=rollout.length.device)
         allreduce_sum_(n)
@@ -148,12 +152,13 @@ def sharded_update(agent, rollout, info: DistInfo, total_episodes: int | None = 
     rollout.n_traj = total_episodes
     if ppo is not None:
         return agent.update_ppo(rollout, allreduce=allreduce_sum_ if info.is_distributed else None, precision=precision,
-                                bootstrap_truncation=bootstrap_truncation, **ppo)
+                                bootstrap_truncation=bootstrap_truncation, entropy_coef=entropy_coef, **ppo)
     if fixed_horizon:
         return agent.update_from_horizon(rollout, allreduce=allreduce_sum_ if info.is_distributed else None,
-                                         precision=precision, exchange=exchange, bootstrap_truncation=bootstrap_truncation)
+                                         precision=precision, exchange=exchange, bootstrap_truncation=bootstrap_truncation,
+                                         entropy_coef=entropy_coef)
     return agent.update_from_rollout(rollout, allreduce=allreduce_sum_ if info.is_distributed else None, precision=precision,
-                                     exchange=exchange, bootstrap_truncation=bootstrap_truncation)
+                                     exchange=exchange, bootstrap_truncation=bootstrap_truncation, entropy_coef=entropy_coef)
 
 
 def episode_rank_weights(total_reward: torch.Tensor, weights_conf, info: DistInfo | None = None) -> torch.Tensor:

@@ -17,6 +17,7 @@ from __future__ import annotations
 
 import ctypes as C
 import logging
+import math
 import os
 from collections.abc import Callable
 from dataclasses import dataclass, replace
@@ -314,23 +315,47 @@ class ReinforceAgent:
         return prec if (n >= 4096 or prec in (0, 2)) else (2 if prec == 3 else 0)
 
     def _backward(self, net: DeviceMLP, boards, mflags, acts, cf: torch.Tensor, n: int, head_mode: int, prec: int, chunk: int,
-                  fell_back: list) -> None:
+                  fell_back: list, ent_cf: torch.Tensor | None = None, ent_acc: torch.Tensor | None = None) -> None:
         """net.grad = b2048_mlp_backward of the n samples (head 0: sum cf log pi(a|s), head 1: sum cf V(s)) at prec.  A
         non-finite split-fp16 gradient (fp16 range exceeded) is never applied: the pass is redone in fp32 and head_mode is
-        appended to fell_back."""
+        appended to fell_back.  ent_cf (policy head): b2048_mlp_backward_entropy, + sum ent_cf H(pi(.|s)), and the pass's
+        sum of H is added to ent_acc (device double[1])."""
         lib, h = self._lib, self._h
         ws_floats = int(lib.b2048_backward_workspace_floats(C.byref(net.desc), min(chunk, n)))
         ws = self._buf("bwd_ws", (ws_floats,), torch.float32)
+        es = self._buf("ent_sum_pass", (1,), torch.float64) if ent_cf is not None else None
         for p_try in ((prec, 0) if prec in (2, 3) else (prec,)):
             net.grad.zero_()
             with torch.cuda.device(self.device):
-                _lib.check(lib.b2048_mlp_backward(h, _ptr(boards), _ptr(mflags) if self._use_mask else None, _ptr(acts),
-                                                  _ptr(cf), C.byref(net.desc), _ptr(net.grad), n, head_mode, _ptr(ws),
-                                                  ws_floats, min(chunk, n), p_try, _stream()), "b2048_mlp_backward")
+                if ent_cf is None:
+                    _lib.check(lib.b2048_mlp_backward(h, _ptr(boards), _ptr(mflags) if self._use_mask else None, _ptr(acts),
+                                                      _ptr(cf), C.byref(net.desc), _ptr(net.grad), n, head_mode, _ptr(ws),
+                                                      ws_floats, min(chunk, n), p_try, _stream()), "b2048_mlp_backward")
+                else:
+                    es.zero_()
+                    _lib.check(lib.b2048_mlp_backward_entropy(
+                        h, _ptr(boards), _ptr(mflags) if self._use_mask else None, _ptr(acts), _ptr(cf), _ptr(ent_cf),
+                        C.byref(net.desc), _ptr(net.grad), n, _ptr(ws), ws_floats, min(chunk, n), p_try, _ptr(es), _stream()),
+                        "b2048_mlp_backward_entropy")
             if p_try == 0 or bool(torch.isfinite(net.grad).all()):
                 break
             fell_back.append(head_mode)
             self._logger.warning("tensor-core gradient not finite (fp16 range exceeded); recomputing on the fp32 kernels")
+        if es is not None and ent_acc is not None:
+            ent_acc += es
+
+    @staticmethod
+    def _check_entropy(entropy_coef: float, exchange: str = "default", precision: int | str = "auto") -> float:
+        """entropy_coef (beta of the bonus beta H(pi(.|s))) as a float; the configurations without an entropy kernel raise."""
+        beta = float(entropy_coef)
+        if not (math.isfinite(beta) and beta >= 0.0):
+            raise ValueError(f"entropy_coef must be finite and >= 0, got {entropy_coef}")
+        if beta > 0.0 and exchange == "one_message":
+            raise ValueError("entropy_coef > 0 is not implemented with exchange='one_message' (the actor gradient is formed "
+                             "as (g_A - mean g_B) / std there; the bonus would need a third backward pass)")
+        if beta > 0.0 and precision != "auto" and int(precision) == 1:
+            raise ValueError("entropy_coef > 0 is not implemented on the single-bf16 path (precision=1)")
+        return beta
 
     def _apply(self, net, lr: float, sign: float, t_adam: int) -> torch.Tensor:
         """b2048_apply_update (global-norm clip, SGD / Adam) of net.grad; returns the device double[1] squared norm."""
@@ -706,7 +731,7 @@ class ReinforceAgent:
 
     def update_from_rollout(self, ro: Rollout, chunk: int = 1 << 20, allreduce=None,
                             precision: int | str = "auto", exchange: str = "default",
-                            bootstrap_truncation: bool = False) -> dict[str, Any]:
+                            bootstrap_truncation: bool = False, entropy_coef: float = 0.0) -> dict[str, Any]:
         """One policy-gradient update from device-resident rollout buffers.  `allreduce(tensor)` (optional) sums
         a tensor over ranks in place: the flat gradients and the advantage statistics are the only exchange.
         precision: 0 = fp32 CUDA cores, "auto" (default) = the float32-grade tensor-core path (split-fp16 forward, fp16
@@ -722,8 +747,13 @@ class ReinforceAgent:
         bootstrap_truncation (needs a critic or a value head): an episode truncated by the env's max_steps (flags[len[b], b]
         has TRUNC) gets the target r + gamma V(boards[len[b], b]) at its last step instead of r, like Gymnasium's `truncated`
         (see _update_bootstrapped).  Episodes cut by rollout_many's own max_steps cap carry no TRUNC flag and are not
-        bootstrapped.  The default keeps update_batch's targets."""
+        bootstrapped.  The default keeps update_batch's targets.
+        entropy_coef (beta >= 0): the actor ascends sum_s coef_s log pi(a_s|s) + ecoef_s H(pi(.|s_s)) with ecoef_s = beta w_b /
+        (len_b n_traj), i.e. beta times the sample's weight in the policy term (b2048_mlp_backward_entropy); info["entropy"] is
+        then the rank-local mean H over the update's samples.  0 (default) runs exactly the calls without the bonus.  Refused
+        with exchange='one_message' and precision=1."""
         cfg = self._check_update_config(exchange)
+        beta = self._check_entropy(entropy_coef, exchange, precision)
         if bootstrap_truncation:
             self._check_bootstrap(ro, window=False)
         if ro.B == 0 or ro.T == 0:
@@ -746,10 +776,11 @@ class ReinforceAgent:
         boot = self._truncated_episode_ends(ro) if bootstrap_truncation else None
         if cfg.augmentation:
             ro = self._augment_rollout(ro)
-        return self._update_bootstrapped(ro, boot, chunk, allreduce, precision, exchange, window=False)
+        return self._update_bootstrapped(ro, boot, chunk, allreduce, precision, exchange, window=False, beta=beta)
 
     def update_from_horizon(self, ro: Rollout, allreduce=None, precision: int | str = "auto", chunk: int = 1 << 20,
-                            exchange: str = "default", bootstrap_truncation: bool = False) -> dict[str, Any]:
+                            exchange: str = "default", bootstrap_truncation: bool = False,
+                            entropy_coef: float = 0.0) -> dict[str, Any]:
         """One policy-gradient update from a fixed-horizon window: a rollout_many(horizon=H) rollout with reset-on-done,
         whose lanes keep playing across updates (synchronous A2C / REINFORCE on segments).  Episode boundaries inside a lane
         (flags DONE | TRUNC after step t) restart the returns, TD targets and advantages (b2048_segment_targets; a truncated
@@ -767,8 +798,11 @@ class ReinforceAgent:
         bootstrap_truncation (needs a critic or a value head, and ro.seed / ro.t0 from rollout_many): a TRUNC boundary
         after step t (the env's max_steps ran out, the game was not over) uses V(s') instead of 0, s' being the board the
         episode was cut on: delta_t = r_t + gamma V(s') - V(s_t).  boards[t + 1] already holds the reset board; s' is replayed
-        on the device from boards[t], actions[t] and the env streams (b2048_replay_pre_reset)."""
+        on the device from boards[t], actions[t] and the env streams (b2048_replay_pre_reset).
+        entropy_coef as in update_from_rollout, with ecoef = beta / (T n_traj) on the samples (every slot with a value
+        function; with REINFORCE the slots t < valid_len[b])."""
         cfg = self._check_update_config(exchange)
+        beta = self._check_entropy(entropy_coef, exchange, precision)
         if not ro.auto_reset:
             raise ValueError("update_from_horizon needs a fixed-horizon rollout with reset-on-done (rollout_many(horizon=H))")
         if cfg.baseline_mode == "each":
@@ -785,12 +819,12 @@ class ReinforceAgent:
         boot = self._truncated_window_steps(ro) if bootstrap_truncation else None
         if cfg.augmentation:
             ro = self._augment_rollout(ro)
-        return self._update_bootstrapped(ro, boot, chunk, allreduce, precision, exchange, window=True)
+        return self._update_bootstrapped(ro, boot, chunk, allreduce, precision, exchange, window=True, beta=beta)
 
     # ------------------------------------------------------------------ PPO on windows
     def update_ppo(self, ro: Rollout, epochs: int = 4, minibatches: int = 4, clip_eps: float = 0.2,
                    value_clip_eps: float | None = None, shuffle_seed: int = 0, allreduce=None, precision: int | str = "auto",
-                   bootstrap_truncation: bool = False) -> dict[str, Any]:
+                   bootstrap_truncation: bool = False, entropy_coef: float = 0.0) -> dict[str, Any]:
         """PPO on a fixed-horizon window (rollout_many(horizon=H), reset-on-done): `epochs` passes over the window's
         N = T n_traj samples, each split into `minibatches` minibatches, one clipped-surrogate step per minibatch
         (epochs x minibatches optimizer steps).  Needs a value function (use_critic=True or SharedTrunkActorCritic).
@@ -811,8 +845,12 @@ class ReinforceAgent:
         buffers, valid until the next update.
         allreduce / precision / bootstrap_truncation as in update_from_horizon.  Refused (ValueError): no value function,
         a rollout without reset-on-done, augmentation, reward rank weights, baseline 'each', epochs < 1, minibatches
-        outside [1, N], clip_eps <= 0, value_clip_eps <= 0, and a shard (n_traj > B) without ro.gid0."""
+        outside [1, N], clip_eps <= 0, value_clip_eps <= 0, and a shard (n_traj > B) without ro.gid0.
+        entropy_coef (beta >= 0): each minibatch step adds beta H(pi(.|s)) / |mb| per sample to the surrogate's gradient
+        (b2048_mlp_backward_entropy, |mb| the global minibatch size as for the surrogate); info["entropy"] is then the per-epoch
+        rank-local mean H at the step's parameters.  Refused with precision=1."""
         cfg = self._check_update_config("default")
+        beta = self._check_entropy(entropy_coef, "default", precision)
         if not (cfg.use_critic and getattr(self, "_critic", None) is not None):
             raise ValueError("update_ppo needs a value function: use_critic=True or SharedTrunkActorCritic")
         if not ro.auto_reset:
@@ -847,7 +885,7 @@ class ReinforceAgent:
             if boot[0].numel():
                 ro = self._fold_truncation(ro, boot, precision)[0]
         return self._ppo(ro, int(epochs), int(minibatches), float(clip_eps), value_clip_eps, int(shuffle_seed), allreduce, prec,
-                         n_traj)
+                         n_traj, beta)
 
     def ppo_minibatch_lists(self, T: int, B: int, n_traj: int, gid0: int, minibatches: int, shuffle_seed: int,
                             epoch: int) -> tuple[torch.Tensor, list[int]]:
@@ -864,7 +902,7 @@ class ReinforceAgent:
         return order, counts
 
     def _ppo(self, ro: Rollout, epochs: int, M: int, clip_eps: float, value_clip_eps, shuffle_seed: int, allreduce, prec: int,
-             n_traj: int) -> dict[str, Any]:
+             n_traj: int, beta: float = 0.0) -> dict[str, Any]:
         cfg = self.agent_config
         lib, h, dev = self._lib, self._h, self.device
         T, B = ro.T, ro.B
@@ -907,6 +945,7 @@ class ReinforceAgent:
         shared = getattr(self, "_shared_net", None)
         ep_stats = torch.zeros((epochs, 5), dtype=torch.float64, device=dev)
         norms = torch.zeros((epochs * M, 2), dtype=torch.float64, device=dev)
+        ent = torch.zeros(epochs, dtype=torch.float64, device=dev) if beta > 0.0 else None
         vclip = float(value_clip_eps) if value_clip_eps is not None else 0.0
         huber = int(cfg.critic_loss_type == "huber")
         chunk = 1 << 20
@@ -933,7 +972,11 @@ class ReinforceAgent:
                             h, _ptr(idx), k, _ptr(z), _ptr(v), _ptr(mflags) if self._use_mask else None, _ptr(acts),
                             _ptr(logp_old), _ptr(adv), _ptr(gae), _ptr(values), float(size), clip_eps, vclip, huber,
                             float(cfg.huber_delta), _ptr(cf), _ptr(gc), _ptr(ep_stats[e]), _stream()), "b2048_ppo_coefficients")
-                    self._backward(self._actor, bx, fx, ax, cf, k, 0, p, chunk, fell_back)
+                    if ent is None:
+                        self._backward(self._actor, bx, fx, ax, cf, k, 0, p, chunk, fell_back)
+                    else:                                      # the bonus beta H / |mb| per sample, like the surrogate's 1 / |mb|
+                        ecf = self._buf("ppo_ent_coef", (k,), torch.float32).fill_(beta / size)
+                        self._backward(self._actor, bx, fx, ax, cf, k, 0, p, chunk, fell_back, ecf, ent[e: e + 1])
                     self._backward(self._critic, bx, fx, ax, gc, k, 1, p, chunk, fell_back)
                 else:                                          # this shard holds none of the minibatch's samples
                     self._actor.grad.zero_()
@@ -954,6 +997,8 @@ class ReinforceAgent:
             "advantages": adv, "gae": gae, "values_old": values, "logp_old": logp_old,
             "precision": self._update_mode_name(prec, n) + (" [fell back to fp32: non-finite fp16 intermediates]" if fell_back else "")}
         info["actor_grad_norm"] = info["actor_grad_norms"][-1]
+        if ent is not None:
+            info["entropy"] = (ent.cpu().numpy() / n).tolist()
         if shared is None:
             info["critic_grad_norms"] = nr[:, 1].tolist()
             info["critic_grad_norm"] = info["critic_grad_norms"][-1]
@@ -995,16 +1040,16 @@ class ReinforceAgent:
         return slots, ro.boards[: T + 1].gather(0, last).reshape(-1)[lanes]
 
     def _update_bootstrapped(self, ro: Rollout, boot, chunk: int, allreduce, precision: int | str, exchange: str,
-                             window: bool) -> dict[str, Any]:
+                             window: bool, beta: float = 0.0) -> dict[str, Any]:
         """_update on a copy of the rewards with gamma V(s') folded in at the truncated steps (boot = (slots, s') of the
         rollout before augmentation; None: no bootstrap).  The target kernels use V = 0 after an episode's last step, so
         r' = r + gamma V(s') (each operation rounded separately, b2048_fold_bootstrap) makes every target, TD error,
         advantage and critic coefficient the bootstrapped one.  With augmentation variant v of step (t, b) is column
         v B + b, and it folds the value of variant v of s'."""
         if boot is None or boot[0].numel() == 0:
-            return self._update(ro, window, chunk, allreduce, precision, exchange)
+            return self._update(ro, window, chunk, allreduce, precision, exchange, beta)
         folded, slots, nxt, values = self._fold_truncation(ro, boot, precision)
-        info = self._update(folded, window, chunk, allreduce, precision, exchange)
+        info = self._update(folded, window, chunk, allreduce, precision, exchange, beta)
         info.update(bootstrap_slots=slots, bootstrap_boards=nxt, bootstrap_values=values)
         return info
 
@@ -1095,9 +1140,10 @@ class ReinforceAgent:
             raise ValueError(f"Unknown critic loss type: {cfg.critic_loss_type}")    # reinforce_agent.py:908
         return cfg
 
-    def _update(self, ro: Rollout, window: bool, chunk: int, allreduce, precision: int | str, exchange: str) -> dict[str, Any]:
+    def _update(self, ro: Rollout, window: bool, chunk: int, allreduce, precision: int | str, exchange: str,
+                beta: float = 0.0) -> dict[str, Any]:
         """The body of update_from_rollout (window=False: one episode per lane, t < length) and update_from_horizon
-        (window=True: a fixed-horizon window, targets from b2048_segment_targets)."""
+        (window=True: a fixed-horizon window, targets from b2048_segment_targets).  beta > 0: the entropy bonus."""
         prec = 2 if precision == "auto" else int(precision)
         cfg = self.agent_config
         T, B = ro.T, ro.B
@@ -1159,11 +1205,33 @@ class ReinforceAgent:
                            "b2048_advantages")
 
         fell_back = []
+        ent_cf = ent_acc = None
+        if beta > 0.0:
+            # ecoef = beta x the sample's weight in the policy term: the advantage kernels in mode 0 on a constant beta give
+            # beta w_b / (len_b n_traj) (episodes) or beta / (T n_traj) (windows), masked and rounded like coef
+            bvals = self._buf("ent_beta", (T, B), torch.float32).fill_(beta)
+            ent_cf = self._buf("ent_coef", (T, B), torch.float32)
+            ent_adv = self._buf("ent_adv", (T, B), torch.float32)
+            ent_acc = self._buf("ent_acc", (1,), torch.float64).zero_()
+            with torch.cuda.device(dev):
+                if window:
+                    _lib.check(lib.b2048_advantages_window(h, _ptr(bvals), _ptr(length), 0, n_traj, T, B, _ptr(ent_adv),
+                                                           _ptr(ent_cf), _ptr(stats), 1, _stream()), "b2048_advantages_window")
+                else:
+                    _lib.check(lib.b2048_advantages(h, _ptr(bvals), _ptr(length), _ptr(ro.ep_weight), 0, n_traj, T, B,
+                                                    _ptr(ent_adv), _ptr(ent_cf), _ptr(stats), 1, _ptr(ep_mean), _stream()),
+                               "b2048_advantages")
+            ent_cf = ent_cf.reshape(-1)
+            if live is not None:
+                ent_cf = ent_cf.index_select(0, live)
 
-        def backward(net: DeviceMLP, cf: torch.Tensor, head_mode: int):
+        def backward(net: DeviceMLP, cf: torch.Tensor, head_mode: int, with_entropy: bool = False):
             if live is not None:
                 cf = cf.index_select(0, live)
-            self._backward(net, boards, mflags, acts, cf, n, head_mode, prec, chunk, fell_back)
+            if with_entropy and ent_cf is not None:
+                self._backward(net, boards, mflags, acts, cf, n, head_mode, prec, chunk, fell_back, ent_cf, ent_acc)
+            else:
+                self._backward(net, boards, mflags, acts, cf, n, head_mode, prec, chunk, fell_back)
 
         if critic:
             # critic block (reinforce_agent.py:403-498): V(s_t) for every stored state, TD(0) errors, critic grads
@@ -1215,7 +1283,7 @@ class ReinforceAgent:
             advantages(base_values, pre=1)   # adv / coef as the default exchange reports them (global statistics)
         else:
             advantages(base_values)
-            backward(self._actor, coef.reshape(-1), 0)
+            backward(self._actor, coef.reshape(-1), 0, with_entropy=True)
             if shared is not None:
                 self._merge_shared_grads()   # trunk gradient = policy part - value_coef x value part
             if allreduce is not None:
@@ -1223,6 +1291,8 @@ class ReinforceAgent:
 
         ss_a, ss_c = self._optimizer_step()
         info["advantages"] = adv
+        if ent_acc is not None:
+            info["entropy"] = float(ent_acc.cpu()[0]) / max(n, 1)
         info["precision"] = self._update_mode_name(prec, n) + (" [fell back to fp32: non-finite fp16 intermediates]" if fell_back else "")
         info["actor_grad_norm"] = float(ss_a.cpu()[0]) ** 0.5
         if ss_c is not None:

@@ -23,6 +23,8 @@ instead of r (``update_from_rollout`` / ``update_from_horizon(bootstrap_truncati
 ``train.ppo`` (default None; needs ``train.horizon`` and ``agent.use_critic`` or a ``shared_trunk`` section): a dict with any of
 ``epochs`` (4), ``minibatches`` (4), ``clip_eps`` (0.2), ``value_clip_eps`` (None) trains every window with
 ``update_ppo`` instead; the shuffle seed of batch k is derived from ``seed`` and k.  The CSV columns are unchanged.
+``train.entropy_coef`` (default 0): the entropy bonus beta H(pi(.|s)) of every update (episodes, horizon windows and PPO);
+refused with ``train.exchange = "one_message"``.
 
     python -m torch.distributed.run ... b2048_runner.py -conf cfg.json      (or: python b2048_runner.py -conf cfg.json)
 """
@@ -126,6 +128,7 @@ def training(cfg: dict[str, Any], info: bd.DistInfo | None = None, device=None, 
         unknown = set(ppo) - PPO_KEYS
         if unknown:
             raise ValueError(f"train.ppo: unknown keys {sorted(unknown)} (allowed: {sorted(PPO_KEYS)})")
+    ReinforceAgent._check_entropy(tr.get("entropy_coef", 0.0), tr.get("exchange", "default"))   # before any device work
     env, agent = build(cfg, int(tr["batch_size"]), info, device)
     out_dir = tr.get("out_dir")
     rows: list[dict[str, Any]] = []
@@ -187,7 +190,8 @@ def training(cfg: dict[str, Any], info: bd.DistInfo | None = None, device=None, 
             if global_step > 30 and is_record and info.rank == 0 and out_dir:
                 agent.save_model(os.path.join(out_dir, f"best_avg_{avg:.2f}_step_{global_step}.npz"))
             upd = bd.sharded_update(agent, ro, info, total_episodes=int(tr["batch_size"]), exchange=tr.get("exchange", "default"),
-                                    bootstrap_truncation=bool(tr.get("bootstrap_truncation", False)))
+                                    bootstrap_truncation=bool(tr.get("bootstrap_truncation", False)),
+                                    entropy_coef=float(tr.get("entropy_coef", 0.0)))
             row = {"batch": global_step, "avg_reward": avg, "max_reward": mx, "min_reward": mn, "max_tile_counts": json.dumps(hist)}
             rows.append(dict(row, steps=int(ro.length.sum().item()), seconds=time.perf_counter() - t0,
                              grad_norm=upd.get("actor_grad_norm")))
@@ -219,7 +223,8 @@ def _horizon_batch(agent, env, info: bd.DistInfo, tr: dict[str, Any], horizon: i
     if ppo is not None:                                    # a fresh minibatch shuffle for every window, the same on every rank
         ppo = dict(ppo, shuffle_seed=(seed * 0x9E3779B97F4A7C15 + 0xBF58476D1CE4E5B9 * global_step) & (2**64 - 1))
     upd = bd.sharded_update(agent, ro, info, total_episodes=int(tr["batch_size"]), exchange=tr.get("exchange", "default"),
-                            fixed_horizon=True, bootstrap_truncation=bool(tr.get("bootstrap_truncation", False)), ppo=ppo)
+                            fixed_horizon=True, bootstrap_truncation=bool(tr.get("bootstrap_truncation", False)), ppo=ppo,
+                            entropy_coef=float(tr.get("entropy_coef", 0.0)))
     es = agent.horizon_episode_stats(reset=True, info=info)
     avg = es["avg_reward"]
     if saving and avg > best:                                                              # runner.py:643-660
