@@ -78,12 +78,12 @@ def phases(agent, ro, M):
     state = {}
 
     def old_pass():
-        agent._forward_checked(agent._critic, ro.boards[: T + 1].reshape(-1), values.view(-1), 2)
+        agent._forward_checked(agent._critic, ro.boards[: T + 1].reshape(-1), values.view(-1), 2, [], 1)
         agent._segment_targets(ro.rewards[:T].contiguous(), ro.flags[: T + 1].contiguous(), values, 0.0, float(B), gae, td,
                                gcoef, valid)
         _lib.check(lib.b2048_advantages_window(h, _ptr(gae), _ptr(valid), 3, float(B), T, B, _ptr(adv), _ptr(coef), _ptr(stats),
                                                0, _stream()))
-        agent._forward_checked(agent._actor, boards, logits, 2)
+        agent._forward_checked(agent._actor, boards, logits, 2, [], 0)
         _lib.check(lib.b2048_ppo_logp(h, _ptr(logits), _ptr(mflags), _ptr(acts), n, _ptr(logp_old), _stream()))
 
     def partition():
@@ -94,8 +94,8 @@ def phases(agent, ro, M):
         idx, k = state["idx"], state["k"]
         state.update(bx=boards.index_select(0, idx), fx=mflags.index_select(0, idx), ax=acts.index_select(0, idx),
                      z=torch.empty((k, 4), dtype=torch.float32, device="cuda"), v=torch.empty(k, dtype=torch.float32, device="cuda"))
-        agent._forward_checked(agent._actor, state["bx"], state["z"], 2)
-        agent._forward_checked(agent._critic, state["bx"], state["v"], 2)
+        agent._forward_checked(agent._actor, state["bx"], state["z"], 2, [], 0)
+        agent._forward_checked(agent._critic, state["bx"], state["v"], 2, [], 1)
 
     def coefficients():
         k = state["k"]

@@ -63,7 +63,7 @@ def bootstrap_only(agent, ro):
     update = agent._update
     agent._update = lambda *a, **k: {}                  # everything of _update_bootstrapped but the unchanged update body
     try:
-        agent._update_bootstrapped(ro, (slots, nxt), 1 << 20, None, "auto", "default", window=True)
+        agent._update_bootstrapped(ro, (slots, nxt), 1 << 20, None, "auto", "default")
     finally:
         agent._update = update
     return int(slots.numel())

@@ -94,6 +94,9 @@ class Rollout:
 
 
 class ReinforceAgent:
+    gae_lambda = 0.0                # set by SharedTrunkActorCritic; 0 = the reference's TD(0) advantages
+    _adam_t_c = 0                   # Adam step counter of a separate critic
+
     def __init__(self, env, mlp_config: MLPConfig, agent_config: ReinforceAgentConfig | None = None,
                  initial_params_path: str | None = None):
         self.env = env
@@ -131,7 +134,6 @@ class ReinforceAgent:
             cparams = init_model_params(input_dim, self.mlp_config.hidden_sizes, 1, self.rng,
                                         self.mlp_config.init_distribution, self.mlp_config.last_init_normal)
             self._critic = self._make_net(cparams)
-            self._adam_t_c = 0
         self._bind_grads()
         self._scratch: dict[str, torch.Tensor] = {}
         self.last_update_info: dict[str, Any] = {}
@@ -198,7 +200,7 @@ class ReinforceAgent:
         """Everything update_batch mutates: actor, critic, Adam moments and step counters (one .npz)."""
         out = {"actor_theta": self._actor.theta.cpu().numpy(), "actor_dims": np.asarray(self._actor.dims, np.int64),
                "actor_adam_m": self._actor.adam_m.cpu().numpy(), "actor_adam_v": self._actor.adam_v.cpu().numpy(),
-               "adam_t": np.int64(self._adam_t), "adam_t_c": np.int64(getattr(self, "_adam_t_c", 0)),
+               "adam_t": np.int64(self._adam_t), "adam_t_c": np.int64(self._adam_t_c),
                "has_critic": np.int64(self._critic is not None)}
         if self._critic is not None:
             out.update(critic_theta=self._critic.theta.cpu().numpy(), critic_dims=np.asarray(self._critic.dims, np.int64),
@@ -207,7 +209,7 @@ class ReinforceAgent:
 
     def save_state(self) -> dict[str, Any]:
         """Device-side snapshot of everything an update mutates (see save_checkpoint), for load_state."""
-        st = {"adam_t": self._adam_t, "adam_t_c": getattr(self, "_adam_t_c", 0)}
+        st = {"adam_t": self._adam_t, "adam_t_c": self._adam_t_c}
         for name, net in (("actor", self._actor), ("critic", self._critic)):
             if net is not None:
                 st[name] = (net.theta.clone(), net.adam_m.clone(), net.adam_v.clone())
@@ -300,14 +302,24 @@ class ReinforceAgent:
             _lib.check(self._lib.b2048_mlp_forward(self._h, _ptr(boards), C.byref(net.desc), _ptr(out), boards.numel(),
                                                    int(precision), _stream()), "b2048_mlp_forward")
 
-    def _forward_checked(self, net: DeviceMLP, boards: torch.Tensor, out: torch.Tensor, prec: int) -> bool:
+    def _forward_checked(self, net: DeviceMLP, boards: torch.Tensor, out: torch.Tensor, prec: int, fell_back: list,
+                         head_mode: int) -> None:
         """b2048_mlp_forward at prec.  The split-fp16 path keeps activations in fp16: a network whose activations leave the
-        fp16 range gives non-finite outputs, which are recomputed on the fp32 kernels.  True when that happened."""
+        fp16 range gives non-finite outputs, which are recomputed on the fp32 kernels; head_mode is then appended to
+        fell_back."""
         self._net_forward(net, boards, out, prec)
         if prec in (2, 3) and not bool(torch.isfinite(out).all()):
             self._net_forward(net, boards, out, 0)
-            return True
-        return False
+            fell_back.append(head_mode)
+
+    @staticmethod
+    def _update_precision(precision: int | str) -> int:
+        """The precision code of the learner's forward / backward passes for an update's `precision` argument."""
+        return 2 if precision == "auto" else int(precision)
+
+    def _precision_info(self, prec: int, n: int, fell_back: list) -> str:
+        """info["precision"] of an update of n samples at prec."""
+        return self._update_mode_name(prec, n) + (" [fell back to fp32: non-finite fp16 intermediates]" if fell_back else "")
 
     @staticmethod
     def _small_batch_precision(prec: int, n: int) -> int:
@@ -369,19 +381,29 @@ class ReinforceAgent:
         return sumsq
 
     def _optimizer_step(self) -> tuple[torch.Tensor, torch.Tensor | None]:
-        """One optimizer step of the actor (or the shared network) and of a separate critic, each Adam counter advanced
-        once; returns their squared gradient norms (device double[1]; None without a separate critic)."""
+        """One optimizer step of the actor and of a separate critic, each Adam counter advanced once; returns their squared
+        gradient norms (device double[1]; None without a critic)."""
         cfg = self.agent_config
-        shared = getattr(self, "_shared_net", None)
         if cfg.optimizer == "adam":
             self._adam_t += 1
-        ss_a = self._apply(self._actor if shared is None else shared, cfg.learning_rate, +1.0, self._adam_t)
+        ss_a = self._apply(self._actor, cfg.learning_rate, +1.0, self._adam_t)
         ss_c = None
-        if cfg.use_critic and self._critic is not None and shared is None:
+        if self._has_value_function():
             if cfg.optimizer == "adam":
                 self._adam_t_c += 1
-            ss_c = self._apply(self._critic, cfg.critic_learning_rate, -1.0, getattr(self, "_adam_t_c", 0))
+            ss_c = self._apply(self._critic, cfg.critic_learning_rate, -1.0, self._adam_t_c)
         return ss_a, ss_c
+
+    def _step(self, allreduce) -> tuple[torch.Tensor, torch.Tensor | None]:
+        """What follows the backward passes of an update step: ONE all-reduce of [actor gradient | critic gradient] when
+        sharded, then _optimizer_step."""
+        if allreduce is not None:
+            allreduce(self._grad_all)
+        return self._optimizer_step()
+
+    def _has_value_function(self) -> bool:
+        """A separate critic (use_critic=True) or SharedTrunkActorCritic's value head."""
+        return bool(self.agent_config.use_critic) and self._critic is not None
 
     # ------------------------------------------------------------------ reference API: acting
     def _obs_to_packed(self, obs) -> tuple[int, int]:
@@ -493,13 +515,7 @@ class ReinforceAgent:
             benv.reset_many()
         fixed = horizon is not None
         cap = int(horizon) if fixed else int(max_steps or benv.config.max_steps or 4096)
-        boards = self._buf("ro_boards", (cap + 1, B), torch.int64)
-        flags = self._buf("ro_flags", (cap + 1, B), torch.uint8)
-        actions = self._buf("ro_actions", (cap, B), torch.uint8)
-        rewards = self._buf("ro_rewards", (cap, B), torch.float32)
-        length = torch.zeros(B, dtype=torch.int32, device=self.device)
-        boards[0].copy_(benv.board)
-        flags[0].copy_(benv.flags)
+        boards, flags, actions, rewards, length = self._rollout_buffers(benv, cap)
         if precision == "auto":
             precision = 1 if (B >= 4096 and self.tc_supported()) else 0
         from .batched_env import make_env_cfg
@@ -551,6 +567,19 @@ class ReinforceAgent:
         benv.flags = flags[T]
         return Rollout(boards[: T + 1], flags[: T + 1], actions[:T], rewards[:T], length, T, auto_reset=fixed, seed=benv.seed,
                        gid0=benv.gid0, t0=t0)
+
+    def _rollout_buffers(self, benv: Batched2048Env, cap: int):
+        """(boards, flags, actions, rewards, length) scratch buffers for up to cap steps of benv's boards, slice 0 holding
+        the current boards and flags, and zeroed lengths."""
+        B = benv.num_envs
+        boards = self._buf("ro_boards", (cap + 1, B), torch.int64)
+        flags = self._buf("ro_flags", (cap + 1, B), torch.uint8)
+        actions = self._buf("ro_actions", (cap, B), torch.uint8)
+        rewards = self._buf("ro_rewards", (cap, B), torch.float32)
+        length = torch.zeros(B, dtype=torch.int32, device=self.device)
+        boards[0].copy_(benv.board)
+        flags[0].copy_(benv.flags)
+        return boards, flags, actions, rewards, length
 
     def _live_chunks(self, launch, length: torch.Tensor, cap: int, check_every: int) -> int:
         """Run-to-termination chunks on the live-board list: launch(T, chunk, slot_map, upper, count) enqueues steps
@@ -606,13 +635,7 @@ class ReinforceAgent:
         policy_rng = np_seed_streams(policy_seeds, self.device)
         benv.reset_many(env_seeds=env_seeds)
         cap = int(max_steps or benv.config.max_steps or 4096)
-        boards = self._buf("ro_boards", (cap + 1, B), torch.int64)
-        flags = self._buf("ro_flags", (cap + 1, B), torch.uint8)
-        actions = self._buf("ro_actions", (cap, B), torch.uint8)
-        rewards = self._buf("ro_rewards", (cap, B), torch.float32)
-        length = torch.zeros(B, dtype=torch.int32, device=self.device)
-        boards[0].copy_(benv.board)
-        flags[0].copy_(benv.flags)
+        boards, flags, actions, rewards, length = self._rollout_buffers(benv, cap)
         actions.zero_()                 # the policy writes no action for a finished board
         rewards.zero_()
         cfg = make_env_cfg(benv.config, "buffer", auto_reset=False, emit_obs=False)
@@ -689,7 +712,8 @@ class ReinforceAgent:
         the policy gradient only").  With a 'batch' / 'batch_norm' baseline the per-sample coefficient is
         (v - mean) / std * w / (T n) with GLOBAL mean / std (reinforce_agent.py:303-322, :864-881); the backward pass is
         linear in it, so g = (g_A - mean g_B) / std with g_A from the coefficients v w / (T n) and g_B from w / (T n).  Both
-        are local sums; they travel with the critic gradient and the four float64 baseline sums in one float64 buffer."""
+        are local sums; they travel with the critic gradient and the four float64 baseline sums in one float64 buffer.
+        Ends with adv / coef as the default exchange reports them (global statistics)."""
         lib, h, dev, T, B = self._lib, self._h, self.device, ro.T, ro.B
         mode = BASELINE[self.agent_config.baseline_mode]
         na = self._actor.n_params
@@ -701,9 +725,7 @@ class ReinforceAgent:
             _lib.check(lib.b2048_weighted_stats(h, _ptr(values), _ptr(ro.length), _ptr(ro.ep_weight), T, B, _ptr(stats),
                                                 _stream()), "b2048_weighted_stats")
         for k, v in enumerate((values, ones)):                       # g_A, then g_B
-            with torch.cuda.device(dev):
-                _lib.check(lib.b2048_advantages(h, _ptr(v), _ptr(ro.length), _ptr(ro.ep_weight), 0, n_traj, T, B, None,
-                                                _ptr(coef), _ptr(stats), 1, _ptr(ep_mean), _stream()), "b2048_advantages")
+            self._advantages(v, ro.length, ro.ep_weight, 0, n_traj, None, coef, stats, ep_mean, window=False, pre=1)
             backward(self._actor, coef.reshape(-1), 0)
             if k == 0:
                 msg[:na].copy_(self._actor.grad)
@@ -719,6 +741,31 @@ class ReinforceAgent:
         g_a, g_b = msg[:na], msg[na: 2 * na]
         self._grad_all.copy_(msg[na: na + self._grad_all.numel()])   # critic part (and g_B, overwritten next)
         self._actor.grad.copy_((g_a - mean32.to(torch.float64) * g_b) / std32.to(torch.float64))
+        self._advantages(values, ro.length, ro.ep_weight, mode, n_traj, adv, coef, stats, ep_mean, window=False, pre=1)
+
+    def _advantages(self, values: torch.Tensor, length: torch.Tensor, ep_weight: torch.Tensor | None, mode: int,
+                    n_traj: float, adv: torch.Tensor | None, coef: torch.Tensor, stats: torch.Tensor,
+                    ep_mean: torch.Tensor | None, window: bool, pre: int = 0, allreduce=None) -> None:
+        """adv / coef of the baseline `mode` on the [T, B] values (the raw advantages, or a constant for the entropy
+        coefficients): b2048_advantages with the weight w_b / (len_b n_traj) on episodes, b2048_advantages_window with
+        1 / (T n_traj) on a window (length = valid_len).  pre=1: stats already holds the baseline sums.  Sharded (allreduce
+        given) with a 'batch' / 'batch_norm' baseline, the local sums are all-reduced first (the 32-byte message)."""
+        lib, h = self._lib, self._h
+        T, B = values.shape
+        with torch.cuda.device(self.device):
+            if allreduce is not None and mode >= 2 and not pre:
+                stats.zero_()
+                _lib.check(lib.b2048_weighted_stats(h, _ptr(values), _ptr(length), _ptr(ep_weight), T, B, _ptr(stats),
+                                                    _stream()), "b2048_weighted_stats")
+                allreduce(stats)
+                pre = 1
+            if window:
+                _lib.check(lib.b2048_advantages_window(h, _ptr(values), _ptr(length), mode, n_traj, T, B, _ptr(adv),
+                                                       _ptr(coef), _ptr(stats), pre, _stream()), "b2048_advantages_window")
+            else:
+                _lib.check(lib.b2048_advantages(h, _ptr(values), _ptr(length), _ptr(ep_weight), mode, n_traj, T, B,
+                                                _ptr(adv), _ptr(coef), _ptr(stats), pre, _ptr(ep_mean), _stream()),
+                           "b2048_advantages")
 
     def update_batch(self, trajectories: list[dict[str, Any]]) -> None:
         """reinforce_agent.py:357-620 on reference-style trajectories (list of dicts from run_episode)."""
@@ -776,7 +823,7 @@ class ReinforceAgent:
         boot = self._truncated_episode_ends(ro) if bootstrap_truncation else None
         if cfg.augmentation:
             ro = self._augment_rollout(ro)
-        return self._update_bootstrapped(ro, boot, chunk, allreduce, precision, exchange, window=False, beta=beta)
+        return self._update_bootstrapped(ro, boot, chunk, allreduce, precision, exchange, beta)
 
     def update_from_horizon(self, ro: Rollout, allreduce=None, precision: int | str = "auto", chunk: int = 1 << 20,
                             exchange: str = "default", bootstrap_truncation: bool = False,
@@ -803,14 +850,7 @@ class ReinforceAgent:
         function; with REINFORCE the slots t < valid_len[b])."""
         cfg = self._check_update_config(exchange)
         beta = self._check_entropy(entropy_coef, exchange, precision)
-        if not ro.auto_reset:
-            raise ValueError("update_from_horizon needs a fixed-horizon rollout with reset-on-done (rollout_many(horizon=H))")
-        if cfg.baseline_mode == "each":
-            raise ValueError("baseline 'each' needs whole episodes: not available on fixed-horizon windows")
-        if cfg.reward_rank_weights or ro.ep_weight is not None:
-            raise ValueError("reward rank weights need whole episodes: not available on fixed-horizon windows")
-        if exchange == "one_message":
-            raise ValueError("exchange='one_message' is not implemented for fixed-horizon windows")
+        self._check_window(ro, exchange, "update_from_horizon")
         if bootstrap_truncation:
             self._check_bootstrap(ro, window=True)
         if ro.B == 0 or ro.T == 0:
@@ -819,7 +859,20 @@ class ReinforceAgent:
         boot = self._truncated_window_steps(ro) if bootstrap_truncation else None
         if cfg.augmentation:
             ro = self._augment_rollout(ro)
-        return self._update_bootstrapped(ro, boot, chunk, allreduce, precision, exchange, window=True, beta=beta)
+        return self._update_bootstrapped(ro, boot, chunk, allreduce, precision, exchange, beta)
+
+    def _check_window(self, ro: Rollout, exchange: str, what: str) -> None:
+        """The configurations a window update refuses (ValueError): a rollout without reset-on-done, and what needs whole
+        episodes or the one-message exchange."""
+        cfg = self.agent_config
+        if not ro.auto_reset:
+            raise ValueError(f"{what} needs a fixed-horizon rollout with reset-on-done (rollout_many(horizon=H))")
+        if cfg.baseline_mode == "each":
+            raise ValueError("baseline 'each' needs whole episodes: not available on fixed-horizon windows")
+        if cfg.reward_rank_weights or ro.ep_weight is not None:
+            raise ValueError("reward rank weights need whole episodes: not available on fixed-horizon windows")
+        if exchange == "one_message":
+            raise ValueError("exchange='one_message' is not implemented for fixed-horizon windows")
 
     # ------------------------------------------------------------------ PPO on windows
     def update_ppo(self, ro: Rollout, epochs: int = 4, minibatches: int = 4, clip_eps: float = 0.2,
@@ -851,16 +904,11 @@ class ReinforceAgent:
         rank-local mean H at the step's parameters.  Refused with precision=1."""
         cfg = self._check_update_config("default")
         beta = self._check_entropy(entropy_coef, "default", precision)
-        if not (cfg.use_critic and getattr(self, "_critic", None) is not None):
+        if not self._has_value_function():
             raise ValueError("update_ppo needs a value function: use_critic=True or SharedTrunkActorCritic")
-        if not ro.auto_reset:
-            raise ValueError("update_ppo needs a fixed-horizon rollout with reset-on-done (rollout_many(horizon=H))")
+        self._check_window(ro, "default", "update_ppo")
         if cfg.augmentation:
             raise ValueError("update_ppo does not implement augmentation")
-        if cfg.reward_rank_weights or ro.ep_weight is not None:
-            raise ValueError("reward rank weights need whole episodes: not available on fixed-horizon windows")
-        if cfg.baseline_mode == "each":
-            raise ValueError("baseline 'each' needs whole episodes: not available on fixed-horizon windows")
         n_traj = int(ro.n_traj if ro.n_traj is not None else ro.B)
         N = ro.T * n_traj
         if int(epochs) < 1:
@@ -879,13 +927,12 @@ class ReinforceAgent:
         if ro.B == 0 or ro.T == 0:
             return {}
         self._horizon_account(ro)
-        prec = 2 if precision == "auto" else int(precision)
         if bootstrap_truncation:
             boot = self._truncated_window_steps(ro)
             if boot[0].numel():
                 ro = self._fold_truncation(ro, boot, precision)[0]
-        return self._ppo(ro, int(epochs), int(minibatches), float(clip_eps), value_clip_eps, int(shuffle_seed), allreduce, prec,
-                         n_traj, beta)
+        return self._ppo(ro, int(epochs), int(minibatches), float(clip_eps), value_clip_eps, int(shuffle_seed), allreduce,
+                         self._update_precision(precision), n_traj, beta)
 
     def ppo_minibatch_lists(self, T: int, B: int, n_traj: int, gid0: int, minibatches: int, shuffle_seed: int,
                             epoch: int) -> tuple[torch.Tensor, list[int]]:
@@ -908,41 +955,20 @@ class ReinforceAgent:
         T, B = ro.T, ro.B
         n, N = T * B, T * n_traj
         gid0 = int(ro.gid0) if n_traj > B else 0
-        lam = float(getattr(self, "gae_lambda", 0.0))
         boards = ro.boards[:T].reshape(-1)
         mflags = ro.flags[:T].reshape(-1)
         acts = ro.actions[:T].reshape(-1)
         fell_back: list = []
         # ---- once per window, at theta_old
-        values = self._buf("values", (T + 1, B), torch.float32)
-        if self._forward_checked(self._critic, ro.boards[: T + 1].reshape(-1), values.view(-1), prec):
-            fell_back.append(1)
-        gae, td, gcoef = (self._buf(k, (T, B), torch.float32) for k in ("gae", "td", "gcoef"))
-        valid = self._buf("valid_len", (B,), torch.int32)
-        self._segment_targets(ro.rewards[:T].contiguous(), ro.flags[: T + 1].contiguous(), values, lam, float(n_traj), gae, td,
-                              gcoef, valid)
-        mode = BASELINE[cfg.baseline_mode]
-        stats = self._buf("stats", (4,), torch.float64)
-        adv, coef = self._buf("adv", (T, B), torch.float32), self._buf("coef", (T, B), torch.float32)
-        pre = 0
-        with torch.cuda.device(dev):
-            if allreduce is not None and mode >= 2:            # the window is sharded: the baseline sums are global
-                stats.zero_()
-                _lib.check(lib.b2048_weighted_stats(h, _ptr(gae), _ptr(valid), None, T, B, _ptr(stats), _stream()),
-                           "b2048_weighted_stats")
-                allreduce(stats)
-                pre = 1
-            _lib.check(lib.b2048_advantages_window(h, _ptr(gae), _ptr(valid), mode, float(n_traj), T, B, _ptr(adv), _ptr(coef),
-                                                   _ptr(stats), pre, _stream()), "b2048_advantages_window")
+        tg = self._window_targets(ro, prec, float(n_traj), allreduce, fell_back)
+        values, gae, adv = tg["values"], tg["raw"], tg["advantages"]
         logits = self._buf("ppo_logits", (n, 4), torch.float32)
-        if self._forward_checked(self._actor, boards, logits, prec):
-            fell_back.append(0)
+        self._forward_checked(self._actor, boards, logits, prec, fell_back, 0)
         logp_old = self._buf("ppo_logp_old", (n,), torch.float64)
         with torch.cuda.device(dev):
             _lib.check(lib.b2048_ppo_logp(h, _ptr(logits), _ptr(mflags) if self._use_mask else None, _ptr(acts), n,
                                           _ptr(logp_old), _stream()), "b2048_ppo_logp")
         # ---- epochs x minibatches clipped steps
-        shared = getattr(self, "_shared_net", None)
         ep_stats = torch.zeros((epochs, 5), dtype=torch.float64, device=dev)
         norms = torch.zeros((epochs * M, 2), dtype=torch.float64, device=dev)
         ent = torch.zeros(epochs, dtype=torch.float64, device=dev) if beta > 0.0 else None
@@ -962,10 +988,8 @@ class ReinforceAgent:
                     bx, fx, ax = boards.index_select(0, idx), mflags.index_select(0, idx), acts.index_select(0, idx)
                     z = self._buf("ppo_z", (k, 4), torch.float32)
                     v = self._buf("ppo_v", (k,), torch.float32)
-                    if self._forward_checked(self._actor, bx, z, p):
-                        fell_back.append(0)
-                    if self._forward_checked(self._critic, bx, v, p):
-                        fell_back.append(1)
+                    self._forward_checked(self._actor, bx, z, p, fell_back, 0)
+                    self._forward_checked(self._critic, bx, v, p, fell_back, 1)
                     cf, gc = self._buf("ppo_coef", (k,), torch.float32), self._buf("ppo_gcoef", (k,), torch.float32)
                     with torch.cuda.device(dev):
                         _lib.check(lib.b2048_ppo_coefficients(
@@ -981,11 +1005,7 @@ class ReinforceAgent:
                 else:                                          # this shard holds none of the minibatch's samples
                     self._actor.grad.zero_()
                     self._critic.grad.zero_()
-                if shared is not None:
-                    self._merge_shared_grads()
-                if allreduce is not None:
-                    allreduce(self._grad_all)                  # ONE message per minibatch step
-                ss_a, ss_c = self._optimizer_step()
+                ss_a, ss_c = self._step(allreduce)             # ONE message per minibatch step
                 norms[e * M + m, 0] = ss_a[0]
                 if ss_c is not None:
                     norms[e * M + m, 1] = ss_c[0]
@@ -995,11 +1015,11 @@ class ReinforceAgent:
             "clip_fraction": st[:, 0].tolist(), "mean_ratio": st[:, 1].tolist(), "approx_kl": st[:, 2].tolist(),
             "surrogate": st[:, 3].tolist(), "value_loss": st[:, 4].tolist(), "actor_grad_norms": nr[:, 0].tolist(),
             "advantages": adv, "gae": gae, "values_old": values, "logp_old": logp_old,
-            "precision": self._update_mode_name(prec, n) + (" [fell back to fp32: non-finite fp16 intermediates]" if fell_back else "")}
+            "precision": self._precision_info(prec, n, fell_back)}
         info["actor_grad_norm"] = info["actor_grad_norms"][-1]
         if ent is not None:
             info["entropy"] = (ent.cpu().numpy() / n).tolist()
-        if shared is None:
+        if ss_c is not None:                                   # a separate critic (not a value head on the shared trunk)
             info["critic_grad_norms"] = nr[:, 1].tolist()
             info["critic_grad_norm"] = info["critic_grad_norms"][-1]
         self.last_update_info = info
@@ -1009,7 +1029,7 @@ class ReinforceAgent:
 
     # ------------------------------------------------------------------ bootstrapping at truncation
     def _check_bootstrap(self, ro: Rollout, window: bool) -> None:
-        if not (self.agent_config.use_critic and getattr(self, "_critic", None) is not None):
+        if not self._has_value_function():
             raise ValueError("bootstrap_truncation needs a value function: use_critic=True or SharedTrunkActorCritic")
         if window and (ro.seed is None or ro.t0 is None):
             raise ValueError("bootstrap_truncation on a window needs its env streams (Rollout.seed and Rollout.t0, which "
@@ -1040,16 +1060,16 @@ class ReinforceAgent:
         return slots, ro.boards[: T + 1].gather(0, last).reshape(-1)[lanes]
 
     def _update_bootstrapped(self, ro: Rollout, boot, chunk: int, allreduce, precision: int | str, exchange: str,
-                             window: bool, beta: float = 0.0) -> dict[str, Any]:
+                             beta: float = 0.0) -> dict[str, Any]:
         """_update on a copy of the rewards with gamma V(s') folded in at the truncated steps (boot = (slots, s') of the
         rollout before augmentation; None: no bootstrap).  The target kernels use V = 0 after an episode's last step, so
         r' = r + gamma V(s') (each operation rounded separately, b2048_fold_bootstrap) makes every target, TD error,
         advantage and critic coefficient the bootstrapped one.  With augmentation variant v of step (t, b) is column
         v B + b, and it folds the value of variant v of s'."""
         if boot is None or boot[0].numel() == 0:
-            return self._update(ro, window, chunk, allreduce, precision, exchange, beta)
+            return self._update(ro, chunk, allreduce, precision, exchange, beta)
         folded, slots, nxt, values = self._fold_truncation(ro, boot, precision)
-        info = self._update(folded, window, chunk, allreduce, precision, exchange, beta)
+        info = self._update(folded, chunk, allreduce, precision, exchange, beta)
         info.update(bootstrap_slots=slots, bootstrap_boards=nxt, bootstrap_values=values)
         return info
 
@@ -1068,9 +1088,9 @@ class ReinforceAgent:
             slots = ((t * B + b).unsqueeze(0) + B0 * torch.arange(8, device=dev).unsqueeze(1)).reshape(-1)
             nxt = nxt8
         K = slots.numel()
-        prec = 2 if precision == "auto" else int(precision)
         values = torch.empty(K, dtype=torch.float32, device=dev)
-        self._forward_checked(self._critic, nxt, values, self._small_batch_precision(prec, K))
+        # a fall-back of this forward is not reported in info["precision"]
+        self._forward_checked(self._critic, nxt, values, self._small_batch_precision(self._update_precision(precision), K), [], 1)
         rewards = torch.empty((T, B), dtype=torch.float32, device=dev)
         with torch.cuda.device(dev):
             _lib.check(lib.b2048_fold_bootstrap(h, _ptr(ro.rewards[:T].contiguous()), _ptr(slots), _ptr(values), K, T * B,
@@ -1140,71 +1160,106 @@ class ReinforceAgent:
             raise ValueError(f"Unknown critic loss type: {cfg.critic_loss_type}")    # reinforce_agent.py:908
         return cfg
 
-    def _update(self, ro: Rollout, window: bool, chunk: int, allreduce, precision: int | str, exchange: str,
+    def _window_targets(self, ro: Rollout, prec: int, n_traj: float, allreduce, fell_back: list) -> dict[str, torch.Tensor]:
+        """The targets of a fixed-horizon window at the current parameters (b2048_segment_targets), then adv / coef of the
+        configured baseline over the window's samples, the slots t < valid_len[b].  With a value function: V on all T + 1
+        slices (V(boards[T]) bootstraps the cut-off tail), the TD errors td, the critic coefficients gcoef and
+        raw = A_t = delta_t + gamma lambda A_{t+1}; every slot is a sample (valid_len = T: the window is never compacted).
+        Without: raw = the segment returns, and the samples are the slots of the episodes that end inside the window.
+        Returns {valid_len, raw, advantages, coef} and, with a value function, {values, td, gcoef}."""
+        T, B = ro.T, ro.B
+        rewards, flags = ro.rewards[:T].contiguous(), ro.flags[: T + 1].contiguous()
+        valid = self._buf("valid_len", (B,), torch.int32)
+        tg: dict[str, torch.Tensor] = {"valid_len": valid}
+        if self._has_value_function():
+            values = self._buf("values", (T + 1, B), torch.float32)
+            self._forward_checked(self._critic, ro.boards[: T + 1].reshape(-1), values.view(-1), prec, fell_back, 1)
+            raw, td, gcoef = (self._buf(k, (T, B), torch.float32) for k in ("gae", "td", "gcoef"))
+            self._segment_targets(rewards, flags, values, self.gae_lambda, n_traj, raw, td, gcoef, valid)
+            tg.update(values=values, td=td, gcoef=gcoef)
+        else:
+            raw = self._buf("returns", (T, B), torch.float32)
+            self._segment_targets(rewards, flags, None, self.gae_lambda, n_traj, raw, None, None, valid)
+        adv, coef = self._buf("adv", (T, B), torch.float32), self._buf("coef", (T, B), torch.float32)
+        self._advantages(raw, valid, None, BASELINE[self.agent_config.baseline_mode], n_traj, adv, coef,
+                         self._buf("stats", (4,), torch.float64), None, window=True, allreduce=allreduce)
+        tg.update(raw=raw, advantages=adv, coef=coef)
+        return tg
+
+    def _live_samples(self, ro: Rollout, length: torch.Tensor):
+        """(live, boards, flags, actions) of the samples t < length[b] of the [T, B] grid, flattened.  Run-to-termination
+        rollouts are ragged: slots with t >= len[b] carry no sample.  The per-sample work (forward / backward GEMMs) then runs
+        on the compacted list of live slots (ONE stream compaction of the live mask; live = their grid indices, None when
+        nothing is compacted); the [T, B] grid is kept for the per-episode time recurrences.  Pure index plumbing (torch)."""
+        T = ro.T
+        boards, mflags, acts = ro.boards[:T].reshape(-1), ro.flags[:T].reshape(-1), ro.actions[:T].reshape(-1)
+        if int(length.sum().item()) >= int(0.9 * T * ro.B):
+            return None, boards, mflags, acts
+        tgrid = torch.arange(T, device=self.device, dtype=torch.int32).unsqueeze(1)
+        live = torch.nonzero((tgrid < length.unsqueeze(0)).reshape(-1)).reshape(-1)
+        return live, boards.index_select(0, live), mflags.index_select(0, live), acts.index_select(0, live)
+
+    def _update(self, ro: Rollout, chunk: int, allreduce, precision: int | str, exchange: str,
                 beta: float = 0.0) -> dict[str, Any]:
-        """The body of update_from_rollout (window=False: one episode per lane, t < length) and update_from_horizon
-        (window=True: a fixed-horizon window, targets from b2048_segment_targets).  beta > 0: the entropy bonus."""
-        prec = 2 if precision == "auto" else int(precision)
+        """The body of update_from_rollout (one episode per lane, t < length) and update_from_horizon (ro.auto_reset: a
+        fixed-horizon window, _window_targets).  beta > 0: the entropy bonus."""
+        prec = self._update_precision(precision)
         cfg = self.agent_config
         T, B = ro.T, ro.B
         n_traj = float(ro.n_traj if ro.n_traj is not None else B)
         lib, h, dev = self._lib, self._h, self.device
-        n = T * B
-        boards = ro.boards[:T].reshape(-1)
-        mflags = ro.flags[:T].reshape(-1)
-        acts = ro.actions[:T].reshape(-1)
-        rewards = ro.rewards[:T].contiguous()
-        critic = cfg.use_critic and self._critic is not None
-        lam = float(getattr(self, "gae_lambda", 0.0))            # shared_trunk.py; 0 = the reference's TD(0) advantages
-        length = ro.length
-        if window:
-            # the samples of lane b are t < valid_len[b]: every slot with a critic, else the slots of the episodes that end
-            # inside the window (known from the flags alone, before the compaction below)
-            length = self._buf("valid_len", (B,), torch.int32)
-            flags_w = ro.flags[: T + 1].contiguous()
-            if critic:
-                length.fill_(T)
-            else:
-                returns = self._buf("returns", (T, B), torch.float32)
-                self._segment_targets(rewards, flags_w, None, lam, n_traj, returns, None, None, length)
-        # Run-to-termination rollouts are ragged: slots with t >= len[b] carry no sample.  The per-sample work
-        # (forward / backward GEMMs) runs on the compacted list of live slots; the [T, B] grid is kept only for
-        # the per-episode time recurrences (returns scan, TD shift).  Pure index plumbing (torch).
-        live = None
-        n_live = int(length.sum().item())
-        if n_live < int(0.9 * n):
-            tgrid = torch.arange(T, device=dev, dtype=torch.int32).unsqueeze(1)
-            # ONE stream compaction (nonzero) of the live mask; everything per-sample is then an index_select by it
-            live = torch.nonzero((tgrid < length.unsqueeze(0)).reshape(-1)).reshape(-1)
-            boards, mflags, acts = boards.index_select(0, live), mflags.index_select(0, live), acts.index_select(0, live)
-            n = n_live
+        critic = self._has_value_function()
+        mode = BASELINE[cfg.baseline_mode]
+        one_msg = exchange == "one_message" and allreduce is not None and mode >= 2
         stats = self._buf("stats", (4,), torch.float64)
         ep_mean = self._buf("ep_mean", (B,), torch.float32)
-        adv = self._buf("adv", (T, B), torch.float32)
-        coef = self._buf("coef", (T, B), torch.float32)
-        info: dict[str, Any] = {}
-        mode = BASELINE[cfg.baseline_mode]
+        fell_back: list = []
+        if ro.auto_reset:
+            tg = self._window_targets(ro, prec, n_traj, allreduce, fell_back)
+            length = tg["valid_len"]
+            info: dict[str, Any] = {"td": tg["td"]} if critic else {"returns": tg["raw"]}
+            info["valid_len"] = length
+            live, boards, mflags, acts = self._live_samples(ro, length)
+        else:
+            length = ro.length
+            live, boards, mflags, acts = self._live_samples(ro, length)
+            rewards = ro.rewards[:T].contiguous()
+            tg = {"advantages": self._buf("adv", (T, B), torch.float32), "coef": self._buf("coef", (T, B), torch.float32)}
+            if critic:
+                # critic block (reinforce_agent.py:403-498): V(s_t) for every stored state, TD(0) errors, critic coefficients
+                values = self._buf("values", (T, B), torch.float32)
+                vc = values.view(-1) if live is None else self._buf("values_c", (boards.numel(),), torch.float32)
+                self._forward_checked(self._critic, boards, vc, prec, fell_back, 1)
+                if live is not None:
+                    values.zero_()
+                    values.view(-1)[live] = vc
+                td = self._buf("td", (T, B), torch.float32)
+                tg["gcoef"] = self._buf("gcoef", (T, B), torch.float32)
+                with torch.cuda.device(dev):
+                    _lib.check(lib.b2048_td_errors(h, _ptr(rewards), _ptr(values), _ptr(length), _ptr(ro.ep_weight),
+                                                   float(cfg.gamma), int(cfg.critic_loss_type == "huber"),
+                                                   float(cfg.huber_delta), n_traj, T, B, _ptr(td), _ptr(tg["gcoef"]), _stream()),
+                               "b2048_td_errors")
+                raw = td                                             # advantages := baseline-processed TD errors (:495-498)
+                lam = float(self.gae_lambda)
+                if lam > 0.0:
+                    raw = self._buf("gae", (T, B), torch.float32)    # A_t = delta_t + gamma lambda A_{t+1}: the returns scan
+                    with torch.cuda.device(dev):
+                        _lib.check(lib.b2048_reverse_scan_f64(_ptr(td), _ptr(raw), _ptr(length), float(cfg.gamma) * lam, T, B,
+                                                              _stream()), "b2048_reverse_scan_f64")
+                info = {"td": td}
+            else:
+                raw = self._buf("returns", (T, B), torch.float32)
+                with torch.cuda.device(dev):
+                    _lib.check(lib.b2048_reverse_scan_f64(_ptr(rewards), _ptr(raw), _ptr(length), float(cfg.gamma), T, B,
+                                                          _stream()), "b2048_reverse_scan_f64")
+                info = {"returns": raw}
+            tg["raw"] = raw
+            if not one_msg:                                          # the one-message exchange forms them after its message
+                self._advantages(raw, length, ro.ep_weight, mode, n_traj, tg["advantages"], tg["coef"], stats, ep_mean,
+                                 window=False, allreduce=allreduce)
+        n = boards.numel()
 
-        one_msg = exchange == "one_message" and allreduce is not None and mode >= 2
-
-        def advantages(values, pre=0):
-            with torch.cuda.device(dev):
-                if allreduce is not None and mode >= 2 and not pre:
-                    # episodes are sharded over ranks: the baseline statistics are global sums
-                    stats.zero_()
-                    _lib.check(lib.b2048_weighted_stats(h, _ptr(values), _ptr(length), _ptr(ro.ep_weight), T, B,
-                                                        _ptr(stats), _stream()), "b2048_weighted_stats")
-                    allreduce(stats)
-                    pre = 1
-                if window:
-                    _lib.check(lib.b2048_advantages_window(h, _ptr(values), _ptr(length), mode, n_traj, T, B, _ptr(adv),
-                                                           _ptr(coef), _ptr(stats), pre, _stream()), "b2048_advantages_window")
-                    return
-                _lib.check(lib.b2048_advantages(h, _ptr(values), _ptr(length), _ptr(ro.ep_weight), mode, n_traj, T, B,
-                                                _ptr(adv), _ptr(coef), _ptr(stats), pre, _ptr(ep_mean), _stream()),
-                           "b2048_advantages")
-
-        fell_back = []
         ent_cf = ent_acc = None
         if beta > 0.0:
             # ecoef = beta x the sample's weight in the policy term: the advantage kernels in mode 0 on a constant beta give
@@ -1213,14 +1268,8 @@ class ReinforceAgent:
             ent_cf = self._buf("ent_coef", (T, B), torch.float32)
             ent_adv = self._buf("ent_adv", (T, B), torch.float32)
             ent_acc = self._buf("ent_acc", (1,), torch.float64).zero_()
-            with torch.cuda.device(dev):
-                if window:
-                    _lib.check(lib.b2048_advantages_window(h, _ptr(bvals), _ptr(length), 0, n_traj, T, B, _ptr(ent_adv),
-                                                           _ptr(ent_cf), _ptr(stats), 1, _stream()), "b2048_advantages_window")
-                else:
-                    _lib.check(lib.b2048_advantages(h, _ptr(bvals), _ptr(length), _ptr(ro.ep_weight), 0, n_traj, T, B,
-                                                    _ptr(ent_adv), _ptr(ent_cf), _ptr(stats), 1, _ptr(ep_mean), _stream()),
-                               "b2048_advantages")
+            self._advantages(bvals, length, ro.ep_weight, 0, n_traj, ent_adv, ent_cf, stats, ep_mean, window=ro.auto_reset,
+                             pre=1)
             ent_cf = ent_cf.reshape(-1)
             if live is not None:
                 ent_cf = ent_cf.index_select(0, live)
@@ -1228,72 +1277,21 @@ class ReinforceAgent:
         def backward(net: DeviceMLP, cf: torch.Tensor, head_mode: int, with_entropy: bool = False):
             if live is not None:
                 cf = cf.index_select(0, live)
-            if with_entropy and ent_cf is not None:
-                self._backward(net, boards, mflags, acts, cf, n, head_mode, prec, chunk, fell_back, ent_cf, ent_acc)
-            else:
-                self._backward(net, boards, mflags, acts, cf, n, head_mode, prec, chunk, fell_back)
+            self._backward(net, boards, mflags, acts, cf, n, head_mode, prec, chunk, fell_back,
+                           ent_cf if with_entropy else None, ent_acc)
 
         if critic:
-            # critic block (reinforce_agent.py:403-498): V(s_t) for every stored state, TD(0) errors, critic grads
-            # (a window also evaluates V(boards[T]), which bootstraps the cut-off tail; none of its slots is compacted)
-            nv = T + 1 if window else T
-            vboards = ro.boards[:nv].reshape(-1) if window else boards
-            values = self._buf("values", (nv, B), torch.float32)
-            vc = values.view(-1) if live is None else self._buf("values_c", (n,), torch.float32)
-            if self._forward_checked(self._critic, vboards, vc, prec):
-                fell_back.append(1)
-            if live is not None:
-                values.zero_()
-                values.view(-1)[live] = vc
-            td = self._buf("td", (T, B), torch.float32)
-            gcoef = self._buf("gcoef", (T, B), torch.float32)
-            if window:                                               # TD errors and A_t = delta_t + gamma lambda A_{t+1}
-                gae = self._buf("gae", (T, B), torch.float32)
-                self._segment_targets(rewards, flags_w, values, lam, n_traj, gae, td, gcoef, length)
-            else:
-                with torch.cuda.device(dev):
-                    _lib.check(lib.b2048_td_errors(h, _ptr(rewards), _ptr(values), _ptr(length), _ptr(ro.ep_weight),
-                                                   float(cfg.gamma), int(cfg.critic_loss_type == "huber"),
-                                                   float(cfg.huber_delta), n_traj, T, B, _ptr(td), _ptr(gcoef), _stream()),
-                               "b2048_td_errors")
-            backward(self._critic, gcoef.reshape(-1), 1)
-            base_values = gae if window else td                      # advantages := baseline-processed TD errors (:495-498)
-            info["td"] = td
-            if lam > 0.0 and not window:
-                gae = self._buf("gae", (T, B), torch.float32)        # A_t = delta_t + gamma lambda A_{t+1}: the returns scan
-                with torch.cuda.device(dev):
-                    _lib.check(lib.b2048_reverse_scan_f64(_ptr(td), _ptr(gae), _ptr(length), float(cfg.gamma) * lam, T, B,
-                                                          _stream()), "b2048_reverse_scan_f64")
-                base_values = gae
-        else:
-            if not window:
-                returns = self._buf("returns", (T, B), torch.float32)
-                with torch.cuda.device(dev):
-                    _lib.check(lib.b2048_reverse_scan_f64(_ptr(rewards), _ptr(returns), _ptr(length), float(cfg.gamma), T, B,
-                                                          _stream()), "b2048_reverse_scan_f64")
-            base_values = returns
-            info["returns"] = returns
-        if window:
-            info["valid_len"] = length
-        shared = getattr(self, "_shared_net", None)                  # shared_trunk.py: one network, two heads, one optimizer
-        if one_msg and shared is not None:
-            raise ValueError("exchange='one_message' is implemented for separate actor / critic networks")
+            backward(self._critic, tg["gcoef"].reshape(-1), 1)
         if one_msg:
-            self._one_message_exchange(base_values, ro, n_traj, adv, coef, stats, ep_mean, backward, allreduce)
-            advantages(base_values, pre=1)   # adv / coef as the default exchange reports them (global statistics)
+            self._one_message_exchange(tg["raw"], ro, n_traj, tg["advantages"], tg["coef"], stats, ep_mean, backward, allreduce)
+            ss_a, ss_c = self._optimizer_step()
         else:
-            advantages(base_values)
-            backward(self._actor, coef.reshape(-1), 0, with_entropy=True)
-            if shared is not None:
-                self._merge_shared_grads()   # trunk gradient = policy part - value_coef x value part
-            if allreduce is not None:
-                allreduce(self._grad_all)    # ONE message per update: [actor gradient | critic gradient]
-
-        ss_a, ss_c = self._optimizer_step()
-        info["advantages"] = adv
+            backward(self._actor, tg["coef"].reshape(-1), 0, with_entropy=True)
+            ss_a, ss_c = self._step(allreduce)
+        info["advantages"] = tg["advantages"]
         if ent_acc is not None:
             info["entropy"] = float(ent_acc.cpu()[0]) / max(n, 1)
-        info["precision"] = self._update_mode_name(prec, n) + (" [fell back to fp32: non-finite fp16 intermediates]" if fell_back else "")
+        info["precision"] = self._precision_info(prec, n, fell_back)
         info["actor_grad_norm"] = float(ss_a.cpu()[0]) ** 0.5
         if ss_c is not None:
             info["critic_grad_norm"] = float(ss_c.cpu()[0]) ** 0.5

@@ -55,6 +55,7 @@ def _view(template: DeviceMLP, dims: list[int], layer_ptrs: list[tuple[int, int]
 class SharedTrunkActorCritic(ReinforceAgent):
     """ReinforceAgent API (select_action / run_episode / rollout_many / update_from_rollout / update_batch) on one network
     with a policy head and a value head.  value_coef weighs the value loss in the joint objective; gae_lambda in [0, 1]."""
+    _shared_net: _FlatNet | None = None                         # set by _install, after the base constructor
 
     def __init__(self, env, mlp_config, agent_config: ReinforceAgentConfig | None = None, value_coef: float = 0.5,
                  gae_lambda: float = 0.0, initial_params_path: str | None = None):
@@ -90,21 +91,34 @@ class SharedTrunkActorCritic(ReinforceAgent):
         ptrs.append((base + 4 * na, base + 4 * (na + H)))
         self._actor = actor
         self._critic = _view(actor, actor.dims[:-1] + [1], ptrs)
-        self._adam_t_c = 0
         self._bind_grads()
 
     def _bind_grads(self) -> None:
-        sn = getattr(self, "_shared_net", None)
+        sn = self._shared_net
         if sn is None:                                          # during the base constructor
             return super()._bind_grads()
         self._grad_all = sn.grad                                # the one buffer a sharded update all-reduces
         self._actor.grad = sn.grad[: self._n_policy]
         self._critic.grad = torch.zeros(self._critic.n_params, dtype=torch.float32, device=self.device)
 
-    def _merge_shared_grads(self) -> None:
+    # ------------------------------------------------------------------ learning
+    def _step(self, allreduce):
+        """Merges the value view's gradient into the one vector (trunk gradient = policy part - value_coef x value part),
+        then the base step: one all-reduce of that vector when sharded and _optimizer_step."""
         g, gc, nt, na = self._shared_net.grad, self._critic.grad, self._n_trunk, self._n_policy
         g[:nt].add_(gc[:nt], alpha=-self.value_coef)            # critic gradients are dL_v/dtheta (descent): minus sign
         g[na:].copy_(gc[nt:]).mul_(-self.value_coef)
+        return super()._step(allreduce)
+
+    def _optimizer_step(self):
+        """One global-norm clip and SGD / Adam step (learning_rate) of the whole vector; no separate critic norm."""
+        cfg = self.agent_config
+        if cfg.optimizer == "adam":
+            self._adam_t += 1
+        return self._apply(self._shared_net, cfg.learning_rate, +1.0, self._adam_t), None
+
+    def _one_message_exchange(self, *args, **kwargs):
+        raise ValueError("exchange='one_message' is implemented for separate actor / critic networks")
 
     @property
     def params(self) -> dict[str, Any]:
@@ -113,7 +127,7 @@ class SharedTrunkActorCritic(ReinforceAgent):
     @params.setter
     def params(self, value: dict[str, Any]) -> None:
         """Policy view (trunk + policy head) in the reference layout; the value head is kept."""
-        vh = self.value_head if getattr(self, "_shared_net", None) is not None else None
+        vh = self.value_head if self._shared_net is not None else None
         if vh is None:                                          # base constructor / load_model before _install
             return ReinforceAgent.params.fset(self, value)
         if np.asarray(value["W"][-1]).shape[0] != vh["W"].shape[0]:
