@@ -429,6 +429,43 @@ int b2048_ppo_coefficients(b2048_handle* h, const int64_t* slots, int64_t n, con
                            const float* a_raw, const float* v_old, double mb_size, double clip_eps, double value_clip_eps,
                            int32_t huber, float huber_delta, float* coef, float* gcoef, double* stats, void* stream);
 
+/* ---------------- one-ply expectimax over the critic ----------------
+ * Playing with the learned value function: Q(s, a) = sum over the spawns s' of p (r + gamma V(s')), the action = the first
+ * argmax of Q over the candidate moves (ties to the lowest index, like greedy selection).  Between the two calls the caller
+ * evaluates the critic on child_board[0 .. *total_dev) (b2048_mlp_forward).  The search draws no random numbers: its result
+ * is a pure function of (board, max_exp, critic).
+ *   candidates   cfg->use_action_mask: the legal moves (flags low nibble, or recomputed when flags == NULL); else all four.
+ *   children     of a candidate a that changes the board, leaving n >= 1 empty cells: 2 n, child 2 k + (v == 4) for
+ *                k = 0 .. n-1 (the k-th empty cell, row-major) and v in {2, 4}, probability 0.9 / n (v = 2) or 0.1 / n
+ *                (v = 4); of a move that changes nothing (mask off only): one, the unchanged board, p = 1.  At most 120
+ *                per board.  Board, float64 reward and done flag of each child are bit-identical to b2048_step_many on
+ *                (s, a) with spawn_replay = 0x80 | k | (v == 4) << 4, auto_reset 0, no step counter (a child is never a
+ *                truncation) and the same max_exp (NULL: no new-max-tile bonus).
+ *   value        t = r + gamma V(s'), V(s') = 0 when the child is terminal; V is the float32 critic output widened.
+ *   Q            changed move: S = sum over k in increasing order of (0.9 t(k, 2) + 0.1 t(k, 4)), Q = S / n; unchanged
+ *                move: Q = t.  Every multiply and add rounded separately in float64.  No candidate: action 0, Q = NaN;
+ *                non-candidate entries of Q are NaN.
+ *
+ * b2048_lookahead_expand: the listed boards (slot_map[0 .. n), or boards 0 .. n-1 without a slot_map; n = n_slots, or
+ * min(n_slots, *n_slots_dev) with n_slots_dev as in b2048_rollout_many) are expanded into one compacted child array.  Per
+ * listed board b and action a: child_first[4 b + a] (the first child, -1 without children) and child_count[4 b + a] (0 for
+ * a non-candidate); rows of boards not listed are not written.  Segments are reserved atomically, so their order varies
+ * from call to call; their contents do not.  *total_dev (zeroed by the call) receives the number of children; when it
+ * exceeds capacity, the boards whose segment did not fit get count 0 and write nothing.  cfg is a host struct (reward
+ * and bonus fields are read); n_slots * 120 and capacity must fit in int32.
+ *
+ * b2048_lookahead_select: for the same listed boards, action[b] (uint8) and, when q != NULL, q[4 b + a] (double [B, 4])
+ * from the child ranges, rewards, done flags and the critic values child_value (float32, indexed like the children). */
+int b2048_lookahead_expand(b2048_handle* h, const uint64_t* board, const uint8_t* flags, const uint8_t* max_exp,
+                           const b2048_env_cfg* cfg /* host */, const int32_t* slot_map, int64_t n_slots,
+                           const int32_t* n_slots_dev, int64_t B, int64_t capacity, uint64_t* child_board,
+                           double* child_reward, uint8_t* child_done, int32_t* child_first, int32_t* child_count,
+                           int32_t* total_dev, void* stream);
+int b2048_lookahead_select(b2048_handle* h, const int32_t* slot_map, int64_t n_slots, const int32_t* n_slots_dev, int64_t B,
+                           const int32_t* child_first, const int32_t* child_count, const double* child_reward,
+                           const uint8_t* child_done, const float* child_value, double gamma, uint8_t* action, double* q,
+                           void* stream);
+
 /* Gradient accumulation of update_batch's actor / critic blocks (reinforce_agent.py:403-555, _backpropagation
  * :639-678) over n samples (flattened [T,B] rollout; samples with coef == 0 contribute nothing).
  * grads is a flat float32 vector laid out W_0, b_0, W_1, b_1, ... and is ACCUMULATED into (zero it first).

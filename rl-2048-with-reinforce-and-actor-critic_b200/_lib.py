@@ -94,6 +94,9 @@ SIGNATURES = {
     "b2048_ppo_logp": [_vp, _vp, _vp, _vp, _i64, _vp, _vp],
     "b2048_ppo_coefficients": [_vp, _vp, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, C.c_double, C.c_double, C.c_double, _i32,
                                _f32, _vp, _vp, _vp, _vp],
+    "b2048_lookahead_expand": [_vp, _vp, _vp, _vp, C.POINTER(EnvCfg), _vp, _i64, _vp, _i64, _i64, _vp, _vp, _vp, _vp, _vp, _vp,
+                               _vp],
+    "b2048_lookahead_select": [_vp, _vp, _i64, _vp, _i64, _vp, _vp, _vp, _vp, _vp, C.c_double, _vp, _vp, _vp],
     "b2048_backward_workspace_floats": [C.POINTER(MlpDesc), _i64],
     "b2048_mlp_backward": [_vp, _vp, _vp, _vp, _vp, C.POINTER(MlpDesc), _vp, _i64, _i32, _vp, _i64, _i64, _i32, _vp],
     "b2048_mlp_backward_entropy": [_vp, _vp, _vp, _vp, _vp, _vp, C.POINTER(MlpDesc), _vp, _i64, _vp, _i64, _i64, _i32, _vp,

@@ -10,7 +10,8 @@ import subprocess
 PKG_DIR = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(PKG_DIR, "csrc")
 LIB_PATH = os.path.join(PKG_DIR, "libb2048.so")
-SOURCES = ["b2048_capi.cu", "b2048_env.cu", "b2048_policy.cu", "b2048_policy_tc.cu", "b2048_learn.cu", "b2048_learn_tc.cu", "b2048_learn_hp.cu", "b2048_mlp_gen.cu"]
+SOURCES = ["b2048_capi.cu", "b2048_env.cu", "b2048_policy.cu", "b2048_policy_tc.cu", "b2048_learn.cu", "b2048_learn_tc.cu", "b2048_learn_hp.cu", "b2048_mlp_gen.cu",
+           "b2048_lookahead.cu"]
 # -cudart shared: torch already loads libcudart; a statically linked runtime would also embed every runtime entry-point
 # name in the shipped binary.
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",

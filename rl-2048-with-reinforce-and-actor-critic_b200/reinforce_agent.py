@@ -11,7 +11,8 @@ Added surface: ``rollout_many`` (run-to-termination or fixed-horizon rollouts of
 into the same rollout buffers and calls the same kernels.  ``update_from_horizon`` trains on fixed-horizon
 windows with reset-on-done (segment-aware returns / TD / GAE, ``horizon_episode_stats`` for logging); ``update_ppo`` runs
 several epochs of clipped-ratio minibatch steps on such a window.  The window updates and ``update_from_rollout`` can
-bootstrap truncated episodes from the critic (``bootstrap_truncation=True``).
+bootstrap truncated episodes from the critic (``bootstrap_truncation=True``).  ``lookahead_actions`` and
+``rollout_lookahead`` play with the critic: a one-ply expectimax over every move and spawn, expanded on the device.
 """
 from __future__ import annotations
 
@@ -653,6 +654,111 @@ class ReinforceAgent:
         benv.board = boards[T]          # the step kernel passes finished boards through: slice T is every final state
         benv.flags = flags[T]
         return Rollout(boards[: T + 1], flags[: T + 1], actions[:T], rewards[:T], length, T)
+
+    # ------------------------------------------------------------------ playing with the critic
+    def _lookahead_precision(self, precision: int | str) -> int:
+        """The critic forward's precision code of a lookahead call; refuses a play without a value function.  Both checks
+        run before any device work."""
+        if not self._has_value_function():
+            raise ValueError("lookahead play needs a value function: agent.use_critic or a SharedTrunkActorCritic")
+        if precision == "auto":
+            return 2
+        if isinstance(precision, bool) or precision not in (0, 1, 2, 3):
+            raise ValueError(f"precision must be 'auto', 0, 1, 2 or 3, got {precision!r}")
+        return int(precision)
+
+    def _lookahead(self, boards: torch.Tensor, flags: torch.Tensor | None, max_exp: torch.Tensor | None, cfg, prec: int,
+                   actions: torch.Tensor, q_out: torch.Tensor | None, slot_map: torch.Tensor | None = None,
+                   count_dev: torch.Tensor | None = None) -> int:
+        """b2048_lookahead_expand of boards (the boards listed in slot_map[:*count_dev] when given), one 4-byte read of the
+        child count, the critic forward on the children, b2048_lookahead_select into actions (and q_out).  Returns the
+        number of children; 0 means no listed board (nothing is selected)."""
+        B = boards.numel()
+        cap = B * 120
+        cb = self._buf("la_child_board", (cap,), torch.int64)
+        cr = self._buf("la_child_reward", (cap,), torch.float64)
+        cd = self._buf("la_child_done", (cap,), torch.uint8)
+        cv = self._buf("la_child_value", (cap,), torch.float32)
+        first = self._buf("la_first", (B, 4), torch.int32)
+        count = self._buf("la_count", (B, 4), torch.int32)
+        total_dev = self._buf("la_total", (1,), torch.int32)
+        total_host = getattr(self, "_la_total_host", None)
+        if total_host is None:
+            total_host = self._la_total_host = torch.zeros(1, dtype=torch.int32).pin_memory()
+        lib, h = self._lib, self._h
+        sm, nd = _ptr(slot_map), _ptr(count_dev)
+        with torch.cuda.device(self.device):
+            _lib.check(lib.b2048_lookahead_expand(h, _ptr(boards), _ptr(flags), _ptr(max_exp), C.byref(cfg), sm, B, nd, B, cap,
+                                                  _ptr(cb), _ptr(cr), _ptr(cd), _ptr(first), _ptr(count), _ptr(total_dev),
+                                                  _stream()), "b2048_lookahead_expand")
+            total_host.copy_(total_dev, non_blocking=True)
+            ev = torch.cuda.Event()
+            ev.record()
+            ev.synchronize()
+            total = int(total_host[0])
+            if total == 0:
+                return 0
+            self._forward_checked(self._critic, cb[:total], cv[:total], self._small_batch_precision(prec, total), [], 1)
+            _lib.check(lib.b2048_lookahead_select(h, sm, B, nd, B, _ptr(first), _ptr(count), _ptr(cr), _ptr(cd), _ptr(cv),
+                                                  float(self.agent_config.gamma), _ptr(actions), _ptr(q_out), _stream()),
+                       "b2048_lookahead_select")
+        return total
+
+    def lookahead_actions(self, boards: torch.Tensor, flags: torch.Tensor | None, max_exp: torch.Tensor | None = None,
+                          precision: int | str = "auto", q_out: torch.Tensor | None = None) -> torch.Tensor:
+        """One-ply expectimax over the critic for a batch of packed boards (include/b2048.h, DESIGN.md K7): every candidate
+        move and every spawn is expanded on the device, the critic values the children, and the action is the first argmax
+        of Q(s, a) = sum p (r + gamma V(s')).  flags: the boards' flags (low nibble = legal mask; None = recomputed);
+        max_exp: the per-board new-max-tile state of the bonus (None = no bonus).  q_out (float64 [n, 4], optional)
+        receives Q, NaN for a non-candidate.  precision: that of the critic forward ("auto" = the split-fp16 tensor cores
+        where they apply, with the fp32 fall-back of the update passes; batches under 4096 children run as "auto" would).
+        Returns the actions (uint8 [n])."""
+        prec = self._lookahead_precision(precision)
+        from .batched_env import make_env_cfg
+        cfg = make_env_cfg(self.env.config, "buffer", auto_reset=False, emit_obs=False)
+        boards = boards.reshape(-1)
+        actions = torch.zeros(boards.numel(), dtype=torch.uint8, device=self.device)
+        if q_out is not None:
+            q_out.fill_(float("nan"))
+        if boards.numel():
+            self._lookahead(boards, flags, max_exp, cfg, prec, actions, q_out)
+        return actions
+
+    def rollout_lookahead(self, benv: Batched2048Env, max_steps: int | None = None, precision: int | str = "auto") -> Rollout:
+        """rollout_many(greedy=True) with the lookahead actions of lookahead_actions instead of the actor's argmax: every
+        board plays to termination (or max_steps, like rollout_many) on the env's Philox streams.  Each step is
+        b2048_compact_live, the lookahead on the boards still playing, and b2048_step_many; the host reads the 4-byte child
+        count once per step.  Returns a run-to-termination Rollout (total_reward(), max tiles 2 ** benv.max_exp)."""
+        prec = self._lookahead_precision(precision)
+        B = benv.num_envs
+        benv.reset_many()
+        cap = int(max_steps or benv.config.max_steps or 4096)
+        boards, flags, actions, rewards, length = self._rollout_buffers(benv, cap)
+        actions.zero_()                 # finished boards get no action
+        from .batched_env import make_env_cfg
+        cfg = make_env_cfg(benv.config, "buffer", auto_reset=False, emit_obs=False)
+        slot = self._buf("ro_slot_map", (B,), torch.int32)
+        count_dev = self._buf("ro_live_count", (1,), torch.int32)
+        t0 = benv.t
+        T = 0
+        while T < cap:
+            with torch.cuda.device(self.device):
+                _lib.check(self._lib.b2048_compact_live(self._h, _ptr(length), B, _ptr(slot), _ptr(count_dev), _stream()),
+                           "b2048_compact_live")
+            if self._lookahead(boards[T], flags[T], benv.max_exp, cfg, prec, actions[T], None, slot, count_dev) == 0:
+                break                   # no board is still playing
+            with torch.cuda.device(self.device):
+                _lib.check(self._lib.b2048_step_many(
+                    self._h, _ptr(boards[T]), _ptr(boards[T + 1]), _ptr(benv.score), _ptr(benv.step_count), _ptr(benv.max_exp),
+                    _ptr(actions[T]), None, _ptr(flags[T]), None, C.byref(cfg), None, _ptr(rewards[T]), None, _ptr(flags[T + 1]),
+                    None, _ptr(length), T + 1, B, benv.seed, benv.gid0, t0 + T + 1, _stream()), "b2048_step_many")
+            T += 1
+        benv.t = t0 + T
+        length = torch.where(length == 0, torch.full_like(length, T), length)   # cut off by the cap
+        benv.board = boards[T]          # the step kernel passes finished boards through: slice T is every final state
+        benv.flags = flags[T]
+        return Rollout(boards[: T + 1], flags[: T + 1], actions[:T], rewards[:T], length, T, seed=benv.seed, gid0=benv.gid0,
+                       t0=t0)
 
     # ------------------------------------------------------------------ reference API: learning
     def compute_returns(self, rewards: list[float]) -> np.ndarray:

@@ -25,6 +25,9 @@ instead of r (``update_from_rollout`` / ``update_from_horizon(bootstrap_truncati
 ``update_ppo`` instead; the shuffle seed of batch k is derived from ``seed`` and k.  The CSV columns are unchanged.
 ``train.entropy_coef`` (default 0): the entropy bonus beta H(pi(.|s)) of every update (episodes, horizon windows and PPO);
 refused with ``train.exchange = "one_message"``.
+``eval.lookahead`` (default false; needs a value function): evaluation plays by the one-ply expectimax over the critic
+(``rollout_lookahead``) instead of the actor; ``eval.checkpoint`` loads a ``save_checkpoint`` file (actor and critic) into an
+agent built by ``evaluation``, which the lookahead requires (``eval.model_path`` loads the actor only).
 
     python -m torch.distributed.run ... b2048_runner.py -conf cfg.json      (or: python b2048_runner.py -conf cfg.json)
 """
@@ -238,15 +241,33 @@ def _horizon_batch(agent, env, info: bd.DistInfo, tr: dict[str, Any], horizon: i
 
 
 def evaluation(cfg: dict[str, Any], info: bd.DistInfo | None = None, device=None, agent=None) -> dict[str, Any]:
+    """Plays ``eval.num_episodes`` games to termination and returns their statistics.  The agent acts with the actor
+    (greedy with ``eval.use_greedy``), or with ``eval.lookahead`` (default false) by the one-ply expectimax over its critic
+    (``rollout_lookahead``).  An agent built here loads ``eval.checkpoint`` (a ``save_checkpoint`` file: actor and critic)
+    or ``eval.model_path`` (the actor alone, which cannot supply a critic for the lookahead)."""
     info = info or bd.DistInfo()
     ev = cfg["eval"]
+    lookahead = bool(ev.get("lookahead", False))
+    if lookahead and agent is None and not ev.get("checkpoint"):
+        raise ValueError("eval.lookahead needs a trained critic: set eval.checkpoint to a save_checkpoint file "
+                         "(eval.model_path holds the actor only)")
+    if lookahead and agent is not None:
+        agent._lookahead_precision("auto")                 # refuses an agent without a value function
+    if lookahead and agent is None and not (cfg["agent"].get("use_critic") or cfg.get("shared_trunk") is not None):
+        raise ValueError("eval.lookahead needs a value function: agent.use_critic or a shared_trunk section")
     env = bd.make_sharded_env(int(ev["num_episodes"]), Game2048EnvConfig(**cfg["env"]), info, seed=int(cfg["seed"]) + 12345,
                               device=device)
     if agent is None:
         agent = make_agent(cfg, env)
-        if ev.get("model_path"):
+        if ev.get("checkpoint"):
+            agent.load_checkpoint(ev["checkpoint"])
+        elif ev.get("model_path"):
             agent.load_model(ev["model_path"])
-    ro = agent.rollout_many(env, greedy=bool(ev.get("use_greedy", True)), precision=cfg["train"].get("precision", "auto"))
+    precision = cfg["train"].get("precision", "auto")
+    if lookahead:
+        ro = agent.rollout_lookahead(env, precision=precision)
+    else:
+        ro = agent.rollout_many(env, greedy=bool(ev.get("use_greedy", True)), precision=precision)
     avg, mx, mn = _global_stats(ro.total_reward(), info)
     return {"avg_reward": avg, "max_reward": mx, "min_reward": mn, "max_tile_counts": tile_histogram(env.max_exp, info),
             "mean_len": float(ro.length.float().mean())}
