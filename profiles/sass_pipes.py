@@ -1,9 +1,10 @@
 #!/usr/bin/env python
 """Per-region, per-pipe instruction counts of the env-step kernel's grid-stride loop (no GPU needed).
 
-The step kernel is bound by the integer ALU pipe (LOP3 / SHF / IADD3 / ISETP ... at 16 lanes per clock per scheduler),
-not by HBM, so the count of ALU-pipe instructions per board is the number to drive down; IMAD runs on the FMA pipe,
-which the step body leaves mostly idle.  The loop is split into:
+The step kernel is bound by instruction issue and the latency of its dependent chain, not by HBM.  ALU-pipe
+(LOP3 / SHF / IADD3 / ISETP ...) and FMA-pipe (IMAD ...) counts are printed apart, but moving work from the first to the
+second does not by itself make the loop faster: an IMAD.HI shift measured slower than the SHF it replaced (DESIGN.md K2).
+The loop is split into:
   main   instructions before the loop's first global store, outside the reset block
   reset  the largest BSSY..BSYNC block between the loop head and its first global store (the auto-reset branch;
          a divergent block: a warp pays all of it when any lane takes it)
@@ -16,7 +17,7 @@ import collections, os, re, subprocess, sys
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 DEFAULT_LIB = os.path.join(ROOT, "rl-2048-with-reinforce-and-actor-critic_b200", "libb2048.so")
-DEFAULT_KERNELS = ["_ZN2b216step_fast_kernelILi3ELb1ELb1EEEvNS_8StepArgsE"]
+DEFAULT_KERNELS = ["_ZN2b216step_fast_kernelILi1ELb1ELb1EEEvNS_8StepArgsE"]   # the kernel bench.py times
 
 ALU = {"LOP3", "LOP", "SHF", "SHL", "SHR", "SEL", "FSEL", "ISETP", "FSETP", "IADD3", "IADD", "VIADD", "VIADDMNMX", "LEA",
        "PRMT", "POPC", "FLO", "BREV", "IMNMX", "VIMNMX", "IABS", "BMSK", "SGXT", "PLOP3", "P2R", "R2P", "MOV", "ICMP",

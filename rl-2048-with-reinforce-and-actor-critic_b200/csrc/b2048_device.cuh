@@ -64,26 +64,21 @@ B2_HD int ffs0(uint32_t x) {  // index of lowest set bit, x != 0
     return __builtin_ctz(x);
 #endif
 }
+B2_HD uint32_t msb(uint32_t x) {  // index of the highest set bit, x != 0 (one FLO; 31 - __clz(x) costs two more ALU ops)
+#if defined(__CUDA_ARCH__)
+    uint32_t r;
+    asm("bfind.u32 %0, %1;" : "=r"(r) : "r"(x));
+    return r;
+#else
+    return 31u - (uint32_t)__builtin_clz(x);
+#endif
+}
 // low 32 bits of ((hi:lo) >> s), 0 <= s < 32
 B2_HD uint32_t funnel_r(uint32_t lo, uint32_t hi, uint32_t s) {
 #if defined(__CUDA_ARCH__)
     return __funnelshift_r(lo, hi, s);
 #else
     return s ? (lo >> s) | (hi << (32 - s)) : lo;
-#endif
-}
-
-// x >> K for a compile-time K, issued on the FMA pipe (IMAD.HI by 2^(32-K)) instead of the integer ALU pipe:
-// the step kernel is bound by the ALU pipe (LOP3 / SHF / IADD3 at 16 lanes per clock per scheduler), the FMA pipe
-// is nearly idle, and ptxas keeps mul.hi with an immediate as IMAD.HI.U32.
-template <int K>
-B2_HD uint32_t shr_fma(uint32_t x) {
-#if defined(__CUDA_ARCH__)
-    uint32_t r;
-    asm("mul.hi.u32 %0, %1, %2;" : "=r"(r) : "r"(x), "n"(1u << (32 - K)));
-    return r;
-#else
-    return x >> K;
 #endif
 }
 
@@ -187,16 +182,16 @@ B2_HD uint32_t blk_transpose(uint32_t x, uint32_t s) {  // s in {0,12}
 B2_HD uint32_t nib_swap(uint32_t x, uint32_t s) {  // s in {0,4}
     return bitsel(0xF0F0F0F0u, x << s, x >> s);
 }
-// The same two transforms without a data-dependent shift, for the ALU-bound fast step: the shifts become IMADs on
-// the FMA pipe and the choice between transform and identity moves into per-action masks / multipliers.
+// The same two transforms without a data-dependent shift, for the fast step: constant shifts, and the choice between
+// transform and identity moves into per-action masks / multipliers.
 //   blk_transpose_m(x, tm) == blk_transpose(x, s) for tm = 0x0F0F0000 (s = 12) or 0 (s = 0)
 //   nib_swap_m(x, nl, nr)  == nib_swap(x, s)      for (nl, nr) = (16, 1) (s = 4) or (1, 16) (s = 0);
 // with s = 0, (x * 16) >> 4 drops only the top nibble, which the 0x0F0F0F0F half of the select does not keep.
 B2_HD uint32_t blk_transpose_m(uint32_t x, uint32_t tm) {
-    return bitsel(tm, x * 4096u, bitsel(shr_fma<12>(tm), shr_fma<12>(x), x));
+    return bitsel(tm, x * 4096u, bitsel(tm >> 12, x >> 12, x));
 }
 B2_HD uint32_t nib_swap_m(uint32_t x, uint32_t nl, uint32_t nr) {
-    return bitsel(0xF0F0F0F0u, x * nl, shr_fma<4>(x * nr));
+    return bitsel(0xF0F0F0F0u, x * nl, (x * nr) >> 4);
 }
 
 B2_HD Board canon_fwd(Board b, const Xform& x) {

@@ -4,14 +4,15 @@
 //
 // Same semantics as step_one (b2048_step.cuh; reference src/game2048.py:40-70, src/env.py:197-302) —
 // the two are checked against each other and against the CPU oracle by tests/host_check — but built
-// to minimise ALU-pipe instructions, which is what bounds the step kernel on sm_100 (profiles/):
+// to minimise issued instructions and the length of their dependent chains, which is what bounds the step kernel on
+// sm_100 (profiles/; a shift issued as IMAD.HI on the FMA pipe instead of SHF measured slower, not faster):
 //   * per-action transform constants come from a 4-entry table (two 128-bit loads), not bit arithmetic;
 //   * merge statistics (score, sum of log2, count, max, overflow) come from a 256-entry table indexed by
 //     each row's merge byte and are combined with two adds and two ors;
-//   * the spawn cell is found with one multiply-prefix-sum per half and a byte-lane compare, and the
+//   * the spawn cell is found with one multiply-prefix-sum per half and one nibble-lane compare, and the
 //     isolated bit (G & -G) is turned into the tile with one multiply (no find-first-set, no shifts);
 //   * the non-zero masks of the moved board are reused for the legal-move test of the new board;
-//   * the canonicalisation has no data-dependent shift (blk_transpose_m / nib_swap_m: IMADs and per-action masks);
+//   * the canonicalisation has no data-dependent shift (blk_transpose_m / nib_swap_m: multiplies and per-action masks);
 //   * auto-reset looks the two-tile start board and its legal mask up by the cells and values its Philox words pick
 //     (start_board) instead of running the generic reset_board + legal_mask.
 // Host+device like the other step headers.
@@ -158,11 +159,11 @@ B2_HD void step_fast_rnd(FastIO& io, const b2048_env_cfg& cfg, const Rand4& rnd,
     const SelEntry s = T.sel[a];
     uint32_t clo = nib_swap_m(blk_transpose_m(io.lo, s.tm), s.nl, s.nr), chi = nib_swap_m(blk_transpose_m(io.hi, s.tm), s.nl, s.nr);
     uint32_t flo = prmt(clo, chi, s.f_lo), fhi = prmt(clo, chi, s.f_hi);
-    uint32_t i0 = flo & 0xFFFFu, i1 = shr_fma<16>(flo), i2 = fhi & 0xFFFFu, i3 = shr_fma<16>(fhi);
+    uint32_t i0 = flo & 0xFFFFu, i1 = flo >> 16, i2 = fhi & 0xFFFFu, i3 = fhi >> 16;
     uint32_t r0 = T.left[i0], r1 = T.left[i1], r2 = T.left[i2], r3 = T.left[i3];
     const AggEntry g0 = T.agg[T.merge[i0]], g1 = T.agg[T.merge[i1]], g2 = T.agg[T.merge[i2]], g3 = T.agg[T.merge[i3]];
     uint32_t agg = g0.agg + g1.agg + g2.agg + g3.agg;
-    uint32_t orm = g0.orm | g1.orm | g2.orm | g3.orm;
+    uint32_t orm = g0.orm | g1.orm | g2.orm | g3.orm | 1u;   // bit 0 (exponent 0) never merges: msb(orm) is defined
     uint32_t mlo = r0 + (r1 << 16), mhi = r2 + (r3 << 16);
     uint32_t plo = prmt(mlo, mhi, s.i_lo), phi = prmt(mlo, mhi, s.i_hi);
     uint32_t vlo = blk_transpose_m(nib_swap_m(plo, s.nl, s.nr), s.tm), vhi = blk_transpose_m(nib_swap_m(phi, s.nl, s.nr), s.tm);
@@ -176,38 +177,36 @@ B2_HD void step_fast_rnd(FastIO& io, const b2048_env_cfg& cfg, const Rand4& rnd,
     }
 
     // ---- spawn: k-th empty cell in row-major order via nibble prefix sums (see file header)
-    const uint32_t nb_lo = shr_fma<3>(nz8(vlo)), nb_hi = shr_fma<3>(nz8(vhi));   // bit 0 of each nibble: cell occupied
+    const uint32_t nb_lo = nz8(vlo) >> 3, nb_hi = nz8(vhi) >> 3;   // bit 0 of each nibble: cell occupied
     const uint32_t zb_lo = nb_lo ^ 0x11111111u, zb_hi = nb_hi ^ 0x11111111u;
     const uint32_t P_lo = zb_lo * 0x11111111u, P_hi = zb_hi * 0x11111111u;   // nibble i = #empty among cells 0..i
-    const uint32_t c_lo = shr_fma<28>(P_lo), c_hi = shr_fma<28>(P_hi);
+    const uint32_t c_lo = P_lo >> 28, c_hi = P_hi >> 28;
     const uint32_t n_empty = c_lo + c_hi;
     uint32_t k = mulhi(rnd.w0, n_empty);
     const bool in_hi = k >= c_lo;
     const uint32_t P = in_hi ? P_hi : P_lo;
     k = in_hi ? k - c_lo : k;
-    const uint32_t addk = (0x7Fu - k) * 0x01010101u;
-    const uint32_t Ge = ((P & 0x0F0F0F0Fu) + addk) & 0x80808080u;           // even cells with prefix > k
-    const uint32_t Go = ((shr_fma<4>(P) & 0x0F0F0F0Fu) + addk) & 0x80808080u;    // odd cells
-    const uint32_t G = shr_fma<7>(Ge) | shr_fma<3>(Go);
+    // nibble i of P + (7 - k) * 0x11111111 is P_i + 7 - k <= 15 (P_i <= 8, k <= 7: no carry between nibbles), so its bit 3
+    // is set exactly for the cells whose prefix exceeds k
+    const uint32_t G = ((P + (7u - k) * 0x11111111u) & 0x88888888u) >> 3;
     const uint32_t iso = G & (0u - G);                                       // 1 << (4 * cell)
-    uint32_t val = rnd.w1 >= 0xE6666667u ? 2u : 1u;
-    val = (changed && n_empty != 0u) ? val : 0u;                             // game2048.py:56-58, :110-111
+    const uint32_t live = (changed && n_empty != 0u) ? 1u : 0u;              // game2048.py:56-58, :110-111
+    const uint32_t val = live * (rnd.w1 >= 0xE6666667u ? 2u : 1u);
     const uint32_t ins = iso * val;
     const uint32_t hsel = in_hi ? 0xFFFFFFFFu : 0u;
     uint32_t nlo = vlo | (ins & ~hsel), nhi = vhi | (ins & hsel);
-    const uint32_t spawned = val ? iso : 0u;
 
     // ---- legal mask of the new board; occupancy bits reused from the spawn stage
-    // N: rows 0,1 at bit 4i, rows 2,3 at bit 4i+1
-    const uint32_t N = (nb_lo | (spawned & ~hsel)) | ((nb_hi | (spawned & hsel)) << 1);
+    // N: rows 0,1 at bit 4i, rows 2,3 at bit 4i+1 (the spawned tile's bit: iso times 1 or 2)
+    const uint32_t N = nb_lo | (nb_hi * 2u) | (iso * (in_hi ? live * 2u : live));
     const uint32_t MH = 0x03330333u, MV = 0x11113333u;
-    const uint32_t Nr = shr_fma<4>(N);
-    const uint32_t EH = shr_fma<3>(nz8(nlo ^ shr_fma<4>(nlo))) | shr_fma<2>(nz8(nhi ^ shr_fma<4>(nhi)));
+    const uint32_t Nr = N >> 4;
+    const uint32_t EH = (nz8(nlo ^ (nlo >> 4)) >> 3) | (nz8(nhi ^ (nhi >> 4)) >> 2);
     const uint32_t hmerge = ~EH & N & MH;
     const uint32_t left = (~N & Nr & MH) | hmerge;
     const uint32_t right = (N & ~Nr & MH) | hmerge;
-    const uint32_t Nd = (shr_fma<16>(N) & 0x00003333u) | ((N * 32768u) & 0x11110000u);
-    const uint32_t EV = shr_fma<3>(nz8(nlo ^ funnel_r(nlo, nhi, 16))) | shr_fma<2>(nz8(nhi ^ shr_fma<16>(nhi)));
+    const uint32_t Nd = ((N >> 16) & 0x00003333u) | ((N * 32768u) & 0x11110000u);
+    const uint32_t EV = (nz8(nlo ^ funnel_r(nlo, nhi, 16)) >> 3) | (nz8(nhi ^ (nhi >> 16)) >> 2);
     const uint32_t vmerge = ~EV & N & MV;
     const uint32_t up = (~N & Nd & MV) | vmerge;
     const uint32_t down = (N & ~Nd & MV) | vmerge;
@@ -215,18 +214,13 @@ B2_HD void step_fast_rnd(FastIO& io, const b2048_env_cfg& cfg, const Rand4& rnd,
     const bool done = (mask == 0u) & ((nlo | nhi) != 0u);
 
     // ---- reward (float64 in the reference's order: base * scale, + step_reward)
-    uint32_t max_merged = 31u - (uint32_t)
-#if defined(__CUDA_ARCH__)
-        __clz((int)(orm | 1u));
-#else
-        __builtin_clz(orm | 1u);
-#endif
-    const uint32_t base = cfg.reward_mode == B2048_REWARD_SUM ? msum : (shr_fma<20>(agg) & 0xFFu);
+    const uint32_t max_merged = msb(orm);
+    const uint32_t base = cfg.reward_mode == B2048_REWARD_SUM ? msum : ((agg >> 20) & 0xFFu);
     double r = dmul((double)base, cfg.base_reward_scale);
     // shaping terms in the reference's order (env.py:226-259, as in step_one): empty cells of the NEW board (after the
     // spawn), number of merges (agg bits 28..31), new-max-tile bonus, step reward, end-game penalty.  All uniform branches
     // on launch constants; the plain configuration skips them.
-    if (kShaped && cfg.empty_tile_reward != 0.0) r = dadd(r, dmul(cfg.empty_tile_reward, (double)(n_empty - (val ? 1u : 0u))));
+    if (kShaped && cfg.empty_tile_reward != 0.0) r = dadd(r, dmul(cfg.empty_tile_reward, (double)(n_empty - live)));
     if (kShaped && cfg.merge_reward != 0.0) r = dadd(r, dmul(cfg.merge_reward, (double)(agg >> 28)));
     if (kTrack && max_merged >= 3u && max_merged > io.max_exp) {                          // env.py:241-250
         io.max_exp = max_merged;
